@@ -210,6 +210,24 @@ int yawb_timer_stop(yawb_ctx *ctx, double *ms);
 int yawb_assign_patches(yawb_ctx *ctx, const double *xyz, int64_t n, const double *centers_xyz, int n_centers,
                         int32_t *out_ids);
 
+/* Spherical k-means for patch centres (replaces treecorr's k-means behind create_patch_centers,
+ * src/yaw/catalog/catalog.py:183-226).  Contract: DESIGN.md §4.4.  xyz n x 3, w n or NULL, host memory;
+ * centers_xyz k x 3 out; labels n out or NULL; *n_iter, *converged out.  Synchronous.
+ *
+ * Deterministic and exact: every sum is an int64 sum of fixed-point coordinates q = rint(x 2^32) (weighted:
+ * q = rint((w x) 2^(32 - e)), e = frexp(max w)), and the centre of a sum s is s / sqrt((sx sx + sy sy) + sz sz)
+ * in correctly rounded double arithmetic.  Initial centres: bisection of the unweighted rows (split the
+ * min(c, k - c) most populated splittable cells along their widest q axis at the mean, q_axis * count > sum q_axis
+ * goes to the high child with id c + rank).  Lloyd iterations: C_i = centre(rows of L_(i-1)), an empty cluster
+ * (s = 0) moved, in ascending order, to the row farthest from its own centre in C_(i-1) (squared vq distance,
+ * ties to the lowest row, rows taken before skipped), L_i = vq(rows, C_i); stop when L_i == L_(i-1)
+ * (*converged = 1) or after max_iter iterations (*n_iter = iterations run; max_iter = 0 returns the initial
+ * centres and their assignment).  labels == vq(xyz, centers) always.
+ * Requirements: 1 <= k <= 4096, k <= n < 2^30, max_iter >= 0, rows finite with |coordinate| <= 1, weights finite,
+ * >= 0, largest weight >= 2^-992; at least k distinct fixed-point positions. */
+int yawb_kmeans(yawb_ctx *ctx, const double *xyz, const double *w, int64_t n, int k, int max_iter,
+                double *centers_xyz, int32_t *labels, int *n_iter, int *converged);
+
 /* Library version and number of SMs of the context's device. */
 int yawb_version(void);
 int yawb_device_sms(const yawb_ctx *ctx);

@@ -27,7 +27,7 @@ EXPORTS = (
     "yawb_build_index", "yawb_drop_index", "yawb_catalog_info", "yawb_sum_weights", "yawb_count",
     "yawb_host_alloc", "yawb_host_free", "yawb_sync", "yawb_version", "yawb_device_sms",
     "yawb_timer_start", "yawb_timer_stop", "yawb_assign_patches", "yawb_upload_catalog_u8", "yawb_count2",
-    "yawb_upload_catalog_z", "yawb_patch_metadata", "yawb_jackknife", "yawb_count4",
+    "yawb_upload_catalog_z", "yawb_patch_metadata", "yawb_jackknife", "yawb_count4", "yawb_kmeans",
 )
 
 
@@ -95,6 +95,9 @@ def load(build_if_missing: bool = False) -> ctypes.CDLL:
     lib.yawb_catalog_info.argtypes = [c_void_p, POINTER(c_int64), POINTER(c_int64)]
     lib.yawb_sum_weights.argtypes = [c_void_p, c_void_p]
     lib.yawb_assign_patches.argtypes = [c_void_p, c_void_p, c_int64, c_void_p, c_int, c_void_p]
+    lib.yawb_kmeans.argtypes = [
+        c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, POINTER(c_int), POINTER(c_int),
+    ]
     lib.yawb_count.argtypes = [
         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_uint32,
         c_void_p, c_void_p, POINTER(YawbStats),

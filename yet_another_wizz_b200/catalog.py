@@ -9,9 +9,11 @@ a `Mapping[int, Patch]` with `get_centers()`, `get_radii()`, `get_num_records()`
 as a structured array with fields `ra`, `dec`, `weights`, `redshifts`.
 
 The reference's ingest pipeline (chunked FITS/HDF5/Parquet readers, writer
-processes, treecorr k-means) is out of scope (SURVEY.md section 2, row 6).  Patches
-here are built in memory from arrays, or opened from a cache directory written
-by the reference (`data.bin` + `meta.yml`, byte-compatible read-only access).
+processes) is out of scope (SURVEY.md section 2, row 6).  Patches here are built in
+memory from arrays, or opened from a cache directory written by the reference
+(`data.bin` + `meta.yml`, byte-compatible read-only access).  Patch centres can be
+given, or computed from a number of patches by the device k-means
+(`create_patch_centers`, in place of the reference's treecorr k-means).
 Real `yaw.Catalog` objects can be handed to the engine directly; both kinds are
 read through the same duck-typed accessors in `measurements.py`.
 """
@@ -26,7 +28,7 @@ import numpy as np
 
 from .coordinates import AngularCoordinates, AngularDistances
 
-__all__ = ["Catalog", "InconsistentPatchesError", "Metadata", "Patch"]
+__all__ = ["Catalog", "InconsistentPatchesError", "Metadata", "Patch", "create_patch_centers"]
 
 ATTR_ORDER = ("ra", "dec", "weights", "redshifts", "patch_ids", "kappa")  # src/yaw/datachunk.py:44
 
@@ -158,6 +160,33 @@ def _nearest_center(xyz: np.ndarray, centers_xyz: np.ndarray, engine=None) -> np
     return ids.astype(np.int32)
 
 
+def create_patch_centers(ra, dec, patch_num: int, *, weights=None, probe_size: int = -1,
+                         engine=None) -> AngularCoordinates:
+    """Centres of `patch_num` patches for the rows `(ra, dec)` (radian): the deterministic spherical k-means of
+    `Engine.kmeans` on their `to_3d` positions, with `weights` if given.  It takes the place of the reference's
+    treecorr k-means (`create_patch_centers`, `src/yaw/catalog/catalog.py:183-226`) but does not reproduce its centres.
+
+    `probe_size > 0` runs the k-means on every `ceil(n / probe_size)`-th row in input order (this package's
+    subsampling rule); the default uses every row.  `engine=None` uses `measurements.get_default_engine()`;
+    there is no CPU fallback."""
+    patch_num = int(patch_num)
+    if patch_num < 1:
+        raise ValueError(f"'patch_num' must be at least 1 (got {patch_num})")
+    if engine is None:
+        from .measurements import get_default_engine
+
+        engine = get_default_engine()
+    xyz = AngularCoordinates(np.column_stack([np.asarray(ra, dtype=np.float64), np.asarray(dec, dtype=np.float64)])).to_3d()
+    if weights is not None:
+        weights = np.asarray(weights, dtype=np.float64)
+    if probe_size > 0:
+        step = -(-len(xyz) // int(probe_size))
+        xyz = xyz[::step]
+        weights = None if weights is None else weights[::step]
+    centers, _, _, _ = engine.kmeans(xyz, patch_num, weights=weights)
+    return AngularCoordinates.from_3d(centers)
+
+
 class Catalog(Mapping):
     """Mapping patch id -> `Patch`; patch ids are 0..P-1 and iterate in sorted order
     (the reference uses them as array indices, `src/yaw/correlation/measurements.py:358-364`)."""
@@ -173,9 +202,13 @@ class Catalog(Mapping):
 
     # ---- constructors -----------------------------------------------------------------------
     @classmethod
-    def from_arrays(cls, ra, dec, *, patch_centers=None, patch_ids=None, weights=None, redshifts=None,
-                    kappa=None, degrees: bool = True, cache_directory=None, engine=None) -> "Catalog":
-        """`engine`: assign rows to the nearest patch centre on the device instead of scipy's vq."""
+    def from_arrays(cls, ra, dec, *, patch_centers=None, patch_ids=None, patch_num=None, probe_size: int = -1,
+                    weights=None, redshifts=None, kappa=None, degrees: bool = True, cache_directory=None,
+                    engine=None) -> "Catalog":
+        """Patches from `patch_centers` (rows go to the nearest centre), else from `patch_ids`, else from
+        `patch_num`: centres of `create_patch_centers` (with the catalog's weights and `probe_size`), then used
+        exactly as if they had been passed as `patch_centers`.  `engine`: assign rows to the nearest patch
+        centre on the device instead of scipy's vq, and run the k-means there (default: the default engine)."""
         ra = np.asarray(ra, dtype=np.float64)
         dec = np.asarray(dec, dtype=np.float64)
         if degrees:
@@ -184,7 +217,10 @@ class Catalog(Mapping):
         redshifts = None if redshifts is None else np.asarray(redshifts, dtype=np.float64)
         kappa = None if kappa is None else np.asarray(kappa, dtype=np.float64)
         if patch_centers is None and patch_ids is None:
-            raise ValueError("one of 'patch_centers' and 'patch_ids' must be provided")
+            if patch_num is None:
+                raise ValueError("one of 'patch_centers', 'patch_ids' and 'patch_num' must be provided")
+            patch_centers = create_patch_centers(ra, dec, patch_num, weights=weights, probe_size=probe_size,
+                                                 engine=engine)
         centers = None
         if patch_centers is not None:
             if isinstance(patch_centers, Mapping):  # another catalog
@@ -212,25 +248,26 @@ class Catalog(Mapping):
     @classmethod
     def from_dataframe(cls, cache_directory, dataframe, *, ra_name, dec_name, weight_name=None,
                        redshift_name=None, patch_centers=None, patch_name=None, patch_num=None,
-                       kappa_name=None, degrees: bool = True, engine=None, **_ignored) -> "Catalog":
-        """Signature of `yaw.Catalog.from_dataframe` (`src/yaw/catalog/catalog.py:980-1108`);
-        `patch_num` (treecorr k-means) is not supported -- pass centres or a patch column."""
-        if patch_num is not None and patch_centers is None and patch_name is None:
-            raise NotImplementedError("automatic patch centres need treecorr; pass patch_centers= or patch_name=")
+                       kappa_name=None, degrees: bool = True, probe_size: int = -1, engine=None,
+                       **_ignored) -> "Catalog":
+        """Signature of `yaw.Catalog.from_dataframe` (`src/yaw/catalog/catalog.py:980-1108`); patches come from
+        `patch_centers`, else `patch_name`, else `patch_num` (see `from_arrays`)."""
         get = lambda name: None if name is None else np.asarray(dataframe[name])  # noqa: E731
         return cls.from_arrays(
             get(ra_name), get(dec_name), patch_centers=patch_centers,
             patch_ids=None if patch_centers is not None else get(patch_name),
-            weights=get(weight_name), redshifts=get(redshift_name), kappa=get(kappa_name), degrees=degrees,
-            cache_directory=cache_directory, engine=engine,
+            patch_num=patch_num, probe_size=probe_size, weights=get(weight_name), redshifts=get(redshift_name),
+            kappa=get(kappa_name), degrees=degrees, cache_directory=cache_directory, engine=engine,
         )
 
     @classmethod
-    def from_random(cls, cache_directory, generator, num_randoms: int, *, patch_centers=None, engine=None,
-                    **_ignored) -> "Catalog":
-        """Signature of `yaw.Catalog.from_random` (`src/yaw/catalog/catalog.py:1245-1343`)."""
+    def from_random(cls, cache_directory, generator, num_randoms: int, *, patch_centers=None, patch_num=None,
+                    probe_size: int = -1, engine=None, **_ignored) -> "Catalog":
+        """Signature of `yaw.Catalog.from_random` (`src/yaw/catalog/catalog.py:1245-1343`); patches come from
+        `patch_centers`, else `patch_num` (see `from_arrays`)."""
         chunk = generator(int(num_randoms))
-        return cls.from_arrays(chunk["ra"], chunk["dec"], patch_centers=patch_centers,
+        return cls.from_arrays(chunk["ra"], chunk["dec"], patch_centers=patch_centers, patch_num=patch_num,
+                               probe_size=probe_size,
                                weights=chunk.get("weights"), redshifts=chunk.get("redshifts"),
                                degrees=False, cache_directory=cache_directory, engine=engine)
 

@@ -11,7 +11,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-SOURCES = ["yawb_api.cu", "yawb_alloc.cu", "yawb_index.cu", "yawb_count.cu"]
+SOURCES = ["yawb_api.cu", "yawb_alloc.cu", "yawb_index.cu", "yawb_count.cu", "yawb_kmeans.cu"]
 HEADERS = ["yawb_internal.cuh", "yawb_count_stream.cuh", os.path.join(ROOT, "include", "yawb.h")]
 OUT = os.environ.get("YAWB_BUILD_OUT") or os.path.join(HERE, "libyawb.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

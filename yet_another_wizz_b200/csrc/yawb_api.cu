@@ -76,8 +76,7 @@ __global__ void k_assign_patches(const double *__restrict__ xyz, long long n, co
         for (int k = threadIdx.x; k < 3 * nc; k += blockDim.x) cs[k] = centers[3 * (size_t)c0 + k];
         __syncthreads();
         for (int c = 0; c < nc; ++c) {
-            const double dx = __dsub_rn(cs[3 * c], x), dy = __dsub_rn(cs[3 * c + 1], y), dz = __dsub_rn(cs[3 * c + 2], z);
-            const double d = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+            const double d = yawb_vq_d2(cs[3 * c], cs[3 * c + 1], cs[3 * c + 2], x, y, z);
             if (d < best) {
                 best = d;
                 arg = c0 + c;

@@ -41,6 +41,13 @@ void yawb_set_error(const char *fmt, ...);
         }                                                                                      \
     } while (0)
 
+// Squared distance of scipy.cluster.vq.vq for fewer than 5 features: differences centre - row, squares summed
+// x -> y -> z, every operation rounded on its own (no FMA).  Shared by patch assignment and k-means.
+__device__ __forceinline__ double yawb_vq_d2(double cx, double cy, double cz, double x, double y, double z) {
+    const double dx = __dsub_rn(cx, x), dy = __dsub_rn(cy, y), dz = __dsub_rn(cz, z);
+    return __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+}
+
 // ---- geometry of one patch: orthonormal frame at the mean direction --------------------
 struct PatchFrame {
     double c[3];   // unit vector of the patch centre (mean direction)

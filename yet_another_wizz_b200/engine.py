@@ -12,7 +12,7 @@ from __future__ import annotations
 import ctypes
 import os
 import weakref
-from ctypes import byref, c_double, c_int64, c_void_p
+from ctypes import byref, c_double, c_int, c_int64, c_void_p
 
 import numpy as np
 
@@ -352,6 +352,24 @@ class Engine:
         _lib.check(self.lib.yawb_assign_patches(self._h, _ptr(xyz), len(xyz), _ptr(centers_xyz), len(centers_xyz),
                                                 _ptr(out)))
         return out
+
+    def kmeans(self, xyz: np.ndarray, k: int, *, weights: np.ndarray | None = None,
+               max_iter: int = 500) -> tuple[np.ndarray, np.ndarray, int, bool]:
+        """Deterministic spherical k-means on the device (`yawb_kmeans`, DESIGN.md section 4.4): patch centres for
+        `k` patches from rows `xyz` (`(n, 3)`, as `AngularCoordinates.to_3d` gives them), optionally weighted.
+        Returns `(centers_xyz (k, 3), labels (n,) int32, n_iter, converged)`; `labels` is the nearest centre of
+        every row (`scipy.cluster.vq.vq` arithmetic).  With `max_iter=0` the initial centres are returned."""
+        xyz = np.ascontiguousarray(xyz, dtype=np.float64).reshape(-1, 3)
+        if weights is not None:
+            weights = np.ascontiguousarray(weights, dtype=np.float64)
+            if len(weights) != len(xyz):
+                raise ValueError("shape of 'xyz' and 'weights' does not match")
+        centers = np.empty((max(int(k), 0), 3), dtype=np.float64)
+        labels = np.empty(len(xyz), dtype=np.int32)
+        n_iter, converged = c_int(), c_int()
+        _lib.check(self.lib.yawb_kmeans(self._h, _ptr(xyz), _ptr(weights), len(xyz), int(k), int(max_iter),
+                                        _ptr(centers), _ptr(labels), byref(n_iter), byref(converged)))
+        return centers, labels, n_iter.value, bool(converged.value)
 
     # ---- resident catalogs across measurement calls -------------------------------------------------
     @staticmethod
