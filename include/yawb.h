@@ -32,6 +32,15 @@ typedef struct yawb_cat yawb_cat;
 /* flags for yawb_count() */
 #define YAWB_FLAG_EXACT_BRUTEFORCE 1u /* FP64 all-pairs kernel, no pruning (validation / cross-check) */
 #define YAWB_FLAG_OUT_DEVICE 2u       /* out_f64 / out_i64 are device pointers (e.g. torch tensors)  */
+/* Labelled second catalogs (library version >= 101): the per-row ids of a binned second catalog are sample labels
+ * 0..L-1 (L = its n_bins; an unbinned second catalog has L = 1), not z-bins.  A row with label l is paired with
+ * every z-bin of the first catalog, as a row of an unbinned catalog is, and its counts go to output block l: each
+ * (first, second) catalog combination writes [L][n_pairs][n_bins][n_edges-1], so the caller's arrays (host or
+ * YAWB_FLAG_OUT_DEVICE) are L times longer.  Block l equals yawb_count(cat1, U_l) for an unbinned upload U_l of
+ * exactly the rows with label l (integer counts bit for bit).  Rows with a label outside [0, L) are dropped (255 in
+ * yawb_upload_catalog_u8).  This is how the tomographic bins of an unknown sample are counted in one pass.  Not
+ * supported with YAWB_FLAG_EXACT_BRUTEFORCE.  Unknown flag bits are rejected. */
+#define YAWB_FLAG_SECOND_LABELS 4u
 
 /* roles for yawb_build_index() */
 #define YAWB_ROLE_FIRST 1  /* catalog used as first argument of yawb_count(): sky-cell index        */
@@ -41,7 +50,7 @@ typedef struct {
     double kernel_ms;          /* device time of planner + pair-count kernel, CUDA events on the ctx stream */
     double index_ms;           /* device time of index builds triggered by this call (0 if prebuilt)      */
     uint64_t pair_tests;       /* pair tests executed (after sky-cell / tile pruning)                     */
-    uint64_t pair_tests_naive; /* sum over requested patch pairs and z-bins of n1 * n2                    */
+    uint64_t pair_tests_naive; /* sum over requested patch pairs and z-bins of n1 * n2 (n2: all labels)   */
     uint64_t rechecks;         /* tests re-evaluated in exact FP64                                        */
     uint64_t work_items;       /* work items written by the planner (tile x linked patch, non-empty)      */
     uint64_t launches;         /* kernels launched by this call                                           */
@@ -184,7 +193,9 @@ int yawb_count2(yawb_ctx *ctx, yawb_cat *cat1a, yawb_cat *cat1b, yawb_cat *cat2,
  * (reference, its randoms, unknown, its randoms).  The planner lists the work items of both second catalogs for
  * one persistent kernel, so a small job (a GPU's share of a multi-GPU run) pays the ramp-up and the tail of a
  * launch, the host synchronisation and the result transfer once instead of twice.  cat2a and cat2b need the same
- * n_patch / n_bins.  out_f64 / out_i64: tables of four pointers each, any of which may be NULL.
+ * n_patch / n_bins; with YAWB_FLAG_SECOND_LABELS only the same n_patch, and each output has the L of its own second
+ * catalog (a labelled unknown sample and a shared unlabelled random catalog in one launch).
+ * out_f64 / out_i64: tables of four pointers each, any of which may be NULL.
  * YAWB_FLAG_EXACT_BRUTEFORCE is not supported.  stats cover all four counts. */
 int yawb_count4(yawb_ctx *ctx, yawb_cat *cat1a, yawb_cat *cat1b, yawb_cat *cat2a, yawb_cat *cat2b, const int32_t *pair_i,
                 const int32_t *pair_j, int n_pairs, const double *r2_edges, int n_edges, uint32_t flags,

@@ -18,6 +18,8 @@ LIB_PATH = os.environ.get("YAWB_LIB") or os.path.join(_HERE, "csrc", "libyawb.so
 
 FLAG_EXACT_BRUTEFORCE = 1
 FLAG_OUT_DEVICE = 2
+FLAG_SECOND_LABELS = 4
+LABELS_MIN_VERSION = 101  # first library version that knows FLAG_SECOND_LABELS
 ROLE_FIRST = 1
 ROLE_SECOND = 2
 

@@ -144,7 +144,7 @@ int yawb_assign_patches(yawb_ctx *ctx, const double *xyz, int64_t n, const doubl
 
 const char *yawb_last_error(void) { return g_err; }
 
-int yawb_version(void) { return 100; }
+int yawb_version(void) { return 101; }
 
 int yawb_create(int device, yawb_ctx **out) {
     YAWB_REQUIRE(out != nullptr, "yawb_create: out is NULL");
@@ -425,11 +425,18 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     YAWB_REQUIRE(n_pairs >= 0, "n_pairs < 0");
     YAWB_REQUIRE(n_edges >= 2 && n_edges <= YAWB_MAX_EDGES, "n_edges must be in 2..%d (got %d)", YAWB_MAX_EDGES, n_edges);
     YAWB_REQUIRE(r2_edges != nullptr, "r2_edges is NULL");
+    YAWB_REQUIRE((flags & ~(uint32_t)(YAWB_FLAG_EXACT_BRUTEFORCE | YAWB_FLAG_OUT_DEVICE | YAWB_FLAG_SECOND_LABELS)) == 0,
+                 "unknown flag bits 0x%x (library version %d)", flags, yawb_version());
+    const bool labels = (flags & YAWB_FLAG_SECOND_LABELS) != 0;
+    YAWB_REQUIRE(!(labels && (flags & YAWB_FLAG_EXACT_BRUTEFORCE)),
+                 "YAWB_FLAG_SECOND_LABELS is not supported by the exact cross-check (YAWB_FLAG_EXACT_BRUTEFORCE)");
     YAWB_REQUIRE(cat1->n_patch == cat2->n_patch, "catalogs have different numbers of patches (%d vs %d)",
                  cat1->n_patch, cat2->n_patch);
-    YAWB_REQUIRE(!(cat2->binned && !cat1->binned), "a binned second catalog needs a binned first catalog");
-    YAWB_REQUIRE(!cat2->binned || cat2->n_bins == cat1->n_bins, "z-bin counts differ (%d vs %d)", cat1->n_bins,
-                 cat2->n_bins);
+    if (!labels) {
+        YAWB_REQUIRE(!(cat2->binned && !cat1->binned), "a binned second catalog needs a binned first catalog");
+        YAWB_REQUIRE(!cat2->binned || cat2->n_bins == cat1->n_bins, "z-bin counts differ (%d vs %d)", cat1->n_bins,
+                     cat2->n_bins);
+    }
     if (cat1b) {
         YAWB_REQUIRE(cat1b != cat1, "yawb_count2: the two first catalogs must differ");
         YAWB_REQUIRE(cat1b->n_patch == cat1->n_patch && cat1b->n_bins == cat1->n_bins && cat1b->binned == cat1->binned,
@@ -439,12 +446,16 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     if (cat2b) {
         YAWB_REQUIRE(cat1b != nullptr, "yawb_count4 needs two first-role catalogs");
         YAWB_REQUIRE(cat2b != cat2 && cat2b->ctx == ctx, "yawb_count4: the two second catalogs must differ and belong to the context");
-        YAWB_REQUIRE(cat2b->n_patch == cat2->n_patch && cat2b->n_bins == cat2->n_bins && cat2b->binned == cat2->binned,
-                     "yawb_count4: the two second catalogs need the same patches and z-bins");
+        YAWB_REQUIRE(cat2b->n_patch == cat2->n_patch, "yawb_count4: the two second catalogs need the same patches");
+        YAWB_REQUIRE(labels || (cat2b->n_bins == cat2->n_bins && cat2b->binned == cat2->binned),
+                     "yawb_count4: the two second catalogs need the same z-bins");
     }
     YAWB_REQUIRE(n_pairs == 0 || (pair_i && pair_j), "pair lists are NULL");
     const int n_types = cat1b ? 2 : 1;
     const int n_src = cat2b ? 2 : 1;  // second catalogs of the launch
+    // output blocks per second catalog: its labels (YAWB_FLAG_SECOND_LABELS on a binned catalog), else one
+    const int n_lab[2] = {labels && cat2->binned ? cat2->n_bins : 1, labels && cat2b && cat2b->binned ? cat2b->n_bins : 1};
+    const int n_blocks = n_lab[0] + (cat2b ? n_lab[1] : 0);
     const int B = cat1->n_bins, P = cat1->n_patch, nsub = n_edges - 1;
     for (int k = 0; k < n_pairs; ++k)
         YAWB_REQUIRE(pair_i[k] >= 0 && pair_i[k] < P && pair_j[k] >= 0 && pair_j[k] < P,
@@ -488,8 +499,8 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     }
 
     const bool weighted = fi->weighted || cat2->weighted || (cat2b && cat2b->weighted);
-    const size_t n_out1 = (size_t)n_pairs * B * nsub;  // one (first, second) catalog combination's results
-    const size_t n_out = n_out1 * n_types * n_src;     // [second catalog][first catalog][pair][bin][sub-bin]
+    const size_t n_out1 = (size_t)n_pairs * B * nsub;  // one (first catalog, output block) combination's results
+    const size_t n_out = n_out1 * n_types * n_blocks;  // [second catalog, label][first catalog][pair][bin][sub-bin]
 
     // host-side preparation of thresholds and the item table
     std::vector<BinPar> binpar(B);
@@ -550,12 +561,12 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
             base[k + 1] = base[k] + nt;
             const int p = pair_i[k];
             if (p == q) flat_diag += nt;
+            long long n2_all = 0;  // a labelled catalog pairs the rows of every label with each z-bin
+            for (int l = 0; l < c2->n_bins; ++l) n2_all += c2->h_counts[(size_t)l * P + q];
             for (int b = 0; b < B; ++b) {
                 long long n1 = cat1->h_counts[(size_t)b * P + p];
                 if (cat1b) n1 += cat1b->h_counts[(size_t)b * P + p];
-                long long n2 = 0;
-                if (c2->binned) n2 = c2->h_counts[(size_t)b * P + q];
-                else n2 = c2->h_counts[q];
+                const long long n2 = c2->binned && !labels ? c2->h_counts[(size_t)b * P + q] : n2_all;
                 s.pair_tests_naive += (uint64_t)(n1 * n2);
             }
         }
@@ -622,6 +633,8 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     a.d_pair_item_base_b = cat2b ? d_base + (n_pairs + 1) : nullptr;
     a.n_items = item_base[n_pairs];
     a.n_items_b = cat2b ? item_base[(size_t)(n_pairs + 1) + n_pairs] : 0;
+    a.labels = labels;
+    a.blk_b = n_lab[0];
     // work-item lists: a patch with itself needs an item per tile (a few more where items are split), of the
     // tiles of neighbouring patches only the boundary strip survives; if a list turns out too small the
     // count is repeated with the exact sizes
@@ -634,6 +647,11 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     int launches = 0;
     unsigned long long h_counters[8] = {0};
     const bool to_device = (flags & YAWB_FLAG_OUT_DEVICE) != 0;
+    // caller array t = (second catalog s, first catalog) holds [label][pair][bin][sub-bin]; on the device, block
+    // (s, label) of first catalog t % n_types sits at this multiple of n_out1
+    auto out_block = [&](int t, int l) -> size_t {
+        return (size_t)((t / n_types ? n_lab[0] : 0) + l) * n_types + (size_t)(t % n_types);
+    };
     // Host results land in page-locked memory of the context first (counters, counts, sums: one copy each, truly
     // asynchronous) and are handed to the caller's -- usually pageable -- arrays after the one synchronisation of
     // the call; a cudaMemcpyAsync into pageable memory is staged by the driver, one blocking round trip per array.
@@ -665,17 +683,19 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
         // been too small -- the host only learns that now -- the count is repeated with the exact sizes
         if (to_device) {
             TRY(cudaMemcpyAsync(h_counters, ctx->d_counters, sizeof(h_counters), cudaMemcpyDeviceToHost, st));
-            for (int t = 0; t < n_types * n_src && n_out1; ++t) {
-                if (out_i64[t]) TRY(cudaMemcpyAsync(out_i64[t], d_cnt + t * n_out1, n_out1 * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
-                if (out_f64[t]) {
-                    if (weighted) {
-                        TRY(cudaMemcpyAsync(out_f64[t], d_w + t * n_out1, n_out1 * sizeof(double), cudaMemcpyDeviceToDevice, st));
-                    } else {
-                        k_u64_to_f64<<<(unsigned)((n_out1 + 255) / 256), 256, 0, st>>>(d_cnt + t * n_out1, out_f64[t], (long long)n_out1);
-                        launches += 1;
+            for (int t = 0; t < n_types * n_src && n_out1; ++t)
+                for (int l = 0; l < n_lab[t / n_types]; ++l) {
+                    const size_t src = out_block(t, l) * n_out1, dst = (size_t)l * n_out1;
+                    if (out_i64[t]) TRY(cudaMemcpyAsync(out_i64[t] + dst, d_cnt + src, n_out1 * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+                    if (out_f64[t]) {
+                        if (weighted) {
+                            TRY(cudaMemcpyAsync(out_f64[t] + dst, d_w + src, n_out1 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+                        } else {
+                            k_u64_to_f64<<<(unsigned)((n_out1 + 255) / 256), 256, 0, st>>>(d_cnt + src, out_f64[t] + dst, (long long)n_out1);
+                            launches += 1;
+                        }
                     }
                 }
-            }
             TRY(cudaStreamSynchronize(st));
         } else {
             TRY(cudaMemcpyAsync(pin, ctx->d_counters, sizeof(h_counters), cudaMemcpyDeviceToHost, st));
@@ -696,16 +716,18 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     if (!to_device) {
         const unsigned long long *h_cnt = reinterpret_cast<const unsigned long long *>(pin + pin_cnt);
         const double *h_w = reinterpret_cast<const double *>(pin + pin_w);
-        for (int t = 0; t < n_types * n_src && n_out1; ++t) {
-            if (out_i64[t]) memcpy(out_i64[t], h_cnt + t * n_out1, n_out1 * sizeof(int64_t));
-            if (out_f64[t]) {
-                if (weighted) {
-                    memcpy(out_f64[t], h_w + t * n_out1, n_out1 * sizeof(double));
-                } else {
-                    for (size_t k = 0; k < n_out1; ++k) out_f64[t][k] = (double)h_cnt[t * n_out1 + k];
+        for (int t = 0; t < n_types * n_src && n_out1; ++t)
+            for (int l = 0; l < n_lab[t / n_types]; ++l) {
+                const size_t src = out_block(t, l) * n_out1, dst = (size_t)l * n_out1;
+                if (out_i64[t]) memcpy(out_i64[t] + dst, h_cnt + src, n_out1 * sizeof(int64_t));
+                if (out_f64[t]) {
+                    if (weighted) {
+                        memcpy(out_f64[t] + dst, h_w + src, n_out1 * sizeof(double));
+                    } else {
+                        for (size_t k = 0; k < n_out1; ++k) out_f64[t][dst + k] = (double)h_cnt[src + k];
+                    }
                 }
             }
-        }
     }
     TRY(cudaGetLastError());
     float t_k = 0.f;

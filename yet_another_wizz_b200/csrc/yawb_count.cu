@@ -78,7 +78,7 @@ struct FastParams {
     int acc_global;               // general sub-bin path: segment histograms go straight to global atomics
     const BinPar *binpar;
     double rmax_all;              // largest search radius over the z-bins
-    unsigned long long *out_cnt;  // [n_src][n_types][n_pairs][n_bins][n_edges - 1] (n_src = second catalogs of the launch)
+    unsigned long long *out_cnt;  // [n_blocks][n_types][n_pairs][n_bins][n_edges - 1] (Item::blk: second catalog, then label)
     double *out_w;
     size_t type_stride;           // n_pairs * n_bins * (n_edges - 1)
     unsigned long long *counters;  // [0] next item, [1] tests, [2] rechecks, [4] heavy items, [5] light items, [6] overflow
@@ -641,6 +641,8 @@ struct PlanParams {
     long long cap_heavy, cap_light;
     int ccap;  // (z-bin, cell row) runs per item: YAWB_CCAP, or less to cut a small job into more, shorter items
     int src;   // which second catalog of a joint launch these tiles belong to (Item::src)
+    int blk;     // first output block of that catalog (Item::blk)
+    int labels;  // the tiles' z-bin ids are sample labels: paired with every z-bin, counts go to block blk + label
     unsigned long long *counters;
 };
 
@@ -684,7 +686,8 @@ __global__ void __launch_bounds__(256) k_plan(const PlanParams Q) {
         const int t = Q.ptile_off[p2] + (int)(f - Q.pair_item_base[k]);
         const Tile tl = Q.tiles[t];
         const PatchFrame &F1 = Q.frames1[p1];
-        const double rmax = tl.bin >= 0 ? (Q.binpar[tl.bin].empty ? 0.0 : Q.binpar[tl.bin].rmax) : Q.rmax_all;
+        const int zb = Q.labels ? -1 : tl.bin;  // z-bin of the tile, -1: paired with every z-bin of the first catalog
+        const double rmax = zb >= 0 ? (Q.binpar[zb].empty ? 0.0 : Q.binpar[zb].rmax) : Q.rmax_all;
         // bounding spheres first (chord distances obey the triangle inequality)
         const double dx = (double)tl.cx - F1.c[0], dy = (double)tl.cy - F1.c[1], dz = (double)tl.cz - F1.c[2];
         const double reach = F1.radius + (double)tl.rad + rmax + 1e-9;
@@ -716,8 +719,9 @@ __global__ void __launch_bounds__(256) k_plan(const PlanParams Q) {
             if (lo3[0] - rmax <= F1.umax && hi3[0] + rmax >= F1.umin && lo3[1] - rmax <= F1.vmax && hi3[1] + rmax >= F1.vmin) {
                 G = Q.sgrid[p1];
                 it.pair = k; it.p1 = p1; it.start = tl.start; it.count = tl.count; it.src = Q.src;
-                it.b_lo = tl.bin >= 0 ? tl.bin : 0;
-                it.b_hi = tl.bin >= 0 ? tl.bin + 1 : Q.n_bins;
+                it.blk = Q.blk + (Q.labels && tl.bin >= 0 ? tl.bin : 0);
+                it.b_lo = zb >= 0 ? zb : 0;
+                it.b_hi = zb >= 0 ? zb + 1 : Q.n_bins;
 #pragma unroll
                 for (int d = 0; d < 3; ++d) { it.lo[d] = lo3[d]; it.hi[d] = hi3[d]; }
                 heavy = p1 == p2;
@@ -906,6 +910,8 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
         Q.counters = ctx->d_counters;
         Q.ccap = ccap;
         Q.src = sc;
+        Q.blk = sc ? a.blk_b : 0;
+        Q.labels = a.labels ? 1 : 0;
         k_plan<<<(unsigned)((n_flat + 255) / 256), 256, 0, ctx->stream>>>(Q);
         *launches += 1;
     }

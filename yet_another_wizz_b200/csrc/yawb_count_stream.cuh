@@ -497,7 +497,7 @@ template <bool WEIGHTED, bool MULTI, bool SAT>
 __device__ __forceinline__ void stream_test_generic(const FastParams &P, const StreamSmem<WEIGHTED> &S, int n_seg,
                                                     const float2 (&rx)[HPL], const float2 (&ry)[HPL],
                                                     const float2 (&rz)[HPL], const Tile &tl,
-                                                    int lane, int nsub, unsigned &n_recheck, int cur_pair, size_t src_off,
+                                                    int lane, int nsub, unsigned &n_recheck, size_t item_off,
                                                     const double (&rwt)[YAWB_RPL]) {
     const size_t nacc1 = (size_t)P.n_bins * nsub;  // accumulators of one type
     for (int sg = 0; sg < n_seg; ++sg) {
@@ -524,7 +524,7 @@ __device__ __forceinline__ void stream_test_generic(const FastParams &P, const S
 #endif
             __syncwarp();
             if (P.acc_global) {  // straight to the result: one atomic per non-empty sub-bin of the segment
-                const size_t o = src_off + (size_t)d.type * P.type_stride + ((size_t)cur_pair * P.n_bins + b) * nsub;
+                const size_t o = item_off + (size_t)d.type * P.type_stride + (size_t)b * nsub;
                 for (int k = lane; k < nsub; k += 32) {
                     if (W.hist[k]) atomicAdd(&P.out_cnt[o + k], (unsigned long long)W.hist[k]);
                     if (WEIGHTED && W.histw[k] != 0.0) atomicAdd(&P.out_w[o + k], W.histw[k]);
@@ -550,6 +550,13 @@ __device__ __forceinline__ void stream_test_generic(const FastParams &P, const S
             }
         }
     }
+}
+
+// Results of an item (first catalog 0): its output block (second catalog of a joint launch, then label; Item::blk), its
+// patch pair.  Read from the item's slot where it is needed rather than kept in registers through the tick.  The
+// accumulators are flushed at the end of every item, so items of different blocks never share them.
+__device__ __forceinline__ size_t item_offset(const FastParams &P, const Item &it, int nsub) {
+    return (size_t)it.blk * P.n_types * P.type_stride + (size_t)it.pair * P.n_bins * nsub;
 }
 
 // ---- the kernel ----------------------------------------------------------------------------------------
@@ -610,12 +617,8 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
         const int c_cnt = raw_cnt, c_slot = raw_slot;
         const bool c_first = raw_first, c_last = raw_last;
         int n_seg = 0;
-        int cur_pair = 0;
-        size_t src_off = 0;  // results of the second catalog of a joint launch follow those of the first
         if (c_cnt >= 0) {
             const Item &it = S.items[c_slot];
-            cur_pair = it.pair;
-            src_off = (size_t)it.src * P.n_types * P.type_stride;
             double dx[YAWB_RPL], dy[YAWB_RPL], dz[YAWB_RPL];
             if (c_first) {
                 // rows of the tile: loads issued now, used after the conversion of the raw chunk
@@ -710,14 +713,16 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
                 if constexpr (!WEIGHTED && !MULTI && SAT)
                     stream_test_sat(P, S, n_seg, rx, ry, rz, tl, lane, n_recheck);
                 else
-                    stream_test_generic<WEIGHTED, MULTI, SAT>(P, S, n_seg, rx, ry, rz, tl, lane, nsub, n_recheck, cur_pair, src_off, rwt);
+                    stream_test_generic<WEIGHTED, MULTI, SAT>(P, S, n_seg, rx, ry, rz, tl, lane, nsub, n_recheck,
+                                                               item_offset(P, S.items[c_slot], nsub), rwt);
             }
-            if (c_last) {  // the item is complete: its counts go to the result of its patch pair
+            if (c_last) {  // the item is complete: its counts go to the result of its patch pair and output block
                 __syncwarp();
                 const size_t nacc1 = (size_t)P.n_bins * nsub;
+                const size_t item_off = item_offset(P, S.items[c_slot], nsub);
                 for (int k = lane; k < nacc; k += 32) {
                     const int type = k >= (int)nacc1 ? 1 : 0;
-                    const size_t o = src_off + (size_t)type * P.type_stride + (size_t)cur_pair * nacc1 + (k - type * nacc1);
+                    const size_t o = item_off + (size_t)type * P.type_stride + (k - type * nacc1);
                     const unsigned long long c = S.acc[k];
                     if (c) {
                         atomicAdd(&P.out_cnt[o], c);

@@ -96,8 +96,9 @@ struct __align__(16) Item {
     int b_lo, b_hi;        // z-bins of the first catalog covered by this item
     int row_lo, row_hi;    // cell rows of the query covered, relative to its first row (whole query: 0, INT_MAX);
                            // a restriction only occurs on items of a single z-bin
-    int src;               // second catalog of a joint launch (0 or 1)
-    int pad[3];
+    int src;               // second catalog of a joint launch (0 or 1): where the tile's rows live
+    int blk;               // output block of the item's counts: second catalog, then label (YAWB_FLAG_SECOND_LABELS)
+    int pad[2];
     double lo[3], hi[3];
 };
 static_assert(sizeof(Item) == 96, "Item is copied as six 16-byte pieces");
@@ -269,6 +270,8 @@ struct CountArgs {
     long long n_items;                  // (patch pair, tile) combinations = threads of the planner
     const long long *d_pair_item_base_b = nullptr;  // the same for c2b
     long long n_items_b = 0;
+    bool labels = false;    // YAWB_FLAG_SECOND_LABELS: the z-bin ids of a binned second catalog are sample labels
+    int blk_b = 1;          // first output block of c2b (= labels of c2)
     long long cap_heavy, cap_light;     // capacities of the two work-item lists
     int n_pairs;
     int n_bins;
@@ -277,7 +280,7 @@ struct CountArgs {
     const float *d_r2f;      // same, rounded to float
     const BinPar *d_binpar;  // [n_bins]
     double rmax_all;         // max search radius over non-empty z-bins
-    unsigned long long *d_out_cnt;  // [n_types][n_pairs][n_bins][n_edges-1]
+    unsigned long long *d_out_cnt;  // [n_blocks][n_types][n_pairs][n_bins][n_edges-1], blocks: second catalog, then label
     double *d_out_w;                // same or nullptr if every catalog is unweighted
     bool weighted;
     // exact all-pairs kernel only (single catalogs): the first catalog's raw (patch, bin)-sorted rows

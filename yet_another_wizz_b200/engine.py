@@ -192,6 +192,20 @@ class Engine:
                                            int(n_bins), _ptr(total), _ptr(samples)))
         return total, samples
 
+    def _labels_flag(self, labels: bool) -> int:
+        if not labels:
+            return 0
+        version = self.lib.yawb_version()
+        if version < _lib.LABELS_MIN_VERSION:
+            raise _lib.YawbError(f"labels=True needs libyawb version >= {_lib.LABELS_MIN_VERSION} (loaded: {version})")
+        return _lib.FLAG_SECOND_LABELS
+
+    @staticmethod
+    def _shape(cat2: DeviceCatalog, labels: bool, n_pairs: int, n_bins: int, n_edges: int) -> tuple:
+        """result shape of one (first, second) catalog combination: a leading label axis with `labels`"""
+        shape = (n_pairs, n_bins, n_edges - 1)
+        return ((cat2.n_bins if cat2.binned else 1), *shape) if labels else shape
+
     def count(
         self,
         cat1: DeviceCatalog,
@@ -201,10 +215,16 @@ class Engine:
         r2_edges: np.ndarray,
         *,
         exact: bool = False,
+        labels: bool = False,
     ) -> tuple[np.ndarray, np.ndarray, dict]:
         """
         Returns `(counts_i64, sums_f64, stats)`, both arrays shaped
         `(n_pairs, n_bins, n_edges - 1)`.
+
+        `labels=True` (`YAWB_FLAG_SECOND_LABELS`): the z-bin ids of a binned `cat2` are sample labels 0..L-1 (L =
+        `cat2.n_bins`, 1 for an unbinned `cat2`); every row is paired with every z-bin of `cat1` and the arrays
+        gain a leading label axis, `(L, n_pairs, n_bins, n_edges - 1)`: entry l is the count against the rows of
+        label l alone.
         """
         pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
         pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
@@ -216,10 +236,11 @@ class Engine:
             raise ValueError(f"r2_edges must have shape (n_bins={n_bins}, n_edges)")
         n_edges = r2_edges.shape[1]
         n_pairs = len(pair_i)
-        out_i = np.zeros((n_pairs, n_bins, n_edges - 1), dtype=np.int64)
-        out_f = np.zeros((n_pairs, n_bins, n_edges - 1), dtype=np.float64)
+        shape = self._shape(cat2, labels, n_pairs, n_bins, n_edges)
+        out_i = np.zeros(shape, dtype=np.int64)
+        out_f = np.zeros(shape, dtype=np.float64)
         stats = _lib.YawbStats()
-        flags = _lib.FLAG_EXACT_BRUTEFORCE if exact else 0
+        flags = (_lib.FLAG_EXACT_BRUTEFORCE if exact else 0) | self._labels_flag(labels)
         _lib.check(
             self.lib.yawb_count(
                 self._h, cat1._h, cat2._h, _ptr(pair_i), _ptr(pair_j), n_pairs, _ptr(r2_edges), n_edges,
@@ -238,13 +259,15 @@ class Engine:
         r2_edges: np.ndarray,
         *,
         out_device: tuple[int, int, int, int] | None = None,
+        labels: bool = False,
     ) -> tuple[tuple[np.ndarray, np.ndarray], tuple[np.ndarray, np.ndarray], dict]:
         """`count(cat1a, cat2)` and `count(cat1b, cat2)` in one pass over a fused index of the two first
         catalogs (`yawb_count2`): returns `((counts_a, sums_a), (counts_b, sums_b), stats)`.
 
         `out_device = (sums_a, counts_a, sums_b, counts_b)`: raw device pointers (0 = not wanted) of
         caller-owned buffers shaped `(n_pairs, n_bins, n_edges - 1)`; the results stay on the device
-        (`YAWB_FLAG_OUT_DEVICE`, e.g. for an NCCL reduce) and the arrays returned are `None`."""
+        (`YAWB_FLAG_OUT_DEVICE`, e.g. for an NCCL reduce) and the arrays returned are `None`.
+        `labels`: as in `count`; the results (and device buffers) gain the leading label axis of `cat2`."""
         pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
         pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
         r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
@@ -254,21 +277,22 @@ class Engine:
         if r2_edges.shape[0] != n_bins:
             raise ValueError(f"r2_edges must have shape (n_bins={n_bins}, n_edges)")
         n_edges = r2_edges.shape[1]
-        shape = (len(pair_i), n_bins, n_edges - 1)
+        shape = self._shape(cat2, labels, len(pair_i), n_bins, n_edges)
         stats = _lib.YawbStats()
+        lab = self._labels_flag(labels)
         if out_device is not None:
             ptrs = [c_void_p(p) if p else None for p in out_device]
             _lib.check(
                 self.lib.yawb_count2(
                     self._h, cat1a._h, cat1b._h, cat2._h, _ptr(pair_i), _ptr(pair_j), len(pair_i), _ptr(r2_edges), n_edges,
-                    _lib.FLAG_OUT_DEVICE, *ptrs, byref(stats),
+                    _lib.FLAG_OUT_DEVICE | lab, *ptrs, byref(stats),
                 )
             )
             return (None, None), (None, None), stats.as_dict()
         out = [(np.zeros(shape, dtype=np.int64), np.zeros(shape, dtype=np.float64)) for _ in range(2)]
         _lib.check(
             self.lib.yawb_count2(
-                self._h, cat1a._h, cat1b._h, cat2._h, _ptr(pair_i), _ptr(pair_j), len(pair_i), _ptr(r2_edges), n_edges, 0,
+                self._h, cat1a._h, cat1b._h, cat2._h, _ptr(pair_i), _ptr(pair_j), len(pair_i), _ptr(r2_edges), n_edges, lab,
                 _ptr(out[0][1]), _ptr(out[0][0]), _ptr(out[1][1]), _ptr(out[1][0]), byref(stats),
             )
         )
@@ -285,6 +309,7 @@ class Engine:
         r2_edges: np.ndarray,
         *,
         out_device: tuple | None = None,
+        labels: bool = False,
     ):
         """The four counts of a cross-correlation in ONE launch (`yawb_count4`): `count(cat1a, cat2a)`,
         `count(cat1b, cat2a)`, `count(cat1a, cat2b)`, `count(cat1b, cat2b)` -- DD, RD, DR, RR for (reference, its
@@ -292,7 +317,9 @@ class Engine:
         `([(counts, sums)] * 4, stats)` in that order.
 
         `out_device = (sums_0, counts_0, ..., sums_3, counts_3)`: raw device pointers (0 = not wanted); the results
-        stay on the device and the arrays returned are `None`."""
+        stay on the device and the arrays returned are `None`.
+        `labels`: as in `count`; each output gains the leading label axis of its own second catalog (e.g. a
+        labelled unknown sample as `cat2a` with a shared, unbinned random catalog as `cat2b`)."""
         pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
         pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
         r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
@@ -302,7 +329,7 @@ class Engine:
         if r2_edges.shape[0] != n_bins:
             raise ValueError(f"r2_edges must have shape (n_bins={n_bins}, n_edges)")
         n_edges = r2_edges.shape[1]
-        shape = (len(pair_i), n_bins, n_edges - 1)
+        shapes = [self._shape(c2, labels, len(pair_i), n_bins, n_edges) for c2 in (cat2a, cat2a, cat2b, cat2b)]
         stats = _lib.YawbStats()
         tab_f, tab_i = (c_void_p * 4)(), (c_void_p * 4)()
         out = None
@@ -312,11 +339,12 @@ class Engine:
                 tab_i[t] = out_device[2 * t + 1] or None
             flags = _lib.FLAG_OUT_DEVICE
         else:
-            out = [(np.zeros(shape, dtype=np.int64), np.zeros(shape, dtype=np.float64)) for _ in range(4)]
+            out = [(np.zeros(s, dtype=np.int64), np.zeros(s, dtype=np.float64)) for s in shapes]
             for t in range(4):
                 tab_i[t] = out[t][0].ctypes.data
                 tab_f[t] = out[t][1].ctypes.data
             flags = 0
+        flags |= self._labels_flag(labels)
         _lib.check(
             self.lib.yawb_count4(
                 self._h, cat1a._h, cat1b._h, cat2a._h, cat2b._h, _ptr(pair_i), _ptr(pair_j), len(pair_i), _ptr(r2_edges),

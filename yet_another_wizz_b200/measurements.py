@@ -20,6 +20,7 @@ from __future__ import annotations
 
 import logging
 import os
+from collections.abc import Sequence
 from copy import deepcopy
 from itertools import compress
 
@@ -34,7 +35,7 @@ from .paircounts import NormalisedCounts, NormalisedScalarCounts, PatchedCounts,
 from .sharding import Shard, assign_pairs_lpt, current_shard, pair_costs
 
 __all__ = ["PatchLinkage", "autocorrelate", "autocorrelate_scalar", "compute_scalar_normalisation", "crosscorrelate",
-           "crosscorrelate_scalar", "get_default_engine", "last_stats"]
+           "crosscorrelate_scalar", "crosscorrelate_tomographic", "get_default_engine", "last_stats"]
 
 logger = logging.getLogger("yaw_b200")
 
@@ -171,20 +172,69 @@ def prepare_catalog_arrays(catalog, binning: Binning | None, *, kappa: bool = Fa
                 ids[ids < 0] = 255
             zb[s:e] = ids
 
-    if workers is None:
-        workers = min(16, os.cpu_count() or 1)
-    if workers > 1 and len(patch_ids) > 1 and n > 200_000:
-        from concurrent.futures import ThreadPoolExecutor
-
-        with ThreadPoolExecutor(max_workers=workers) as pool:
-            list(pool.map(fill, patch_ids))
-    else:
-        for pid in patch_ids:
-            fill(pid)
+    _run_fill(fill, patch_ids, n, workers)
     out = dict(xyz=xyz, patch_off=off, weights=ws, zbin=zb, n_bins=len(binning) if binning is not None else 1)
     if zr is not None:
         out.update(redshifts=zr, edges=np.asarray(binning.edges, dtype=np.float64), closed=str(binning.closed))
     return out
+
+
+def _run_fill(fill, tasks, n_rows: int, workers: int | None) -> None:
+    """`fill(task)` for every task; by a small thread pool (numpy releases the GIL) when the rows are many"""
+    if workers is None:
+        workers = min(16, os.cpu_count() or 1)
+    if workers > 1 and len(tasks) > 1 and n_rows > 200_000:
+        from concurrent.futures import ThreadPoolExecutor
+
+        with ThreadPoolExecutor(max_workers=workers) as pool:
+            list(pool.map(fill, tasks))
+    else:
+        for task in tasks:
+            fill(task)
+
+
+def prepare_labelled_arrays(catalogs, *, workers: int | None = None, alloc=None) -> dict:
+    """Host preparation of ONE labelled catalog from several (`YAWB_FLAG_SECOND_LABELS`): per patch the rows of
+    `catalogs[0]`, `catalogs[1]`, ..., each row labelled with the position of its catalog (byte-sized ids, at
+    most 254 catalogs).  The rows and their unit vectors are those `prepare_catalog_arrays` gives each catalog.
+    Returns the keyword arguments of `Engine.upload_catalog`."""
+    alloc = alloc or np.empty
+    catalogs = list(catalogs)
+    if not 1 <= len(catalogs) <= 254:
+        raise ValueError("a labelled catalog holds 1 to 254 catalogs")
+    has_w = bool(catalogs[0].has_weights)
+    if any(bool(c.has_weights) != has_w for c in catalogs):
+        raise ValueError("the catalogs of a labelled upload must all have weights or all have none")
+    n_patch = len(catalogs[0])
+    for c in catalogs:
+        if list(c.keys()) != list(range(n_patch)):
+            raise InconsistentPatchesError("patch IDs must be 0..num_patches-1")
+    sizes = np.array([[int(n) for n in c.get_num_records()] for c in catalogs], dtype=np.int64)  # (label, patch)
+    # row offset of (patch, label): patch-major, the labels of a patch one after the other
+    start = np.concatenate([[0], np.cumsum(sizes.T.ravel())]).astype(np.int64)
+    off = np.ascontiguousarray(start[:: len(catalogs)])
+    n = int(off[-1])
+    xyz = alloc((n, 3), np.float64)
+    ws = alloc(n, np.float64) if has_w else None
+    lab = alloc(n, np.uint8)
+
+    def fill(task) -> None:
+        label, pid = task
+        ra, dec, weights, _, _ = _patch_rows(catalogs[label][pid])
+        s = int(start[pid * len(catalogs) + label])
+        e = s + int(sizes[label, pid])
+        if len(ra) != e - s:
+            raise InconsistentPatchesError(f"patch {pid} holds {len(ra)} rows, its meta data says {e - s}")
+        cos_dec = np.cos(dec)  # same operations, same order as prepare_catalog_arrays
+        np.multiply(np.cos(ra), cos_dec, out=xyz[s:e, 0])
+        np.multiply(np.sin(ra), cos_dec, out=xyz[s:e, 1])
+        np.sin(dec, out=xyz[s:e, 2])
+        if has_w:
+            ws[s:e] = weights
+        lab[s:e] = label
+
+    _run_fill(fill, [(label, pid) for pid in range(n_patch) for label in range(len(catalogs))], n, workers)
+    return dict(xyz=xyz, patch_off=off, weights=ws, zbin=lab, n_bins=len(catalogs))
 
 
 def _prepare_for(engine, catalog, binning: Binning | None, kappa: bool) -> dict:
@@ -628,6 +678,139 @@ def crosscorrelate(config, reference, unknown, *, ref_rand=None, unk_rand=None, 
         links._uploads.free()
         links._uploads = None
     return [CorrFunc(dd, dr, rd, rr) for dd, dr, rd, rr in zip(DD, DR, RD, RR)]
+
+
+def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, unk_rand=None, progress: bool = False,
+                               max_workers=None, engine=None, shard: Shard | None = None) -> list[list[CorrFunc]]:
+    """`crosscorrelate` of the reference sample with every tomographic bin of the unknown sample in one pass:
+    `result[i]` is `crosscorrelate(config, reference, unknowns[i], ref_rand=ref_rand, unk_rand=<randoms of bin
+    i>)`, the loop of the reference CLI's `CrossCorrTask` (`cli/tasks.py:536-550`) as one call.
+
+    `unknowns`: 1 to 254 catalogs, one per bin, all with weights or all without.  `unk_rand`: None, one catalog
+    shared by every bin, or a sequence of one catalog per bin.  The bins travel to the device as ONE labelled
+    catalog (`YAWB_FLAG_SECOND_LABELS`), per-bin randoms likewise; every count runs once over the union of the
+    bins' patch-pair lists, and each bin is packaged from its own linkage.  A shared `unk_rand` is counted once
+    (DR and RR) for all bins.  Everything a per-bin call would raise is raised before any counting.
+    `progress` / `max_workers` are accepted and ignored."""
+    unknowns = list(unknowns)
+    n_tomo = len(unknowns)
+    if n_tomo == 0:
+        raise ValueError("'unknowns' must hold at least one catalog")
+    if n_tomo > 254:
+        raise ValueError(f"at most 254 tomographic bins are supported (got {n_tomo})")
+    shared = unk_rand is not None and not isinstance(unk_rand, Sequence)
+    if unk_rand is None or shared:
+        rands = [unk_rand] * n_tomo
+    else:
+        rands = list(unk_rand)
+        if len(rands) != n_tomo:
+            raise ValueError(f"'unk_rand' holds {len(rands)} catalogs for {n_tomo} tomographic bins")
+        if any(r is None for r in rands):
+            raise ValueError("a per-bin 'unk_rand' must hold one catalog for every bin")
+    for unknown, rand in zip(unknowns, rands):
+        _ensure_unique_catalogs(reference, unknown, ref_rand, rand)
+    if ref_rand is None and unk_rand is None:
+        raise ValueError("at least one random dataset must be provided")
+    if len({bool(c.has_weights) for c in unknowns}) > 1:
+        raise ValueError("the tomographic bins must all have weights or all have none")
+    if not shared and unk_rand is not None and len({bool(c.has_weights) for c in rands}) > 1:
+        raise ValueError("the per-bin randoms must all have weights or all have none")
+    # the linkage of every bin, exactly as its own call would build it: the largest catalog decides the links
+    links = [PatchLinkage.from_catalogs(config, reference, unknown, *[c for c in (ref_rand, rand) if c is not None],
+                                        engine=engine, shard=shard) for unknown, rand in zip(unknowns, rands)]
+    bin_pairs = [lk.get_patch_id_pairs(auto=False) for lk in links]
+    union: dict[tuple[int, int], int] = {}
+    for pi, pj in bin_pairs:
+        for pair in zip(pi.tolist(), pj.tolist()):
+            union.setdefault(pair, len(union))
+    union_ij = np.array(list(union), dtype=np.int32).reshape(-1, 2)
+    # rows of the union that make up each bin's pair list, in that bin's order
+    bin_rows = [np.array([union[p] for p in zip(pi.tolist(), pj.tolist())], dtype=np.int64) for pi, pj in bin_pairs]
+
+    driver = links[0]
+    eng = engine or get_default_engine()
+    shard = shard or current_shard()
+    binning = _as_binning(config)
+    plan = driver._get_plan()
+    num_patches = len(reference)
+    _last_stats.clear()
+    uploads = _Uploads(eng)
+    labelled = []  # device catalogs of this call only
+
+    def upload_labelled(catalogs):
+        arrays = prepare_labelled_arrays(catalogs)
+        dev = eng.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
+        labelled.append(dev)
+        return dev
+
+    own = np.arange(len(union_ij))
+    if shard.active:  # a pair's cost sums the rows of every bin
+        first = reference if ref_rand is None or sum(reference.get_num_records()) >= sum(ref_rand.get_num_records()) \
+            else ref_rand
+        n2 = np.sum([u.get_num_records() for u in unknowns], axis=0)
+        costs = pair_costs(union_ij[:, 0], union_ij[:, 1], first.get_num_records(), n2,
+                           radii1=np.asarray(first.get_radii().data))
+        own = assign_pairs_lpt(costs, shard.world_size)[shard.rank]
+    pi_own, pj_own = union_ij[own, 0], union_ij[own, 1]
+
+    def gather(hist):
+        """(L, own pairs, ...) -> (L, union pairs, ...) summed over the ranks: one reduce per count tensor"""
+        return np.moveaxis(driver._gather_shards(shard, np.moveaxis(hist, 1, 0), own, len(union_ij)), 0, 1)
+
+    fuse = (ref_rand is not None and bool(reference.has_weights) == bool(ref_rand.has_weights)
+            and hasattr(eng, "count2") and os.environ.get("YAWB_FUSE", "1") != "0")
+    hists: dict[str, np.ndarray] = {}
+    try:
+        uploads.enqueue(((reference, binning), (ref_rand, binning), (unk_rand if shared else None, None)))
+        dev_ref = uploads.get(reference, binning)
+        dev_rr = uploads.get(ref_rand, binning) if ref_rand is not None else None
+        dev_unk = upload_labelled(unknowns)
+        dev_ur = None
+        if unk_rand is not None:
+            dev_ur = uploads.get(unk_rand, None) if shared else upload_labelled(rands)
+        sw = dict(ref=dev_ref.sum_weights(), unk=dev_unk.sum_weights())
+        if dev_rr is not None:
+            sw["rr"] = dev_rr.sum_weights()
+        if dev_ur is not None:
+            sw["ur"] = dev_ur.sum_weights()
+        if fuse:
+            for second, kinds in ((dev_unk, ("DD", "RD")), (dev_ur, ("DR", "RR"))):
+                if second is None:
+                    continue
+                out_a, out_b, stats = eng.count2(dev_ref, dev_rr, second, pi_own, pj_own, plan.r2, labels=True)
+                weighted = dev_ref.weighted or dev_rr.weighted or second.weighted
+                hists[kinds[0]] = gather(out_a[1] if weighted else out_a[0])
+                hists[kinds[1]] = gather(out_b[1] if weighted else out_b[0])
+                _last_stats["+".join(kinds)] = stats
+        else:
+            for kind, dev1, dev2 in (("DD", dev_ref, dev_unk), ("RD", dev_rr, dev_unk), ("DR", dev_ref, dev_ur),
+                                     ("RR", dev_rr, dev_ur)):
+                if dev1 is None or dev2 is None:
+                    continue
+                hist_i, hist_f, stats = eng.count(dev1, dev2, pi_own, pj_own, plan.r2, labels=True)
+                hists[kind] = gather(hist_f if (dev1.weighted or dev2.weighted) else hist_i)
+                _last_stats[kind] = stats
+    finally:
+        for dev in labelled:
+            dev.free()
+        uploads.free()
+
+    none = [None for _ in range(config.scales.num_scales)]
+    result = []
+    for i, ((pi, pj), rows) in enumerate(zip(bin_pairs, bin_rows)):
+        def package(kind, sw1, sw2, label):
+            if kind not in hists:
+                return none
+            return PatchLinkage._package(hists[kind][label][rows], plan, binning, num_patches, pi, pj, sw[sw1],
+                                         sw[sw2][label:label + 1], False)
+
+        rand_label = 0 if shared else i
+        DD = package("DD", "ref", "unk", i)
+        RD = package("RD", "rr", "unk", i)
+        DR = package("DR", "ref", "ur", rand_label)
+        RR = package("RR", "rr", "ur", rand_label)
+        result.append([CorrFunc(dd, dr, rd, rr) for dd, dr, rd, rr in zip(DD, DR, RD, RR)])
+    return result
 
 
 # ---- scalar-field correlations (NK / KK) ----------------------------------------------------------------
