@@ -324,11 +324,9 @@ def test_four_counts_in_one_launch_equal_four_counts(engine):
             d.free()
 
 
-@pytest.mark.parametrize("variant", ["sat", "pred"])
-def test_pair_test_variants_exact(engine, variant, monkeypatch):
-    """both FP32 pair-test formulations (7-instruction saturating ramp / 8-instruction predicated) must
-    reproduce the reference's counts on the adversarial on-edge set and on dense random data"""
-    monkeypatch.setenv("YAWB_PAIR_TEST", variant)
+def test_pair_test_variants_exact(engine):
+    """the saturating-ramp FP32 pair test of the unweighted single-bin kernel must reproduce the reference's
+    counts on the adversarial on-edge set and on dense random data"""
     g = golden_io.load("edge_adversarial")
     a, b = g["a_xyz"], g["b_xyz"]
     for key in ("upper", "lower"):

@@ -89,21 +89,18 @@ def _same(got, want, weighted):
         assert_array_equal(got, want)
 
 
-VARIANTS = {  # name: (weighted, n_edges, YAWB_PAIR_TEST)
-    "single": (False, 2, None),
-    "single_pred": (False, 2, "pred"),
-    "cumulative": (False, 4, None),
-    "subbins": (False, 24, None),
-    "weighted_single": (True, 2, None),
-    "weighted_multi": (True, 5, None),
+VARIANTS = {  # name: (weighted, n_edges)
+    "single": (False, 2),
+    "cumulative": (False, 4),
+    "subbins": (False, 24),
+    "weighted_single": (True, 2),
+    "weighted_multi": (True, 5),
 }
 
 
 @pytest.mark.parametrize("variant", list(VARIANTS))
-def test_labelled_equals_per_label_uploads(engine, variant, monkeypatch):
-    weighted, n_edges, pair_test = VARIANTS[variant]
-    if pair_test:
-        monkeypatch.setenv("YAWB_PAIR_TEST", pair_test)
+def test_labelled_equals_per_label_uploads(engine, variant):
+    weighted, n_edges = VARIANTS[variant]
     s = Setup(engine, weighted=weighted)
     try:
         r2 = s.r2(n_edges)

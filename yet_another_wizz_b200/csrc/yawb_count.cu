@@ -7,7 +7,7 @@
 // k_plan          -- one thread per (patch pair, register tile of the second catalog): the tile's bounding box is
 //   rotated into the frame of the first catalog's patch, tested against that patch's box grown by the largest
 //   search radius, and the survivors are written as self-contained work items (split so that an item never
-//   holds more than YAWB_CCAP (z-bin, cell row) runs).
+//   holds more than CCAP (z-bin, cell row) runs).
 // k_count_stream  -- the production kernel (yawb_count_stream.cuh).  One warp owns a register tile of YAWB_TILE
 //   second-catalog points (YAWB_RPL per lane).  For every z-bin it gathers the first-catalog rows of the linked
 //   patch that fall into the tile's bounding box grown by the bin's search radius (sky-cell rows -> contiguous
@@ -23,8 +23,6 @@
 // k_count_exact   -- all-pairs FP64 kernel without pruning (validation and cross-check).
 #include <cfloat>
 #include <climits>
-#include <cstdlib>
-#include <cstring>
 
 #include "yawb_internal.cuh"
 
@@ -32,22 +30,13 @@ namespace {
 
 constexpr unsigned FULL = 0xffffffffu;
 constexpr float EPS32 = 5.9604645e-8f;  // 2^-24
-#ifndef YAWB_CHUNK
-#define YAWB_CHUNK 8
-#endif
-constexpr int CHUNK = YAWB_CHUNK;       // candidates between consistency checks (power of two)
+constexpr int CHUNK = 8;                // candidates between consistency checks (power of two)
 // Coordinates of the padding rows of a short tile: NaN.  u = NaN fails |u| < h, and a saturating FMA flushes NaN to +0
 // (PTX: "NaN results are flushed to +0.0f"), so every form of the pair test counts such a row as decided and outside.
 #define PAD_ROW __int_as_float(0x7fffffff)
-#ifndef YAWB_CCAP
-#define YAWB_CCAP 160
-#endif
-#ifndef YAWB_CCAP_SMALL
-#define YAWB_CCAP_SMALL 24
-#endif
-#ifndef YAWB_SMALL_JOB_ITEMS
-#define YAWB_SMALL_JOB_ITEMS 30
-#endif
+constexpr int CCAP = 160;               // (z-bin, cell row) runs per item; the planner splits items to fit
+constexpr int CCAP_SMALL = 24;          // the same for a small job (yawb_launch_count_fast)
+constexpr int SMALL_JOB_ITEMS = 30;     // (pair, tile) combinations per warp below which a job is small
 
 struct FastParams {
     // first-role index (one catalog, or two fused).  The exact rows of a candidate are only needed by the FP64
@@ -68,7 +57,6 @@ struct FastParams {
     // work items written by the planner: patch-diagonal items first, then the boundary items
     const Item *items_heavy, *items_light;
     long long cap_heavy, cap_light;
-    int debug;
     int n_pairs, n_bins, n_edges;
     const double *r2;
     const float *r2f;
@@ -152,42 +140,85 @@ __device__ __forceinline__ double warp_sum(double v) {
 typedef float4 Cand;
 constexpr int HPL = YAWB_RPL / 2;  // row pairs per lane
 
-// ---- view of a warp's staged list for the phase-2 functions --------------------------------------
-template <bool WEIGHTED>
-struct WarpSmem {
-    Cand *list;               // [LCAP] staged candidates
-    double *lw;               // [LCAP] their weights (WEIGHTED)
-    unsigned long long *acc;  // [n_bins * nsub] pair counts of the current patch pair
-    double *accw;             // same, weighted sums (WEIGHTED)
-    double *histw;            // [nsub] scratch histogram of one z-bin (MULTI && WEIGHTED)
-    float4 *binrec;           // [n_bins] half extents of the query box (x, y, z) and mid
-    float2 *binthr;           // [n_bins] (h - eps, h + eps)
-    int *lidx;                // [LCAP] row of the candidate in the sorted first catalog
-    int *bin_iv0;             // [n_bins] first cell row of the query box
-    int *bin_iu;              // [n_bins] iu0 | iu1 << 16
-    int *cstart;              // [n_bins + 1] prefix of cell rows per z-bin
-    int *rs0;                 // [CCAP] first candidate row of a (bin, cell-row) run
-    int *rpre;                // [CCAP] inclusive prefix of run lengths
-    int *cbin;                // [CCAP] z-bin of the run
-    unsigned *hist;           // [nsub] (MULTI)
-    unsigned short *lbin;     // [LCAP] z-bin of the candidate
-    unsigned short *seg;      // [LCAP] first entry of every z-bin segment of the staged list
-    float *cum;               // [n_bins][CUM_EDGES] ramp offsets K (e_k - mid) + 1/2 of the item (MULTI && SAT)
-    unsigned *cumtot;         // [CUM_EDGES] cumulative counts of one z-bin segment (MULTI && SAT)
+// ---- the paths of the streaming kernel; the host picks one per count (yawb_launch_count_fast) ---------------
+enum class CountPath {
+    Single,             // unweighted, one sub-bin: saturating ramp (stream_test_sat)
+    SingleWeighted,     // weighted, one sub-bin: predicated test, weighted sums (phase2_single)
+    Cumulative,         // unweighted, a few sub-bins: cumulative counts with the saturating ramp (phase2_cumul)
+    Histogram,          // unweighted, many sub-bins: in-range tests classified into a histogram (phase2_multi_queue)
+    HistogramWeighted,  // weighted, several sub-bins: the same with weighted sums
+};
+__host__ __device__ constexpr bool path_weighted(CountPath p) {
+    return p == CountPath::SingleWeighted || p == CountPath::HistogramWeighted;
+}
+__host__ __device__ constexpr bool path_multi(CountPath p) { return p != CountPath::Single && p != CountPath::SingleWeighted; }
+
+// ---- a warp's block of shared memory in the streaming kernel (yawb_count_stream.cuh) ----------------------
+constexpr int LB = 128;   // rows per raw chunk = capacity of the staged list
+constexpr int NSLOT = 4;  // items in flight per warp: consumed, produced, planned, fetched
+
+// The staged frame of an item ("tile frame"): origin O = the point of the unit sphere in the direction of the centre of
+// the tile box, axes (t1, t2, n) with n = O - (centre of the sphere).  For a row P of the tile (a unit vector)
+// |P - O|^2 = -2 (P - O).n, so the squared chord to a candidate s needs no |r|^2 term:
+//     |r - s|^2 - mid = (|s|^2 - mid) + r . (-2 s_x, -2 s_y, -2 (1 + s_z))        (three FMAs per test)
+struct __align__(16) ItemAux {
+    double R[9];        // rows t1, t2, n of the tile frame, in coordinates of the frame of p1
+    double O[3];        // origin of the tile frame, in coordinates of the frame of p1
+    double dq[3];       // lattice origin - O:  (row of the index) - O = (k - ko) * qinv + dq
+    int ko[3];          // lattice origin: the lattice point nearest to the centre of the tile box
+    int n_combo;        // runs of the item
+    float qinv;         // lattice spacing (a power of two)
+    float eu, ev, et;   // half extents of the tile box about the lattice origin, rounded up
+    float g;            // |lattice origin - O|, rounded up
+    int end;            // 1: the work list is exhausted, this slot holds no item
+    int pad[2];
+};
+static_assert(sizeof(ItemAux) % 16 == 0, "ItemAux layout");
+
+struct __align__(16) SegDesc {
+    short ea, eb;  // entries [ea, eb) of the staged list
+    short bin;     // their z-bin
+    short type;    // catalog of a fused first-role index (0 / 1)
+};
+
+struct StreamSmem {
+    Item *items;               // [NSLOT]
+    ItemAux *aux;              // [NSLOT]
+    int *bin_iv0, *bin_iu;     // [n_bins] plan: first cell row of the query, iu0 | iu1 << 16
+    int *cstart;               // [n_bins + 1] prefix of cell rows per z-bin
+    int2 *cs;                  // [CCAP] cell_start at the two ends of every run (lands asynchronously)
+    unsigned short *csbin;     // [CCAP] z-bin of the run
+    int2 *run;                 // [CCAP] run table of the item being produced: (inclusive prefix of the run lengths,
+                               //        row of the index that flat position 0 would have if the run started there)
+    unsigned short *cbin;      // [CCAP]
+    SRec *raw;                 // [LB] raw chunk (lands asynchronously)
+    unsigned short *rawbin;    // [LB]
+    double *rawlw;             // [LB] weights of the raw rows (weighted paths)
+    Cand *list;                // [LB] staged candidates: type 0 from the bottom, type 1 from the top
+    int *lidx;                 // [LB] row of the candidate in its catalog | catalog bit (SRec::aux)
+    unsigned short *lbin;      // [LB]
+    double *lw;                // [LB] (weighted paths)
+    SegDesc *seg;              // [n_types * n_bins]
+    float4 *binrec;            // [n_bins] half extents of the query box (x, y, z) and mid
+    float2 *binthr;            // [n_bins] thresholds of the pair test
+    unsigned long long *acc;   // [n_types][n_bins * nsub]
+    double *accw;              // same (weighted paths)
+    unsigned *hist;            // [nsub] scratch histogram of one z-bin segment (sub-bin paths)
+    double *histw;             // [nsub] (HistogramWeighted)
+    float *cum;                // [n_bins][CUM_EDGES] ramp offsets K (e_k - mid) + 1/2 of the item (sub-bin paths)
+    unsigned *cumtot;          // [CUM_EDGES] cumulative counts of one z-bin segment
 };
 
 // ---- exact re-evaluation of one lane's share of a chunk, done by the whole warp ----------------
 // Lane `src` saw a test inside the FP32 uncertainty band.  Its (YAWB_RPL x chunk) tests are
-// re-evaluated with the reference's FP64 expression, two or more per lane, and summed.
-template <bool WEIGHTED>
-__device__ __forceinline__ void recheck_chunk(const FastParams &P, const WarpSmem<WEIGHTED> &S, int e0, int e1,
+// re-evaluated with the reference's FP64 expression, two or more per lane, and summed (weighted single-bin path).
+__device__ __forceinline__ void recheck_chunk(const FastParams &P, const StreamSmem &S, int e0, int e1,
                                               const Tile &tl, int lane, int src, double lo, double hi,
                                               unsigned &cnt_out, double &w_out, unsigned &n_recheck) {
     unsigned cnt = 0;
     double wsum = 0.0;
     const double *const trow = YAWB_TILE_ROWS(P, tl);
     const double *const tw = YAWB_TILE_WEIGHTS(P, tl);
-    (void)tw;
     for (int t = lane; t < CHUNK * YAWB_RPL; t += 32) {
         const int e = e0 + (t & (CHUNK - 1));
         const int k = src + 32 * (t / CHUNK);
@@ -198,32 +229,28 @@ __device__ __forceinline__ void recheck_chunk(const FastParams &P, const WarpSme
             const double d2 = exact_d2(cxx, cyy, czz, trow[(size_t)YAWB_RSTRIDE * j], trow[(size_t)YAWB_RSTRIDE * j + 1], trow[(size_t)YAWB_RSTRIDE * j + 2]);
             if (d2 > lo && d2 <= hi) {
                 cnt += 1;
-                if (WEIGHTED) wsum += S.lw[e] * (tw ? tw[j] : 1.0);
+                wsum += S.lw[e] * (tw ? tw[j] : 1.0);
             }
             n_recheck += 1;
         }
     }
     cnt_out = __reduce_add_sync(FULL, cnt);
-    if (WEIGHTED) w_out = warp_sum(wsum);
+    w_out = warp_sum(wsum);
 }
 
 // The same for a span [e0, e1) of at most 16 entries (the streaming kernel checks once per <= 16 candidates): lane t
 // takes row t & 7 of lane `src` against candidates t >> 3, t >> 3 + 4, ...; all operands of a lane's (up to four)
-// tests are requested before the first is used, so the warp pays the memory latency once.
-template <bool WEIGHTED>
-__device__ __forceinline__ void recheck_span(const FastParams &P, const WarpSmem<WEIGHTED> &S, int e0, int e1,
+// tests are requested before the first is used, so the warp pays the memory latency once (unweighted single-bin path).
+__device__ __forceinline__ void recheck_span(const FastParams &P, const StreamSmem &S, int e0, int e1,
                                              const Tile &tl, int lane, int src, double lo, double hi,
-                                             unsigned &cnt_out, double &w_out, unsigned &n_recheck) {
+                                             unsigned &cnt_out, unsigned &n_recheck) {
     static_assert(YAWB_RPL == 8, "one lane per row of the flagged lane");
     constexpr int Q = 4;  // 16 candidates x 8 rows / 32 lanes
     unsigned cnt = 0;
-    double wsum = 0.0;
     const int k = src + 32 * (lane & 7);
     const bool row_ok = k < tl.count;
     const int j = tl.start + (row_ok ? k : 0);
     const double *const trow = YAWB_TILE_ROWS(P, tl);
-    const double *const tw = YAWB_TILE_WEIGHTS(P, tl);
-    (void)tw;
     const double bx = trow[(size_t)YAWB_RSTRIDE * j], by = trow[(size_t)YAWB_RSTRIDE * j + 1], bz = trow[(size_t)YAWB_RSTRIDE * j + 2];
     double ax[Q], ay[Q], az[Q];
     bool ok[Q];
@@ -238,26 +265,22 @@ __device__ __forceinline__ void recheck_span(const FastParams &P, const WarpSmem
     for (int q = 0; q < Q; ++q) {
         const double d2 = exact_d2(ax[q], ay[q], az[q], bx, by, bz);
         if (ok[q]) {
-            if (d2 > lo && d2 <= hi) {
-                cnt += 1;
-                if (WEIGHTED) wsum += S.lw[e0 + (lane >> 3) + 4 * q] * (tw ? tw[j] : 1.0);
-            }
+            if (d2 > lo && d2 <= hi) cnt += 1;
             n_recheck += 1;
         }
     }
     cnt_out = __reduce_add_sync(FULL, cnt);
-    if (WEIGHTED) w_out = warp_sum(wsum);
 }
 
 // ---- phase 2, single sub-bin (n_edges == 2): the hot loop ----------------------------------
 // One candidate against the lane's YAWB_RPL rows:  u = (rn + s.w) + rx s.x + ry s.y + rz s.z = d2 - mid.
-//   predicated: |u| < h - eps, |u| < h + eps (2 FSETP) + 2 predicated FADD, also feeds the weighted sums;
-//   SAT: v = sat(C - K |u|) is a ramp through the uncertainty band: exactly 1 well inside the bin,
+//   unweighted: v = sat(C - K |u|) is a ramp through the uncertainty band: exactly 1 well inside the bin,
 //        exactly 0 well outside, in [0.1, 0.9] wherever FP32 cannot decide (K = 0.4 / eps,
 //        C = 1/2 + h K).  sum(v) and sum(v*v) are equal iff every v of the chunk was 0 or 1 (then
-//        sum(v) is the exact count); an undecidable test makes them differ by >= 0.09.
+//        sum(v) is the exact count); an undecidable test makes them differ by >= 0.09;
+//   weighted (predicated): |u| < h - eps, |u| < h + eps (2 FSETP) + 2 predicated FADD, also feeds the weighted sums.
 // Two accumulator pairs (even / odd rows) halve the length of the dependent add chains.
-template <bool WEIGHTED, bool SAT>
+template <bool WEIGHTED>
 __device__ __forceinline__ void test_candidate(const Cand c, double swt, const float2 (&rx)[HPL],
                                                const float2 (&ry)[HPL], const float2 (&rz)[HPL],
                                                float ta, float tb, float2 &acc_a,
@@ -270,7 +293,7 @@ __device__ __forceinline__ void test_candidate(const Cand c, double swt, const f
         float2 u = __ffma2_rn(rx[k], sx, sw);
         u = __ffma2_rn(ry[k], sy, u);
         u = __ffma2_rn(rz[k], sz, u);
-        if (SAT) {
+        if constexpr (!WEIGHTED) {
             float2 v;
             v.x = __saturatef(fmaf(fabsf(u.x), ta, tb));  // ta = -K, tb = C
             v.y = __saturatef(fmaf(fabsf(u.y), ta, tb));
@@ -283,19 +306,16 @@ __device__ __forceinline__ void test_candidate(const Cand c, double swt, const f
             if (in1) acc_a.y += 1.f;
             if (a0 < tb) acc_b.x += 1.f;
             if (a1 < tb) acc_b.y += 1.f;
-            if (WEIGHTED) {
-                // ws += [in] * swt as one select on the high word of a 0.0 / 1.0 double plus one DFMA (a
-                // conditional FP64 add is lowered to an add plus two selects)
-                ws[2 * k] = fma(__hiloint2double(in0 ? 0x3ff00000 : 0, 0), swt, ws[2 * k]);
-                ws[2 * k + 1] = fma(__hiloint2double(in1 ? 0x3ff00000 : 0, 0), swt, ws[2 * k + 1]);
-            }
+            // ws += [in] * swt as one select on the high word of a 0.0 / 1.0 double plus one DFMA (a
+            // conditional FP64 add is lowered to an add plus two selects)
+            ws[2 * k] = fma(__hiloint2double(in0 ? 0x3ff00000 : 0, 0), swt, ws[2 * k]);
+            ws[2 * k + 1] = fma(__hiloint2double(in1 ? 0x3ff00000 : 0, 0), swt, ws[2 * k + 1]);
         }
     }
 }
 
-// entries [ea, eb) of the list belong to one z-bin
-template <bool WEIGHTED, bool SAT>
-__device__ __forceinline__ void phase2_single(const FastParams &P, const WarpSmem<WEIGHTED> &S, int ea, int eb,
+// ---- phase 2, weighted, single sub-bin: entries [ea, eb) of the list belong to one z-bin ---------------
+__device__ __forceinline__ void phase2_single(const FastParams &P, const StreamSmem &S, int ea, int eb,
                                               const float2 (&rx)[HPL], const float2 (&ry)[HPL],
                                               const float2 (&rz)[HPL],
                                               float ta, float tb, const Tile &tl, int lane, double lo,
@@ -305,41 +325,35 @@ __device__ __forceinline__ void phase2_single(const FastParams &P, const WarpSme
         const int e1 = min(e0 + CHUNK, eb);
         float2 acc_a = make_float2(0.f, 0.f), acc_b = make_float2(0.f, 0.f);
         double ws[YAWB_RPL];
-        if (WEIGHTED) {
 #pragma unroll
-            for (int r = 0; r < YAWB_RPL; ++r) ws[r] = 0.0;
-        }
+        for (int r = 0; r < YAWB_RPL; ++r) ws[r] = 0.0;
         if (e1 - e0 == CHUNK) {  // common case: fully unrolled, no loop bookkeeping
 #pragma unroll
             for (int k = 0; k < CHUNK; ++k)
-                test_candidate<WEIGHTED, SAT>(S.list[e0 + k], WEIGHTED ? S.lw[e0 + k] : 0.0, rx, ry, rz, ta, tb,
-                                              acc_a, acc_b, ws);
+                test_candidate<true>(S.list[e0 + k], S.lw[e0 + k], rx, ry, rz, ta, tb, acc_a, acc_b, ws);
         } else {
             for (int e = e0; e < e1; ++e)
-                test_candidate<WEIGHTED, SAT>(S.list[e], WEIGHTED ? S.lw[e] : 0.0, rx, ry, rz, ta, tb, acc_a,
-                                              acc_b, ws);
+                test_candidate<true>(S.list[e], S.lw[e], rx, ry, rz, ta, tb, acc_a, acc_b, ws);
         }
         const float sa = acc_a.x + acc_a.y, sb = acc_b.x + acc_b.y;
         unsigned c = (unsigned)(sa + 0.5f);
         double wsum = 0.0;
-        if (WEIGHTED) {
 #pragma unroll
-            for (int r = 0; r < YAWB_RPL; ++r) wsum += ws[r] * rwt[r];  // row weights live in registers
-        }
+        for (int r = 0; r < YAWB_RPL; ++r) wsum += ws[r] * rwt[r];  // row weights live in registers
         unsigned flagged = __ballot_sync(FULL, sa != sb);
         while (flagged) {  // warp-uniform: some lane met the uncertainty band of an edge
             const int src = __ffs(flagged) - 1;
             flagged &= flagged - 1;
             unsigned cx = 0;
             double wx = 0.0;
-            recheck_chunk<WEIGHTED>(P, S, e0, e1, tl, lane, src, lo, hi, cx, wx, n_recheck);
+            recheck_chunk(P, S, e0, e1, tl, lane, src, lo, hi, cx, wx, n_recheck);
             if (lane == src) {
                 c = cx;
                 wsum = wx;
             }
         }
         cnt_total += c;
-        if (WEIGHTED) w_total += wsum;
+        w_total += wsum;
     }
 }
 
@@ -380,9 +394,9 @@ __device__ __forceinline__ void recheck_cumul(const FastParams &P, const int *li
     for (int g = 0; g < G; ++g) cnt_out[g] = __reduce_add_sync(FULL, cnt[g]);
 }
 
-// entries [ea, eb) of the list belong to z-bin b; adds the sub-bin counts of the segment to S.acc
+// entries [ea, eb) of the list belong to z-bin b; adds the sub-bin counts of the segment to acc
 template <int CUM_GROUP>
-__device__ __forceinline__ void phase2_cumul_g(const FastParams &P, const WarpSmem<false> &S, int ea, int eb,
+__device__ __forceinline__ void phase2_cumul_g(const FastParams &P, const StreamSmem &S, unsigned long long *acc, int ea, int eb,
                                              const float2 (&rx)[HPL], const float2 (&ry)[HPL],
                                              const float2 (&rz)[HPL], float nk,
                                              const Tile &tl, int lane, int b, unsigned &n_recheck) {
@@ -449,85 +463,30 @@ __device__ __forceinline__ void phase2_cumul_g(const FastParams &P, const WarpSm
     }
     __syncwarp();
     // pairs with r2[s] < d2 <= r2[s + 1]: difference of the cumulative counts
-    if (lane < ne - 1) S.acc[(size_t)b * (ne - 1) + lane] += (unsigned long long)(S.cumtot[lane + 1] - S.cumtot[lane]);
+    if (lane < ne - 1) acc[(size_t)b * (ne - 1) + lane] += (unsigned long long)(S.cumtot[lane + 1] - S.cumtot[lane]);
     __syncwarp();
 }
 
-__device__ __forceinline__ void phase2_cumul(const FastParams &P, const WarpSmem<false> &S, int ea, int eb,
+__device__ __forceinline__ void phase2_cumul(const FastParams &P, const StreamSmem &S, unsigned long long *acc, int ea, int eb,
                                              const float2 (&rx)[HPL], const float2 (&ry)[HPL],
                                              const float2 (&rz)[HPL], float nk,
                                              const Tile &tl, int lane, int b, unsigned &n_recheck) {
     const int ne = P.n_edges;  // measured on C4 (6 edges): one pass of 6 beats two of 3 beats three of 2
-    if (ne <= 3) phase2_cumul_g<3>(P, S, ea, eb, rx, ry, rz, nk, tl, lane, b, n_recheck);
-    else if (ne == 5 || ne == 6) phase2_cumul_g<6>(P, S, ea, eb, rx, ry, rz, nk, tl, lane, b, n_recheck);
-    else phase2_cumul_g<4>(P, S, ea, eb, rx, ry, rz, nk, tl, lane, b, n_recheck);
+    if (ne <= 3) phase2_cumul_g<3>(P, S, acc, ea, eb, rx, ry, rz, nk, tl, lane, b, n_recheck);
+    else if (ne == 5 || ne == 6) phase2_cumul_g<6>(P, S, acc, ea, eb, rx, ry, rz, nk, tl, lane, b, n_recheck);
+    else phase2_cumul_g<4>(P, S, acc, ea, eb, rx, ry, rz, nk, tl, lane, b, n_recheck);
 }
 
-// ---- phase 2, several sub-bins (r-weights, multi-scale) ------------------------------------
-template <bool WEIGHTED>
-__device__ __forceinline__ void phase2_multi(const FastParams &P, const WarpSmem<WEIGHTED> &S, int ea, int eb,
-                                             const float2 (&rx)[HPL], const float2 (&ry)[HPL],
-                                             const float2 (&rz)[HPL],
-                                             float h_out, float eps, float mid, const Tile &tl, int lane, int b,
-                                             unsigned &n_recheck) {
-    const int ne = P.n_edges;
-    const float *ef = P.r2f + (size_t)b * ne;
-    const double *ed = P.r2 + (size_t)b * ne;
-    const int nc = P.lg_cells;
-    const float lg_scale = P.lgpar[2 * b], lg_off = P.lgpar[2 * b + 1];
-    const unsigned short *lgT = P.lgT + (size_t)b * nc;
-    const double *const trow = YAWB_TILE_ROWS(P, tl);
-    const double *const tw = YAWB_TILE_WEIGHTS(P, tl);
-    (void)tw;
-    for (int e = ea; e < eb; ++e) {
-        const Cand c = S.list[e];
-        const float2 sx = make_float2(c.x, c.x), sy = make_float2(c.y, c.y);
-        const float2 sz = make_float2(c.z, c.z), sw = make_float2(c.w, c.w);
-#pragma unroll
-        for (int r = 0; r < YAWB_RPL; ++r) {
-            float2 u2 = __ffma2_rn(rx[r >> 1], sx, sw);
-            u2 = __ffma2_rn(ry[r >> 1], sy, u2);
-            u2 = __ffma2_rn(rz[r >> 1], sz, u2);
-            const float u = (r & 1) ? u2.y : u2.x;  // the compiler merges the two halves of a row pair
-            if (fabsf(u) < h_out) {  // possibly inside [lo, hi]
-                const float d2f = u + mid;
-                // number of edges strictly below d2f (float copy of the edges): the edges are close to
-                // log-spaced, so a table over uniform cells of lg2(d2) gives a lower bound that is rarely
-                // off by more than one
-                const int cell = min(max((int)fmaf(__log2f(d2f), lg_scale, lg_off), 0), nc - 1);
-                int k = lgT[cell];
-                while (k < ne && ef[k] < d2f) ++k;
-                // distance to the neighbouring edges decides whether FP32 was good enough
-                float gap = FLT_MAX;
-                if (k > 0) gap = fminf(gap, d2f - ef[k - 1]);
-                if (k < ne) gap = fminf(gap, ef[k] - d2f);
-                const int j = tl.start + min(lane + 32 * r, tl.count - 1);
-                if (!(gap > eps)) {
-                    const int i = S.lidx[e];
-                    double cxx, cyy, czz;
-                    YAWB_CAND_ROW(P, i, cxx, cyy, czz);
-                    const double d2 = exact_d2(cxx, cyy, czz, trow[(size_t)YAWB_RSTRIDE * j], trow[(size_t)YAWB_RSTRIDE * j + 1], trow[(size_t)YAWB_RSTRIDE * j + 2]);
-                    k = edges_below(ed, ne, d2);
-                    n_recheck += 1;
-                }
-                if (k >= 1 && k < ne) {
-                    atomicAdd(&S.hist[k - 1], 1u);
-                    if (WEIGHTED) atomicAdd(&S.histw[k - 1], S.lw[e] * (tw ? tw[j] : 1.0));
-                }
-            }
-        }
-    }
-}
-
-// ---- the same classification, dense: in-range tests are queued warp-wide and classified 32 at a time -----------
+// ---- phase 2, several sub-bins (r-weights, multi-scale): in-range tests queued warp-wide, classified 32 at a time ----
 // With ~50 sub-bins the scale range of a z-bin is a wide annulus: some 11 % of the executed tests fall inside, spread
-// over most of the eight row slots of a candidate, so the in-place form above walks through the classification code
-// for nearly every (candidate, row slot) with one lane in seven active (ncu: 2.15e10 warp instructions per C3w count
-// against 3.9e9 for the single-bin kernel, a quarter of them in the edge fix-up loop).  Here every in-range test is
-// appended to a queue of the warp (position by ballot + popcount; entry = d2 as float and candidate << 8 | row slot
-// << 5 | lane), and whenever 32 entries are waiting every lane classifies one.
+// over most of the eight row slots of a candidate, so classifying in place, inside the test loop (round 1), walked
+// through the classification code for nearly every (candidate, row slot) with one lane in seven active (ncu: 2.15e10
+// warp instructions per C3w count against 3.9e9 for the single-bin kernel, a quarter of them in the edge fix-up loop;
+// C3w count kernels 38.5 ms against 34.7 with the queue).  Here every in-range test is appended to a queue of the warp
+// (position by ballot + popcount; entry = d2 as float and candidate << 8 | row slot << 5 | lane), and whenever 32
+// entries are waiting every lane classifies one.
 template <bool WEIGHTED>
-__device__ __forceinline__ void classify_queued(const FastParams &P, const WarpSmem<WEIGHTED> &S, float d2f, unsigned code,
+__device__ __forceinline__ void classify_queued(const FastParams &P, const StreamSmem &S, float d2f, unsigned code,
                                                 float eps, const Tile &tl, const float *__restrict__ ef,
                                                 const double *__restrict__ ed, const unsigned short *__restrict__ lgT,
                                                 float lg_scale, float lg_off, int nc, int ne, const double *trow,
@@ -555,7 +514,7 @@ __device__ __forceinline__ void classify_queued(const FastParams &P, const WarpS
 }
 
 template <bool WEIGHTED>
-__device__ __forceinline__ void phase2_multi_queue(const FastParams &P, const WarpSmem<WEIGHTED> &S, int ea, int eb,
+__device__ __forceinline__ void phase2_multi_queue(const FastParams &P, const StreamSmem &S, int ea, int eb,
                                                    const float2 (&rx)[HPL], const float2 (&ry)[HPL],
                                                    const float2 (&rz)[HPL],
                                                    float h_out, float eps, float mid, const Tile &tl, int lane, int b,
@@ -619,7 +578,7 @@ __device__ __forceinline__ void phase2_multi_queue(const FastParams &P, const Wa
 // of its own patch, is carried into the frame of the first catalog's patch as the hull of its eight rotated
 // corners (a box is convex and the map is affine, so the hull contains every row).  The item survives if that
 // box, grown by the largest search radius, meets the (u, v) box of the first catalog's patch and holds at least
-// one cell row of some z-bin.  Items are split so that none exceeds YAWB_CCAP (z-bin, cell row) runs: by z-bin
+// one cell row of some z-bin.  Items are split so that none exceeds CCAP (z-bin, cell row) runs: by z-bin
 // ranges, and a single z-bin with more rows than that by row ranges.  Items of a patch with itself (nearly
 // all of the work) are listed first, the boundary items of neighbouring patches after them, so that the tail of
 // the launch consists of light items.
@@ -639,7 +598,7 @@ struct PlanParams {
     double rmax_all;
     Item *heavy, *light;
     long long cap_heavy, cap_light;
-    int ccap;  // (z-bin, cell row) runs per item: YAWB_CCAP, or less to cut a small job into more, shorter items
+    int ccap;  // (z-bin, cell row) runs per item: CCAP, or less to cut a small job into more, shorter items
     int src;   // which second catalog of a joint launch these tiles belong to (Item::src)
     int blk;     // first output block of that catalog (Item::blk)
     int labels;  // the tiles' z-bin ids are sample labels: paired with every z-bin, counts go to block blk + label
@@ -884,13 +843,12 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
 
     // planner: self-contained work items (patch-diagonal ones first)
     // a small job (a rank's share of a strong-scaling run) is cut into more, shorter items, so that the warps of
-    // the persistent grid finish together: below YAWB_SMALL_JOB_ITEMS flat (pair, tile) combinations per warp the
-    // items hold at most YAWB_CCAP_SMALL runs (swept on an eighth of C3: 16 / 24 / 32 / 48 / 72 / 112 runs ->
+    // the persistent grid finish together: below SMALL_JOB_ITEMS flat (pair, tile) combinations per warp the
+    // items hold at most CCAP_SMALL runs (swept on an eighth of C3: 16 / 24 / 32 / 48 / 72 / 112 runs ->
     // count kernels 1.02 / 1.01 / 1.05 / 1.10 / 1.18 / 1.17 ms); the lists grow by the same factor
     const long long warps = (long long)ctx->sms * STREAM_CTAS * STREAM_WARPS;
-    int ccap = n_items_all < YAWB_SMALL_JOB_ITEMS * warps ? YAWB_CCAP_SMALL : YAWB_CCAP;
-    if (const char *e = getenv("YAWB_CCAP_RUNTIME")) ccap = std::max(8, std::min(YAWB_CCAP, atoi(e)));
-    const long long cap_scale = (YAWB_CCAP + ccap - 1) / ccap;
+    const int ccap = n_items_all < SMALL_JOB_ITEMS * warps ? CCAP_SMALL : CCAP;
+    const long long cap_scale = (CCAP + ccap - 1) / ccap;
     const long long cap_heavy = a.cap_heavy * cap_scale, cap_light = a.cap_light * cap_scale;
     Item *d_items = nullptr;
     if (yawb_dalloc(ctx, (void **)&d_items, (size_t)(cap_heavy + cap_light) * sizeof(Item), ctx->stream)) return 1;
@@ -920,39 +878,33 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
 
     const bool multi = a.n_edges > 2;
     const int nsub = a.n_edges - 1;
-    if (const char *dbg = getenv("YAWB_DEBUG_MODE")) P.debug = atoi(dbg);
-    // unweighted single-bin counts use the 7-instruction saturating test unless YAWB_PAIR_TEST=pred
-    const char *variant = getenv("YAWB_PAIR_TEST");
-    const bool sat = !(variant && strcmp(variant, "pred") == 0);
+    // few sub-bins (multi-scale without r-weights): cumulative counts with the saturating test
+    const bool cumul = multi && !a.weighted && a.n_edges <= CUM_MAX_EDGES;
     {
         // many z-bins x sub-bins: per-warp accumulators in shared memory would cost most of the occupancy, so
         // the general sub-bin path sends every segment histogram straight to global atomics instead
-        const bool cumul = multi && !a.weighted && sat && a.n_edges <= CUM_MAX_EDGES;
         const size_t acc_bytes = (size_t)fi->n_types * a.n_bins * nsub * (a.weighted ? 16 : 8);
         P.acc_global = multi && !cumul && acc_bytes > 2048;
-        const size_t per_warp = a.weighted
-                                    ? stream_carve<true>(nullptr, nullptr, multi, a.n_bins, nsub, fi->n_types, P.acc_global)
-                                    : stream_carve<false>(nullptr, nullptr, multi, a.n_bins, nsub, fi->n_types, P.acc_global);
+        const size_t per_warp = stream_carve(nullptr, nullptr, a.weighted, multi, a.n_bins, nsub, fi->n_types, P.acc_global);
         const size_t smem = STREAM_WARPS * per_warp;
         YAWB_REQUIRE(smem <= 227 * 1024, "too many z-bins x sub-bins for the shared-memory accumulators (%zu B)", smem);
         // persistent grid: a multiple of the SM count, warps pull items from a global counter
-        int per_sm = std::max(1, std::min(STREAM_CTAS, (int)((227 * 1024) / (smem + 1024))));
-        if (const char *e = getenv("YAWB_CTAS_PER_SM")) per_sm = std::max(1, std::min(per_sm, atoi(e)));
+        const int per_sm = std::max(1, std::min(STREAM_CTAS, (int)((227 * 1024) / (smem + 1024))));
         const int ctas = ctx->sms * per_sm;
-#define LAUNCH(W, M, T)                                                                                      \
+#define LAUNCH(PATH)                                                                                         \
     do {                                                                                                     \
-        YAWB_CUDA(cudaFuncSetAttribute(k_count_stream<W, M, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+        YAWB_CUDA(cudaFuncSetAttribute(k_count_stream<PATH>, cudaFuncAttributeMaxDynamicSharedMemorySize,    \
                                        (int)smem));                                                          \
-        k_count_stream<W, M, T><<<ctas, STREAM_WARPS * 32, smem, ctx->stream>>>(P);                         \
+        k_count_stream<PATH><<<ctas, STREAM_WARPS * 32, smem, ctx->stream>>>(P);                            \
     } while (0)
         if (a.weighted) {
-            if (multi) LAUNCH(true, true, false); else LAUNCH(true, false, false);
+            if (multi) LAUNCH(CountPath::HistogramWeighted); else LAUNCH(CountPath::SingleWeighted);
+        } else if (cumul) {
+            LAUNCH(CountPath::Cumulative);
+        } else if (multi) {
+            LAUNCH(CountPath::Histogram);
         } else {
-            // few sub-bins (multi-scale without r-weights): cumulative counts with the saturating test
-            if (cumul) LAUNCH(false, true, true);
-            else if (multi) LAUNCH(false, true, false);
-            else if (sat) LAUNCH(false, false, true);
-            else LAUNCH(false, false, false);
+            LAUNCH(CountPath::Single);
         }
 #undef LAUNCH
     }

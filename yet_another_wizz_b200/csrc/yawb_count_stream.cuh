@@ -1,5 +1,5 @@
 // The production pair-count kernel k_count_stream (included by yawb_count.cu after the shared device
-// functions): a software-pipelined stream of work items per warp.
+// functions and the layout of a warp's shared memory, StreamSmem): a software-pipelined stream of work items per warp.
 //
 // A work item (written by the planner k_plan) is a register tile of the second catalog against some z-bins of
 // one linked patch of the first catalog, with the tile's bounding box already expressed in the frame of that
@@ -21,80 +21,14 @@
 // chunks of 192 rows: C3 count kernels 6.37 -> 6.16 ms).
 #pragma once
 
-#ifndef YAWB_LB
-#define YAWB_LB 128
-#endif
-#ifndef YAWB_STREAM_WARPS
-#define YAWB_STREAM_WARPS 4
-#endif
-#ifndef YAWB_STREAM_CTAS
-#define YAWB_STREAM_CTAS 4
-#endif
-constexpr int LB = YAWB_LB;                    // rows per raw chunk = capacity of the staged list
-constexpr int CCAP = YAWB_CCAP;                // (z-bin, cell row) runs per item; the planner splits items to fit
-constexpr int NSLOT = 4;                       // items in flight per warp: consumed, produced, planned, fetched
-constexpr int STREAM_WARPS = YAWB_STREAM_WARPS;
-constexpr int STREAM_CTAS = YAWB_STREAM_CTAS;
-
-// The staged frame of an item ("tile frame"): origin O = the point of the unit sphere in the direction of the centre of
-// the tile box, axes (t1, t2, n) with n = O - (centre of the sphere).  For a row P of the tile (a unit vector)
-// |P - O|^2 = -2 (P - O).n, so the squared chord to a candidate s needs no |r|^2 term:
-//     |r - s|^2 - mid = (|s|^2 - mid) + r . (-2 s_x, -2 s_y, -2 (1 + s_z))        (three FMAs per test)
-struct __align__(16) ItemAux {
-    double R[9];        // rows t1, t2, n of the tile frame, in coordinates of the frame of p1
-    double O[3];        // origin of the tile frame, in coordinates of the frame of p1
-    double dq[3];       // lattice origin - O:  (row of the index) - O = (k - ko) * qinv + dq
-    int ko[3];          // lattice origin: the lattice point nearest to the centre of the tile box
-    int n_combo;        // runs of the item
-    float qinv;         // lattice spacing (a power of two)
-    float eu, ev, et;   // half extents of the tile box about the lattice origin, rounded up
-    float g;            // |lattice origin - O|, rounded up
-    int end;            // 1: the work list is exhausted, this slot holds no item
-    int pad[2];
-};
-static_assert(sizeof(ItemAux) % 16 == 0, "ItemAux layout");
-
-struct __align__(16) SegDesc {
-    short ea, eb;  // entries [ea, eb) of the staged list
-    short bin;     // their z-bin
-    short type;    // catalog of a fused first-role index (0 / 1)
-};
-
-template <bool WEIGHTED>
-struct StreamSmem {
-    Item *items;               // [NSLOT]
-    ItemAux *aux;              // [NSLOT]
-    int *bin_iv0, *bin_iu;     // [n_bins] plan: first cell row of the query, iu0 | iu1 << 16
-    int *cstart;               // [n_bins + 1] prefix of cell rows per z-bin
-    int2 *cs;                  // [CCAP] cell_start at the two ends of every run (lands asynchronously)
-    unsigned short *csbin;     // [CCAP] z-bin of the run
-    int2 *run;                 // [CCAP] run table of the item being produced: (inclusive prefix of the run lengths,
-                               //        row of the index that flat position 0 would have if the run started there)
-    unsigned short *cbin;      // [CCAP]
-    SRec *raw;                 // [LB] raw chunk (lands asynchronously)
-    unsigned short *rawbin;    // [LB]
-    double *rawlw;             // [LB] weights of the raw rows (WEIGHTED)
-    Cand *list;                // [LB] staged candidates: type 0 from the bottom, type 1 from the top
-    int *lidx;                 // [LB]
-    unsigned short *lbin;      // [LB]
-    double *lw;                // [LB] (WEIGHTED)
-    SegDesc *seg;              // [n_types * n_bins]
-    float4 *binrec;            // [n_bins] half extents of the query box (x, y, z) and mid
-    float2 *binthr;            // [n_bins] thresholds of the pair test
-    unsigned long long *acc;   // [n_types][n_bins * nsub]
-    double *accw;              // same (WEIGHTED)
-    unsigned *hist;            // [nsub] (MULTI)
-    double *histw;             // [nsub] (MULTI && WEIGHTED)
-    float *cum;                // [n_bins][CUM_EDGES] (MULTI && SAT)
-    unsigned *cumtot;          // [CUM_EDGES]
-};
+constexpr int STREAM_WARPS = 4;  // warps per CTA
+constexpr int STREAM_CTAS = 4;   // CTAs per SM the kernel is compiled for (128 registers)
 
 __host__ __device__ inline size_t up16(size_t b) { return (b + 15) & ~(size_t)15; }
 
-// Walks the layout of a warp's block; with `base == nullptr` only the size is of interest.
-template <bool WEIGHTED>
-__host__ __device__ inline size_t stream_carve(StreamSmem<WEIGHTED> *S, unsigned char *base, bool multi, int n_bins, int nsub,
-                                               int n_types, bool acc_global) {
+// Walks the layout of a warp's block (StreamSmem); with `base == nullptr` only the size is of interest.
+__host__ __device__ inline size_t stream_carve(StreamSmem *S, unsigned char *base, bool weighted, bool multi, int n_bins,
+                                               int nsub, int n_types, bool acc_global) {
     size_t o = 0;
     auto take = [&](size_t bytes) {
         unsigned char *p = base + o;
@@ -114,18 +48,18 @@ __host__ __device__ inline size_t stream_carve(StreamSmem<WEIGHTED> *S, unsigned
     p = take(CCAP * sizeof(unsigned short)); if (S) S->cbin = (unsigned short *)p;
     p = take(LB * sizeof(SRec)); if (S) S->raw = (SRec *)p;
     p = take(LB * sizeof(unsigned short)); if (S) S->rawbin = (unsigned short *)p;
-    p = take(WEIGHTED ? LB * sizeof(double) : 0); if (S) S->rawlw = WEIGHTED ? (double *)p : nullptr;
+    p = take(weighted ? LB * sizeof(double) : 0); if (S) S->rawlw = weighted ? (double *)p : nullptr;
     p = take(LB * sizeof(Cand)); if (S) S->list = (Cand *)p;
     p = take(LB * sizeof(int)); if (S) S->lidx = (int *)p;
     p = take(LB * sizeof(unsigned short)); if (S) S->lbin = (unsigned short *)p;
-    p = take(WEIGHTED ? LB * sizeof(double) : 0); if (S) S->lw = WEIGHTED ? (double *)p : nullptr;
+    p = take(weighted ? LB * sizeof(double) : 0); if (S) S->lw = weighted ? (double *)p : nullptr;
     p = take((size_t)n_types * n_bins * sizeof(SegDesc)); if (S) S->seg = (SegDesc *)p;
     p = take(n_bins * sizeof(float4)); if (S) S->binrec = (float4 *)p;
     p = take(n_bins * sizeof(float2)); if (S) S->binthr = (float2 *)p;
     p = take(nacc * sizeof(unsigned long long)); if (S) S->acc = (unsigned long long *)p;
-    p = take(WEIGHTED ? nacc * sizeof(double) : 0); if (S) S->accw = WEIGHTED ? (double *)p : nullptr;
+    p = take(weighted ? nacc * sizeof(double) : 0); if (S) S->accw = weighted ? (double *)p : nullptr;
     p = take(multi ? nsub * sizeof(unsigned) : 0); if (S) S->hist = multi ? (unsigned *)p : nullptr;
-    p = take(multi && WEIGHTED ? nsub * sizeof(double) : 0); if (S) S->histw = (multi && WEIGHTED) ? (double *)p : nullptr;
+    p = take(multi && weighted ? nsub * sizeof(double) : 0); if (S) S->histw = (multi && weighted) ? (double *)p : nullptr;
     // (at least 128 words: the general sub-bin path keeps its queue of in-range tests here, phase2_multi_queue)
     p = take(multi ? ((size_t)n_bins * CUM_EDGES > 128 ? (size_t)n_bins * CUM_EDGES : 128) * sizeof(float) : 0); if (S) S->cum = multi ? (float *)p : nullptr;
     p = take(multi ? CUM_EDGES * sizeof(unsigned) : 0); if (S) S->cumtot = multi ? (unsigned *)p : nullptr;
@@ -150,8 +84,7 @@ __device__ __forceinline__ const Item *item_ptr(const FastParams &P, long long i
 }
 
 // ---- fetch: the record of work item `idx` into a slot (asynchronous), or the end marker -------------------
-template <bool WEIGHTED, typename SM = StreamSmem<WEIGHTED>>
-__device__ __forceinline__ void stream_fetch(const FastParams &P, const SM &S, int slot, long long idx,
+__device__ __forceinline__ void stream_fetch(const FastParams &P, const StreamSmem &S, int slot, long long idx,
                                              long long n_heavy, long long n_live, int lane) {
     if (idx >= n_live) {
         if (lane == 0) S.aux[slot].end = 1;
@@ -163,8 +96,7 @@ __device__ __forceinline__ void stream_fetch(const FastParams &P, const SM &S, i
 }
 
 // ---- plan: cell rows of the query per z-bin, then request the cell boundaries of every run ----------------
-template <bool WEIGHTED, typename SM = StreamSmem<WEIGHTED>>
-__device__ __forceinline__ void stream_plan(const FastParams &P, const SM &S, int slot, int lane) {
+__device__ __forceinline__ void stream_plan(const FastParams &P, const StreamSmem &S, int slot, int lane) {
     ItemAux &ax = S.aux[slot];
     if (ax.end) return;
     const Item &it = S.items[slot];
@@ -255,8 +187,7 @@ __device__ __forceinline__ void stream_plan(const FastParams &P, const SM &S, in
 }
 
 // ---- run table of the item whose cell boundaries have landed; returns the number of candidate rows -------
-template <bool WEIGHTED, typename SM = StreamSmem<WEIGHTED>>
-__device__ __forceinline__ int stream_runs(const SM &S, int n_combo, int lane) {
+__device__ __forceinline__ int stream_runs(const StreamSmem &S, int n_combo, int lane) {
     int running = 0;
     for (int k0 = 0; k0 < n_combo; k0 += 32) {
         const int k = k0 + lane;
@@ -285,8 +216,8 @@ __device__ __forceinline__ int stream_runs(const SM &S, int n_combo, int lane) {
 // ---- request the rows [t0, t0 + cnt) of the item's flat candidate range: one lane per row ----------------
 // Every lane walks the run table forwards (its flat positions grow by 32 per round, a run holds a handful of
 // rows), starting from a binary search.
-template <bool WEIGHTED, typename SM = StreamSmem<WEIGHTED>>
-__device__ __forceinline__ void stream_issue(const FastParams &P, const SM &S, int n_combo, int t0, int cnt,
+template <bool WEIGHTED>
+__device__ __forceinline__ void stream_issue(const FastParams &P, const StreamSmem &S, int n_combo, int t0, int cnt,
                                              int lane) {
     if (cnt <= 0) return;
     int cur;
@@ -317,8 +248,8 @@ __device__ __forceinline__ void stream_issue(const FastParams &P, const SM &S, i
 }
 
 // ---- per-item tables of the consumer: half extents of the query box, FP32 error bound, thresholds --------
-template <bool WEIGHTED, bool MULTI, bool SAT>
-__device__ __forceinline__ void stream_begin(const FastParams &P, const StreamSmem<WEIGHTED> &S, int slot, int lane) {
+template <CountPath PATH>
+__device__ __forceinline__ void stream_begin(const FastParams &P, const StreamSmem &S, int slot, int lane) {
     const Item &it = S.items[slot];
     const ItemAux &ax = S.aux[slot];
     const float eu = ax.eu, ev = ax.ev, et = ax.et;
@@ -340,7 +271,7 @@ __device__ __forceinline__ void stream_begin(const FastParams &P, const StreamSm
         // |delta| (2 |d| + |delta|) <= 0.87 q (4 M + q) < 4 M q + q^2
         const float eps = (EPS32 * (24.0f * m2 + 8.0f * bp.mid) + 4.0f * m1 * 1.0001f * q + q * q + P.zeta) * 1.0001f;
         S.binrec[b] = make_float4(hx, hy, hz, bp.mid);
-        if (MULTI && SAT) {
+        if constexpr (PATH == CountPath::Cumulative) {
             // cumulative counts per edge: v_k = sat(K (e_k - mid - u) + 1/2); the float copy of
             // e_k - mid adds at most eps32 |e_k - mid| to the error of u
             const float K = 0.4f / (eps + 4.0f * EPS32 * (float)bp.hi);
@@ -349,12 +280,12 @@ __device__ __forceinline__ void stream_begin(const FastParams &P, const StreamSm
             for (int k = 0; k < CUM_EDGES; ++k)
                 S.cum[b * CUM_EDGES + k] =
                     k < ne ? fmaf(K, (float)(P.r2[(size_t)b * ne + k] - (double)bp.mid), 0.5f) : -1.0e30f;
-        } else if (MULTI) {
+        } else if constexpr (path_multi(PATH)) {  // Histogram, HistogramWeighted
             S.binthr[b] = make_float2(bp.h + eps, eps + 4.0f * EPS32 * (float)bp.hi);
-        } else if (SAT) {
+        } else if constexpr (PATH == CountPath::Single) {
             const float K = 0.4f / eps;  // undecidable tests land in v = [0.1, 0.9]: v (1 - v) >= 0.09
             S.binthr[b] = make_float2(-K, 0.5f + bp.h * K);
-        } else {
+        } else {  // SingleWeighted
             S.binthr[b] = make_float2(bp.h - eps, bp.h + eps);
         }
     }
@@ -362,7 +293,7 @@ __device__ __forceinline__ void stream_begin(const FastParams &P, const StreamSm
 
 // ---- convert the landed raw chunk into the staged list; returns (entries of type 0, entries of type 1) ----
 template <bool WEIGHTED>
-__device__ __forceinline__ int2 stream_convert(const StreamSmem<WEIGHTED> &S, int slot, int cnt, int lane) {
+__device__ __forceinline__ int2 stream_convert(const StreamSmem &S, int slot, int cnt, int lane) {
     const ItemAux &ax = S.aux[slot];
     const int k0 = ax.ko[0], k1 = ax.ko[1], k2 = ax.ko[2];
     const float qinv = ax.qinv;
@@ -411,8 +342,7 @@ __device__ __forceinline__ int2 stream_convert(const StreamSmem<WEIGHTED> &S, in
 }
 
 // ---- segment table: runs of equal z-bin in the two regions of the staged list; returns their number -------
-template <bool WEIGHTED>
-__device__ __forceinline__ int stream_segments(const StreamSmem<WEIGHTED> &S, int L0, int L1, int lane) {
+__device__ __forceinline__ int stream_segments(const StreamSmem &S, int L0, int L1, int lane) {
     int n_seg = 0;
 #pragma unroll
     for (int region = 0; region < 2; ++region) {
@@ -441,14 +371,9 @@ __device__ __forceinline__ int stream_segments(const StreamSmem<WEIGHTED> &S, in
 // Per z-bin segment: groups of four candidates fully unrolled plus a fall-through tail, the decided /
 // undecided check once per <= 16 candidates, the warp total of a segment added to the accumulator while the
 // next segment is already running.
-__device__ __forceinline__ void stream_test_sat(const FastParams &P, const StreamSmem<false> &S, int n_seg,
+__device__ __forceinline__ void stream_test_sat(const FastParams &P, const StreamSmem &S, int n_seg,
                                                 const float2 (&rx)[HPL], const float2 (&ry)[HPL], const float2 (&rz)[HPL],
                                                 const Tile &tl, int lane, unsigned &n_recheck) {
-    WarpSmem<false> W{};
-    W.list = S.list;
-    W.lidx = S.lidx;
-    const double dummy_w[YAWB_RPL] = {};
-    (void)dummy_w;
     unsigned pend_tot = 0;
     int pend_acc = -1;
     for (int sg = 0; sg < n_seg; ++sg) {
@@ -461,7 +386,7 @@ __device__ __forceinline__ void stream_test_sat(const FastParams &P, const Strea
             float2 acc_a = make_float2(0.f, 0.f), acc_b = make_float2(0.f, 0.f);
             double ws[YAWB_RPL];
             int e = c0;
-#define YAWB_T(idx) test_candidate<false, true>(S.list[idx], 0.0, rx, ry, rz, ta, tb, acc_a, acc_b, ws)
+#define YAWB_T(idx) test_candidate<false>(S.list[idx], 0.0, rx, ry, rz, ta, tb, acc_a, acc_b, ws)
             for (; e + 4 <= c1; e += 4) {
                 YAWB_T(e); YAWB_T(e + 1); YAWB_T(e + 2); YAWB_T(e + 3);
             }
@@ -479,8 +404,7 @@ __device__ __forceinline__ void stream_test_sat(const FastParams &P, const Strea
                 const int src = __ffs(flagged) - 1;
                 flagged &= flagged - 1;
                 unsigned cx = 0;
-                double wx = 0.0;
-                recheck_span<false>(P, W, c0, c1, tl, lane, src, P.binpar[d.bin].lo, P.binpar[d.bin].hi, cx, wx, n_recheck);
+                recheck_span(P, S, c0, c1, tl, lane, src, P.binpar[d.bin].lo, P.binpar[d.bin].hi, cx, n_recheck);
                 if (lane == src) c = cx;
             }
             cnt_total += c;
@@ -492,61 +416,54 @@ __device__ __forceinline__ void stream_test_sat(const FastParams &P, const Strea
     if (lane == 0 && pend_acc >= 0) S.acc[pend_acc] += pend_tot;
 }
 
-// ---- every other variant: the shared phase-2 functions, one pass per segment ------------------------------
-template <bool WEIGHTED, bool MULTI, bool SAT>
-__device__ __forceinline__ void stream_test_generic(const FastParams &P, const StreamSmem<WEIGHTED> &S, int n_seg,
+// ---- every other path: the shared phase-2 functions, one pass per segment ------------------------------
+template <CountPath PATH>
+__device__ __forceinline__ void stream_test_generic(const FastParams &P, const StreamSmem &S, int n_seg,
                                                     const float2 (&rx)[HPL], const float2 (&ry)[HPL],
                                                     const float2 (&rz)[HPL], const Tile &tl,
                                                     int lane, int nsub, unsigned &n_recheck, size_t item_off,
                                                     const double (&rwt)[YAWB_RPL]) {
+    constexpr bool WEIGHTED = path_weighted(PATH);
     const size_t nacc1 = (size_t)P.n_bins * nsub;  // accumulators of one type
     for (int sg = 0; sg < n_seg; ++sg) {
         const SegDesc d = S.seg[sg];
         const int ea = d.ea, eb = d.eb, b = d.bin;
-        WarpSmem<WEIGHTED> W{};
-        W.list = S.list; W.lw = S.lw; W.lidx = S.lidx; W.lbin = S.lbin;
-        W.hist = S.hist; W.histw = S.histw; W.cum = S.cum; W.cumtot = S.cumtot;
-        W.acc = S.acc ? S.acc + d.type * nacc1 : nullptr;
-        W.accw = (WEIGHTED && S.accw) ? S.accw + d.type * nacc1 : nullptr;
+        unsigned long long *const acc = S.acc ? S.acc + d.type * nacc1 : nullptr;
+        double *const accw = (WEIGHTED && S.accw) ? S.accw + d.type * nacc1 : nullptr;
         const float2 thr = S.binthr[b];
-        if (MULTI && SAT && !WEIGHTED) {
-            if constexpr (!WEIGHTED) phase2_cumul(P, W, ea, eb, rx, ry, rz, thr.x, tl, lane, b, n_recheck);
-        } else if (MULTI) {
+        if constexpr (PATH == CountPath::Cumulative) {
+            phase2_cumul(P, S, acc, ea, eb, rx, ry, rz, thr.x, tl, lane, b, n_recheck);
+        } else if constexpr (path_multi(PATH)) {  // Histogram, HistogramWeighted
             for (int k = lane; k < nsub; k += 32) {
-                W.hist[k] = 0u;
-                if (WEIGHTED) W.histw[k] = 0.0;
+                S.hist[k] = 0u;
+                if (WEIGHTED) S.histw[k] = 0.0;
             }
             __syncwarp();
-#ifdef YAWB_MULTI_INPLACE  // round 1's form: classification inside the test loop (C3w count kernels 38.5 ms against 34.7)
-            phase2_multi<WEIGHTED>(P, W, ea, eb, rx, ry, rz, thr.x, thr.y, S.binrec[b].w, tl, lane, b, n_recheck);
-#else
-            phase2_multi_queue<WEIGHTED>(P, W, ea, eb, rx, ry, rz, thr.x, thr.y, S.binrec[b].w, tl, lane, b, n_recheck);
-#endif
+            phase2_multi_queue<WEIGHTED>(P, S, ea, eb, rx, ry, rz, thr.x, thr.y, S.binrec[b].w, tl, lane, b, n_recheck);
             __syncwarp();
             if (P.acc_global) {  // straight to the result: one atomic per non-empty sub-bin of the segment
                 const size_t o = item_off + (size_t)d.type * P.type_stride + (size_t)b * nsub;
                 for (int k = lane; k < nsub; k += 32) {
-                    if (W.hist[k]) atomicAdd(&P.out_cnt[o + k], (unsigned long long)W.hist[k]);
-                    if (WEIGHTED && W.histw[k] != 0.0) atomicAdd(&P.out_w[o + k], W.histw[k]);
+                    if (S.hist[k]) atomicAdd(&P.out_cnt[o + k], (unsigned long long)S.hist[k]);
+                    if (WEIGHTED && S.histw[k] != 0.0) atomicAdd(&P.out_w[o + k], S.histw[k]);
                 }
             } else {
                 for (int k = lane; k < nsub; k += 32) {
-                    W.acc[(size_t)b * nsub + k] += W.hist[k];
-                    if (WEIGHTED) W.accw[(size_t)b * nsub + k] += W.histw[k];
+                    acc[(size_t)b * nsub + k] += S.hist[k];
+                    if (WEIGHTED) accw[(size_t)b * nsub + k] += S.histw[k];
                 }
             }
             __syncwarp();
-        } else {
+        } else {  // SingleWeighted
             unsigned cnt_total = 0;
             double w_total = 0.0;
-            phase2_single<WEIGHTED, SAT && !WEIGHTED>(P, W, ea, eb, rx, ry, rz, thr.x, thr.y, tl, lane,
-                                                      P.binpar[b].lo, P.binpar[b].hi, cnt_total, w_total, n_recheck, rwt);
+            phase2_single(P, S, ea, eb, rx, ry, rz, thr.x, thr.y, tl, lane, P.binpar[b].lo, P.binpar[b].hi, cnt_total,
+                          w_total, n_recheck, rwt);
             const unsigned tot = __reduce_add_sync(FULL, cnt_total);
-            double wtot = 0.0;
-            if (WEIGHTED) wtot = warp_sum(w_total);
+            const double wtot = warp_sum(w_total);
             if (lane == 0) {
-                W.acc[b] += tot;
-                if (WEIGHTED) W.accw[b] += wtot;
+                acc[b] += tot;
+                accw[b] += wtot;
             }
         }
     }
@@ -560,17 +477,18 @@ __device__ __forceinline__ size_t item_offset(const FastParams &P, const Item &i
 }
 
 // ---- the kernel ----------------------------------------------------------------------------------------
-template <bool WEIGHTED, bool MULTI, bool SAT>
+template <CountPath PATH>
 __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream(const FastParams P) {
+    constexpr bool WEIGHTED = path_weighted(PATH), MULTI = path_multi(PATH);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int nsub = P.n_edges - 1;
     const bool acc_global = MULTI && P.acc_global;
     const int nacc = acc_global ? 0 : P.n_types * P.n_bins * nsub;  // accumulators kept in shared memory
-    StreamSmem<WEIGHTED> S;
-    const size_t per_warp = stream_carve<WEIGHTED>(nullptr, nullptr, MULTI, P.n_bins, nsub, P.n_types, acc_global);
-    stream_carve<WEIGHTED>(&S, smem_raw + warp * per_warp, MULTI, P.n_bins, nsub, P.n_types, acc_global);
+    StreamSmem S;
+    const size_t per_warp = stream_carve(nullptr, nullptr, WEIGHTED, MULTI, P.n_bins, nsub, P.n_types, acc_global);
+    stream_carve(&S, smem_raw + warp * per_warp, WEIGHTED, MULTI, P.n_bins, nsub, P.n_types, acc_global);
     for (int k = lane; k < nacc; k += 32) {
         S.acc[k] = 0ull;
         if (WEIGHTED) S.accw[k] = 0.0;
@@ -587,12 +505,12 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
     if (lane == 0) next_idx = (long long)atomicAdd(&P.counters[0], 2ull);
     next_idx = __shfl_sync(FULL, next_idx, 0);
 #pragma unroll
-    for (int j = 0; j < 2; ++j) stream_fetch<WEIGHTED>(P, S, j, next_idx + j, n_heavy, n_live, lane);
+    for (int j = 0; j < 2; ++j) stream_fetch(P, S, j, next_idx + j, n_heavy, n_live, lane);
     if (next_idx + 1 >= n_live) grabbing = false;
     cp_async_commit();
     cp_async_wait_all();
     __syncwarp();
-    stream_plan<WEIGHTED>(P, S, 0, lane);
+    stream_plan(P, S, 0, lane);
     if (grabbing && lane == 0) next_idx = (long long)atomicAdd(&P.counters[0], 1ull);
     if (!grabbing) next_idx = n_live;
     cp_async_commit();
@@ -636,7 +554,7 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
                         if (WEIGHTED) rwt[r] = rws ? rws[j] : 1.0;
                     }
                 }
-                stream_begin<WEIGHTED, MULTI, SAT>(P, S, c_slot, lane);
+                stream_begin<PATH>(P, S, c_slot, lane);
                 __syncwarp();
             }
             if (c_first) {
@@ -666,7 +584,7 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
             }
             const int2 L = stream_convert<WEIGHTED>(S, c_slot, c_cnt, lane);
             __syncwarp();
-            n_seg = stream_segments<WEIGHTED>(S, L.x, L.y, lane);
+            n_seg = stream_segments(S, L.x, L.y, lane);
             n_tests += (unsigned long long)(L.x + L.y) * (unsigned long long)it.count;
         }
 
@@ -680,12 +598,12 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
                     prod_done = true;
                 } else {
                     p_ncombo = S.aux[slot].n_combo;
-                    p_ncand = stream_runs<WEIGHTED>(S, p_ncombo, lane);
+                    p_ncand = stream_runs(S, p_ncombo, lane);
                     p_t0 = 0;
                     prod_exhausted = false;
-                    stream_plan<WEIGHTED>(P, S, (ip + 1) & (NSLOT - 1), lane);
+                    stream_plan(P, S, (ip + 1) & (NSLOT - 1), lane);
                     const long long idx = __shfl_sync(FULL, next_idx, 0);
-                    stream_fetch<WEIGHTED>(P, S, (ip + 2) & (NSLOT - 1), idx, n_heavy, n_live, lane);
+                    stream_fetch(P, S, (ip + 2) & (NSLOT - 1), idx, n_heavy, n_live, lane);
                     if (idx >= n_live) grabbing = false;
                     if (grabbing) {
                         if (lane == 0) next_idx = (long long)atomicAdd(&P.counters[0], 1ull);
@@ -710,11 +628,11 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
         // ---- test ----
         if (c_cnt >= 0) {
             if (n_seg > 0) {
-                if constexpr (!WEIGHTED && !MULTI && SAT)
+                if constexpr (PATH == CountPath::Single)
                     stream_test_sat(P, S, n_seg, rx, ry, rz, tl, lane, n_recheck);
                 else
-                    stream_test_generic<WEIGHTED, MULTI, SAT>(P, S, n_seg, rx, ry, rz, tl, lane, nsub, n_recheck,
-                                                               item_offset(P, S.items[c_slot], nsub), rwt);
+                    stream_test_generic<PATH>(P, S, n_seg, rx, ry, rz, tl, lane, nsub, n_recheck,
+                                              item_offset(P, S.items[c_slot], nsub), rwt);
             }
             if (c_last) {  // the item is complete: its counts go to the result of its patch pair and output block
                 __syncwarp();

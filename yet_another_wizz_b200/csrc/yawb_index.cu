@@ -24,15 +24,9 @@
 namespace {
 
 constexpr int kThreads = 256;
-#ifndef YAWB_TARGET_PER_CELL
-#define YAWB_TARGET_PER_CELL 5.5
-#endif
-constexpr double kTargetPerCell = YAWB_TARGET_PER_CELL;  // rows per sky cell and z-bin the grid is sized for
+constexpr double kTargetPerCell = 5.5;  // rows per sky cell and z-bin the grid is sized for
 constexpr long long kMaxCellsPerPatchBin = 1ll << 24;
-#ifndef YAWB_CELL_ASPECT
-#define YAWB_CELL_ASPECT 4.0
-#endif
-constexpr double kCellAspect = YAWB_CELL_ASPECT;  // cell height / cell width
+constexpr double kCellAspect = 4.0;  // cell height / cell width
 
 inline int blocks_for(int64_t n, int per_block = kThreads) {
     return (int)std::min<int64_t>((n + per_block - 1) / per_block, 1 << 30);
@@ -978,10 +972,7 @@ int build_second_sorted(yawb_cat *cat, int hbits) {
 }  // namespace
 
 // -------------------------------------------------------------------------------------------
-#ifndef YAWB_COPY_CHUNK_MB
-#define YAWB_COPY_CHUNK_MB 64
-#endif
-static constexpr size_t kCopyChunk = (size_t)YAWB_COPY_CHUNK_MB << 20;
+static constexpr size_t kCopyChunk = (size_t)64 << 20;
 
 int yawb_index_upload(yawb_ctx *ctx, yawb_cat *cat, const double *xyz, const double *w, const uint8_t *zbin8,
                       const int32_t *zbin, const double *zred, const int64_t *patch_off) {
@@ -1263,7 +1254,7 @@ static int findex_build(yawb_ctx *ctx, yawb_cat *a, yawb_cat *b, FIndex **out) {
     // bounded, dense keys: counting sort (the radix sort only for grids with more cells than the key counts may take)
     // (weighted rows keep the stable radix sort: the order of the rows of a cell is the order their weights are
     // summed in, and a counting sort's atomics would make the last bits of the sums vary from run to run)
-    if (base <= kCountingSortMaxKeys && !fi->weighted && !getenv("YAWB_RADIX_SORT")) {
+    if (base <= kCountingSortMaxKeys && !fi->weighted) {
         if (build_first_counting(fi, base)) return fail();
     } else if (base < 0xffffffffll ? build_first_sorted<unsigned>(fi, base) : build_first_sorted<unsigned long long>(fi, base)) {
         return fail();
@@ -1347,12 +1338,10 @@ int yawb_index_build_second(yawb_cat *cat) {
         // at most about ONE key per row (the cells then hold 1-4 rows, in arbitrary order; swept on C3: 4 / 1 / 0.25 /
         // 0.06 keys per row -> index build 1.80 / 1.60 / 1.57 / 2.89 ms, count kernels 6.05 / 6.07 / 6.11 / 6.31 ms)
         int kc = k;
-        double keys_per_row = 1.0;
-        if (const char *e = getenv("YAWB_KEYS_PER_ROW")) keys_per_row = std::max(0.001, atof(e));
-        const long long key_budget = std::max<long long>((long long)(keys_per_row * (double)cat->n_in), 1 << 16);
+        const long long key_budget = std::max<long long>(cat->n_in, 1 << 16);
         while (kc > 1 && (((long long)P * B) << (2 * kc)) > key_budget) --kc;
         const long long n_keys = ((long long)P * B) << (2 * kc);
-        if (n_keys <= kCountingSortMaxKeys && !cat->weighted && !getenv("YAWB_RADIX_SORT")) {
+        if (n_keys <= kCountingSortMaxKeys && !cat->weighted) {
             if (build_second_counting(cat, 2 * kc, n_keys)) return 1;
         } else if (hbits32 >= 16) {
             if (build_second_sorted<unsigned>(cat, std::min(hbits32, 2 * k))) return 1;

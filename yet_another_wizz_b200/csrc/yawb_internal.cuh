@@ -66,7 +66,7 @@ struct PatchFrame {
 // vector), and the exact doubles stay available for the FP64 recheck.
 struct SGrid {
     double u0, v0;         // cell (iu, iv) covers u0 + iu / inv_cu ..., v0 + iv / inv_cv ...
-    double inv_cu, inv_cv; // cells are narrower along u, the direction of the contiguous runs (YAWB_CELL_ASPECT)
+    double inv_cu, inv_cv; // cells are narrower along u, the direction of the contiguous runs (kCellAspect)
     int gu, gv;            // cells per row / number of rows
     long long cell_base;   // global cell id of (bin 0, iv 0, iu 0); bin stride = gu * gv
     double t0;             // origin of the third coordinate (t = (P - c).c <= 0)
@@ -126,14 +126,6 @@ constexpr int YAWB_RPL = 8;               // second-role points per lane
 constexpr int YAWB_TILE = 32 * YAWB_RPL;  // points per register tile (one warp)
 constexpr int YAWB_LG_CELLS_PER_EDGE = 4;  // cells of the lg2(d2) lookup per edge (sub-bin paths): finer cells = fewer fix-up steps
 constexpr int YAWB_RSTRIDE = 4;           // doubles per second-role row record (x, y, z, unused): one 32-byte sector
-constexpr int YAWB_LCAP = 256;            // candidate list capacity per warp
-constexpr int YAWB_WARPS = 4;             // warps per CTA in the count kernel
-#ifndef YAWB_MIN_CTAS_VALUE
-#define YAWB_MIN_CTAS_VALUE 5
-#endif
-constexpr int YAWB_MIN_CTAS_WEIGHTED = 4;   // weighted kernels (FP64 row sums) and the cumulative sub-bin kernel (up to 12
-                                            // packed accumulators): 128 registers, 4 CTAs per SM
-constexpr int YAWB_MIN_CTAS = YAWB_MIN_CTAS_VALUE;  // CTAs per SM the count kernel is compiled for (register budget)
 constexpr int YAWB_MAX_EDGES = 256;
 
 struct yawb_ctx {
