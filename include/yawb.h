@@ -106,6 +106,21 @@ int yawb_upload_catalog_u8(yawb_ctx *ctx, const double *xyz, const double *w, co
  *   z       n redshifts;   edges   n_bins + 1 strictly increasing doubles (copied by the call) */
 int yawb_upload_catalog_z(yawb_ctx *ctx, const double *xyz, const double *w, const double *z, const double *edges,
                           int closed_right, const int64_t *patch_off, int n_patch, int n_bins, yawb_cat **out);
+/* Binned labels (library version >= 102): declares the ids of a catalog uploaded with yawb_upload_catalog or
+ * yawb_upload_catalog_u8 to be  id = label * B + zbin  with L = n_labels labels and B = n_bins / L z-bins, e.g. the
+ * tomographic bins of a sample, each z-binned.  Rejects unbinned catalogs, yawb_upload_catalog_z catalogs,
+ * n_labels < 1 and an n_bins that L does not divide.  Indexes and yawb_sum_weights ([n_bins][n_patch] =
+ * [L][B][n_patch]) do not depend on it.  yawb_count then takes r2_edges as [B][n_edges] and writes
+ * [L][n_pairs][B][n_edges-1] (block l = label l, as with YAWB_FLAG_SECOND_LABELS), under two rules:
+ *   (a) cat1 and cat2 both labelled, with the same L and B (cat1 == cat2 included): the rows (l, z) of cat2 are
+ *       counted against the rows (l, z) of cat1 -- per label, the z-binned count of its own two catalogs;
+ *   (b) cat1 binned with B z-bins and no labels, cat2 labelled: the rows (l, z) of cat2 against the rows z of cat1.
+ *       Pair counts are symmetric (d2 and w1 * w2 are the same doubles either way round), so a labelled sample
+ *       against shared randoms is counted with the randoms as cat1 and the pair lists swapped.
+ * Rejected with a message (the context stays usable): a labelled cat1 with an unlabelled cat2 (swap the roles),
+ * different L or B, YAWB_FLAG_EXACT_BRUTEFORCE, YAWB_FLAG_SECOND_LABELS, and labelled catalogs in yawb_count2 /
+ * yawb_count4. */
+int yawb_catalog_set_labels(yawb_cat *cat, int n_labels);
 int yawb_free_catalog(yawb_cat *cat);
 
 /* Build (or rebuild) the device-side index for a role ahead of time; otherwise

@@ -1,7 +1,8 @@
-"""A loop of `crosscorrelate` calls over tomographic bins against one `crosscorrelate_tomographic` call; prints one
-JSON line and writes it to --out (default profiles/r04_tomographic_timing.json).
+"""A loop of `crosscorrelate` calls over tomographic bins against one `crosscorrelate_tomographic` call (`--mode
+cross`), or a loop of `autocorrelate` calls against one `autocorrelate_tomographic` call (`--mode auto`); prints one
+JSON line and writes it to --out (default profiles/r05_<mode>_tomographic_timing.json).
 
-    python tools/tomographic_timing.py [--out PATH] [--small] [--repeats R]
+    python tools/tomographic_timing.py [--mode cross|auto] [--out PATH] [--small] [--repeats R]
 
 Inputs (seeded `BoxRandoms` in the benchmark's C3 box, 64 patches, 30 z-bins, 100-1000 kpc): reference 1e6 rows,
 its randoms 1e7, an unknown sample of 1e7 rows split into N = 5 bins by a seeded label.  Cases: (A) one shared
@@ -10,6 +11,9 @@ calls (the first call of each form is a warm-up; the reference catalogs stay res
 way), the sums of `kernel_ms`, `index_ms` and `pair_tests` from `last_stats()`, and a check that both forms give
 equal results.  Also the GPU name and power limit, read in the same run.  `--small` divides every size by 100 (a
 rehearsal).
+
+Auto mode: the unknown sample of 1e7 rows carries redshifts and is split into the same N = 5 bins; cases (A) one
+shared random catalog of 1e7 rows with redshifts, (B) per-bin randoms of 2e6 rows each with redshifts.
 """
 
 import argparse
@@ -68,6 +72,32 @@ def inputs(scale: float):
     return config, ref, ref_rand, unknowns, dict(A=unk_rand, B=per_bin_rand, C=None)
 
 
+def auto_inputs(scale: float):
+    """the unknown sample with redshifts, split into N_TOMO bins, and its randoms with redshifts (shared, per bin)"""
+    nx, ny = 8, 8
+    ras = BOX[0] + (np.arange(nx) + 0.5) * (BOX[1] - BOX[0]) / nx
+    decs = BOX[2] + (np.arange(ny) + 0.5) * (BOX[3] - BOX[2]) / ny
+    centers = yb.AngularCoordinates(np.deg2rad([[r, d] for d in decs for r in ras]))
+    pool = np.random.default_rng(7).uniform(0.07, 1.42, 1_000_000)
+
+    def box(name, n, seed):
+        gen = yb.BoxRandoms(*BOX, redshifts=pool, seed=seed)
+        return yb.Catalog.from_random(name, gen, max(int(n * scale), 1000), patch_centers=centers)
+
+    unk, shared = box("unk", 1e7, 2), box("unk_rand", 1e7, 4)
+    per_bin_rand = [box(f"unk_rand_{i}", 2e6, 40 + i) for i in range(N_TOMO)]
+    rows = {p: unk[p].load_data() for p in unk}
+    lab = {p: np.random.default_rng(1000 + p).integers(0, N_TOMO, len(rows[p])) for p in unk}
+    data = []
+    for i in range(N_TOMO):
+        col = lambda k: np.concatenate([rows[p][k][lab[p] == i] for p in unk])  # noqa: E731
+        ids = np.concatenate([np.full(int((lab[p] == i).sum()), p) for p in unk])
+        data.append(yb.Catalog.from_arrays(col("ra"), col("dec"), patch_ids=ids, patch_centers=centers,
+                                           redshifts=col("redshifts"), degrees=False, cache_directory=f"unk_{i}"))
+    config = yb.Configuration.create(rmin=100, rmax=1000, zmin=0.07, zmax=1.42, num_bins=30)
+    return config, data, dict(A=shared, B=per_bin_rand)
+
+
 def stat_sums():
     st = measurements.last_stats()
     return {k: sum(s[k] for s in st.values()) for k in ("kernel_ms", "index_ms", "pair_tests")}
@@ -94,28 +124,55 @@ def run_one(eng, config, ref, ref_rand, unknowns, unk_rand):
     return time.perf_counter() - t0, stat_sums(), out
 
 
+def run_loop_auto(eng, config, data, random):
+    rands = random if isinstance(random, list) else [random] * len(data)
+    sums, out = {}, []
+    t0 = time.perf_counter()
+    for d, rand in zip(data, rands):
+        out.append(yb.autocorrelate(config, d, rand, engine=eng))
+        add(sums, stat_sums())
+    return time.perf_counter() - t0, sums, out
+
+
+def run_one_auto(eng, config, data, random):
+    t0 = time.perf_counter()
+    out = yb.autocorrelate_tomographic(config, data, random, engine=eng)
+    return time.perf_counter() - t0, stat_sums(), out
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r04_tomographic_timing.json"))
+    ap.add_argument("--mode", choices=("cross", "auto"), default="cross")
+    ap.add_argument("--out", default=None)
     ap.add_argument("--small", action="store_true")
     ap.add_argument("--repeats", type=int, default=3)
     args = ap.parse_args()
-    config, ref, ref_rand, unknowns, rand_forms = inputs(0.01 if args.small else 1.0)
+    out_path = args.out or os.path.join(ROOT, "profiles", f"r05_{args.mode}_tomographic_timing.json")
+    scale = 0.01 if args.small else 1.0
+    if args.mode == "cross":
+        config, ref, ref_rand, unknowns, rand_forms = inputs(scale)
+        loop = lambda eng, r: run_loop(eng, config, ref, ref_rand, unknowns, r)  # noqa: E731
+        one = lambda eng, r: run_one(eng, config, ref, ref_rand, unknowns, r)  # noqa: E731
+        rows = dict(ref=sum(ref.get_num_records()), ref_rand=sum(ref_rand.get_num_records()),
+                    unknown=sum(sum(u.get_num_records()) for u in unknowns))
+    else:
+        config, data, rand_forms = auto_inputs(scale)
+        loop = lambda eng, r: run_loop_auto(eng, config, data, r)  # noqa: E731
+        one = lambda eng, r: run_one_auto(eng, config, data, r)  # noqa: E731
+        rows = dict(unknown=sum(sum(d.get_num_records()) for d in data))
     eng = yb.Engine(0)
-    result = dict(gpu=gpu_info(), n_tomo=N_TOMO, rows=dict(ref=sum(ref.get_num_records()),
-                  ref_rand=sum(ref_rand.get_num_records()), unknown=sum(sum(u.get_num_records()) for u in unknowns)),
-                  cases={})
+    result = dict(gpu=gpu_info(), mode=args.mode, n_tomo=N_TOMO, rows=rows, cases={})
     for case, unk_rand in rand_forms.items():
-        # warm-up of both forms, then alternate them: the reference catalogs stay resident in the engine either way
-        _, _, loop_out = run_loop(eng, config, ref, ref_rand, unknowns, unk_rand)
-        _, _, one_out = run_one(eng, config, ref, ref_rand, unknowns, unk_rand)
+        # warm-up of both forms, then alternate them: every catalog stays resident in the engine's cache either way
+        _, _, loop_out = loop(eng, unk_rand)
+        _, _, one_out = one(eng, unk_rand)
         for a, b in zip(loop_out, one_out):
-            assert a == b, f"case {case}: crosscorrelate_tomographic differs from the loop"
+            assert a == b, f"case {case}: the one-call form differs from the loop"
         loop_t, one_t = [], []
         for _ in range(args.repeats):
-            t, loop_stats, _ = run_loop(eng, config, ref, ref_rand, unknowns, unk_rand)
+            t, loop_stats, _ = loop(eng, unk_rand)
             loop_t.append(t)
-            t, one_stats, _ = run_one(eng, config, ref, ref_rand, unknowns, unk_rand)
+            t, one_stats, _ = one(eng, unk_rand)
             one_t.append(t)
         result["cases"][case] = dict(
             unk_rand={"A": "shared 1e7", "B": f"per bin {N_TOMO} x 2e6", "C": "none"}[case],
@@ -132,8 +189,8 @@ def main() -> None:
     eng.close()
     line = json.dumps(result)
     print(line)
-    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-    with open(args.out, "w") as f:
+    os.makedirs(os.path.dirname(os.path.abspath(out_path)), exist_ok=True)
+    with open(out_path, "w") as f:
         f.write(line + "\n")
 
 

@@ -20,6 +20,7 @@ FLAG_EXACT_BRUTEFORCE = 1
 FLAG_OUT_DEVICE = 2
 FLAG_SECOND_LABELS = 4
 LABELS_MIN_VERSION = 101  # first library version that knows FLAG_SECOND_LABELS
+BINNED_LABELS_MIN_VERSION = 102  # first library version with yawb_catalog_set_labels
 ROLE_FIRST = 1
 ROLE_SECOND = 2
 
@@ -30,6 +31,7 @@ EXPORTS = (
     "yawb_host_alloc", "yawb_host_free", "yawb_sync", "yawb_version", "yawb_device_sms",
     "yawb_timer_start", "yawb_timer_stop", "yawb_assign_patches", "yawb_upload_catalog_u8", "yawb_count2",
     "yawb_upload_catalog_z", "yawb_patch_metadata", "yawb_jackknife", "yawb_count4", "yawb_kmeans",
+    "yawb_catalog_set_labels",
 )
 
 
@@ -112,8 +114,11 @@ def load(build_if_missing: bool = False) -> ctypes.CDLL:
         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_uint32,
         POINTER(c_void_p), POINTER(c_void_p), POINTER(YawbStats),
     ]
+    if hasattr(lib, "yawb_catalog_set_labels"):  # older libraries lack it: Engine.upload_catalog(n_labels=) refuses
+        lib.yawb_catalog_set_labels.argtypes = [c_void_p, c_int]
+        lib.yawb_catalog_set_labels.restype = c_int
     for name in EXPORTS:
-        if name not in ("yawb_last_error",):
+        if name not in ("yawb_last_error", "yawb_catalog_set_labels"):
             getattr(lib, name).restype = c_int
     lib.yawb_last_error.restype = c_char_p
     _lib = lib

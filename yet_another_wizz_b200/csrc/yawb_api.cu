@@ -144,7 +144,7 @@ int yawb_assign_patches(yawb_ctx *ctx, const double *xyz, int64_t n, const doubl
 
 const char *yawb_last_error(void) { return g_err; }
 
-int yawb_version(void) { return 101; }
+int yawb_version(void) { return 102; }
 
 int yawb_create(int device, yawb_ctx **out) {
     YAWB_REQUIRE(out != nullptr, "yawb_create: out is NULL");
@@ -306,6 +306,17 @@ int yawb_upload_catalog_z(yawb_ctx *ctx, const double *xyz, const double *w, con
     return upload_common(ctx, xyz, w, nullptr, nullptr, z, edges, closed_right, patch_off, n_patch, n_bins, out);
 }
 
+int yawb_catalog_set_labels(yawb_cat *cat, int n_labels) {
+    YAWB_REQUIRE(cat != nullptr, "yawb_catalog_set_labels: cat is NULL");
+    YAWB_REQUIRE(cat->binned, "yawb_catalog_set_labels: the catalog has no z-bin ids");
+    YAWB_REQUIRE(cat->h_edges.empty(), "yawb_catalog_set_labels: a catalog binned on the device (yawb_upload_catalog_z) "
+                                       "holds z-bins, not binned labels");
+    YAWB_REQUIRE(n_labels >= 1 && cat->n_bins % n_labels == 0,
+                 "yawb_catalog_set_labels: n_labels must be >= 1 and divide n_bins = %d (got %d)", cat->n_bins, n_labels);
+    cat->n_labels = n_labels;
+    return 0;
+}
+
 int yawb_free_catalog(yawb_cat *cat) {
     if (!cat) return 0;
     cudaSetDevice(cat->ctx->device);
@@ -432,7 +443,25 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
                  "YAWB_FLAG_SECOND_LABELS is not supported by the exact cross-check (YAWB_FLAG_EXACT_BRUTEFORCE)");
     YAWB_REQUIRE(cat1->n_patch == cat2->n_patch, "catalogs have different numbers of patches (%d vs %d)",
                  cat1->n_patch, cat2->n_patch);
-    if (!labels) {
+    // binned labels (yawb_catalog_set_labels): (a) both catalogs labelled alike, row (l, z) of cat2 meets (l, z) of
+    // cat1; (b) cat1 binned without labels, (l, z) meets z.  Counts of label l go to output block l.
+    const int L1 = cat1->n_labels, L2 = cat2->n_labels;
+    if (L1 || L2 || (cat1b && cat1b->n_labels) || (cat2b && cat2b->n_labels)) {
+        YAWB_REQUIRE(!cat1b && !cat2b, "catalogs with binned labels are not supported by yawb_count2 / yawb_count4");
+        YAWB_REQUIRE(!labels, "catalogs with binned labels cannot be combined with YAWB_FLAG_SECOND_LABELS");
+        YAWB_REQUIRE(!(flags & YAWB_FLAG_EXACT_BRUTEFORCE),
+                     "catalogs with binned labels are not supported by the exact cross-check (YAWB_FLAG_EXACT_BRUTEFORCE)");
+        YAWB_REQUIRE(L2, "a first catalog with binned labels needs a second catalog with the same labels; "
+                         "swap the roles (pair counts are symmetric)");
+        YAWB_REQUIRE(cat1->binned, "a second catalog with binned labels needs a binned first catalog");
+        if (L1)
+            YAWB_REQUIRE(L1 == L2 && cat1->n_bins == cat2->n_bins,
+                         "catalogs with binned labels differ (%d labels x %d z-bins vs %d x %d)", L1, cat1->n_bins / L1, L2,
+                         cat2->n_bins / L2);
+        else
+            YAWB_REQUIRE(cat1->n_bins == cat2->n_bins / L2, "z-bin counts differ (%d vs %d per label)", cat1->n_bins,
+                         cat2->n_bins / L2);
+    } else if (!labels) {
         YAWB_REQUIRE(!(cat2->binned && !cat1->binned), "a binned second catalog needs a binned first catalog");
         YAWB_REQUIRE(!cat2->binned || cat2->n_bins == cat1->n_bins, "z-bin counts differ (%d vs %d)", cat1->n_bins,
                      cat2->n_bins);
@@ -453,10 +482,12 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     YAWB_REQUIRE(n_pairs == 0 || (pair_i && pair_j), "pair lists are NULL");
     const int n_types = cat1b ? 2 : 1;
     const int n_src = cat2b ? 2 : 1;  // second catalogs of the launch
-    // output blocks per second catalog: its labels (YAWB_FLAG_SECOND_LABELS on a binned catalog), else one
-    const int n_lab[2] = {labels && cat2->binned ? cat2->n_bins : 1, labels && cat2b && cat2b->binned ? cat2b->n_bins : 1};
+    // output blocks per second catalog: its labels (binned labels, or YAWB_FLAG_SECOND_LABELS on a binned catalog), else one
+    const int n_lab[2] = {L2 ? L2 : labels && cat2->binned ? cat2->n_bins : 1,
+                          labels && cat2b && cat2b->binned ? cat2b->n_bins : 1};
     const int n_blocks = n_lab[0] + (cat2b ? n_lab[1] : 0);
-    const int B = cat1->n_bins, P = cat1->n_patch, nsub = n_edges - 1;
+    // B: z-bins of the thresholds and of every output block
+    const int B = L2 ? cat2->n_bins / L2 : cat1->n_bins, P = cat1->n_patch, nsub = n_edges - 1;
     for (int k = 0; k < n_pairs; ++k)
         YAWB_REQUIRE(pair_i[k] >= 0 && pair_i[k] < P && pair_j[k] >= 0 && pair_j[k] < P,
                      "patch pair %d = (%d, %d) out of range", k, pair_i[k], pair_j[k]);
@@ -561,6 +592,13 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
             base[k + 1] = base[k] + nt;
             const int p = pair_i[k];
             if (p == q) flat_diag += nt;
+            if (L2) {  // binned labels: (l, z) of the second catalog against (l, z) or z of the first
+                for (int l = 0; l < L2; ++l)
+                    for (int b = 0; b < B; ++b)
+                        s.pair_tests_naive += (uint64_t)(cat1->h_counts[((size_t)(L1 ? l * B : 0) + b) * P + p] *
+                                                         c2->h_counts[((size_t)l * B + b) * P + q]);
+                continue;
+            }
             long long n2_all = 0;  // a labelled catalog pairs the rows of every label with each z-bin
             for (int l = 0; l < c2->n_bins; ++l) n2_all += c2->h_counts[(size_t)l * P + q];
             for (int b = 0; b < B; ++b) {
@@ -635,6 +673,8 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
     a.n_items_b = cat2b ? item_base[(size_t)(n_pairs + 1) + n_pairs] : 0;
     a.labels = labels;
     a.blk_b = n_lab[0];
+    a.lab_bins = L2 ? B : 0;
+    a.lab_first = L1 > 0;
     // work-item lists: a patch with itself needs an item per tile (a few more where items are split), of the
     // tiles of neighbouring patches only the boundary strip survives; if a list turns out too small the
     // count is repeated with the exact sizes

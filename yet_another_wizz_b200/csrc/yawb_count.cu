@@ -602,6 +602,9 @@ struct PlanParams {
     int src;   // which second catalog of a joint launch these tiles belong to (Item::src)
     int blk;     // first output block of that catalog (Item::blk)
     int labels;  // the tiles' z-bin ids are sample labels: paired with every z-bin, counts go to block blk + label
+    int lab_bins;   // binned labels: a tile's id t is (label t / lab_bins, z-bin t % lab_bins); counts go to block
+                    // blk + label (0: none)
+    int lab_first;  // ... and the first catalog's ids are binned labels too: the item reads id label * lab_bins + z-bin
     unsigned long long *counters;
 };
 
@@ -645,7 +648,9 @@ __global__ void __launch_bounds__(256) k_plan(const PlanParams Q) {
         const int t = Q.ptile_off[p2] + (int)(f - Q.pair_item_base[k]);
         const Tile tl = Q.tiles[t];
         const PatchFrame &F1 = Q.frames1[p1];
-        const int zb = Q.labels ? -1 : tl.bin;  // z-bin of the tile, -1: paired with every z-bin of the first catalog
+        // z-bin of the tile (-1: paired with every z-bin of the first catalog) and its label (output block)
+        const int zb = Q.lab_bins ? tl.bin % Q.lab_bins : Q.labels ? -1 : tl.bin;
+        const int lab = Q.lab_bins ? tl.bin / Q.lab_bins : Q.labels && tl.bin >= 0 ? tl.bin : 0;
         const double rmax = zb >= 0 ? (Q.binpar[zb].empty ? 0.0 : Q.binpar[zb].rmax) : Q.rmax_all;
         // bounding spheres first (chord distances obey the triangle inequality)
         const double dx = (double)tl.cx - F1.c[0], dy = (double)tl.cy - F1.c[1], dz = (double)tl.cz - F1.c[2];
@@ -678,7 +683,8 @@ __global__ void __launch_bounds__(256) k_plan(const PlanParams Q) {
             if (lo3[0] - rmax <= F1.umax && hi3[0] + rmax >= F1.umin && lo3[1] - rmax <= F1.vmax && hi3[1] + rmax >= F1.vmin) {
                 G = Q.sgrid[p1];
                 it.pair = k; it.p1 = p1; it.start = tl.start; it.count = tl.count; it.src = Q.src;
-                it.blk = Q.blk + (Q.labels && tl.bin >= 0 ? tl.bin : 0);
+                it.blk = Q.blk + lab;
+                it.b_off = Q.lab_first ? lab * Q.lab_bins : 0;
                 it.b_lo = zb >= 0 ? zb : 0;
                 it.b_hi = zb >= 0 ? zb + 1 : Q.n_bins;
 #pragma unroll
@@ -870,6 +876,8 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
         Q.src = sc;
         Q.blk = sc ? a.blk_b : 0;
         Q.labels = a.labels ? 1 : 0;
+        Q.lab_bins = a.lab_bins;
+        Q.lab_first = a.lab_first ? 1 : 0;
         k_plan<<<(unsigned)((n_flat + 255) / 256), 256, 0, ctx->stream>>>(Q);
         *launches += 1;
     }

@@ -165,7 +165,7 @@ __device__ __forceinline__ void stream_plan(const FastParams &P, const StreamSme
         ax.n_combo = n_combo;
     }
     __syncwarp();
-    const int b_lo = it.b_lo, b_hi = it.b_hi;
+    const int b_lo = it.b_lo, b_hi = it.b_hi, b_off = it.b_off;
     for (int k = lane; k < n_combo; k += 32) {
         int lo = b_lo, hi = b_hi;  // last z-bin with cstart[b] <= k
         while (hi - lo > 1) {
@@ -175,7 +175,9 @@ __device__ __forceinline__ void stream_plan(const FastParams &P, const StreamSme
         const int b = lo;
         const int iv = S.bin_iv0[b] + (k - S.cstart[b]);
         const int iu = S.bin_iu[b];
-        const long long row = G.cell_base + ((long long)b * G.gv + iv) * G.gu;
+        // the first catalog's cells of z-bin b of the item's label (binned labels: id b + b_off); every table of
+        // the warp stays indexed by the z-bin b
+        const long long row = G.cell_base + ((long long)(b + b_off) * G.gv + iv) * G.gu;
         cp_async4(&S.cs[k].x, P.cell_start + row + (iu & 0xffff));
         cp_async4(&S.cs[k].y, P.cell_start + row + (iu >> 16) + 1);
         S.csbin[k] = (unsigned short)b;

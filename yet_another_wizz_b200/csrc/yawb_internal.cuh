@@ -98,7 +98,9 @@ struct __align__(16) Item {
                            // a restriction only occurs on items of a single z-bin
     int src;               // second catalog of a joint launch (0 or 1): where the tile's rows live
     int blk;               // output block of the item's counts: second catalog, then label (YAWB_FLAG_SECOND_LABELS)
-    int pad[2];
+    int b_off;             // first-catalog id of z-bin 0 of the item's label (label * B when both catalogs carry
+                           // binned labels, else 0): the cell rows of z-bin b are those of id b + b_off
+    int pad;
     double lo[3], hi[3];
 };
 static_assert(sizeof(Item) == 96, "Item is copied as six 16-byte pieces");
@@ -159,6 +161,7 @@ struct yawb_cat {
     int64_t n = 0;        // rows kept (z-bin in range)
     int n_patch = 0;
     int n_bins = 1;       // 1 for an unbinned catalog
+    int n_labels = 0;     // binned labels (yawb_catalog_set_labels): ids are label * (n_bins / n_labels) + z-bin; 0: none
     bool binned = false;
     bool weighted = false;
     int64_t device_bytes = 0;
@@ -264,6 +267,8 @@ struct CountArgs {
     long long n_items_b = 0;
     bool labels = false;    // YAWB_FLAG_SECOND_LABELS: the z-bin ids of a binned second catalog are sample labels
     int blk_b = 1;          // first output block of c2b (= labels of c2)
+    int lab_bins = 0;       // binned labels of c2: z-bins per label B (id = label * B + z-bin), 0: none
+    bool lab_first = false;  // ... and the first catalog carries the same binned labels
     long long cap_heavy, cap_light;     // capacities of the two work-item lists
     int n_pairs;
     int n_bins;

@@ -33,6 +33,7 @@ class DeviceCatalog:
         self.n_bins = n_bins
         self.binned = binned
         self.weighted = weighted
+        self.n_labels = None  # binned labels (`Engine.upload_catalog(n_labels=)`): id = label * (n_bins // n_labels) + z-bin
 
     def sum_weights(self) -> np.ndarray:
         """`(n_bins, n_patch)` sum of weights (row counts if unweighted)."""
@@ -85,8 +86,10 @@ class Engine:
         functions stay resident, with their indexes, keyed by (catalog, z-binning) -- the counterpart of the
         reference's on-disk tree cache (`BinnedTrees.build` skips the rebuild while the `binning` file matches,
         `src/yaw/catalog/trees.py:515-526`).  A loop of `crosscorrelate` calls over tomographic bins then uploads and
-        indexes only the catalogs that changed.  Least recently used entries are dropped beyond `cache_bytes` of
-        device memory (default 64 GB, YAWB_CACHE_GB).
+        indexes only the catalogs that changed.  A labelled upload of several catalogs (`crosscorrelate_tomographic`,
+        `autocorrelate_tomographic`) is kept the same way, keyed by the tuple of its members and dropped as soon as
+        any of them dies.  Least recently used entries are dropped beyond `cache_bytes` of device memory (default
+        64 GB, YAWB_CACHE_GB).
 
         `staging=True` (or YAWB_STAGING=1): measurement calls prepare large catalogs straight into a
         cache of page-locked buffers, so their copies are asynchronous and run at full PCIe rate.  Worth it
@@ -105,7 +108,7 @@ class Engine:
         self._catalogs = weakref.WeakSet()  # live device catalogs: freed before the context goes away
         self.cache_catalogs = (os.environ.get("YAWB_CACHE", "1") != "0") if cache_catalogs is None else bool(cache_catalogs)
         self.cache_bytes = int(float(os.environ.get("YAWB_CACHE_GB", "64")) * 2**30) if cache_bytes is None else int(cache_bytes)
-        self._cat_cache: dict = {}  # (identity, kappa) -> [signature of the binning, DeviceCatalog, bytes, weakref | None]
+        self._cat_cache: dict = {}  # (identity, kappa) -> [signature of the binning, DeviceCatalog, bytes, weakrefs, tick]
         self._cat_cache_tick = 0
         self._pinned: list[c_void_p] = []
         self._stage_free: list[tuple[c_void_p, int]] = []
@@ -126,10 +129,22 @@ class Engine:
         redshifts: np.ndarray | None = None,
         edges: np.ndarray | None = None,
         closed: str = "right",
+        n_labels: int | None = None,
     ) -> DeviceCatalog:
         """`zbin` (+ `n_bins`): z-bin ids assigned on the host; or `redshifts` + `edges` (+ `closed`): the raw
         redshifts travel and the device assigns the bins with np.digitize's comparisons (`yawb_upload_catalog_z`,
-        reference `src/yaw/catalog/trees.py:408-414`)."""
+        reference `src/yaw/catalog/trees.py:408-414`).
+
+        `n_labels` (with `zbin`): binned labels (`yawb_catalog_set_labels`), the ids are `label * B + z-bin` with
+        `B = n_bins // n_labels`, e.g. the tomographic bins of a sample, each z-binned (`prepare_labelled_arrays`
+        with a binning).  `count` then pairs label by label; see there."""
+        if n_labels is not None:
+            if zbin is None:
+                raise ValueError("'n_labels' needs z-bin ids ('zbin')")
+            version = self.lib.yawb_version()
+            if version < _lib.BINNED_LABELS_MIN_VERSION:
+                raise _lib.YawbError(f"n_labels needs libyawb version >= {_lib.BINNED_LABELS_MIN_VERSION} "
+                                     f"(loaded: {version})")
         xyz = np.ascontiguousarray(xyz, dtype=np.float64).reshape(-1, 3)
         patch_off = np.ascontiguousarray(patch_off, dtype=np.int64)
         n = len(xyz)
@@ -172,6 +187,13 @@ class Engine:
             )
         binned = zbin is not None or redshifts is not None
         cat = DeviceCatalog(self, h, len(patch_off) - 1, int(n_bins) if binned else 1, binned, weights is not None)
+        if n_labels is not None:
+            try:
+                _lib.check(self.lib.yawb_catalog_set_labels(h, int(n_labels)))
+            except Exception:
+                cat.free()
+                raise
+            cat.n_labels = int(n_labels)
         # the upload is asynchronous: keep the host buffers alive as long as the handle
         cat._keepalive = (xyz, weights, zbin, redshifts, patch_off)
         self._catalogs.add(cat)
@@ -202,8 +224,12 @@ class Engine:
 
     @staticmethod
     def _shape(cat2: DeviceCatalog, labels: bool, n_pairs: int, n_bins: int, n_edges: int) -> tuple:
-        """result shape of one (first, second) catalog combination: a leading label axis with `labels`"""
+        """result shape of one (first, second) catalog combination: a leading label axis with `labels` or with the
+        binned labels of `cat2`"""
         shape = (n_pairs, n_bins, n_edges - 1)
+        n_labels = getattr(cat2, "n_labels", None)
+        if n_labels is not None:
+            return (n_labels, *shape)
         return ((cat2.n_bins if cat2.binned else 1), *shape) if labels else shape
 
     def count(
@@ -225,11 +251,18 @@ class Engine:
         `cat2.n_bins`, 1 for an unbinned `cat2`); every row is paired with every z-bin of `cat1` and the arrays
         gain a leading label axis, `(L, n_pairs, n_bins, n_edges - 1)`: entry l is the count against the rows of
         label l alone.
+
+        Binned labels (`cat2` uploaded with `n_labels=L`, `B = cat2.n_bins // L` z-bins per label): `r2_edges` is
+        `(B, n_edges)` and the arrays are `(L, n_pairs, B, n_edges - 1)`, also for L = 1.  Entry l is the z-binned
+        count of label l of `cat2` against label l of `cat1` when `cat1` carries the same binned labels (`cat1` may
+        be `cat2`), or against the whole of `cat1` when `cat1` is binned with B z-bins and unlabelled.  A labelled
+        `cat1` needs a labelled `cat2`: pair counts are symmetric, swap the catalogs and the pair lists.
         """
         pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
         pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
         r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
-        n_bins = cat1.n_bins
+        lab = cat2 if getattr(cat2, "n_labels", None) else cat1  # binned labels: r2_edges per z-bin of a label
+        n_bins = lab.n_bins // lab.n_labels if getattr(lab, "n_labels", None) else cat1.n_bins
         if r2_edges.ndim == 1:
             r2_edges = np.ascontiguousarray(np.broadcast_to(r2_edges, (n_bins, len(r2_edges))))
         if r2_edges.shape[0] != n_bins:
@@ -403,7 +436,10 @@ class Engine:
     @staticmethod
     def _cache_identity(catalog):
         # the catalog OBJECT (an entry lives exactly as long as it does); a cache directory is only a label for
-        # this package's in-memory catalogs, and on disk it can be overwritten, so paths are not identities
+        # this package's in-memory catalogs, and on disk it can be overwritten, so paths are not identities.  A
+        # labelled upload (`prepare_labelled_arrays`) is keyed by the tuple of its member catalogs.
+        if isinstance(catalog, tuple):
+            return ("labelled", tuple(id(c) for c in catalog))
         return ("id", id(catalog))
 
     def cache_lookup(self, catalog, signature, kappa: bool):
@@ -427,8 +463,9 @@ class Engine:
             return False
         ident = self._cache_identity(catalog)
         key = (ident, bool(kappa))
-        try:
-            ref = weakref.ref(catalog, lambda _r, k=key: self._cache_drop(k))
+        members = catalog if isinstance(catalog, tuple) else (catalog,)
+        try:  # the entry is dropped as soon as any member dies
+            ref = [weakref.ref(c, lambda _r, k=key: self._cache_drop(k)) for c in members]
         except TypeError:
             return False
         self._cache_drop(key)

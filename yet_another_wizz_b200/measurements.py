@@ -34,8 +34,9 @@ from .corrfunc import CorrFunc, ScalarCorrFunc
 from .paircounts import NormalisedCounts, NormalisedScalarCounts, PatchedCounts, PatchedSumWeights
 from .sharding import Shard, assign_pairs_lpt, current_shard, pair_costs
 
-__all__ = ["PatchLinkage", "autocorrelate", "autocorrelate_scalar", "compute_scalar_normalisation", "crosscorrelate",
-           "crosscorrelate_scalar", "crosscorrelate_tomographic", "get_default_engine", "last_stats"]
+__all__ = ["PatchLinkage", "autocorrelate", "autocorrelate_scalar", "autocorrelate_tomographic",
+           "compute_scalar_normalisation", "crosscorrelate", "crosscorrelate_scalar", "crosscorrelate_tomographic",
+           "get_default_engine", "last_stats"]
 
 logger = logging.getLogger("yaw_b200")
 
@@ -193,11 +194,16 @@ def _run_fill(fill, tasks, n_rows: int, workers: int | None) -> None:
             fill(task)
 
 
-def prepare_labelled_arrays(catalogs, *, workers: int | None = None, alloc=None) -> dict:
+def prepare_labelled_arrays(catalogs, binning: Binning | None = None, *, workers: int | None = None,
+                            alloc=None) -> dict:
     """Host preparation of ONE labelled catalog from several (`YAWB_FLAG_SECOND_LABELS`): per patch the rows of
     `catalogs[0]`, `catalogs[1]`, ..., each row labelled with the position of its catalog (byte-sized ids, at
     most 254 catalogs).  The rows and their unit vectors are those `prepare_catalog_arrays` gives each catalog.
-    Returns the keyword arguments of `Engine.upload_catalog`."""
+    Returns the keyword arguments of `Engine.upload_catalog`.
+
+    With `binning` the ids are binned labels (`n_labels` = number of catalogs): `label * B + z-bin`, the z-bins
+    digitised as `prepare_catalog_arrays` does.  A row outside the binning is dropped (id 255 when `L * B <= 254`,
+    else -1), never given a neighbouring label's id."""
     alloc = alloc or np.empty
     catalogs = list(catalogs)
     if not 1 <= len(catalogs) <= 254:
@@ -205,6 +211,11 @@ def prepare_labelled_arrays(catalogs, *, workers: int | None = None, alloc=None)
     has_w = bool(catalogs[0].has_weights)
     if any(bool(c.has_weights) != has_w for c in catalogs):
         raise ValueError("the catalogs of a labelled upload must all have weights or all have none")
+    if binning is not None and not all(c.has_redshifts for c in catalogs):
+        raise ValueError("patch has no 'redshifts' attached")  # as prepare_catalog_arrays
+    n_zbins = len(binning) if binning is not None else 1
+    n_ids = len(catalogs) * n_zbins
+    small_ids = n_ids <= 254
     n_patch = len(catalogs[0])
     for c in catalogs:
         if list(c.keys()) != list(range(n_patch)):
@@ -216,11 +227,11 @@ def prepare_labelled_arrays(catalogs, *, workers: int | None = None, alloc=None)
     n = int(off[-1])
     xyz = alloc((n, 3), np.float64)
     ws = alloc(n, np.float64) if has_w else None
-    lab = alloc(n, np.uint8)
+    lab = alloc(n, np.uint8 if small_ids else np.int32)
 
     def fill(task) -> None:
         label, pid = task
-        ra, dec, weights, _, _ = _patch_rows(catalogs[label][pid])
+        ra, dec, weights, redshifts, _ = _patch_rows(catalogs[label][pid])
         s = int(start[pid * len(catalogs) + label])
         e = s + int(sizes[label, pid])
         if len(ra) != e - s:
@@ -231,10 +242,17 @@ def prepare_labelled_arrays(catalogs, *, workers: int | None = None, alloc=None)
         np.sin(dec, out=xyz[s:e, 2])
         if has_w:
             ws[s:e] = weights
-        lab[s:e] = label
+        if binning is None:
+            lab[s:e] = label
+        else:
+            z = binning.digitize(redshifts)  # -1 below, len(binning) above the binning
+            lab[s:e] = np.where((z >= 0) & (z < n_zbins), label * n_zbins + z, 255 if small_ids else -1)
 
     _run_fill(fill, [(label, pid) for pid in range(n_patch) for label in range(len(catalogs))], n, workers)
-    return dict(xyz=xyz, patch_off=off, weights=ws, zbin=lab, n_bins=len(catalogs))
+    out = dict(xyz=xyz, patch_off=off, weights=ws, zbin=lab, n_bins=n_ids)
+    if binning is not None:
+        out["n_labels"] = len(catalogs)
+    return out
 
 
 def _prepare_for(engine, catalog, binning: Binning | None, kappa: bool) -> dict:
@@ -273,6 +291,8 @@ class _Uploads:
     def _signature(catalog, binning):
         """what a resident device catalog depends on besides the catalog object: the z-binning (the reference's
         `binning` file) and, as a guard against catalogs refilled in place, the rows per patch"""
+        if isinstance(catalog, tuple):  # a labelled upload: the signatures of its members
+            return tuple(_Uploads._signature(c, binning) for c in catalog)
         rows = tuple(int(n) for n in catalog.get_num_records())
         if binning is None:
             return (rows, None)
@@ -326,6 +346,18 @@ class _Uploads:
             return self._resolve(key)
         if key not in self._cache and not self._resident_lookup(key, catalog, binning, kappa):
             self._store(key, catalog, binning, kappa, upload_catalog(self.engine, catalog, binning, kappa=kappa))
+        return self._cache[key]
+
+    def get_labelled(self, catalogs, binning: Binning | None = None):
+        """ONE device catalog holding the rows of `catalogs`, labelled by position (`prepare_labelled_arrays`; with
+        `binning`, binned labels).  Kept in the engine's cache like a single catalog, keyed by the tuple of its
+        members, and dropped there as soon as any member dies."""
+        catalogs = tuple(catalogs)
+        key = (("labelled", *map(id, catalogs)), binning is not None, False)
+        if key not in self._cache and not self._resident_lookup(key, catalogs, binning, False):
+            arrays = prepare_labelled_arrays(catalogs, binning)
+            dev = self.engine.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
+            self._store(key, catalogs, binning, False, dev)
         return self._cache[key]
 
     def free(self) -> None:
@@ -688,8 +720,9 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
 
     `unknowns`: 1 to 254 catalogs, one per bin, all with weights or all without.  `unk_rand`: None, one catalog
     shared by every bin, or a sequence of one catalog per bin.  The bins travel to the device as ONE labelled
-    catalog (`YAWB_FLAG_SECOND_LABELS`), per-bin randoms likewise; every count runs once over the union of the
-    bins' patch-pair lists, and each bin is packaged from its own linkage.  A shared `unk_rand` is counted once
+    catalog (`YAWB_FLAG_SECOND_LABELS`), per-bin randoms likewise, and stay in the engine's cache like single
+    catalogs; every count runs once over the union of the bins' patch-pair lists, and each bin is packaged from its
+    own linkage.  A shared `unk_rand` is counted once
     (DR and RR) for all bins.  Everything a per-bin call would raise is raised before any counting.
     `progress` / `max_workers` are accepted and ignored."""
     unknowns = list(unknowns)
@@ -719,13 +752,7 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
     links = [PatchLinkage.from_catalogs(config, reference, unknown, *[c for c in (ref_rand, rand) if c is not None],
                                         engine=engine, shard=shard) for unknown, rand in zip(unknowns, rands)]
     bin_pairs = [lk.get_patch_id_pairs(auto=False) for lk in links]
-    union: dict[tuple[int, int], int] = {}
-    for pi, pj in bin_pairs:
-        for pair in zip(pi.tolist(), pj.tolist()):
-            union.setdefault(pair, len(union))
-    union_ij = np.array(list(union), dtype=np.int32).reshape(-1, 2)
-    # rows of the union that make up each bin's pair list, in that bin's order
-    bin_rows = [np.array([union[p] for p in zip(pi.tolist(), pj.tolist())], dtype=np.int64) for pi, pj in bin_pairs]
+    union_ij, bin_rows = _union_pairs(bin_pairs)
 
     driver = links[0]
     eng = engine or get_default_engine()
@@ -735,13 +762,6 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
     num_patches = len(reference)
     _last_stats.clear()
     uploads = _Uploads(eng)
-    labelled = []  # device catalogs of this call only
-
-    def upload_labelled(catalogs):
-        arrays = prepare_labelled_arrays(catalogs)
-        dev = eng.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
-        labelled.append(dev)
-        return dev
 
     own = np.arange(len(union_ij))
     if shard.active:  # a pair's cost sums the rows of every bin
@@ -764,10 +784,10 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
         uploads.enqueue(((reference, binning), (ref_rand, binning), (unk_rand if shared else None, None)))
         dev_ref = uploads.get(reference, binning)
         dev_rr = uploads.get(ref_rand, binning) if ref_rand is not None else None
-        dev_unk = upload_labelled(unknowns)
+        dev_unk = uploads.get_labelled(unknowns)
         dev_ur = None
         if unk_rand is not None:
-            dev_ur = uploads.get(unk_rand, None) if shared else upload_labelled(rands)
+            dev_ur = uploads.get(unk_rand, None) if shared else uploads.get_labelled(rands)
         sw = dict(ref=dev_ref.sum_weights(), unk=dev_unk.sum_weights())
         if dev_rr is not None:
             sw["rr"] = dev_rr.sum_weights()
@@ -791,8 +811,6 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
                 hists[kind] = gather(hist_f if (dev1.weighted or dev2.weighted) else hist_i)
                 _last_stats[kind] = stats
     finally:
-        for dev in labelled:
-            dev.free()
         uploads.free()
 
     none = [None for _ in range(config.scales.num_scales)]
@@ -810,6 +828,132 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
         DR = package("DR", "ref", "ur", rand_label)
         RR = package("RR", "rr", "ur", rand_label)
         result.append([CorrFunc(dd, dr, rd, rr) for dd, dr, rd, rr in zip(DD, DR, RD, RR)])
+    return result
+
+
+def _union_pairs(bin_pairs) -> tuple[np.ndarray, list[np.ndarray]]:
+    """union of the bins' patch-pair lists (first appearance order) and, per bin, the rows of the union that make up
+    its own list, in its order"""
+    union: dict[tuple[int, int], int] = {}
+    for pi, pj in bin_pairs:
+        for pair in zip(pi.tolist(), pj.tolist()):
+            union.setdefault(pair, len(union))
+    union_ij = np.array(list(union), dtype=np.int32).reshape(-1, 2)
+    rows = [np.array([union[p] for p in zip(pi.tolist(), pj.tolist())], dtype=np.int64) for pi, pj in bin_pairs]
+    return union_ij, rows
+
+
+def autocorrelate_tomographic(config, data, random, *, count_rr: bool = True, progress: bool = False,
+                              max_workers=None, engine=None, shard: Shard | None = None) -> list[list[CorrFunc]]:
+    """`autocorrelate` of every tomographic bin of a sample in one pass: `result[i]` is `autocorrelate(config,
+    data[i], <randoms of bin i>, count_rr=count_rr)`, the per-bin unknown autocorrelation of the reference CLI
+    (`auto_unk`) as one call.
+
+    `data`: 1 to 254 z-binned catalogs, one per bin, all with weights or all without.  `random`: one catalog shared
+    by every bin, or a sequence of one catalog per bin.  The bins travel to the device as ONE catalog with binned
+    labels (id = bin * B + z-bin, `Engine.upload_catalog(n_labels=)`), per-bin randoms likewise.  DD is one
+    labelled autocount; DR one labelled count, or with shared randoms one count with the randoms as the first
+    catalog (pair counts are symmetric); RR one count, with shared randoms a plain z-binned autocount for all bins.
+    Every count runs once over the union of the bins' patch-pair lists, and each bin is packaged from its own
+    linkage.  Everything a per-bin call would raise is raised before any counting.  The labelled uploads stay in
+    the engine's cache like single catalogs.  `progress` / `max_workers` are accepted and ignored."""
+    data = list(data)
+    n_tomo = len(data)
+    if n_tomo == 0:
+        raise ValueError("'data' must hold at least one catalog")
+    if n_tomo > 254:
+        raise ValueError(f"at most 254 tomographic bins are supported (got {n_tomo})")
+    shared = not isinstance(random, Sequence)
+    rands = [random] * n_tomo if shared else list(random)
+    if len(rands) != n_tomo:
+        raise ValueError(f"'random' holds {len(rands)} catalogs for {n_tomo} tomographic bins")
+    if any(r is None for r in rands):
+        raise ValueError("'random' must hold a catalog for every bin")
+    for d, r in zip(data, rands):
+        _ensure_unique_catalogs(d, r)
+    # the linkage of every bin, exactly as its own call would build it
+    links = [PatchLinkage.from_catalogs(config, d, r, engine=engine, shard=shard) for d, r in zip(data, rands)]
+    if not all(c.has_redshifts for c in (*data, *rands)):
+        raise ValueError("patch has no 'redshifts' attached")
+    if len({bool(c.has_weights) for c in data}) > 1:
+        raise ValueError("the tomographic bins must all have weights or all have none")
+    if not shared and len({bool(c.has_weights) for c in rands}) > 1:
+        raise ValueError("the per-bin randoms must all have weights or all have none")
+    binning = _as_binning(config)
+    n_zbins = len(binning)
+    if n_tomo * n_zbins > 4096:
+        raise ValueError(f"bins x z-bins must not exceed 4096 (got {n_tomo} x {n_zbins})")
+
+    auto_pairs = [lk.get_patch_id_pairs(auto=True) for lk in links]
+    cross_pairs = [lk.get_patch_id_pairs(auto=False) for lk in links]
+    auto_ij, auto_rows = _union_pairs(auto_pairs)
+    cross_ij, cross_rows = _union_pairs(cross_pairs)
+
+    driver = links[0]
+    eng = engine or get_default_engine()
+    shard = shard or current_shard()
+    plan = driver._get_plan()
+    num_patches = len(data[0])
+    _last_stats.clear()
+    uploads = _Uploads(eng)
+
+    def own_pairs(ij, n1, n2):
+        if not shard.active:
+            return np.arange(len(ij))
+        costs = pair_costs(ij[:, 0], ij[:, 1], n1, n2, radii1=np.asarray(rands[0].get_radii().data))
+        return assign_pairs_lpt(costs, shard.world_size)[shard.rank]
+
+    n_data = np.sum([d.get_num_records() for d in data], axis=0)
+    n_rand = rands[0].get_num_records() if shared else np.sum([r.get_num_records() for r in rands], axis=0)
+    own_auto_dd = own_pairs(auto_ij, n_data, n_data)
+    own_cross = own_pairs(cross_ij, n_data, n_rand)
+    own_auto_rr = own_pairs(auto_ij, n_rand, n_rand)
+
+    def gather(hist, own, n_pairs, labelled=True):
+        """(L, own pairs, ...) -> (L, union pairs, ...) summed over the ranks (unlabelled: no leading axis)"""
+        if not labelled:
+            return driver._gather_shards(shard, hist, own, n_pairs)
+        return np.moveaxis(driver._gather_shards(shard, np.moveaxis(hist, 1, 0), own, n_pairs), 0, 1)
+
+    def count(kind, dev1, dev2, ij, own, swap=False):
+        pi, pj = ij[own, 0], ij[own, 1]
+        hist_i, hist_f, stats = eng.count(dev1, dev2, pj if swap else pi, pi if swap else pj, plan.r2)
+        hist = hist_f if (dev1.weighted or dev2.weighted) else hist_i
+        _last_stats[kind] = stats
+        return gather(hist, own, len(ij), labelled=getattr(dev2, "n_labels", None) is not None)
+
+    hists: dict[str, np.ndarray] = {}
+    try:
+        dev_d = uploads.get_labelled(data, binning)
+        dev_r = uploads.get(random, binning) if shared else uploads.get_labelled(rands, binning)
+        sw_d = dev_d.sum_weights().reshape(n_tomo, n_zbins, num_patches)
+        sw_r = dev_r.sum_weights().reshape(-1, n_zbins, num_patches)
+        hists["DD"] = count("DD", dev_d, dev_d, auto_ij, own_auto_dd)
+        if shared:  # the randoms as the first catalog, every bin's rows against their z-bin: pair lists swapped
+            hists["DR"] = count("DR", dev_r, dev_d, cross_ij, own_cross, swap=True)
+        else:
+            hists["DR"] = count("DR", dev_d, dev_r, cross_ij, own_cross)
+        if count_rr:
+            rr = count("RR", dev_r, dev_r, auto_ij, own_auto_rr)
+            hists["RR"] = rr[None] if shared else rr
+    finally:
+        uploads.free()
+
+    none = [None for _ in range(config.scales.num_scales)]
+    result = []
+    for i in range(n_tomo):
+        r = 0 if shared else i
+
+        def package(kind, rows, pairs, sw1, sw2, auto):
+            if kind not in hists:
+                return none
+            lab = r if kind == "RR" else i
+            return PatchLinkage._package(hists[kind][lab][rows], plan, binning, num_patches, *pairs, sw1, sw2, auto)
+
+        DD = package("DD", auto_rows[i], auto_pairs[i], sw_d[i], sw_d[i], True)
+        DR = package("DR", cross_rows[i], cross_pairs[i], sw_d[i], sw_r[r], False)
+        RR = package("RR", auto_rows[i], auto_pairs[i], sw_r[r], sw_r[r], True)
+        result.append([CorrFunc(dd, dr, None, rr) for dd, dr, rr in zip(DD, DR, RR)])
     return result
 
 
