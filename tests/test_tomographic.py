@@ -100,13 +100,11 @@ def _inputs(name):
     return g, config, ref, ref_rand, unk_rand, split_catalog(g, "unk")
 
 
-@pytest.mark.parametrize("fuse", ["1", "0"])
 @pytest.mark.parametrize("rand_form", ["shared", "per_bin", "none"])
 @pytest.mark.parametrize("name", ["cross_unweighted", "cross_weighted_multiscale"])
-def test_equals_per_bin_calls(name, rand_form, fuse, monkeypatch):
+def test_equals_per_bin_calls(name, rand_form):
     import yet_another_wizz_b200 as yb
 
-    monkeypatch.setenv("YAWB_FUSE", fuse)
     g, config, ref, ref_rand, unk_rand, unknowns = _inputs(name)
     if rand_form == "shared":
         arg, rands = unk_rand, [unk_rand] * N_TOMO
@@ -124,7 +122,7 @@ def test_equals_per_bin_calls(name, rand_form, fuse, monkeypatch):
     assert eng.log[0][1].binned and eng.log[0][1].n_bins == N_TOMO
     assert all(cat2.binned == (rand_form != "shared" or cat2 is eng.log[0][1]) for _, cat2 in eng.log)
     n_second = 1 + (rand_form != "none")
-    fused = fuse == "1" and bool(ref.has_weights) == bool(ref_rand.has_weights)  # crosscorrelate's decision
+    fused = bool(ref.has_weights) == bool(ref_rand.has_weights)  # crosscorrelate's decision
     assert len(eng.log) == (n_second if fused else 2 * n_second)
 
 

@@ -23,6 +23,19 @@ def _ptr(a: np.ndarray | None):
     return None if a is None else a.ctypes.data_as(c_void_p)
 
 
+def _pairs_and_edges(pair_i, pair_j, r2_edges, n_bins: int) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """the pair lists as contiguous int32 and `r2_edges` as contiguous `(n_bins, n_edges)` doubles (one row of
+    thresholds stands for every z-bin)"""
+    pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
+    pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
+    r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
+    if r2_edges.ndim == 1:
+        r2_edges = np.ascontiguousarray(np.broadcast_to(r2_edges, (n_bins, len(r2_edges))))
+    if r2_edges.shape[0] != n_bins:
+        raise ValueError(f"r2_edges must have shape (n_bins={n_bins}, n_edges)")
+    return pair_i, pair_j, r2_edges
+
+
 class DeviceCatalog:
     """Handle of a catalog uploaded with `Engine.upload_catalog`."""
 
@@ -258,15 +271,9 @@ class Engine:
         be `cat2`), or against the whole of `cat1` when `cat1` is binned with B z-bins and unlabelled.  A labelled
         `cat1` needs a labelled `cat2`: pair counts are symmetric, swap the catalogs and the pair lists.
         """
-        pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
-        pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
-        r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
         lab = cat2 if getattr(cat2, "n_labels", None) else cat1  # binned labels: r2_edges per z-bin of a label
         n_bins = lab.n_bins // lab.n_labels if getattr(lab, "n_labels", None) else cat1.n_bins
-        if r2_edges.ndim == 1:
-            r2_edges = np.ascontiguousarray(np.broadcast_to(r2_edges, (n_bins, len(r2_edges))))
-        if r2_edges.shape[0] != n_bins:
-            raise ValueError(f"r2_edges must have shape (n_bins={n_bins}, n_edges)")
+        pair_i, pair_j, r2_edges = _pairs_and_edges(pair_i, pair_j, r2_edges, n_bins)
         n_edges = r2_edges.shape[1]
         n_pairs = len(pair_i)
         shape = self._shape(cat2, labels, n_pairs, n_bins, n_edges)
@@ -301,14 +308,8 @@ class Engine:
         caller-owned buffers shaped `(n_pairs, n_bins, n_edges - 1)`; the results stay on the device
         (`YAWB_FLAG_OUT_DEVICE`, e.g. for an NCCL reduce) and the arrays returned are `None`.
         `labels`: as in `count`; the results (and device buffers) gain the leading label axis of `cat2`."""
-        pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
-        pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
-        r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
         n_bins = cat1a.n_bins
-        if r2_edges.ndim == 1:
-            r2_edges = np.ascontiguousarray(np.broadcast_to(r2_edges, (n_bins, len(r2_edges))))
-        if r2_edges.shape[0] != n_bins:
-            raise ValueError(f"r2_edges must have shape (n_bins={n_bins}, n_edges)")
+        pair_i, pair_j, r2_edges = _pairs_and_edges(pair_i, pair_j, r2_edges, n_bins)
         n_edges = r2_edges.shape[1]
         shape = self._shape(cat2, labels, len(pair_i), n_bins, n_edges)
         stats = _lib.YawbStats()
@@ -353,14 +354,8 @@ class Engine:
         stay on the device and the arrays returned are `None`.
         `labels`: as in `count`; each output gains the leading label axis of its own second catalog (e.g. a
         labelled unknown sample as `cat2a` with a shared, unbinned random catalog as `cat2b`)."""
-        pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
-        pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
-        r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
         n_bins = cat1a.n_bins
-        if r2_edges.ndim == 1:
-            r2_edges = np.ascontiguousarray(np.broadcast_to(r2_edges, (n_bins, len(r2_edges))))
-        if r2_edges.shape[0] != n_bins:
-            raise ValueError(f"r2_edges must have shape (n_bins={n_bins}, n_edges)")
+        pair_i, pair_j, r2_edges = _pairs_and_edges(pair_i, pair_j, r2_edges, n_bins)
         n_edges = r2_edges.shape[1]
         shapes = [self._shape(c2, labels, len(pair_i), n_bins, n_edges) for c2 in (cat2a, cat2a, cat2b, cat2b)]
         stats = _lib.YawbStats()
@@ -390,9 +385,7 @@ class Engine:
 
     def count_into_device(self, cat1, cat2, pair_i, pair_j, r2_edges, out_f64_ptr: int, out_i64_ptr: int):
         """Variant writing into caller-owned device buffers (raw pointers)."""
-        pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
-        pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
-        r2_edges = np.ascontiguousarray(r2_edges, dtype=np.float64)
+        pair_i, pair_j, r2_edges = _pairs_and_edges(pair_i, pair_j, r2_edges, cat1.n_bins)
         stats = _lib.YawbStats()
         _lib.check(
             self.lib.yawb_count(

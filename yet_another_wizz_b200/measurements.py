@@ -153,18 +153,11 @@ def prepare_catalog_arrays(catalog, binning: Binning | None, *, kappa: bool = Fa
     def fill(pid: int) -> None:
         ra, dec, weights, redshifts, kappa_vals = _patch_rows(catalog[pid])
         s, e = int(off[pid]), int(off[pid + 1])
-        if len(ra) != e - s:
-            raise InconsistentPatchesError(f"patch {pid} holds {len(ra)} rows, its meta data says {e - s}")
-        cos_dec = np.cos(dec)  # same operations, same order as coordinates.py:134-147
-        np.multiply(np.cos(ra), cos_dec, out=xyz[s:e, 0])
-        np.multiply(np.sin(ra), cos_dec, out=xyz[s:e, 1])
-        np.sin(dec, out=xyz[s:e, 2])
         if kappa:
             if kappa_vals is None:
                 raise ValueError("missing required 'kappa'")
-            ws[s:e] = kappa_vals if weights is None else kappa_vals * weights
-        elif has_w:
-            ws[s:e] = weights
+            weights = kappa_vals if weights is None else kappa_vals * weights
+        _fill_rows(xyz, ws, s, e, pid, ra, dec, weights)
         if zr is not None:
             zr[s:e] = redshifts
         elif binning is not None:
@@ -178,6 +171,19 @@ def prepare_catalog_arrays(catalog, binning: Binning | None, *, kappa: bool = Fa
     if zr is not None:
         out.update(redshifts=zr, edges=np.asarray(binning.edges, dtype=np.float64), closed=str(binning.closed))
     return out
+
+
+def _fill_rows(xyz, ws, s: int, e: int, pid: int, ra, dec, weights) -> None:
+    """rows `s:e` of the output arrays from the rows of patch `pid`: unit vectors with the reference's formula and, when
+    the catalog is weighted (`ws` is not None), the weights"""
+    if len(ra) != e - s:
+        raise InconsistentPatchesError(f"patch {pid} holds {len(ra)} rows, its meta data says {e - s}")
+    cos_dec = np.cos(dec)  # same operations, same order as coordinates.py:134-147
+    np.multiply(np.cos(ra), cos_dec, out=xyz[s:e, 0])
+    np.multiply(np.sin(ra), cos_dec, out=xyz[s:e, 1])
+    np.sin(dec, out=xyz[s:e, 2])
+    if ws is not None:
+        ws[s:e] = weights
 
 
 def _run_fill(fill, tasks, n_rows: int, workers: int | None) -> None:
@@ -234,14 +240,7 @@ def prepare_labelled_arrays(catalogs, binning: Binning | None = None, *, workers
         ra, dec, weights, redshifts, _ = _patch_rows(catalogs[label][pid])
         s = int(start[pid * len(catalogs) + label])
         e = s + int(sizes[label, pid])
-        if len(ra) != e - s:
-            raise InconsistentPatchesError(f"patch {pid} holds {len(ra)} rows, its meta data says {e - s}")
-        cos_dec = np.cos(dec)  # same operations, same order as prepare_catalog_arrays
-        np.multiply(np.cos(ra), cos_dec, out=xyz[s:e, 0])
-        np.multiply(np.sin(ra), cos_dec, out=xyz[s:e, 1])
-        np.sin(dec, out=xyz[s:e, 2])
-        if has_w:
-            ws[s:e] = weights
+        _fill_rows(xyz, ws, s, e, pid, ra, dec, weights)
         if binning is None:
             lab[s:e] = label
         else:
@@ -503,9 +502,8 @@ class PatchLinkage:
         uploads = self._uploads or _Uploads(engine)
 
         binning = _as_binning(self.config)
-        num_bins, num_patches = len(binning), len(main_catalog)
         plan = self._get_plan()
-        pair_i, pair_j = self.get_patch_id_pairs(auto=auto)
+        ij = self.get_patch_id_pairs(auto=auto)
         # the "k" side of a scalar-field count carries kappa x weight per row (trees.py:270-301)
         has1, has2 = _has_kappa(main_catalog), _has_kappa(second)
         if kappa1 and kappa2 and not (has1 and has2):
@@ -523,33 +521,13 @@ class PatchLinkage:
             sw1_all = (uploads.get(main_catalog, binning) if kappa1 else dev1).sum_weights()
             sw2_all = (uploads.get(second, bins2) if kappa2 else dev2).sum_weights()
 
-            own = self._own_pairs(shard, pair_i, pair_j, main_catalog, second)
-            hist_i, hist_f, stats = engine.count(dev1, dev2, pair_i[own], pair_j[own], plan.r2)
-            hist = hist_f if (dev1.weighted or dev2.weighted) else hist_i
-            hist = self._gather_shards(shard, hist, own, len(pair_i))
-            _last_stats[count_type_info or ("auto" if auto else "cross")] = stats
+            own = _own_pairs(shard, ij, main_catalog.get_num_records(), second.get_num_records(),
+                             main_catalog.get_radii().data)
+            hist = _count(engine, shard, count_type_info or ("auto" if auto else "cross"), dev1, dev2, ij, own, plan.r2)
         finally:
             if self._uploads is None:
                 uploads.free()
-        return self._package(hist, plan, binning, num_patches, pair_i, pair_j, sw1_all, sw2_all, auto)
-
-    @staticmethod
-    def _own_pairs(shard, pair_i, pair_j, cat1, cat2) -> np.ndarray:
-        """patch pairs counted by this rank (all of them without sharding)"""
-        if not shard.active:
-            return np.arange(len(pair_i))
-        costs = pair_costs(pair_i, pair_j, cat1.get_num_records(), cat2.get_num_records(),
-                           radii1=np.asarray(cat1.get_radii().data))
-        return assign_pairs_lpt(costs, shard.world_size)[shard.rank]
-
-    def _gather_shards(self, shard, hist: np.ndarray, own: np.ndarray, n_pairs: int) -> np.ndarray:
-        if not shard.active:
-            return hist
-        full = np.zeros((n_pairs, *hist.shape[1:]), dtype=hist.dtype)
-        full[own] = hist
-        engine = self.engine or get_default_engine()
-        device = getattr(engine, "device", None)
-        return shard.reduce_to_root(full, device=None if device is None else f"cuda:{device}")
+        return self._package(hist, plan, binning, len(main_catalog), *ij, sw1_all, sw2_all, auto)
 
     @staticmethod
     def _package(hist, plan, binning, num_patches, pair_i, pair_j, sw1_all, sw2_all, auto) -> list[NormalisedCounts]:
@@ -585,25 +563,20 @@ class PatchLinkage:
         shard = self.shard or current_shard()
         uploads = self._uploads or _Uploads(engine)
         binning = _as_binning(self.config)
-        num_patches = len(main_a)
         plan = self._get_plan()
-        pair_i, pair_j = self.get_patch_id_pairs(auto=False)
+        ij = self.get_patch_id_pairs(auto=False)
         try:
             dev_a, dev_b = uploads.get(main_a, binning), uploads.get(main_b, binning)
             dev2 = uploads.get(second, None)
             sw_a, sw_b, sw2 = dev_a.sum_weights(), dev_b.sum_weights(), dev2.sum_weights()
             larger = main_a if sum(main_a.get_num_records()) >= sum(main_b.get_num_records()) else main_b
-            own = self._own_pairs(shard, pair_i, pair_j, larger, second)
-            (ia, fa), (ib, fb), stats = engine.count2(dev_a, dev_b, dev2, pair_i[own], pair_j[own], plan.r2)
-            weighted = dev_a.weighted or dev_b.weighted or dev2.weighted
-            hist_a = self._gather_shards(shard, fa if weighted else ia, own, len(pair_i))
-            hist_b = self._gather_shards(shard, fb if weighted else ib, own, len(pair_i))
-            _last_stats["+".join(count_type_info)] = stats
+            own = _own_pairs(shard, ij, larger.get_num_records(), second.get_num_records(), larger.get_radii().data)
+            hist_a, hist_b = _count(engine, shard, "+".join(count_type_info), (dev_a, dev_b), dev2, ij, own, plan.r2)
         finally:
             if self._uploads is None:
                 uploads.free()
-        return (self._package(hist_a, plan, binning, num_patches, pair_i, pair_j, sw_a, sw2, False),
-                self._package(hist_b, plan, binning, num_patches, pair_i, pair_j, sw_b, sw2, False))
+        return (self._package(hist_a, plan, binning, len(main_a), *ij, sw_a, sw2, False),
+                self._package(hist_b, plan, binning, len(main_a), *ij, sw_b, sw2, False))
 
     def count_pairs_optional(self, main_catalog, *optional_catalog, **kwargs):
         if any(cat is None for cat in (main_catalog, *optional_catalog)):
@@ -630,6 +603,56 @@ class PatchLinkage:
                 self._uploads.free()
                 self._uploads = None
         return [NormalisedScalarCounts(kk.counts, nn.counts) for kk, nn in zip(counts[mode], counts["nn"])]
+
+
+# ---- the count step of every measurement --------------------------------------------------------------
+def _own_pairs(shard: Shard, ij, n1_per_patch, n2_per_patch, radii1) -> np.ndarray:
+    """rows of the pair list `ij = (pair_i, pair_j)` counted by this rank (all of them without sharding)"""
+    if not shard.active:
+        return np.arange(len(ij[0]))
+    costs = pair_costs(*ij, n1_per_patch, n2_per_patch, radii1=np.asarray(radii1))
+    return assign_pairs_lpt(costs, shard.world_size)[shard.rank]
+
+
+def _reduce(engine, shard: Shard, hist: np.ndarray, own: np.ndarray, n_pairs: int, *, labelled: bool) -> np.ndarray:
+    """the histograms of the pairs `own` placed into the full pair axis (behind the leading label axis if `labelled`)
+    and summed over the ranks"""
+    if not shard.active:
+        return hist
+    axis = 1 if labelled else 0
+    full = np.zeros((*hist.shape[:axis], n_pairs, *hist.shape[axis + 1:]), dtype=hist.dtype)
+    full[(slice(None),) * axis + (own,)] = hist
+    device = getattr(engine, "device", None)
+    return shard.reduce_to_root(full, device=None if device is None else f"cuda:{device}")
+
+
+def _count(engine, shard: Shard, tag: str, first, second, ij, own: np.ndarray, r2: np.ndarray, *,
+           swap: bool = False, labels: bool = False):
+    """`first` (a device catalog, or a tuple of two counted in one pass by `Engine.count2`) against `second` over the
+    rows `own` of the pair list `ij` (`swap`: `pair_i` and `pair_j` exchanged), statistics recorded under `tag`.
+    Returns the histogram of each first catalog, float if any catalog is weighted, summed over the ranks."""
+    pi, pj = ij[0][own], ij[1][own]
+    if swap:
+        pi, pj = pj, pi
+    kw = dict(labels=True) if labels else {}
+    fused = isinstance(first, tuple)
+    if fused:
+        *outs, stats = engine.count2(*first, second, pi, pj, r2, **kw)
+    else:
+        *out, stats = engine.count(first, second, pi, pj, r2, **kw)
+        outs = [out]
+    _last_stats[tag] = stats
+    weighted = any(c.weighted for c in (*(first if fused else (first,)), second))
+    labelled = labels or getattr(second, "n_labels", None) is not None  # a leading label axis
+    hists = [_reduce(engine, shard, out[1] if weighted else out[0], own, len(ij[0]), labelled=labelled) for out in outs]
+    return tuple(hists) if fused else hists[0]
+
+
+def _fuse(engine, reference, ref_rand) -> bool:
+    """whether the reference sample and its randoms are counted against a second catalog in one pass
+    (`Engine.count2`): they share patches, z-bins and thresholds, unless only one of them carries weights"""
+    return (ref_rand is not None and bool(reference.has_weights) == bool(ref_rand.has_weights)
+            and hasattr(engine, "count2"))
 
 
 def _has_kappa(catalog) -> bool:
@@ -691,11 +714,7 @@ def crosscorrelate(config, reference, unknown, *, ref_rand=None, unk_rand=None, 
         # `pipeline.count_cross_pipelined`)
         binning = _as_binning(config)
         links._uploads.enqueue(((reference, binning), (unknown, None), (ref_rand, binning), (unk_rand, None)))
-        # the reference sample and its randoms share patches, z-bins and thresholds: counted together against
-        # each unbinned catalog (one pass instead of two) unless only one of them carries weights
-        fuse = (ref_rand is not None and bool(reference.has_weights) == bool(ref_rand.has_weights)
-                and hasattr(links.engine or get_default_engine(), "count2") and os.environ.get("YAWB_FUSE", "1") != "0")
-        if fuse:
+        if _fuse(links.engine or get_default_engine(), reference, ref_rand):
             DD, RD = links.count_pairs_fused(reference, ref_rand, unknown, count_type_info=("DD", "RD"))
             if unk_rand is not None:
                 DR, RR = links.count_pairs_fused(reference, ref_rand, unk_rand, count_type_info=("DR", "RR"))
@@ -725,61 +744,31 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
     own linkage.  A shared `unk_rand` is counted once
     (DR and RR) for all bins.  Everything a per-bin call would raise is raised before any counting.
     `progress` / `max_workers` are accepted and ignored."""
-    unknowns = list(unknowns)
-    n_tomo = len(unknowns)
-    if n_tomo == 0:
-        raise ValueError("'unknowns' must hold at least one catalog")
-    if n_tomo > 254:
-        raise ValueError(f"at most 254 tomographic bins are supported (got {n_tomo})")
-    shared = unk_rand is not None and not isinstance(unk_rand, Sequence)
-    if unk_rand is None or shared:
-        rands = [unk_rand] * n_tomo
-    else:
-        rands = list(unk_rand)
-        if len(rands) != n_tomo:
-            raise ValueError(f"'unk_rand' holds {len(rands)} catalogs for {n_tomo} tomographic bins")
-        if any(r is None for r in rands):
-            raise ValueError("a per-bin 'unk_rand' must hold one catalog for every bin")
-    for unknown, rand in zip(unknowns, rands):
-        _ensure_unique_catalogs(reference, unknown, ref_rand, rand)
+    unknowns, rands, shared = _check_tomographic(unknowns, unk_rand, "unknowns", "unk_rand", (reference, ref_rand))
     if ref_rand is None and unk_rand is None:
         raise ValueError("at least one random dataset must be provided")
-    if len({bool(c.has_weights) for c in unknowns}) > 1:
-        raise ValueError("the tomographic bins must all have weights or all have none")
-    if not shared and unk_rand is not None and len({bool(c.has_weights) for c in rands}) > 1:
-        raise ValueError("the per-bin randoms must all have weights or all have none")
+    _check_tomographic_weights(unknowns, rands, shared)
     # the linkage of every bin, exactly as its own call would build it: the largest catalog decides the links
     links = [PatchLinkage.from_catalogs(config, reference, unknown, *[c for c in (ref_rand, rand) if c is not None],
                                         engine=engine, shard=shard) for unknown, rand in zip(unknowns, rands)]
     bin_pairs = [lk.get_patch_id_pairs(auto=False) for lk in links]
-    union_ij, bin_rows = _union_pairs(bin_pairs)
+    ij, bin_rows = _union_pairs(bin_pairs)
 
-    driver = links[0]
     eng = engine or get_default_engine()
     shard = shard or current_shard()
     binning = _as_binning(config)
-    plan = driver._get_plan()
+    plan = links[0]._get_plan()
     num_patches = len(reference)
     _last_stats.clear()
     uploads = _Uploads(eng)
 
-    own = np.arange(len(union_ij))
-    if shard.active:  # a pair's cost sums the rows of every bin
-        first = reference if ref_rand is None or sum(reference.get_num_records()) >= sum(ref_rand.get_num_records()) \
-            else ref_rand
-        n2 = np.sum([u.get_num_records() for u in unknowns], axis=0)
-        costs = pair_costs(union_ij[:, 0], union_ij[:, 1], first.get_num_records(), n2,
-                           radii1=np.asarray(first.get_radii().data))
-        own = assign_pairs_lpt(costs, shard.world_size)[shard.rank]
-    pi_own, pj_own = union_ij[own, 0], union_ij[own, 1]
-
-    def gather(hist):
-        """(L, own pairs, ...) -> (L, union pairs, ...) summed over the ranks: one reduce per count tensor"""
-        return np.moveaxis(driver._gather_shards(shard, np.moveaxis(hist, 1, 0), own, len(union_ij)), 0, 1)
-
-    fuse = (ref_rand is not None and bool(reference.has_weights) == bool(ref_rand.has_weights)
-            and hasattr(eng, "count2") and os.environ.get("YAWB_FUSE", "1") != "0")
-    hists: dict[str, np.ndarray] = {}
+    # a pair's cost sums the rows of every bin
+    first = reference if ref_rand is None or sum(reference.get_num_records()) >= sum(ref_rand.get_num_records()) \
+        else ref_rand
+    own = _own_pairs(shard, ij, first.get_num_records(), np.sum([u.get_num_records() for u in unknowns], axis=0),
+                     first.get_radii().data)
+    fuse = _fuse(eng, reference, ref_rand)
+    counts: dict[str, tuple] = {}
     try:
         uploads.enqueue(((reference, binning), (ref_rand, binning), (unk_rand if shared else None, None)))
         dev_ref = uploads.get(reference, binning)
@@ -788,50 +777,61 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
         dev_ur = None
         if unk_rand is not None:
             dev_ur = uploads.get(unk_rand, None) if shared else uploads.get_labelled(rands)
-        sw = dict(ref=dev_ref.sum_weights(), unk=dev_unk.sum_weights())
-        if dev_rr is not None:
-            sw["rr"] = dev_rr.sum_weights()
-        if dev_ur is not None:
-            sw["ur"] = dev_ur.sum_weights()
-        if fuse:
-            for second, kinds in ((dev_unk, ("DD", "RD")), (dev_ur, ("DR", "RR"))):
-                if second is None:
-                    continue
-                out_a, out_b, stats = eng.count2(dev_ref, dev_rr, second, pi_own, pj_own, plan.r2, labels=True)
-                weighted = dev_ref.weighted or dev_rr.weighted or second.weighted
-                hists[kinds[0]] = gather(out_a[1] if weighted else out_a[0])
-                hists[kinds[1]] = gather(out_b[1] if weighted else out_b[0])
-                _last_stats["+".join(kinds)] = stats
-        else:
-            for kind, dev1, dev2 in (("DD", dev_ref, dev_unk), ("RD", dev_rr, dev_unk), ("DR", dev_ref, dev_ur),
-                                     ("RR", dev_rr, dev_ur)):
-                if dev1 is None or dev2 is None:
-                    continue
-                hist_i, hist_f, stats = eng.count(dev1, dev2, pi_own, pj_own, plan.r2, labels=True)
-                hists[kind] = gather(hist_f if (dev1.weighted or dev2.weighted) else hist_i)
-                _last_stats[kind] = stats
+        # sums of weights with a leading label axis: (1, z-bins, patches) for the reference sample and its randoms,
+        # (labels, 1, patches) for the unknown side
+        sw_ref, sw_unk = dev_ref.sum_weights()[None], dev_unk.sum_weights()[:, None]
+        sw_rr = dev_rr.sum_weights()[None] if dev_rr is not None else None
+        sw_ur = dev_ur.sum_weights()[:, None] if dev_ur is not None else None
+        for second, sw2, kinds in ((dev_unk, sw_unk, ("DD", "RD")), (dev_ur, sw_ur, ("DR", "RR"))):
+            if second is None:
+                continue
+            if fuse:
+                hists = _count(eng, shard, "+".join(kinds), (dev_ref, dev_rr), second, ij, own, plan.r2, labels=True)
+            else:
+                hists = [None if dev1 is None else _count(eng, shard, kind, dev1, second, ij, own, plan.r2, labels=True)
+                         for kind, dev1 in zip(kinds, (dev_ref, dev_rr))]
+            counts.update((kind, (h, sw1, sw2)) for kind, h, sw1 in zip(kinds, hists, (sw_ref, sw_rr)) if h is not None)
     finally:
         uploads.free()
 
-    none = [None for _ in range(config.scales.num_scales)]
     result = []
-    for i, ((pi, pj), rows) in enumerate(zip(bin_pairs, bin_rows)):
-        def package(kind, sw1, sw2, label):
-            if kind not in hists:
-                return none
-            return PatchLinkage._package(hists[kind][label][rows], plan, binning, num_patches, pi, pj, sw[sw1],
-                                         sw[sw2][label:label + 1], False)
-
-        rand_label = 0 if shared else i
-        DD = package("DD", "ref", "unk", i)
-        RD = package("RD", "rr", "unk", i)
-        DR = package("DR", "ref", "ur", rand_label)
-        RR = package("RR", "rr", "ur", rand_label)
+    for i, (pairs, rows) in enumerate(zip(bin_pairs, bin_rows)):
+        DD, DR, RD, RR = (_package_bin(counts.get(kind), i, rows, pairs, False, plan, binning, num_patches)
+                          for kind in ("DD", "DR", "RD", "RR"))
         result.append([CorrFunc(dd, dr, rd, rr) for dd, dr, rd, rr in zip(DD, DR, RD, RR)])
     return result
 
 
-def _union_pairs(bin_pairs) -> tuple[np.ndarray, list[np.ndarray]]:
+def _check_tomographic(bins, rand, bins_name: str, rand_name: str, others=(), *, rand_required: bool = False
+                       ) -> tuple[list, list, bool]:
+    """`bins`: 1 to 254 catalogs; `rand`: None (unless `rand_required`), one catalog shared by every bin or one per
+    bin; no catalog twice among a bin, its randoms and `others`.  Returns (bins, randoms of every bin, shared)."""
+    bins = list(bins)
+    n_tomo = len(bins)
+    if n_tomo == 0:
+        raise ValueError(f"'{bins_name}' must hold at least one catalog")
+    if n_tomo > 254:
+        raise ValueError(f"at most 254 tomographic bins are supported (got {n_tomo})")
+    per_bin = isinstance(rand, Sequence)
+    rands = list(rand) if per_bin else [rand] * n_tomo
+    if len(rands) != n_tomo:
+        raise ValueError(f"'{rand_name}' holds {len(rands)} catalogs for {n_tomo} tomographic bins")
+    if (per_bin or rand_required) and any(r is None for r in rands):
+        raise ValueError(f"'{rand_name}' must hold a catalog for every bin")
+    for b, r in zip(bins, rands):
+        _ensure_unique_catalogs(*others, b, r)
+    return bins, rands, rand is not None and not per_bin
+
+
+def _check_tomographic_weights(bins, rands, shared: bool) -> None:
+    """the bins, and per-bin randoms, travel as one labelled catalog each: all with weights or all without"""
+    if len({bool(c.has_weights) for c in bins}) > 1:
+        raise ValueError("the tomographic bins must all have weights or all have none")
+    if not shared and rands[0] is not None and len({bool(c.has_weights) for c in rands}) > 1:
+        raise ValueError("the per-bin randoms must all have weights or all have none")
+
+
+def _union_pairs(bin_pairs) -> tuple[tuple[np.ndarray, np.ndarray], list[np.ndarray]]:
     """union of the bins' patch-pair lists (first appearance order) and, per bin, the rows of the union that make up
     its own list, in its order"""
     union: dict[tuple[int, int], int] = {}
@@ -840,7 +840,18 @@ def _union_pairs(bin_pairs) -> tuple[np.ndarray, list[np.ndarray]]:
             union.setdefault(pair, len(union))
     union_ij = np.array(list(union), dtype=np.int32).reshape(-1, 2)
     rows = [np.array([union[p] for p in zip(pi.tolist(), pj.tolist())], dtype=np.int64) for pi, pj in bin_pairs]
-    return union_ij, rows
+    return (union_ij[:, 0], union_ij[:, 1]), rows
+
+
+def _package_bin(count, i: int, rows: np.ndarray, pairs, auto: bool, plan, binning, num_patches: int
+                 ) -> list[NormalisedCounts | None]:
+    """bin `i`'s share of a count over the union of the bins' pair lists: `rows` of the union are its own `pairs`.
+    `count`: (histogram, sums of weights of the first and second catalog), each with a leading axis of one entry per
+    bin or one shared by every bin; None: a count not made."""
+    if count is None:
+        return [None] * plan.n_scales
+    hist, sw1, sw2 = (x[i if len(x) > 1 else 0] for x in count)
+    return PatchLinkage._package(hist[rows], plan, binning, num_patches, *pairs, sw1, sw2, auto)
 
 
 def autocorrelate_tomographic(config, data, random, *, count_rr: bool = True, progress: bool = False,
@@ -857,28 +868,13 @@ def autocorrelate_tomographic(config, data, random, *, count_rr: bool = True, pr
     Every count runs once over the union of the bins' patch-pair lists, and each bin is packaged from its own
     linkage.  Everything a per-bin call would raise is raised before any counting.  The labelled uploads stay in
     the engine's cache like single catalogs.  `progress` / `max_workers` are accepted and ignored."""
-    data = list(data)
+    data, rands, shared = _check_tomographic(data, random, "data", "random", rand_required=True)
     n_tomo = len(data)
-    if n_tomo == 0:
-        raise ValueError("'data' must hold at least one catalog")
-    if n_tomo > 254:
-        raise ValueError(f"at most 254 tomographic bins are supported (got {n_tomo})")
-    shared = not isinstance(random, Sequence)
-    rands = [random] * n_tomo if shared else list(random)
-    if len(rands) != n_tomo:
-        raise ValueError(f"'random' holds {len(rands)} catalogs for {n_tomo} tomographic bins")
-    if any(r is None for r in rands):
-        raise ValueError("'random' must hold a catalog for every bin")
-    for d, r in zip(data, rands):
-        _ensure_unique_catalogs(d, r)
     # the linkage of every bin, exactly as its own call would build it
     links = [PatchLinkage.from_catalogs(config, d, r, engine=engine, shard=shard) for d, r in zip(data, rands)]
     if not all(c.has_redshifts for c in (*data, *rands)):
         raise ValueError("patch has no 'redshifts' attached")
-    if len({bool(c.has_weights) for c in data}) > 1:
-        raise ValueError("the tomographic bins must all have weights or all have none")
-    if not shared and len({bool(c.has_weights) for c in rands}) > 1:
-        raise ValueError("the per-bin randoms must all have weights or all have none")
+    _check_tomographic_weights(data, rands, shared)
     binning = _as_binning(config)
     n_zbins = len(binning)
     if n_tomo * n_zbins > 4096:
@@ -889,73 +885,45 @@ def autocorrelate_tomographic(config, data, random, *, count_rr: bool = True, pr
     auto_ij, auto_rows = _union_pairs(auto_pairs)
     cross_ij, cross_rows = _union_pairs(cross_pairs)
 
-    driver = links[0]
     eng = engine or get_default_engine()
     shard = shard or current_shard()
-    plan = driver._get_plan()
+    plan = links[0]._get_plan()
     num_patches = len(data[0])
     _last_stats.clear()
     uploads = _Uploads(eng)
 
-    def own_pairs(ij, n1, n2):
-        if not shard.active:
-            return np.arange(len(ij))
-        costs = pair_costs(ij[:, 0], ij[:, 1], n1, n2, radii1=np.asarray(rands[0].get_radii().data))
-        return assign_pairs_lpt(costs, shard.world_size)[shard.rank]
-
     n_data = np.sum([d.get_num_records() for d in data], axis=0)
     n_rand = rands[0].get_num_records() if shared else np.sum([r.get_num_records() for r in rands], axis=0)
-    own_auto_dd = own_pairs(auto_ij, n_data, n_data)
-    own_cross = own_pairs(cross_ij, n_data, n_rand)
-    own_auto_rr = own_pairs(auto_ij, n_rand, n_rand)
+    radii = rands[0].get_radii().data
+    own_auto_dd = _own_pairs(shard, auto_ij, n_data, n_data, radii)
+    own_cross = _own_pairs(shard, cross_ij, n_data, n_rand, radii)
+    own_auto_rr = _own_pairs(shard, auto_ij, n_rand, n_rand, radii)
 
-    def gather(hist, own, n_pairs, labelled=True):
-        """(L, own pairs, ...) -> (L, union pairs, ...) summed over the ranks (unlabelled: no leading axis)"""
-        if not labelled:
-            return driver._gather_shards(shard, hist, own, n_pairs)
-        return np.moveaxis(driver._gather_shards(shard, np.moveaxis(hist, 1, 0), own, n_pairs), 0, 1)
-
-    def count(kind, dev1, dev2, ij, own, swap=False):
-        pi, pj = ij[own, 0], ij[own, 1]
-        hist_i, hist_f, stats = eng.count(dev1, dev2, pj if swap else pi, pi if swap else pj, plan.r2)
-        hist = hist_f if (dev1.weighted or dev2.weighted) else hist_i
-        _last_stats[kind] = stats
-        return gather(hist, own, len(ij), labelled=getattr(dev2, "n_labels", None) is not None)
-
-    hists: dict[str, np.ndarray] = {}
+    counts: dict[str, tuple] = {}
     try:
         dev_d = uploads.get_labelled(data, binning)
         dev_r = uploads.get(random, binning) if shared else uploads.get_labelled(rands, binning)
         sw_d = dev_d.sum_weights().reshape(n_tomo, n_zbins, num_patches)
         sw_r = dev_r.sum_weights().reshape(-1, n_zbins, num_patches)
-        hists["DD"] = count("DD", dev_d, dev_d, auto_ij, own_auto_dd)
+        dd = _count(eng, shard, "DD", dev_d, dev_d, auto_ij, own_auto_dd, plan.r2)
         if shared:  # the randoms as the first catalog, every bin's rows against their z-bin: pair lists swapped
-            hists["DR"] = count("DR", dev_r, dev_d, cross_ij, own_cross, swap=True)
+            dr = _count(eng, shard, "DR", dev_r, dev_d, cross_ij, own_cross, plan.r2, swap=True)
         else:
-            hists["DR"] = count("DR", dev_d, dev_r, cross_ij, own_cross)
+            dr = _count(eng, shard, "DR", dev_d, dev_r, cross_ij, own_cross, plan.r2)
+        counts.update(DD=(dd, sw_d, sw_d), DR=(dr, sw_d, sw_r))
         if count_rr:
-            rr = count("RR", dev_r, dev_r, auto_ij, own_auto_rr)
-            hists["RR"] = rr[None] if shared else rr
+            rr = _count(eng, shard, "RR", dev_r, dev_r, auto_ij, own_auto_rr, plan.r2)
+            counts["RR"] = (rr[None] if shared else rr, sw_r, sw_r)
     finally:
         uploads.free()
 
-    none = [None for _ in range(config.scales.num_scales)]
     result = []
     for i in range(n_tomo):
-        r = 0 if shared else i
-
-        def package(kind, rows, pairs, sw1, sw2, auto):
-            if kind not in hists:
-                return none
-            lab = r if kind == "RR" else i
-            return PatchLinkage._package(hists[kind][lab][rows], plan, binning, num_patches, *pairs, sw1, sw2, auto)
-
-        DD = package("DD", auto_rows[i], auto_pairs[i], sw_d[i], sw_d[i], True)
-        DR = package("DR", cross_rows[i], cross_pairs[i], sw_d[i], sw_r[r], False)
-        RR = package("RR", auto_rows[i], auto_pairs[i], sw_r[r], sw_r[r], True)
+        DD = _package_bin(counts["DD"], i, auto_rows[i], auto_pairs[i], True, plan, binning, num_patches)
+        DR = _package_bin(counts["DR"], i, cross_rows[i], cross_pairs[i], False, plan, binning, num_patches)
+        RR = _package_bin(counts.get("RR"), i, auto_rows[i], auto_pairs[i], True, plan, binning, num_patches)
         result.append([CorrFunc(dd, dr, None, rr) for dd, dr, rr in zip(DD, DR, RR)])
     return result
-
 
 # ---- scalar-field correlations (NK / KK) ----------------------------------------------------------------
 def compute_scalar_normalisation(catalog, binning: Binning, *, engine=None, uploads: "_Uploads | None" = None
