@@ -213,6 +213,105 @@ def pair_histogram(xyz1, xyz2, w1, w2, r2, *, use_c: bool | None = None):
     return hist
 
 
+def binned_pair_counts(
+    xyz1, patch1, zbin1, xyz2, patch2, pair_i, pair_j, r2, *,
+    w1=None, w2=None, zbin2=None, label1=None, label2=None, n_labels: int = 1,
+):
+    """
+    `pair_histogram` of every (patch pair, z-bin) of a pair list at once, for catalogs far too large for a brute
+    force per (pair, z-bin): the layout of `yawb_count`'s results, `(n_labels, n_pairs, n_bins, n_edges - 1)`.
+
+    Row a of the first catalog (patch `patch1[a]`, z-bin `zbin1[a]`; < 0 = dropped) meets row b of the second one
+    iff `zbin2` is None (unbinned) or `zbin2[b] == zbin1[a]`, and `label1` is None or `label1[a] == label2[b]`.
+    The pair goes to output block `label2[b]` (0 without labels; < 0 = dropped), patch pair k with
+    `(pair_i[k], pair_j[k]) == (patch1[a], patch2[b])`, z-bin `zbin1[a]`, and sub-bin k with
+    `r2[z][k-1] < d2 <= r2[z][k]` (`r2`: `(n_bins, n_edges)`).
+
+    A k-d tree only SELECTS candidate pairs, with the search radius of the device kernel
+    (`sqrt(max r2) (1 + 1e-9) + 1e-14`, far beyond the rounding of its own distances); every candidate is then
+    decided by the reference expression `(dx*dx + dy*dy) + dz*dz` in float64 and `searchsorted(..., "left")`, as in
+    `pair_histogram`.  Returns `(counts int64, sums float64)`: counts exact, sums of `w1[a] * w2[b]` correctly
+    rounded (`math.fsum` per entry; the counts as floats if neither catalog is weighted).
+    """
+    from scipy.spatial import cKDTree
+
+    xyz1 = np.ascontiguousarray(xyz1, dtype=np.float64).reshape(-1, 3)
+    xyz2 = np.ascontiguousarray(xyz2, dtype=np.float64).reshape(-1, 3)
+    r2 = np.atleast_2d(np.asarray(r2, dtype=np.float64))
+    n_bins, n_edges = r2.shape
+    nsub = n_edges - 1
+    pair_i = np.asarray(pair_i, dtype=np.int64)
+    pair_j = np.asarray(pair_j, dtype=np.int64)
+    n_pairs = len(pair_i)
+    patch1 = np.asarray(patch1, dtype=np.int64)
+    patch2 = np.asarray(patch2, dtype=np.int64)
+    zb1 = np.asarray(zbin1, dtype=np.int64)
+    lab2 = np.zeros(len(xyz2), dtype=np.int64) if label2 is None else np.asarray(label2, dtype=np.int64)
+    shape = (n_labels, n_pairs, n_bins, nsub)
+    counts = np.zeros(int(np.prod(shape)), dtype=np.int64)
+    weighted = w1 is not None or w2 is not None
+    sums = np.zeros(counts.shape, dtype=np.float64)
+    if n_pairs == 0 or len(xyz1) == 0 or len(xyz2) == 0:
+        return counts.reshape(shape), sums.reshape(shape)
+
+    n_patch = int(max(patch1.max(initial=0), patch2.max(initial=0), pair_i.max(), pair_j.max())) + 1
+    pair_of = np.full((n_patch, n_patch), -1, dtype=np.int64)
+    if len(set(zip(pair_i.tolist(), pair_j.tolist()))) != n_pairs:
+        raise ValueError("pair list has repeated patch pairs")
+    pair_of[pair_i, pair_j] = np.arange(n_pairs)
+
+    # rows that can meet share a group key: (z-bin if the second catalog is binned, label if the first is labelled)
+    live1 = (zb1 >= 0) & (zb1 < n_bins)
+    if label1 is not None:
+        live1 &= np.asarray(label1) >= 0
+    live2 = (lab2 >= 0) & (lab2 < n_labels)
+    g1 = np.zeros(len(xyz1), dtype=np.int64)
+    g2 = np.zeros(len(xyz2), dtype=np.int64)
+    if zbin2 is not None:
+        zb2 = np.asarray(zbin2, dtype=np.int64)
+        live2 &= zb2 >= 0
+        g1 = g1 * (n_bins + 1) + zb1
+        g2 = g2 * (n_bins + 1) + zb2
+    if label1 is not None:
+        g1 = g1 * (n_labels + 1) + np.asarray(label1, dtype=np.int64)
+        g2 = g2 * (n_labels + 1) + lab2
+    rmax = math.sqrt(float(r2[:, -1].max())) * (1.0 + 1e-9) + 1e-14
+
+    flat_all, prod_all = [], []
+    for g in np.intersect1d(g1[live1], g2[live2]):
+        ia = np.flatnonzero(live1 & (g1 == g))
+        ib = np.flatnonzero(live2 & (g2 == g))
+        cand = cKDTree(xyz1[ia]).sparse_distance_matrix(cKDTree(xyz2[ib]), rmax, output_type="coo_matrix")
+        a, b = ia[cand.row], ib[cand.col]
+        kp = pair_of[patch1[a], patch2[b]]
+        a, b, kp = a[kp >= 0], b[kp >= 0], kp[kp >= 0]
+        d = xyz1[a] - xyz2[b]
+        dx, dy, dz = d[:, 0], d[:, 1], d[:, 2]
+        d2 = (dx * dx + dy * dy) + dz * dz  # separate roundings, x -> y -> z
+        z = zb1[a]
+        k = np.zeros(len(a), dtype=np.int64)
+        for zz in np.unique(z):
+            m = z == zz
+            k[m] = np.searchsorted(r2[zz], d2[m], side="left")
+        keep = (k >= 1) & (k <= nsub)
+        a, b, kp, z, k = a[keep], b[keep], kp[keep], z[keep], k[keep]
+        flat = ((lab2[b] * n_pairs + kp) * n_bins + z) * nsub + (k - 1)
+        counts += np.bincount(flat, minlength=len(counts))
+        if weighted:
+            flat_all.append(flat)
+            prod_all.append((np.ones(len(a)) if w1 is None else np.asarray(w1)[a]) *
+                            (np.ones(len(b)) if w2 is None else np.asarray(w2)[b]))
+    if weighted and flat_all:
+        flat, prod = np.concatenate(flat_all), np.concatenate(prod_all)
+        order = np.argsort(flat, kind="stable")
+        flat, prod = flat[order], prod[order]
+        cells, start = np.unique(flat, return_index=True)
+        sums[cells] = [math.fsum(c) for c in np.split(prod, start[1:])]
+    elif not weighted:
+        sums = counts.astype(np.float64)
+    return counts.reshape(shape), sums.reshape(shape)
+
+
 def tree_count(
     xyz1, w1, xyz2, w2, ang_min, ang_max, *, weight_scale=None, weight_res=50, use_c=None
 ) -> np.ndarray:

@@ -245,3 +245,73 @@ def test_cpu_port_counts_equal_reference(name, workers):
             else:
                 assert_array_equal(got, want)
             assert want.sum() > 0
+
+
+def _brute_binned(xyz1, patch1, zbin1, xyz2, patch2, pairs, r2, w1, w2, zbin2=None, label1=None, label2=None,
+                  n_labels=1):
+    """`binned_pair_counts` spelled out: one `pair_histogram` per (label, patch pair, z-bin)"""
+    out_i = np.zeros((n_labels, len(pairs), r2.shape[0], r2.shape[1] - 1), dtype=np.int64)
+    out_f = np.zeros(out_i.shape)
+    lab2 = np.zeros(len(xyz2), dtype=int) if label2 is None else label2
+    for ell in range(n_labels):
+        for k, (i, j) in enumerate(pairs):
+            for b in range(r2.shape[0]):
+                m1 = (patch1 == i) & (zbin1 == b) & (True if label1 is None else label1 == ell)
+                m2 = (patch2 == j) & (lab2 == ell) & (True if zbin2 is None else zbin2 == b)
+                args = (xyz1[m1], xyz2[m2], None if w1 is None else w1[m1], None if w2 is None else w2[m2], r2[b])
+                out_i[ell, k, b] = oracle.pair_histogram(*args[:2], None, None, r2[b])
+                out_f[ell, k, b] = oracle.pair_histogram(*args)
+    return out_i, out_f
+
+
+@pytest.mark.parametrize("weights", ["none", "first", "second", "both"])
+@pytest.mark.parametrize("mode", ["unbinned", "binned", "labels", "binned_labels"])
+def test_binned_pair_counts_equal_pair_histogram(weights, mode):
+    """the k-d-tree-pruned oracle (`binned_pair_counts`) against `pair_histogram` per (label, patch pair, z-bin):
+    dropped rows, duplicated rows (d2 = 0 against a lower edge of 0), equal neighbouring edges, an empty z-bin
+    (hi == lo), thresholds that differ per z-bin, patch pairs that are not in the list"""
+    rng = np.random.default_rng(["none", "first", "second", "both"].index(weights) * 7 + len(mode))
+    n_patch, n_bins, n_labels = 3, 4, 3
+    n1, n2 = 900, 1100
+    def rows(n):
+        ra = rng.uniform(0.0, 0.06, n); dec = np.arcsin(rng.uniform(-0.02, 0.02, n))
+        return oracle.radec_to_xyz(ra, dec), np.minimum((ra / 0.02).astype(int), n_patch - 1)
+    xyz1, patch1 = rows(n1)
+    xyz2, patch2 = rows(n2)
+    xyz2[:150], patch2[:150] = xyz1[:150], patch1[:150]  # duplicates
+    zbin1 = rng.integers(-1, n_bins, n1)
+    zbin2 = rng.integers(-1, n_bins, n2) if mode in ("binned", "binned_labels") else None
+    label1 = rng.integers(0, n_labels, n1) if mode == "binned_labels" else None
+    label2 = rng.integers(-1, n_labels, n2) if mode in ("labels", "binned_labels") else None
+    w1 = rng.uniform(0.5, 1.5, n1) if weights in ("first", "both") else None
+    w2 = rng.uniform(0.5, 1.5, n2) if weights in ("second", "both") else None
+    r2 = oracle.chord_sq_edges(np.array([0.0, 1e-3, 2e-3, 2e-3, 4e-3, 6e-3]))
+    r2 = np.array([r2, r2 * 1.3, np.full(6, r2[3]), r2 * 0.7])
+    r2[1, 0] = 1e-7
+    pairs = [(0, 0), (0, 1), (1, 0), (1, 1), (2, 1), (1, 2), (2, 2)]  # (0, 2) and (2, 0) are not linked
+    pi, pj = np.array(pairs).T
+    L = n_labels if label2 is not None else 1
+    got_i, got_f = oracle.binned_pair_counts(xyz1, patch1, zbin1, xyz2, patch2, pi, pj, r2, w1=w1, w2=w2,
+                                             zbin2=zbin2, label1=label1, label2=label2, n_labels=L)
+    want_i, want_f = _brute_binned(xyz1, patch1, zbin1, xyz2, patch2, pairs, r2, w1, w2, zbin2, label1, label2, L)
+    assert_array_equal(got_i, want_i)
+    assert_allclose(got_f, want_f, rtol=1e-13, atol=0)  # pair_histogram sums in plain order
+    assert want_i.sum() > 1000 and not want_i[:, :, 2].any()
+
+
+@pytest.mark.parametrize("weights", ["none", "both"])
+def test_binned_pair_counts_on_edge_adversarial(weights):
+    """rows within a few ulp of the bin edges: the pruned oracle decides them as `pair_histogram` does"""
+    g = golden_io.load("edge_adversarial")
+    a, b = g["a_xyz"], g["b_xyz"]
+    rng = np.random.default_rng(8)
+    w1 = rng.uniform(0.5, 1.5, len(a)) if weights == "both" else None
+    w2 = rng.uniform(0.5, 1.5, len(b)) if weights == "both" else None
+    for key in ("upper", "lower", "multi"):
+        lim = oracle.parse_ang_limits(g[f"{key}_ang_min"], g[f"{key}_ang_max"])
+        r2 = oracle.chord_sq_edges(oracle.get_ang_bins(lim, None, 50))
+        got_i, got_f = oracle.binned_pair_counts(a, np.zeros(len(a)), np.zeros(len(a)), b, np.zeros(len(b)), [0], [0],
+                                                 r2, w1=w1, w2=w2)
+        assert_array_equal(got_i[0, 0, 0], oracle.pair_histogram(a, b, None, None, r2))
+        assert_allclose(got_f[0, 0, 0], oracle.pair_histogram(a, b, w1, w2, r2), rtol=1e-14, atol=0)
+        assert got_i.sum() > 0
