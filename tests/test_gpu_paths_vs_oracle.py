@@ -3,8 +3,8 @@ The pair-count kernels against the host oracle, at every place where `yawb_launc
 switches to other code or other constants: the five kernel paths and where their accumulators live, the group size of
 the cumulative path, sub-bin counts up to `YAWB_MAX_EDGES`, z-bin counts around the 32 lanes of a warp, small and
 large jobs (items of `CCAP_SMALL` or `CCAP` cell-row runs) with the row-range split of the planner, weights on either
-side, per-bin thresholds with lower edges of 0, equal edges and empty z-bins, extreme geometry, short tiles, the three
-kinds of z-bin upload, both kinds of labels, and the two rejections.
+side, per-bin thresholds with lower edges of 0, equal edges and empty z-bins, extreme geometry, short tiles and tiles cut
+by the straggler guard, the three kinds of z-bin upload, both kinds of labels, and the two rejections.
 
 Every result is compared with `oracle.binned_pair_counts` (the reference expression in float64 on k-d-tree candidates),
 never with another device kernel: the exact kernel `k_count_exact` reads the same index data as the streaming one, so
@@ -168,6 +168,7 @@ PATH_CASES = [
     ("histw-e6-both-count2-B16-global", 6, 16, "both", 2, True),
     ("histw-e34-both-B1", 34, 1, "both", 1, False),
     ("histw-e256-second-B2", 256, 2, "second", 1, False),
+    ("singlew-first-count2-binned", 2, 5, "first", 2, True),
 ]
 
 
@@ -211,6 +212,8 @@ def _path_catalogs(rng, n_bins, weights, n_types, binned2):
         patch = np.minimum((r / 0.01).astype(int), n_patch - 1)
         z = rng.integers(0, n_bins, n)
         z[rng.random(n) < 0.05] = -1
+        if w:  # 400 rows at one position in one z-bin: one sort key, whose rows the index stores in any order
+            xyz[1000:1400], patch[1000:1400], z[1000:1400] = xyz[1000].copy(), patch[1000], 0
         return xyz, patch, z, rng.uniform(0.5, 1.5, n) if w else None
 
     firsts = []
@@ -347,7 +350,8 @@ def test_large_job_with_row_split(engine, n_edges, weights):
 
 
 # --------------------------------------------------------------------------------------------------------------------
-# 3. geometry: pole, RA = 0, a patch of more than 90 degrees, very large and very small angles, short tiles
+# 3. geometry: pole, RA = 0, a patch of more than 90 degrees, very large and very small angles, short tiles, hollow
+# patches, and a strip among thousands of patches
 # --------------------------------------------------------------------------------------------------------------------
 def _geometry(rng, name):
     """(first catalog, second catalog, n_patch, (theta_lo, theta_hi) in radian)"""
@@ -385,6 +389,24 @@ def _geometry(rng, name):
         p2 = np.repeat(np.arange(5), sizes2)
         p1 = np.repeat(np.arange(5), sizes1)
         return Rows(x1, p1, 5), Rows(x2, p2, 5), 5, (5e-4, 6e-3)
+    if name == "irregular":  # a ring and an L: the Hilbert curve of a patch box crosses empty parts of the patch
+        def cat(n):
+            r, phi = np.sqrt(rng.uniform(0.012**2, 0.02**2, n)), rng.uniform(0.0, 2.0 * np.pi, n)
+            u, v = rng.uniform(0.0, 0.04, 4 * n), rng.uniform(0.0, 0.04, 4 * n)
+            keep = (u < 0.008) | (v < 0.008)
+            ra = np.concatenate([0.05 + r * np.cos(phi), 0.08 + u[keep][:n]])
+            dec = np.concatenate([r * np.sin(phi), -0.02 + v[keep][:n]])
+            return oracle.radec_to_xyz(ra, dec), np.repeat([0, 1], n)
+        (x1, p1), (x2, p2) = cat(6000), cat(10000)
+        return Rows(x1, p1, 2), Rows(x2, p2, 2), 2, (2e-4, 1e-3)
+    if name == "strip":  # 5000 patches, all but two empty: 5000 x 16 > 2^16 Hilbert cells leave one level of the curve
+        # (two key bits) below each (patch, z-bin), and patch 0 is a 6 : 1 strip, wide enough for more than 4 squares
+        def cat(n_strip, n_box):
+            xs = sky(rng, n_strip, (0.0, 0.06), (-0.005, 0.005))[0]
+            xb = sky(rng, n_box, (0.1, 0.11), (-0.005, 0.005))[0]
+            return np.concatenate([xs, xb]), np.repeat([0, 1], [n_strip, n_box])
+        (x1, p1), (x2, p2) = cat(3000, 500), cat(4000, 600)
+        return Rows(x1, p1, 5000), Rows(x2, p2, 5000), 5000, (2e-4, 3e-3)
     if name == "off-sphere":  # rows 1e-6 off the unit sphere: the FP32 test widens its undecided band by that much
         def cat(n, dev):
             xyz, r, _ = sky(rng, n, (0.0, 0.02), (-0.01, 0.01))
@@ -394,7 +416,17 @@ def _geometry(rng, name):
     raise ValueError(name)
 
 
-GEOMETRIES = ["pole", "ra0", "wide100", "wide150", "wide179", "tiny", "tiles", "off-sphere"]
+GEOMETRIES = ["pole", "ra0", "wide100", "wide150", "wide179", "tiny", "tiles", "off-sphere", "irregular", "strip"]
+
+
+def second_role_index_bytes(engine, rows: Rows) -> int:
+    """device bytes that the second-role index of the unbinned catalog `rows` adds to it"""
+    dev = rows.upload(engine)
+    before = dev.info()[1]
+    dev.build_index(2)  # YAWB_ROLE_SECOND
+    extra = dev.info()[1] - before
+    dev.free()
+    return extra
 
 
 @pytest.mark.parametrize("name", GEOMETRIES)
@@ -404,7 +436,11 @@ def test_geometry_against_oracle(engine, name):
     n_bins = 3
     r1.zbin = rng.integers(0, n_bins, len(r1.xyz))
     r2.w = rng.uniform(0.5, 1.5, len(r2.xyz))
-    pi, pj = all_pairs(n_patch)
+    if name == "irregular":  # the straggler guard cut tiles: more tiles than for as many rows per patch in compact patches
+        compact = Rows(sky(rng, len(r2.xyz), (0.0, 0.04), (-0.02, 0.02))[0], r2.patch, n_patch, w=r2.w)
+        assert second_role_index_bytes(engine, r2) > second_role_index_bytes(engine, compact)
+    live = np.flatnonzero(np.diff(r1.off) * np.diff(r2.off))  # patches with rows in both catalogs
+    pi, pj = (live[k].astype(np.int32) for k in all_pairs(len(live)))
     d1 = r1.upload(engine, n_bins)
     plain, weighted = Rows(r2.xyz, r2.patch, n_patch), r2
     for n_edges, second in ((2, plain), (5, plain), (12, plain), (2, weighted), (9, weighted)):

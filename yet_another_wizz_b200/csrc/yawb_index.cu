@@ -3,7 +3,7 @@
 // Replaces the reference's tree build (src/yaw/catalog/trees.py:365-429,
 // BinnedTrees.build :483-545, Catalog.build_trees catalog.py:1406-1460): instead of
 // one pickled cKDTree per (patch, z-bin) the rows stay resident in HBM in two sort
-// orders, each built with one key kernel + one radix sort + one gather:
+// orders, each built by a counting sort (one histogram pass, one scan, one scatter pass):
 //
 //   first role  (cat1 of yawb_count): rows sorted by global sky-cell id
 //               (patch, z-bin, row-major cell of a per-patch tangent-plane grid),
@@ -13,8 +13,6 @@
 //
 // Everything here is HBM-bound streaming work: coalesced SoA double arrays, one pass
 // per step, grids sized from the row count.
-#include <cub/device/device_radix_sort.cuh>
-
 #include <algorithm>
 #include <cmath>
 #include <cstring>
@@ -26,6 +24,7 @@ namespace {
 constexpr int kThreads = 256;
 constexpr double kTargetPerCell = 5.5;  // rows per sky cell and z-bin the grid is sized for
 constexpr long long kMaxCellsPerPatchBin = 1ll << 24;
+constexpr long long kMaxGridCells = 1ll << 30;  // sky cells of a first-role index, all patches and z-bins
 constexpr double kCellAspect = 4.0;  // cell height / cell width
 
 inline int blocks_for(int64_t n, int per_block = kThreads) {
@@ -380,21 +379,6 @@ __device__ __forceinline__ long long key_first(double X, double Y, double Z, int
     return g.cell_base + ((long long)b * g.gv + iv) * g.gu + iu;
 }
 
-template <typename K>
-__global__ void k_keys_first(const double *__restrict__ x, const double *__restrict__ y,
-                             const double *__restrict__ z, const int *__restrict__ bin,
-                             const int *__restrict__ patch, long long n, int n_bins,
-                             const PatchFrame *__restrict__ frames, const SGrid *__restrict__ grids,
-                             K *__restrict__ keys, unsigned *__restrict__ vals, long long off) {
-    long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    keys += off;  // rows of the second catalog of a fused index follow those of the first
-    vals += off;
-    vals[i] = (unsigned)(off + i);
-    const long long key = key_first(x[3 * i], y[3 * i], z[3 * i], bin ? bin[i] : 0, patch[i], n_bins, frames, grids);
-    keys[i] = key < 0 ? (K)~(K)0 : (K)key;
-}
-
 // Hilbert index of a cell on a 65536 x 65536 grid.  Unlike the Morton (Z) curve the Hilbert curve has
 // no jumps: consecutive cells are always neighbours, so every run of YAWB_TILE consecutive rows is a
 // compact clump and no register tile straddles a quadrant boundary with a patch-sized bounding box.
@@ -429,7 +413,8 @@ __device__ __forceinline__ unsigned hilbert16(unsigned x, unsigned y, int levels
 // the cells -- hence the tiles -- stay close to square instead of being stretched k : 1 (a 4 : 1 strip in one
 // square: every tile trips the straggler guard and is cut into 32-row sub-tiles).  Below 2 : 1 a single
 // stretched square is better (C3's 5 x 3 degree patches: 3.6 % fewer executed tests than with two squares).
-// The square index takes its bits from the Hilbert resolution.
+// The square index takes its bits from the Hilbert resolution: a key of hbits = 2 bits below the (patch, z-bin)
+// segment has room for at most 4 squares (with more, the rows of squares 4-7 would carry the key of the next segment).
 struct HMap {
     double c[3], e_long[3], e_short[3];  // centre of the patch; tangent axes along the long / short side of the box
     double o_long, o_short;              // lower edge of the box along the two axes
@@ -444,7 +429,7 @@ __global__ void k_hilbert_map(const PatchFrame *__restrict__ frames, int n_patch
     const double du = f.umax - f.umin, dv = f.vmax - f.vmin;
     const bool swap = dv > du;  // the long axis is the x of the curve (which runs from (0, 0) to (max, 0))
     const double lng = swap ? dv : du, sht = swap ? du : dv;
-    const int k = sht > 0.0 && lng >= 2.0 * sht ? min((int)rint(lng / sht), 8) : 1;
+    const int k = sht > 0.0 && lng >= 2.0 * sht ? min((int)rint(lng / sht), hbits >= 3 ? 8 : 1 << hbits) : 1;
     const int kb = k > 4 ? 3 : k > 2 ? 2 : k > 1 ? 1 : 0;  // bits of the square index
     HMap m;
     for (int d = 0; d < 3; ++d) {
@@ -478,27 +463,15 @@ __device__ __forceinline__ long long key_second(double X, double Y, double Z, in
     return (long long)(((unsigned long long)((long long)p * n_bins + b) << hbits) | ((unsigned long long)sq << (2 * levels)) | h);
 }
 
-template <typename K>
-__global__ void k_keys_second(const double *__restrict__ x, const double *__restrict__ y,
-                              const double *__restrict__ z, const int *__restrict__ bin,
-                              const int *__restrict__ patch, long long n, int n_bins, int hbits,
-                              const HMap *__restrict__ maps, K *__restrict__ keys,
-                              unsigned *__restrict__ vals) {
-    long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    vals[i] = (unsigned)i;
-    const long long key = key_second(x[3 * i], y[3 * i], z[3 * i], bin ? bin[i] : 0, patch[i], n_bins, hbits, maps);
-    keys[i] = key < 0 ? (K)~(K)0 : (K)key;
-}
-
 // ---- counting sort ------------------------------------------------------------------------------------
 // The sort keys are bounded and dense (sky-cell ids, (patch, z-bin, Hilbert cell) ids: about as many keys as rows),
 // so the rows are put in order by ONE histogram pass that also hands every row its rank among the rows of its
 // key (the value the atomic returns), an in-place exclusive scan of the key counts, and ONE scatter pass without
 // atomics: position = first slot of the key + rank.  (key, rank) of a row travel from the first pass to the second
 // in an 8-byte side array, so the second pass neither walks the curve again nor waits for an atomic.  The order of
-// rows with the same key is arbitrary (it has no meaning: pair counts are sums over all rows of a cell).  After the
-// scan cur[k] is the first slot of key k, i.e. the cell_start table of a first-role index (entry n_keys = row count).
+// rows with the same key is arbitrary (it has no meaning: pair counts are sums over all rows of a cell, and the
+// count kernel adds weighted sums in an order that its warps settle at run time anyway).  After the scan cur[k] is
+// the first slot of key k, i.e. the cell_start table of a first-role index (entry n_keys = row count).
 __global__ void k_hist_first(const double *__restrict__ x, const double *__restrict__ y, const double *__restrict__ z,
                              const int *__restrict__ bin, const int *__restrict__ patch, long long n, int n_bins,
                              const PatchFrame *__restrict__ frames, const SGrid *__restrict__ grids,
@@ -662,67 +635,6 @@ __global__ void k_scatter_first(const double *__restrict__ x, const double *__re
     orec[pos] = r;
 }
 
-__global__ void k_gather(const unsigned *__restrict__ perm, long long n, const double *__restrict__ x,
-                         const double *__restrict__ y, const double *__restrict__ z,
-                         const double *__restrict__ w, double *__restrict__ ox, double *__restrict__ oy,
-                         double *__restrict__ oz, double *__restrict__ ow) {
-    long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    unsigned j = perm[i];
-    double2 *const o = reinterpret_cast<double2 *>(ox + (size_t)YAWB_RSTRIDE * i);
-    o[0] = make_double2(x[3 * (size_t)j], y[3 * (size_t)j]);
-    o[1] = make_double2(z[3 * (size_t)j], 0.0);
-    if (w) ow[i] = w[j];
-}
-
-// first-role gather (rows of one catalog, or of two for a fused index): the exact rows in sorted order plus
-// their fixed-point record in the frame of the patch (SGrid: origin and power-of-two scale)
-__global__ void k_gather_rec(const unsigned *__restrict__ perm, long long n, long long n_a,
-                             const double *__restrict__ ax, const double *__restrict__ ay, const double *__restrict__ az,
-                             const double *__restrict__ aw, const int *__restrict__ apatch,
-                             const double *__restrict__ bx, const double *__restrict__ by, const double *__restrict__ bz,
-                             const double *__restrict__ bw, const int *__restrict__ bpatch,
-                             const PatchFrame *__restrict__ frames, const SGrid *__restrict__ grids,
-                             double *__restrict__ ow, SRec *__restrict__ orec) {
-    long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    long long j = perm[i];
-    const bool second = j >= n_a;
-    if (second) j -= n_a;
-    const double X = second ? bx[3 * j] : ax[3 * j], Y = second ? by[3 * j] : ay[3 * j], Z = second ? bz[3 * j] : az[3 * j];
-    if (ow) {
-        const double *w = second ? bw : aw;
-        ow[i] = w ? w[j] : 1.0;  // fused index of a weighted and an unweighted catalog
-    }
-    const int p = second ? bpatch[j] : apatch[j];
-    const PatchFrame &f = frames[p];
-    const SGrid &g = grids[p];
-    const double dx = X - f.c[0], dy = Y - f.c[1], dz = Z - f.c[2];
-    const double u = dx * f.e1[0] + dy * f.e1[1] + dz * f.e1[2];
-    const double v = dx * f.e2[0] + dy * f.e2[1] + dz * f.e2[2];
-    const double t = dx * f.c[0] + dy * f.c[1] + dz * f.c[2];
-    SRec r;
-    r.ku = (int)fmin(fmax(rint((u - g.u0) * g.qscale), 0.0), 2147483647.0);
-    r.kv = (int)fmin(fmax(rint((v - g.v0) * g.qscale), 0.0), 2147483647.0);
-    r.kt = (int)fmin(fmax(rint((t - g.t0) * g.qscale), 0.0), 2147483647.0);
-    r.aux = (unsigned)j | (second ? 0x80000000u : 0u);  // row of its catalog | catalog bit
-    orec[i] = r;
-}
-
-// cell_start[g] = first sorted row whose key is >= g (one thread per cell, binary search)
-template <typename K>
-__global__ void k_cell_start(const K *__restrict__ keys, long long n, long long n_cells,
-                             int *__restrict__ cell_start) {
-    long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (g > n_cells) return;
-    long long lo = 0, hi = n;
-    while (lo < hi) {
-        long long mid = (lo + hi) >> 1;
-        if ((unsigned long long)keys[mid] < (unsigned long long)g) lo = mid + 1; else hi = mid;
-    }
-    cell_start[g] = (int)lo;
-}
-
 // bounding sphere of each register tile, and its bounding box in the frame of its own patch: one warp per tile
 __global__ void k_tile_spheres(const double *__restrict__ x, const double *__restrict__ y,
                                const double *__restrict__ z, Tile *__restrict__ tiles, int n_tiles,
@@ -827,25 +739,6 @@ __global__ void k_count_oversized(const Tile *__restrict__ tiles, int n_tiles, c
     if (t < n_tiles && tiles[t].count > 32 && tiles[t].rad > thr[tiles[t].patch]) atomicAdd(n_big, 1u);
 }
 
-template <typename K>
-int sort_pairs(yawb_ctx *ctx, Scratch &scr, K *keys_in, K *keys_out, unsigned *vals_in, unsigned *vals_out,
-               long long n, int end_bit) {
-    size_t temp_bytes = 0;
-    YAWB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, keys_in, keys_out, vals_in, vals_out,
-                                              (int)n, 0, end_bit, ctx->stream));
-    void *temp = scr.get<unsigned char>(std::max<size_t>(temp_bytes, 16));
-    YAWB_REQUIRE(temp != nullptr, "out of device memory (radix sort scratch)");
-    YAWB_CUDA(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys_in, keys_out, vals_in, vals_out, (int)n, 0,
-                                              end_bit, ctx->stream));
-    return 0;
-}
-
-int bits_for(unsigned long long max_key) {
-    int b = 1;
-    while (b < 64 && (max_key >> b)) ++b;
-    return b;
-}
-
 template <typename T>
 int fi_alloc(FIndex *fi, T **ptr, size_t count) {
     *ptr = nullptr;
@@ -864,9 +757,6 @@ int exclusive_scan_inplace(yawb_ctx *ctx, Scratch &scr, int *cur, long long n) {
     k_scan_lookback<<<n_blocks, kThreads, 0, ctx->stream>>>(cur, n, desc);
     return 0;
 }
-
-// keys up to this many go through the counting sort (one int per key); beyond, the radix sort
-constexpr long long kCountingSortMaxKeys = 1ll << 30;
 
 // first-role rows in sky-cell order by counting sort; fills cell_start (base + 1 entries)
 int build_first_counting(FIndex *fi, long long base) {
@@ -912,61 +802,20 @@ int build_second_counting(yawb_cat *cat, int hbits, long long n_keys) {
     return 0;
 }
 
-template <typename K>
-int build_first_sorted(FIndex *fi, long long base) {
-    yawb_ctx *ctx = fi->ctx;
-    cudaStream_t st = ctx->stream;
-    const yawb_cat *a = fi->a, *b = fi->b;
-    const long long na_in = a->n_in, nb_in = b ? b->n_in : 0, n_in = na_in + nb_in, n = fi->n;
-    Scratch scr(ctx, st);
-    const size_t nn = std::max<long long>(n_in, 1);
-    K *k0 = scr.get<K>(nn), *k1 = scr.get<K>(nn);
-    unsigned *v0 = scr.get<unsigned>(nn), *v1 = scr.get<unsigned>(nn);
-    YAWB_REQUIRE(k0 && k1 && v0 && v1, "out of device memory (sort buffers)");
-    if (n_in > 0) {
-        if (na_in > 0)
-            k_keys_first<K><<<blocks_for(na_in), kThreads, 0, st>>>(a->x, a->y, a->z, a->bin, a->patch, na_in, fi->n_bins,
-                                                                    fi->d_frames, fi->d_sgrid, k0, v0, 0);
-        if (nb_in > 0)
-            k_keys_first<K><<<blocks_for(nb_in), kThreads, 0, st>>>(b->x, b->y, b->z, b->bin, b->patch, nb_in, fi->n_bins,
-                                                                    fi->d_frames, fi->d_sgrid, k0, v0, na_in);
-        // dropped rows carry the all-ones key: sort every bit only if something was dropped
-        const int end_bit = (n == n_in) ? bits_for((unsigned long long)std::max<long long>(base, 1)) : (int)(8 * sizeof(K));
-        if (sort_pairs<K>(ctx, scr, k0, k1, v0, v1, n_in, end_bit)) return 1;
+// cells of edge c in a first-role grid of a patch box du x dv, grown by 1.5 until a z-bin has at most
+// kMaxCellsPerPatchBin cells and a cell row at most 32767
+void size_cells(SGrid &g, double du, double dv, double c) {
+    auto dims = [&]() {
+        g.inv_cv = 1.0 / c;
+        g.inv_cu = kCellAspect / c;
+        g.gu = std::max(1, (int)std::floor(du * g.inv_cu) + 1);
+        g.gv = std::max(1, (int)std::floor(dv * g.inv_cv) + 1);
+    };
+    dims();
+    while ((long long)g.gu * g.gv > kMaxCellsPerPatchBin || g.gu > 32767) {
+        c *= 1.5;
+        dims();
     }
-    if (n > 0)
-        k_gather_rec<<<blocks_for(n), kThreads, 0, st>>>(v1, n, na_in, a->x, a->y, a->z, a->w, a->patch, b ? b->x : nullptr,
-                                                         b ? b->y : nullptr, b ? b->z : nullptr, b ? b->w : nullptr,
-                                                         b ? b->patch : nullptr, fi->d_frames, fi->d_sgrid, fi->sw, fi->rec);
-    k_cell_start<K><<<blocks_for(base + 1), kThreads, 0, st>>>(k1, n, base, fi->cell_start);
-    return 0;
-}
-
-template <typename K>
-int build_second_sorted(yawb_cat *cat, int hbits) {
-    yawb_ctx *ctx = cat->ctx;
-    cudaStream_t st = ctx->stream;
-    const long long n_in = cat->n_in, n = cat->n;
-    const int P = cat->n_patch, B = cat->n_bins;
-    Scratch scr(ctx, st);
-    const size_t nn = std::max<long long>(n_in, 1);
-    K *k0 = scr.get<K>(nn), *k1 = scr.get<K>(nn);
-    unsigned *v0 = scr.get<unsigned>(nn), *v1 = scr.get<unsigned>(nn);
-    YAWB_REQUIRE(k0 && k1 && v0 && v1, "out of device memory (sort buffers)");
-    if (n_in > 0) {
-        HMap *maps = scr.get<HMap>((size_t)P);
-        YAWB_REQUIRE(maps != nullptr, "out of device memory (sort buffers)");
-        k_hilbert_map<<<(P + 127) / 128, 128, 0, st>>>(cat->d_frames, P, hbits, maps);
-        k_keys_second<K><<<blocks_for(n_in), kThreads, 0, st>>>(cat->x, cat->y, cat->z, cat->bin, cat->patch, n_in, B,
-                                                                hbits, maps, k0, v0);
-        const int end_bit = (n == n_in) ? hbits + bits_for((unsigned long long)std::max<long long>((long long)P * B, 1))
-                                        : (int)(8 * sizeof(K));
-        if (sort_pairs<K>(ctx, scr, k0, k1, v0, v1, n_in, std::min(end_bit, (int)(8 * sizeof(K))))) return 1;
-    }
-    if (n > 0)
-        k_gather<<<blocks_for(n), kThreads, 0, st>>>(v1, n, cat->x, cat->y, cat->z, cat->w, cat->rx, cat->ry,
-                                                     cat->rz, cat->rw);
-    return 0;
 }
 
 }  // namespace
@@ -1200,6 +1049,7 @@ static int findex_build(yawb_ctx *ctx, yawb_cat *a, yawb_cat *b, FIndex **out) {
 
     // grid per patch: cell edge from the mean density of one z-bin of this patch; fixed-point scale of the rows
     fi->h_sgrid.assign(P, SGrid{});
+    std::vector<double> edge(P);  // cell edge of every patch before the bound on the whole grid below
     long long base = 0;
     for (int p = 0; p < P; ++p) {
         const PatchFrame &f = fi->h_frames[p];
@@ -1215,20 +1065,11 @@ static int findex_build(yawb_ctx *ctx, yawb_cat *a, yawb_cat *b, FIndex **out) {
         double span = std::max(du, dv);
         if (!(c > 0.0) || span <= 0.0) c = 1.0;
         c = std::max(c, span / 2048.0);  // bound the grid, <= 8192 x 2048 cells
+        edge[p] = c;
         SGrid &g = fi->h_sgrid[p];
         g.u0 = f.umin;
         g.v0 = f.vmin;
-        auto dims = [&]() {
-            g.inv_cv = 1.0 / c;
-            g.inv_cu = kCellAspect / c;
-            g.gu = std::max(1, (int)std::floor(du * g.inv_cu) + 1);
-            g.gv = std::max(1, (int)std::floor(dv * g.inv_cv) + 1);
-        };
-        dims();
-        while ((long long)g.gu * g.gv > kMaxCellsPerPatchBin || g.gu > 32767) {
-            c *= 1.5;
-            dims();
-        }
+        size_cells(g, du, dv, c);
         g.cell_base = base;
         base += (long long)B * g.gu * g.gv;
         // t = (P - c).c = -chord^2 / 2 lies in [-radius^2 / 2, 0]; one power-of-two scale for (u, v, t)
@@ -1240,25 +1081,26 @@ static int findex_build(yawb_ctx *ctx, yawb_cat *a, yawb_cat *b, FIndex **out) {
         g.qscale = std::ldexp(1.0, m);
         g.qinv = std::ldexp(1.0, -m);
     }
-    fi->n_cells = base;
-    if (base >= (1ll << 40)) {
-        yawb_set_error("sky-cell index too large (%lld cells)", base);
-        return fail();
+    // cell_start takes one int per cell: while the grids of all patches have more than kMaxGridCells cells together,
+    // the cells of every patch grow by 1.5 (the grid only prunes pair tests, the counts do not depend on it).  With
+    // one cell per patch and z-bin there are P B < 2^28.
+    for (double grow = 1.5; base > kMaxGridCells; grow *= 1.5) {
+        base = 0;
+        for (int p = 0; p < P; ++p) {
+            const PatchFrame &f = fi->h_frames[p];
+            SGrid &g = fi->h_sgrid[p];
+            size_cells(g, std::max(f.umax - f.umin, 0.0), std::max(f.vmax - f.vmin, 0.0), edge[p] * grow);
+            g.cell_base = base;
+            base += (long long)B * g.gu * g.gv;
+        }
     }
+    fi->n_cells = base;
     if (fi_alloc(fi, &fi->d_sgrid, P)) return fail();
     if (yawb_h2d_small(ctx, fi->d_sgrid, fi->h_sgrid.data(), P * sizeof(SGrid))) return fail();
     if (fi_alloc(fi, &fi->rec, n)) return fail();
     if (fi->weighted && fi_alloc(fi, &fi->sw, n)) return fail();
     if (fi_alloc(fi, &fi->cell_start, base + 1)) return fail();
-    // 32-bit sort keys whenever the cell ids fit (they nearly always do): a third less radix-sort traffic
-    // bounded, dense keys: counting sort (the radix sort only for grids with more cells than the key counts may take)
-    // (weighted rows keep the stable radix sort: the order of the rows of a cell is the order their weights are
-    // summed in, and a counting sort's atomics would make the last bits of the sums vary from run to run)
-    if (base <= kCountingSortMaxKeys && !fi->weighted) {
-        if (build_first_counting(fi, base)) return fail();
-    } else if (base < 0xffffffffll ? build_first_sorted<unsigned>(fi, base) : build_first_sorted<unsigned long long>(fi, base)) {
-        return fail();
-    }
+    if (build_first_counting(fi, base)) return fail();
     if (cudaGetLastError() != cudaSuccess) {
         yawb_set_error("first-role index build failed");
         return fail();
@@ -1323,31 +1165,20 @@ int yawb_index_build_second(yawb_cat *cat) {
     cat->ry = cat->rrow + 1;
     cat->rz = cat->rrow + 2;
     if (cat->weighted && dev_alloc(cat, &cat->rw, n)) return 1;
-    // 32-bit sort keys when (patch, bin) leaves at least 16 bits (an even number) for the Hilbert index
+    // The curve only has to order the rows down to about one row per Hilbert cell: with m rows in the largest
+    // (patch, bin) segment, 2^k x 2^k >= 1.5 m cells are enough.  The counting sort takes one count per (patch, bin,
+    // Hilbert cell), so the resolution is capped at about ONE key per row (the cells then hold 1-4 rows, in arbitrary
+    // order; swept on C3: 4 / 1 / 0.25 / 0.06 keys per row -> index build 1.80 / 1.60 / 1.57 / 2.89 ms, count
+    // kernels 6.05 / 6.07 / 6.11 / 6.31 ms).  Keys are ints: n_keys <= max(4 P B, n_in, 2^16) < 2^31.
     {
-        const int seg_bits = bits_for((unsigned long long)std::max<long long>((long long)P * B, 1));
-        const int hbits32 = ((31 - seg_bits) / 2) * 2;  // the all-ones key stays reserved for dropped rows
-        // The curve only has to order the rows down to about one row per Hilbert cell: with m rows in the
-        // largest (patch, bin) segment, 2^k x 2^k >= 1.5 m cells are enough.  Fewer key bits = fewer radix passes.
         long long m = 1;
         for (size_t sgm = 0; sgm + 1 < cat->h_seg_off.size(); ++sgm)
             m = std::max<long long>(m, cat->h_seg_off[sgm + 1] - cat->h_seg_off[sgm]);
         int k = 4;
         while (k < 16 && (1ll << (2 * k)) < m + m / 2) ++k;
-        // counting sort: one count per (patch, bin, Hilbert cell); the Hilbert resolution is capped so that there are
-        // at most about ONE key per row (the cells then hold 1-4 rows, in arbitrary order; swept on C3: 4 / 1 / 0.25 /
-        // 0.06 keys per row -> index build 1.80 / 1.60 / 1.57 / 2.89 ms, count kernels 6.05 / 6.07 / 6.11 / 6.31 ms)
-        int kc = k;
         const long long key_budget = std::max<long long>(cat->n_in, 1 << 16);
-        while (kc > 1 && (((long long)P * B) << (2 * kc)) > key_budget) --kc;
-        const long long n_keys = ((long long)P * B) << (2 * kc);
-        if (n_keys <= kCountingSortMaxKeys && !cat->weighted) {
-            if (build_second_counting(cat, 2 * kc, n_keys)) return 1;
-        } else if (hbits32 >= 16) {
-            if (build_second_sorted<unsigned>(cat, std::min(hbits32, 2 * k))) return 1;
-        } else {
-            if (build_second_sorted<unsigned long long>(cat, 32)) return 1;
-        }
+        while (k > 1 && (((long long)P * B) << (2 * k)) > key_budget) --k;
+        if (build_second_counting(cat, 2 * k, ((long long)P * B) << (2 * k))) return 1;
     }
 
     // tiles: chunks of YAWB_TILE rows inside each (patch, bin) segment; the host only needs their number per segment
