@@ -13,8 +13,12 @@
  *     library owns every device buffer;
  *   - every function returns 0 on success, non-zero on failure with a message
  *     available from yawb_last_error() (thread local);
- *   - one context per process/GPU, not re-entrant per context; all work of a
- *     context is issued on one CUDA stream owned by the context;
+ *   - any number of contexts per process, on the same or on different devices
+ *     (library version >= 103); every entry point selects the device of the
+ *     context it is given, and contexts share no state, so each context may be
+ *     driven by its own host thread.  A context is not re-entrant: one thread
+ *     at a time per context and its catalogs.  All work of a context is issued
+ *     on CUDA streams owned by the context;
  *   - there is no CPU fallback: without a CUDA device yawb_create() fails.
  */
 #ifndef YAWB_H
@@ -121,6 +125,31 @@ int yawb_upload_catalog_z(yawb_ctx *ctx, const double *xyz, const double *w, con
  * different L or B, YAWB_FLAG_EXACT_BRUTEFORCE, YAWB_FLAG_SECOND_LABELS, and labelled catalogs in yawb_count2 /
  * yawb_count4. */
 int yawb_catalog_set_labels(yawb_cat *cat, int n_labels);
+
+/* Partial upload (library version >= 103): the rows of the patches with keep[p] != 0 only, taken from the full host
+ * arrays (xyz, w, zbin / zbin8 / z and patch_off describe the whole catalog, as for the uploads above; at most one of
+ * zbin, zbin8 and z with edges / closed_right).  Patch ids keep their numbers and an unkept patch is an empty patch:
+ * for a kept patch the sums of weights, frames and indexes are those of a full upload (up to the order of FP64
+ * sums), for an unkept one the sums are 0.  Each run of consecutive kept patches travels straight from the caller's
+ * arrays, as one copy per array; no host-side gather.  This is how one device of several holds only the patches it
+ * counts and their neighbours. */
+int yawb_upload_catalog_patches(yawb_ctx *ctx, const double *xyz, const double *w, const int32_t *zbin,
+                                const uint8_t *zbin8, const double *z, const double *edges, int closed_right,
+                                const int64_t *patch_off, int n_patch, int n_bins, const uint8_t *keep, yawb_cat **out);
+
+/* Second-role row mask (library version >= 103): mask holds one byte per uploaded row (for a partial upload: the rows
+ * of the kept patches, in patch order); a row with mask 0 is left out of the second-role index (tiles, Hilbert order,
+ * tile spheres) as a row outside the z-binning is.  NULL clears the mask.  The first-role index, yawb_sum_weights,
+ * yawb_patch_metadata and yawb_catalog_info keep every row.  Setting or clearing the mask drops a built second-role
+ * index (first-role and fused indexes stay).  Synchronous.
+ * Contract: for masks m and !m on two uploads A_m, A_!m of the same rows (and A_full without a mask),
+ *     count(c1, A_m) + count(c1, A_!m) == count(c1, A_full)
+ * bit for bit for integer counts and to 1e-12 for weighted sums, for every count path, for labelled and binned-label
+ * catalogs, in yawb_count / yawb_count2 / yawb_count4, and for auto counts (the masked upload as the second catalog,
+ * the same or a full upload as the first).  The mask carries the caller's choice of rows: equal sort keys have no
+ * defined order and frames are FP64 atomic sums, so no rule stated in the index's own order would split the rows
+ * alike on two devices. */
+int yawb_catalog_set_second_rows(yawb_cat *cat, const uint8_t *mask);
 int yawb_free_catalog(yawb_cat *cat);
 
 /* Build (or rebuild) the device-side index for a role ahead of time; otherwise

@@ -13,14 +13,14 @@ from .catalog import Catalog, InconsistentPatchesError
 from .config import Configuration
 from .coordinates import AngularCoordinates, AngularDistances
 from .corrfunc import CorrFunc, ScalarCorrFunc
-from .engine import DeviceCatalog, Engine
+from .engine import DeviceCatalog, Engine, EngineGroup
 from .measurements import (PatchLinkage, autocorrelate, autocorrelate_scalar, autocorrelate_tomographic,
                            crosscorrelate, crosscorrelate_scalar, crosscorrelate_tomographic)
 from .randoms import BoxRandoms
 
 __all__ = [
     "AngularCoordinates", "AngularDistances", "Binning", "BoxRandoms", "Catalog", "Configuration", "CorrFunc",
-    "DeviceCatalog", "Engine", "InconsistentPatchesError", "PatchLinkage", "ScalarCorrFunc", "YawbError",
+    "DeviceCatalog", "Engine", "EngineGroup", "InconsistentPatchesError", "PatchLinkage", "ScalarCorrFunc", "YawbError",
     "autocorrelate", "autocorrelate_scalar", "autocorrelate_tomographic", "crosscorrelate", "crosscorrelate_scalar",
     "crosscorrelate_tomographic",
 ]

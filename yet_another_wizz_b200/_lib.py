@@ -21,6 +21,7 @@ FLAG_OUT_DEVICE = 2
 FLAG_SECOND_LABELS = 4
 LABELS_MIN_VERSION = 101  # first library version that knows FLAG_SECOND_LABELS
 BINNED_LABELS_MIN_VERSION = 102  # first library version with yawb_catalog_set_labels
+PARTIAL_MIN_VERSION = 103  # first library version with partial uploads and second-role row masks
 ROLE_FIRST = 1
 ROLE_SECOND = 2
 
@@ -31,7 +32,7 @@ EXPORTS = (
     "yawb_host_alloc", "yawb_host_free", "yawb_sync", "yawb_version", "yawb_device_sms",
     "yawb_timer_start", "yawb_timer_stop", "yawb_assign_patches", "yawb_upload_catalog_u8", "yawb_count2",
     "yawb_upload_catalog_z", "yawb_patch_metadata", "yawb_jackknife", "yawb_count4", "yawb_kmeans",
-    "yawb_catalog_set_labels",
+    "yawb_catalog_set_labels", "yawb_upload_catalog_patches", "yawb_catalog_set_second_rows",
 )
 
 
@@ -91,6 +92,11 @@ def load(build_if_missing: bool = False) -> ctypes.CDLL:
     lib.yawb_upload_catalog_z.argtypes = [
         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, POINTER(c_void_p),
     ]
+    lib.yawb_upload_catalog_patches.argtypes = [
+        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p,
+        POINTER(c_void_p),
+    ]
+    lib.yawb_catalog_set_second_rows.argtypes = [c_void_p, c_void_p]
     lib.yawb_patch_metadata.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p]
     lib.yawb_jackknife.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]
     lib.yawb_free_catalog.argtypes = [c_void_p]

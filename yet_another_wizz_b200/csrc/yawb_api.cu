@@ -144,7 +144,7 @@ int yawb_assign_patches(yawb_ctx *ctx, const double *xyz, int64_t n, const doubl
 
 const char *yawb_last_error(void) { return g_err; }
 
-int yawb_version(void) { return 102; }
+int yawb_version(void) { return 103; }
 
 int yawb_create(int device, yawb_ctx **out) {
     YAWB_REQUIRE(out != nullptr, "yawb_create: out is NULL");
@@ -214,6 +214,7 @@ int yawb_device_sms(const yawb_ctx *ctx) { return ctx ? ctx->sms : 0; }
 
 int yawb_sync(yawb_ctx *ctx) {
     YAWB_REQUIRE(ctx != nullptr, "yawb_sync: ctx is NULL");
+    YAWB_CUDA(cudaSetDevice(ctx->device));
     YAWB_CUDA(cudaStreamSynchronize(ctx->copy_stream));
     YAWB_CUDA(cudaStreamSynchronize(ctx->stream));
     return 0;
@@ -221,12 +222,14 @@ int yawb_sync(yawb_ctx *ctx) {
 
 int yawb_timer_start(yawb_ctx *ctx) {
     YAWB_REQUIRE(ctx != nullptr, "yawb_timer_start: ctx is NULL");
+    YAWB_CUDA(cudaSetDevice(ctx->device));
     YAWB_CUDA(cudaEventRecord(ctx->ev_t0, ctx->stream));
     return 0;
 }
 
 int yawb_timer_stop(yawb_ctx *ctx, double *ms) {
     YAWB_REQUIRE(ctx && ms, "yawb_timer_stop: NULL argument");
+    YAWB_CUDA(cudaSetDevice(ctx->device));
     YAWB_CUDA(cudaEventRecord(ctx->ev_t1, ctx->stream));
     YAWB_CUDA(cudaEventSynchronize(ctx->ev_t1));
     float t = 0.f;
@@ -246,9 +249,10 @@ int yawb_host_free(void *ptr) {
     return 0;
 }
 
+// keep: NULL (every patch) or one byte per patch; the rows of the kept patches travel, an unkept patch is empty
 static int upload_common(yawb_ctx *ctx, const double *xyz, const double *w, const int32_t *zbin, const uint8_t *zbin8,
                          const double *zred, const double *edges, int closed_right, const int64_t *patch_off,
-                         int n_patch, int n_bins, yawb_cat **out) {
+                         int n_patch, int n_bins, const uint8_t *keep, yawb_cat **out) {
     YAWB_REQUIRE(ctx && out && patch_off, "yawb_upload_catalog: NULL argument");
     *out = nullptr;
     YAWB_REQUIRE(n_patch >= 1 && n_patch <= 65535, "n_patch must be in 1..65535 (got %d)", n_patch);
@@ -259,7 +263,19 @@ static int upload_common(yawb_ctx *ctx, const double *xyz, const double *w, cons
     YAWB_REQUIRE(patch_off[0] == 0, "patch_off[0] must be 0");
     for (int p = 0; p < n_patch; ++p)
         YAWB_REQUIRE(patch_off[p + 1] >= patch_off[p], "patch_off must be non-decreasing");
-    const int64_t n = patch_off[n_patch];
+    // rows on the device: the kept patches one after the other, each run of consecutive kept patches one copy
+    std::vector<int64_t> dev_off(n_patch + 1, 0);
+    std::vector<RowRun> runs;
+    for (int p = 0; p < n_patch; ++p) {
+        const int64_t rows = keep && !keep[p] ? 0 : patch_off[p + 1] - patch_off[p];
+        dev_off[p + 1] = dev_off[p] + rows;
+        if (rows == 0) continue;
+        if (!runs.empty() && runs.back().src + runs.back().rows == patch_off[p])
+            runs.back().rows += rows;
+        else
+            runs.push_back({patch_off[p], dev_off[p], rows});
+    }
+    const int64_t n = dev_off[n_patch];
     YAWB_REQUIRE(n < (1ll << 31) - 1024, "catalogs are limited to 2^31 rows (got %lld)", (long long)n);
     YAWB_REQUIRE(n == 0 || xyz != nullptr, "xyz is NULL");
     YAWB_CUDA(cudaSetDevice(ctx->device));
@@ -273,12 +289,13 @@ static int upload_common(yawb_ctx *ctx, const double *xyz, const double *w, cons
     cat->binned = binned;
     cat->weighted = w != nullptr;
     cat->h_rows_per_patch.resize(n_patch);
-    for (int p = 0; p < n_patch; ++p) cat->h_rows_per_patch[p] = patch_off[p + 1] - patch_off[p];
+    for (int p = 0; p < n_patch; ++p) cat->h_rows_per_patch[p] = dev_off[p + 1] - dev_off[p];
     if (zred) {
         cat->h_edges.assign(edges, edges + n_bins + 1);
         cat->closed_right = closed_right != 0;
     }
-    if (yawb_index_upload(ctx, cat, xyz, w, zbin8, zbin, zred, patch_off)) {
+    cat->h_dev_off.swap(dev_off);  // the device copies its row offsets from here, asynchronously
+    if (yawb_index_upload(ctx, cat, xyz, w, zbin8, zbin, zred, cat->h_dev_off.data(), runs)) {
         yawb_index_free(cat, true);
         delete cat;
         return 1;
@@ -289,21 +306,45 @@ static int upload_common(yawb_ctx *ctx, const double *xyz, const double *w, cons
 
 int yawb_upload_catalog(yawb_ctx *ctx, const double *xyz, const double *w, const int32_t *zbin,
                         const int64_t *patch_off, int n_patch, int n_bins, yawb_cat **out) {
-    return upload_common(ctx, xyz, w, zbin, nullptr, nullptr, nullptr, 1, patch_off, n_patch, n_bins, out);
+    return upload_common(ctx, xyz, w, zbin, nullptr, nullptr, nullptr, 1, patch_off, n_patch, n_bins, nullptr, out);
 }
 
 int yawb_upload_catalog_u8(yawb_ctx *ctx, const double *xyz, const double *w, const uint8_t *zbin,
                            const int64_t *patch_off, int n_patch, int n_bins, yawb_cat **out) {
-    return upload_common(ctx, xyz, w, nullptr, zbin, nullptr, nullptr, 1, patch_off, n_patch, n_bins, out);
+    return upload_common(ctx, xyz, w, nullptr, zbin, nullptr, nullptr, 1, patch_off, n_patch, n_bins, nullptr, out);
+}
+
+static int check_edges(const double *edges, int n_bins) {
+    YAWB_REQUIRE(n_bins >= 1, "yawb_upload_catalog_z: n_bins must be >= 1 (got %d)", n_bins);
+    for (int b = 0; b < n_bins; ++b)
+        YAWB_REQUIRE(edges[b] < edges[b + 1], "yawb_upload_catalog_z: z-bin edges must increase (edge %d)", b);
+    return 0;
 }
 
 int yawb_upload_catalog_z(yawb_ctx *ctx, const double *xyz, const double *w, const double *z, const double *edges,
                           int closed_right, const int64_t *patch_off, int n_patch, int n_bins, yawb_cat **out) {
     YAWB_REQUIRE(z && edges, "yawb_upload_catalog_z: redshifts or edges are NULL");
-    YAWB_REQUIRE(n_bins >= 1, "yawb_upload_catalog_z: n_bins must be >= 1 (got %d)", n_bins);
-    for (int b = 0; b < n_bins; ++b)
-        YAWB_REQUIRE(edges[b] < edges[b + 1], "yawb_upload_catalog_z: z-bin edges must increase (edge %d)", b);
-    return upload_common(ctx, xyz, w, nullptr, nullptr, z, edges, closed_right, patch_off, n_patch, n_bins, out);
+    if (int rc = check_edges(edges, n_bins)) return rc;
+    return upload_common(ctx, xyz, w, nullptr, nullptr, z, edges, closed_right, patch_off, n_patch, n_bins, nullptr, out);
+}
+
+int yawb_upload_catalog_patches(yawb_ctx *ctx, const double *xyz, const double *w, const int32_t *zbin,
+                                const uint8_t *zbin8, const double *z, const double *edges, int closed_right,
+                                const int64_t *patch_off, int n_patch, int n_bins, const uint8_t *keep, yawb_cat **out) {
+    YAWB_REQUIRE(keep != nullptr, "yawb_upload_catalog_patches: keep is NULL");
+    YAWB_REQUIRE((zbin != nullptr) + (zbin8 != nullptr) + (z != nullptr) <= 1,
+                 "yawb_upload_catalog_patches: pass at most one of zbin, zbin8 and z");
+    if (z) {
+        YAWB_REQUIRE(edges != nullptr, "yawb_upload_catalog_patches: z-bin edges are NULL");
+        if (int rc = check_edges(edges, n_bins)) return rc;
+    }
+    return upload_common(ctx, xyz, w, zbin, zbin8, z, edges, closed_right, patch_off, n_patch, n_bins, keep, out);
+}
+
+int yawb_catalog_set_second_rows(yawb_cat *cat, const uint8_t *mask) {
+    YAWB_REQUIRE(cat != nullptr, "yawb_catalog_set_second_rows: cat is NULL");
+    YAWB_CUDA(cudaSetDevice(cat->ctx->device));
+    return yawb_index_set_second_rows(cat, mask);
 }
 
 int yawb_catalog_set_labels(yawb_cat *cat, int n_labels) {
@@ -354,6 +395,7 @@ int yawb_drop_index(yawb_cat *cat) {
 
 int yawb_catalog_info(const yawb_cat *cat, int64_t *n_rows, int64_t *device_bytes) {
     YAWB_REQUIRE(cat != nullptr, "yawb_catalog_info: cat is NULL");
+    YAWB_CUDA(cudaSetDevice(cat->ctx->device));
     if (yawb_cat_finalize(const_cast<yawb_cat *>(cat))) return 1;
     if (n_rows) *n_rows = cat->n;
     if (device_bytes) *device_bytes = cat->device_bytes;
@@ -362,6 +404,7 @@ int yawb_catalog_info(const yawb_cat *cat, int64_t *n_rows, int64_t *device_byte
 
 int yawb_sum_weights(const yawb_cat *cat, double *out) {
     YAWB_REQUIRE(cat && out, "yawb_sum_weights: NULL argument");
+    YAWB_CUDA(cudaSetDevice(cat->ctx->device));
     if (yawb_cat_finalize(const_cast<yawb_cat *>(cat))) return 1;
     std::memcpy(out, cat->h_sumw.data(), cat->h_sumw.size() * sizeof(double));
     return 0;
@@ -415,6 +458,7 @@ int yawb_jackknife(yawb_ctx *ctx, const double *values, const int32_t *pair_i, c
 
 int yawb_patch_metadata(const yawb_cat *cat, double *center_xyz, double *radius_chord, int64_t *num_records) {
     YAWB_REQUIRE(cat != nullptr, "yawb_patch_metadata: NULL catalog");
+    YAWB_CUDA(cudaSetDevice(cat->ctx->device));
     if (yawb_cat_finalize(const_cast<yawb_cat *>(cat))) return 1;
     for (int p = 0; p < cat->n_patch; ++p) {
         const PatchFrame &f = cat->h_frames[p];
@@ -596,15 +640,16 @@ static int count_impl(yawb_ctx *ctx, yawb_cat *cat1, yawb_cat *cat1b, yawb_cat *
                 for (int l = 0; l < L2; ++l)
                     for (int b = 0; b < B; ++b)
                         s.pair_tests_naive += (uint64_t)(cat1->h_counts[((size_t)(L1 ? l * B : 0) + b) * P + p] *
-                                                         c2->h_counts[((size_t)l * B + b) * P + q]);
+                                                         c2->second_counts()[((size_t)l * B + b) * P + q]);
                 continue;
             }
             long long n2_all = 0;  // a labelled catalog pairs the rows of every label with each z-bin
-            for (int l = 0; l < c2->n_bins; ++l) n2_all += c2->h_counts[(size_t)l * P + q];
+            const std::vector<long long> &cnt2 = c2->second_counts();
+            for (int l = 0; l < c2->n_bins; ++l) n2_all += cnt2[(size_t)l * P + q];
             for (int b = 0; b < B; ++b) {
                 long long n1 = cat1->h_counts[(size_t)b * P + p];
                 if (cat1b) n1 += cat1b->h_counts[(size_t)b * P + p];
-                const long long n2 = c2->binned && !labels ? c2->h_counts[(size_t)b * P + q] : n2_all;
+                const long long n2 = c2->binned && !labels ? cnt2[(size_t)b * P + q] : n2_all;
                 s.pair_tests_naive += (uint64_t)(n1 * n2);
             }
         }

@@ -927,7 +927,7 @@ int yawb_launch_count_exact(yawb_ctx *ctx, const CountArgs &a, int *launches) {
     ExactParams P{};
     P.cx = a.c1_cat->x; P.cy = a.c1_cat->y; P.cz = a.c1_cat->z; P.rec = a.c1->rec;
     P.sw = a.c1->sw; P.s_seg = a.c1_cat->d_seg_off;
-    P.rx = a.c2->rx; P.ry = a.c2->ry; P.rz = a.c2->rz; P.rw = a.c2->rw; P.r_seg = a.c2->d_seg_off;
+    P.rx = a.c2->rx; P.ry = a.c2->ry; P.rz = a.c2->rz; P.rw = a.c2->rw; P.r_seg = a.c2->second_d_seg_off();
     P.b1 = a.c1_cat->n_bins; P.b2 = a.c2->n_bins;
     P.pair_i = a.d_pair_i; P.pair_j = a.d_pair_j;
     P.n_pairs = a.n_pairs; P.n_bins = a.n_bins; P.n_edges = a.n_edges;

@@ -486,10 +486,13 @@ __global__ void k_hist_first(const double *__restrict__ x, const double *__restr
 
 __global__ void k_hist_second(const double *__restrict__ x, const double *__restrict__ y, const double *__restrict__ z,
                               const int *__restrict__ bin, const int *__restrict__ patch, long long n, int n_bins,
-                              int hbits, const HMap *__restrict__ maps, int *__restrict__ cur, int2 *__restrict__ kr) {
+                              int hbits, const HMap *__restrict__ maps, const unsigned char *__restrict__ mask,
+                              int *__restrict__ cur, int2 *__restrict__ kr) {
     long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const long long key = key_second(x[3 * i], y[3 * i], z[3 * i], bin ? bin[i] : 0, patch[i], n_bins, hbits, maps);
+    // a row outside the mask (yawb_catalog_set_second_rows) is dropped like a row outside the z-binning
+    const long long key = mask && !mask[i] ? -1
+                                           : key_second(x[3 * i], y[3 * i], z[3 * i], bin ? bin[i] : 0, patch[i], n_bins, hbits, maps);
     int rank = 0;
     if (key >= 0) rank = atomicAdd(&cur[key], 1);
     kr[i] = make_int2((int)key, rank);  // -1: dropped row
@@ -739,6 +742,19 @@ __global__ void k_count_oversized(const Tile *__restrict__ tiles, int n_tiles, c
     if (t < n_tiles && tiles[t].count > 32 && tiles[t].rad > thr[tiles[t].patch]) atomicAdd(n_big, 1u);
 }
 
+// rows per (z-bin, patch) inside the second-role mask; rows are grouped by patch, so the lanes of a warp mostly share
+// a key and one lane adds for all of them
+__global__ void k_second_counts(const int *__restrict__ bin, const int *__restrict__ patch, const unsigned char *__restrict__ mask,
+                                long long n, int n_bins, int n_patch, unsigned long long *__restrict__ counts) {
+    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int b = bin ? bin[i] : 0;
+    if (!mask[i] || b < 0 || b >= n_bins) return;
+    const int key = b * n_patch + patch[i];
+    const unsigned peers = __match_any_sync(__activemask(), key);
+    if ((threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&counts[key], (unsigned long long)__popc(peers));
+}
+
 template <typename T>
 int fi_alloc(FIndex *fi, T **ptr, size_t count) {
     *ptr = nullptr;
@@ -795,7 +811,7 @@ int build_second_counting(yawb_cat *cat, int hbits, long long n_keys) {
     YAWB_CUDA(cudaMemsetAsync(cur, 0, (size_t)n_keys * sizeof(int), st));
     k_hilbert_map<<<(cat->n_patch + 127) / 128, 128, 0, st>>>(cat->d_frames, cat->n_patch, hbits, maps);
     k_hist_second<<<blocks_for(cat->n_in), kThreads, 0, st>>>(cat->x, cat->y, cat->z, cat->bin, cat->patch, cat->n_in,
-                                                              cat->n_bins, hbits, maps, cur, keys);
+                                                              cat->n_bins, hbits, maps, cat->d_second_mask, cur, keys);
     if (exclusive_scan_inplace(ctx, scr, cur, n_keys)) return 1;
     k_scatter_second<<<blocks_for(cat->n_in), kThreads, 0, st>>>(cat->x, cat->y, cat->z, cat->w, keys, cat->n_in, cur,
                                                                  cat->rx, cat->ry, cat->rz, cat->rw);
@@ -824,7 +840,7 @@ void size_cells(SGrid &g, double du, double dv, double c) {
 static constexpr size_t kCopyChunk = (size_t)64 << 20;
 
 int yawb_index_upload(yawb_ctx *ctx, yawb_cat *cat, const double *xyz, const double *w, const uint8_t *zbin8,
-                      const int32_t *zbin, const double *zred, const int64_t *patch_off) {
+                      const int32_t *zbin, const double *zred, const int64_t *patch_off, const std::vector<RowRun> &runs) {
     YawbRange range("yawb:upload");
     const long long n = cat->n_in;
     const int P = cat->n_patch, B = cat->n_bins;
@@ -846,22 +862,27 @@ int yawb_index_upload(yawb_ctx *ctx, yawb_cat *cat, const double *xyz, const dou
     if (dev_alloc(cat, &cat->d_frames, P, st) || dev_alloc(cat, &cat->d_seg_off, (size_t)P * B + 1, st)) return 1;
     if (dev_alloc(cat, &cat->d_stage_poff, P + 1, st)) return 1;
 
-    // Bulk copies go out in pieces so that other users of the copy engine never wait behind a whole
-    // catalog (the small tables of a concurrent pair count avoid the engine altogether: yawb_h2d_small).
-    auto h2d = [&](void *dst, const void *src, size_t bytes) -> cudaError_t {
-        for (size_t o = 0; o < bytes; o += kCopyChunk) {
-            cudaError_t e = cudaMemcpyAsync((char *)dst + o, (const char *)src + o, std::min(kCopyChunk, bytes - o),
-                                            cudaMemcpyHostToDevice, st);
-            if (e != cudaSuccess) return e;
+    // Each run of rows (the whole catalog, or a run of consecutive kept patches of a partial upload) travels straight
+    // from the caller's array.  Bulk copies go out in pieces so that other users of the copy engine never wait behind
+    // a whole catalog (the small tables of a concurrent pair count avoid the engine altogether: yawb_h2d_small).
+    auto h2d = [&](void *dst, const void *src, size_t row_bytes) -> cudaError_t {
+        for (const RowRun &r : runs) {
+            const size_t bytes = (size_t)r.rows * row_bytes;
+            char *d = (char *)dst + (size_t)r.dst * row_bytes;
+            const char *s = (const char *)src + (size_t)r.src * row_bytes;
+            for (size_t o = 0; o < bytes; o += kCopyChunk) {
+                cudaError_t e = cudaMemcpyAsync(d + o, s + o, std::min(kCopyChunk, bytes - o), cudaMemcpyHostToDevice, st);
+                if (e != cudaSuccess) return e;
+            }
         }
         return cudaSuccess;
     };
-    if (n > 0) YAWB_CUDA(h2d(cat->xyz, xyz, n * 3 * sizeof(double)));
+    if (n > 0) YAWB_CUDA(h2d(cat->xyz, xyz, 3 * sizeof(double)));
     YAWB_CUDA(cudaMemcpyAsync(cat->d_stage_poff, patch_off, (P + 1) * sizeof(long long), cudaMemcpyHostToDevice, st));
-    if (w && n > 0) YAWB_CUDA(h2d(cat->w, w, n * sizeof(double)));
-    if (zbin && n > 0) YAWB_CUDA(h2d(cat->bin, zbin, n * sizeof(int32_t)));
-    if (zbin8 && n > 0) YAWB_CUDA(h2d(cat->d_stage_bin8, zbin8, n));
-    if (zred && n > 0) YAWB_CUDA(h2d(cat->d_stage_z, zred, n * sizeof(double)));
+    if (w && n > 0) YAWB_CUDA(h2d(cat->w, w, sizeof(double)));
+    if (zbin && n > 0) YAWB_CUDA(h2d(cat->bin, zbin, sizeof(int32_t)));
+    if (zbin8 && n > 0) YAWB_CUDA(h2d(cat->d_stage_bin8, zbin8, 1));
+    if (zred && n > 0) YAWB_CUDA(h2d(cat->d_stage_z, zred, sizeof(double)));
     YAWB_CUDA(cudaEventCreateWithFlags(&cat->ev_meta, cudaEventDisableTiming));
     YAWB_CUDA(cudaEventRecord(cat->ev_meta, st));
     YAWB_CUDA(cudaGetLastError());
@@ -1157,8 +1178,9 @@ int yawb_index_build_second(yawb_cat *cat) {
     YawbRange range("yawb:index_second");
     yawb_ctx *ctx = cat->ctx;
     cudaStream_t st = ctx->stream;
-    const long long n = cat->n;
+    const long long n = cat->second_rows();
     const int P = cat->n_patch, B = cat->n_bins;
+    const std::vector<int> &seg_off = cat->second_seg_off();
 
     if (dev_alloc(cat, &cat->rrow, (size_t)n * YAWB_RSTRIDE)) return 1;
     cat->rx = cat->rrow;
@@ -1172,8 +1194,8 @@ int yawb_index_build_second(yawb_cat *cat) {
     // kernels 6.05 / 6.07 / 6.11 / 6.31 ms).  Keys are ints: n_keys <= max(4 P B, n_in, 2^16) < 2^31.
     {
         long long m = 1;
-        for (size_t sgm = 0; sgm + 1 < cat->h_seg_off.size(); ++sgm)
-            m = std::max<long long>(m, cat->h_seg_off[sgm + 1] - cat->h_seg_off[sgm]);
+        for (size_t sgm = 0; sgm + 1 < seg_off.size(); ++sgm)
+            m = std::max<long long>(m, seg_off[sgm + 1] - seg_off[sgm]);
         int k = 4;
         while (k < 16 && (1ll << (2 * k)) < m + m / 2) ++k;
         const long long key_budget = std::max<long long>(cat->n_in, 1 << 16);
@@ -1190,7 +1212,7 @@ int yawb_index_build_second(yawb_cat *cat) {
     for (int p = 0; p < P; ++p) {
         cat->h_ptile_off[p] = seg_tile_off[(size_t)p * B];
         for (int b = 0; b < B; ++b) {
-            const int len = cat->h_seg_off[(size_t)p * B + b + 1] - cat->h_seg_off[(size_t)p * B + b];
+            const int len = seg_off[(size_t)p * B + b + 1] - seg_off[(size_t)p * B + b];
             seg_tile_off[(size_t)p * B + b + 1] = seg_tile_off[(size_t)p * B + b] + (len + YAWB_TILE - 1) / YAWB_TILE;
         }
     }
@@ -1217,7 +1239,7 @@ int yawb_index_build_second(yawb_cat *cat) {
         std::vector<float> thr(P, 3.0e38f);
         for (int p = 0; p < P; ++p) {
             const PatchFrame &f = cat->h_frames[p];
-            const long long np = cat->h_seg_off[(size_t)(p + 1) * B] - cat->h_seg_off[(size_t)p * B];
+            const long long np = seg_off[(size_t)(p + 1) * B] - seg_off[(size_t)p * B];
             const double area = std::max(f.umax - f.umin, 0.0) * std::max(f.vmax - f.vmin, 0.0);
             if (np >= 8 * YAWB_TILE && area > 0.0)  // radius of a disc holding YAWB_TILE rows of one z-bin
                 thr[p] = (float)(3.0 * std::sqrt((double)YAWB_TILE * B * area / (3.14159265358979 * (double)np)));
@@ -1225,7 +1247,7 @@ int yawb_index_build_second(yawb_cat *cat) {
         if (yawb_h2d_small(ctx, d_seg_tile_off, seg_tile_off.data(), seg_tile_off.size() * sizeof(int))) return 1;
         if (yawb_h2d_small(ctx, d_thr, thr.data(), P * sizeof(float))) return 1;
         YAWB_CUDA(cudaMemsetAsync(d_nbig, 0, sizeof(unsigned), st));
-        k_make_tiles<<<blocks_for((long long)n_tiles0), kThreads, 0, st>>>(cat->d_seg_off, d_seg_tile_off, P * B, B,
+        k_make_tiles<<<blocks_for((long long)n_tiles0), kThreads, 0, st>>>(cat->second_d_seg_off(), d_seg_tile_off, P * B, B,
                                                                           cat->binned ? 1 : 0, n_tiles0, d_tmp);
         TileBox *d_box_tmp = nullptr;
         if (dev_alloc(cat, &d_box_tmp, (size_t)n_tiles0)) return 1;
@@ -1283,23 +1305,84 @@ int yawb_index_build_second(yawb_cat *cat) {
     return 0;
 }
 
+void yawb_index_free_second(yawb_cat *cat) {
+    const size_t n = (size_t)cat->second_rows(), P = (size_t)cat->n_patch;
+    dev_free(cat, cat->rrow, n * YAWB_RSTRIDE);
+    cat->rx = cat->ry = cat->rz = nullptr;
+    dev_free(cat, cat->rw, n);
+    dev_free(cat, cat->d_tiles, (size_t)cat->n_tiles);
+    dev_free(cat, cat->d_tile_box, (size_t)cat->n_tiles);
+    dev_free(cat, cat->d_ptile_off, P + 1);
+    cat->has_rtiles = false;
+}
+
+// The mask is copied to the device and its rows are counted per (z-bin, patch) right away: the second-role index
+// needs those counts on the host to size its segments and tiles.
+int yawb_index_set_second_rows(yawb_cat *cat, const uint8_t *mask) {
+    if (yawb_cat_finalize(cat)) return 1;
+    yawb_ctx *ctx = cat->ctx;
+    cudaStream_t st = ctx->stream;
+    const int P = cat->n_patch, B = cat->n_bins;
+    YAWB_CUDA(cudaStreamSynchronize(st));  // nothing in flight still reads the second-role index
+    yawb_index_free_second(cat);
+    dev_free(cat, cat->d_second_mask, (size_t)cat->n_in);
+    dev_free(cat, cat->d_seg_off2, (size_t)P * B + 1);
+    cat->h_counts2.clear();
+    cat->h_seg_off2.clear();
+    cat->n2 = 0;
+    if (!mask) return 0;
+    const long long n = cat->n_in;
+    unsigned char *d_mask = nullptr;
+    int *d_seg = nullptr;
+    std::vector<unsigned long long> counts((size_t)B * P, 0);
+    {
+        Scratch scr(ctx, st);
+        unsigned long long *d_counts = scr.get<unsigned long long>((size_t)B * P);
+        // the catalog takes the mask only once everything has worked: on failure it stays without one
+        auto fail = [&]() {
+            dev_free(cat, d_mask, (size_t)n);
+            dev_free(cat, d_seg, (size_t)P * B + 1);
+            return 1;
+        };
+        if (!d_counts || dev_alloc(cat, &d_mask, (size_t)n) || dev_alloc(cat, &d_seg, (size_t)P * B + 1)) {
+            yawb_set_error("out of device memory (second-role mask)");
+            return fail();
+        }
+        cudaError_t e = cudaMemsetAsync(d_counts, 0, (size_t)B * P * sizeof(unsigned long long), st);
+        if (e == cudaSuccess && n > 0) {
+            e = cudaMemcpyAsync(d_mask, mask, (size_t)n, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess)
+                k_second_counts<<<blocks_for(n), kThreads, 0, st>>>(cat->bin, cat->patch, d_mask, n, B, P, d_counts);
+        }
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(counts.data(), d_counts, counts.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e != cudaSuccess) {
+            yawb_set_error("yawb_catalog_set_second_rows: %s", cudaGetErrorString(e));
+            return fail();
+        }
+    }
+    cat->d_second_mask = d_mask;
+    cat->d_seg_off2 = d_seg;
+    cat->h_counts2.assign(counts.begin(), counts.end());
+    cat->h_seg_off2.assign((size_t)P * B + 1, 0);
+    for (int p = 0; p < P; ++p)
+        for (int b = 0; b < B; ++b)
+            cat->h_seg_off2[(size_t)p * B + b + 1] = cat->h_seg_off2[(size_t)p * B + b] + (int)counts[(size_t)b * P + p];
+    cat->n2 = cat->h_seg_off2.back();
+    return yawb_h2d_small(ctx, cat->d_seg_off2, cat->h_seg_off2.data(), cat->h_seg_off2.size() * sizeof(int));
+}
+
 void yawb_index_free(yawb_cat *cat, bool everything) {
-    const size_t n = (size_t)cat->n, P = (size_t)cat->n_patch;
+    const size_t P = (size_t)cat->n_patch;
     if (cat->findex) {
         cat->device_bytes -= cat->findex->device_bytes;
         yawb_findex_free(cat->findex);
         cat->findex = nullptr;
     }
     yawb_findex_drop_fused(cat->ctx, cat);
-    if (cat->has_rtiles || everything) {
-        dev_free(cat, cat->rrow, n * YAWB_RSTRIDE);
-        cat->rx = cat->ry = cat->rz = nullptr;
-        dev_free(cat, cat->rw, n);
-        dev_free(cat, cat->d_tiles, (size_t)cat->n_tiles);
-        dev_free(cat, cat->d_tile_box, (size_t)cat->n_tiles);
-        dev_free(cat, cat->d_ptile_off, P + 1);
-        cat->has_rtiles = false;
-    }
+    if (cat->has_rtiles || everything) yawb_index_free_second(cat);
     if (everything) {
         release_staging(cat);
         // a catalog that was never used may still have copies in flight: frees are ordered behind them
@@ -1316,5 +1399,7 @@ void yawb_index_free(yawb_cat *cat, bool everything) {
         dev_free(cat, cat->patch, ni);
         dev_free(cat, cat->d_frames, P);
         dev_free(cat, cat->d_seg_off, P * (size_t)cat->n_bins + 1);
+        dev_free(cat, cat->d_second_mask, ni);
+        dev_free(cat, cat->d_seg_off2, P * (size_t)cat->n_bins + 1);
     }
 }

@@ -193,12 +193,25 @@ struct yawb_cat {
     // per (bin, patch): number of rows and sum of weights, host copies
     std::vector<long long> h_counts;   // [n_bins][n_patch]
     std::vector<long long> h_rows_per_patch;  // [n_patch] rows uploaded, whatever their z-bin
+    std::vector<int64_t> h_dev_off;           // [n_patch + 1] row offsets on the device (source of an async copy)
     std::vector<double> h_sumw;        // [n_bins][n_patch]
     std::vector<int> h_seg_off;        // [(n_patch * n_bins) + 1], patch-major, bin-minor
     int *d_seg_off = nullptr;
 
     // first-role index: rows sorted by global sky-cell id (built on first use)
     struct FIndex *findex = nullptr;
+
+    // rows of the second-role index (yawb_catalog_set_second_rows): a byte per uploaded row, nullptr = every row.
+    // With a mask the second-role index has its own row counts and segments; everything else keeps all rows.
+    unsigned char *d_second_mask = nullptr;
+    std::vector<long long> h_counts2;  // [n_bins][n_patch] masked rows (with a mask only)
+    std::vector<int> h_seg_off2;       // [(n_patch * n_bins) + 1] segments of the masked rows
+    int *d_seg_off2 = nullptr;
+    int64_t n2 = 0;                    // masked rows
+    int64_t second_rows() const { return d_second_mask ? n2 : n; }
+    const std::vector<int> &second_seg_off() const { return d_second_mask ? h_seg_off2 : h_seg_off; }
+    const std::vector<long long> &second_counts() const { return d_second_mask ? h_counts2 : h_counts; }
+    int *second_d_seg_off() const { return d_second_mask ? d_seg_off2 : d_seg_off; }
 
     // second-role index: rows sorted by (patch, bin, Hilbert index), cut into register tiles
     bool has_rtiles = false;
@@ -234,8 +247,16 @@ struct FIndex {
 };
 
 // index construction (yawb_index.cu)
+// A run of rows copied from the caller's arrays: rows [src, src + rows) go to device rows [dst, dst + rows).
+struct RowRun {
+    int64_t src, dst, rows;
+};
+// patch_off: row offsets of the patches ON THE DEVICE; runs: where those rows come from in the host arrays
 int yawb_index_upload(yawb_ctx *ctx, yawb_cat *cat, const double *xyz, const double *w, const uint8_t *zbin8,
-                      const int32_t *zbin, const double *zred, const int64_t *patch_off);
+                      const int32_t *zbin, const double *zred, const int64_t *patch_off, const std::vector<RowRun> &runs);
+// second-role row mask (nullptr clears it); drops a built second-role index
+int yawb_index_set_second_rows(yawb_cat *cat, const uint8_t *mask);
+void yawb_index_free_second(yawb_cat *cat);
 // device memory (yawb_alloc.cu): stream-aware caching allocator on top of cudaMalloc
 int yawb_dalloc(yawb_ctx *ctx, void **out, size_t bytes, cudaStream_t st);
 void yawb_dfree(yawb_ctx *ctx, void *ptr, cudaStream_t st);

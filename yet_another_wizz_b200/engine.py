@@ -1,6 +1,8 @@
 """
-Thin object wrappers over the C ABI: `Engine` (one per process / GPU) and
-`DeviceCatalog` (one patch-partitioned catalog resident in HBM).
+Thin object wrappers over the C ABI: `Engine` (one context on one GPU),
+`DeviceCatalog` (one patch-partitioned catalog resident in HBM) and
+`EngineGroup` (several engines driven from one process, each holding its share of
+a measurement's catalogs).
 
 These are the B200 counterparts of the reference's worker pool
 (`src/yaw/utils/parallel.py:318-343`) and of its per-patch `BinnedTrees` cache
@@ -12,6 +14,7 @@ from __future__ import annotations
 import ctypes
 import os
 import weakref
+from concurrent.futures import ThreadPoolExecutor
 from ctypes import byref, c_double, c_int, c_int64, c_void_p
 
 import numpy as np
@@ -63,6 +66,17 @@ class DeviceCatalog:
         num = np.empty(self.n_patch, dtype=np.int64)
         _lib.check(self.engine.lib.yawb_patch_metadata(self._h, _ptr(center), _ptr(chord), _ptr(num)))
         return center, 2.0 * np.arcsin(np.minimum(chord / 2.0, 1.0)), num
+
+    def set_second_rows(self, mask: np.ndarray | None) -> None:
+        """Rows of the second-role index (`yawb_catalog_set_second_rows`): one byte per uploaded row (for a partial
+        upload the rows of the kept patches, in patch order), 0 = left out; None clears the mask.  The first role,
+        `sum_weights` and `info` keep every row."""
+        if mask is not None:
+            mask = np.ascontiguousarray(mask, dtype=np.uint8)
+            n_rows = self._n_uploaded
+            if len(mask) != n_rows:
+                raise ValueError(f"the mask needs one byte per uploaded row ({n_rows}), got {len(mask)}")
+        _lib.check(self.engine.lib.yawb_catalog_set_second_rows(self._h, _ptr(mask)))
 
     def info(self) -> tuple[int, int]:
         n, nbytes = c_int64(), c_int64()
@@ -143,6 +157,8 @@ class Engine:
         edges: np.ndarray | None = None,
         closed: str = "right",
         n_labels: int | None = None,
+        keep: np.ndarray | None = None,
+        second_rows: np.ndarray | None = None,
     ) -> DeviceCatalog:
         """`zbin` (+ `n_bins`): z-bin ids assigned on the host; or `redshifts` + `edges` (+ `closed`): the raw
         redshifts travel and the device assigns the bins with np.digitize's comparisons (`yawb_upload_catalog_z`,
@@ -150,7 +166,11 @@ class Engine:
 
         `n_labels` (with `zbin`): binned labels (`yawb_catalog_set_labels`), the ids are `label * B + z-bin` with
         `B = n_bins // n_labels`, e.g. the tomographic bins of a sample, each z-binned (`prepare_labelled_arrays`
-        with a binning).  `count` then pairs label by label; see there."""
+        with a binning).  `count` then pairs label by label; see there.
+
+        `keep` (one flag per patch): only the rows of the kept patches travel (`yawb_upload_catalog_patches`), straight
+        from these arrays; an unkept patch is an empty patch.  `second_rows`: the mask of `DeviceCatalog.set_second_rows`,
+        one byte per row that travels."""
         if n_labels is not None:
             if zbin is None:
                 raise ValueError("'n_labels' needs z-bin ids ('zbin')")
@@ -185,6 +205,21 @@ class Engine:
             if len(redshifts) != n:
                 raise ValueError("shape of 'xyz' and 'redshifts' does not match")
             n_bins = len(edges) - 1
+        n_rows = n
+        if keep is not None:
+            keep = np.ascontiguousarray(keep, dtype=np.uint8)
+            if len(keep) != len(patch_off) - 1:
+                raise ValueError("'keep' needs one flag per patch")
+            n_rows = int(np.diff(patch_off)[keep != 0].sum())
+            z8 = zbin is not None and zbin.dtype == np.uint8
+            _lib.check(
+                self.lib.yawb_upload_catalog_patches(
+                    self._h, _ptr(xyz), _ptr(weights), None if z8 else _ptr(zbin), _ptr(zbin) if z8 else None,
+                    _ptr(redshifts), _ptr(edges), int(str(closed) == "right"), _ptr(patch_off), len(patch_off) - 1,
+                    int(n_bins), _ptr(keep), byref(h),
+                )
+            )
+        elif redshifts is not None:
             _lib.check(
                 self.lib.yawb_upload_catalog_z(
                     self._h, _ptr(xyz), _ptr(weights), _ptr(redshifts), _ptr(edges), int(str(closed) == "right"),
@@ -200,13 +235,16 @@ class Engine:
             )
         binned = zbin is not None or redshifts is not None
         cat = DeviceCatalog(self, h, len(patch_off) - 1, int(n_bins) if binned else 1, binned, weights is not None)
-        if n_labels is not None:
-            try:
+        cat._n_uploaded = n_rows
+        try:
+            if n_labels is not None:
                 _lib.check(self.lib.yawb_catalog_set_labels(h, int(n_labels)))
-            except Exception:
-                cat.free()
-                raise
-            cat.n_labels = int(n_labels)
+                cat.n_labels = int(n_labels)
+            if second_rows is not None:
+                cat.set_second_rows(second_rows)
+        except Exception:
+            cat.free()
+            raise
         # the upload is asynchronous: keep the host buffers alive as long as the handle
         cat._keepalive = (xyz, weights, zbin, redshifts, patch_off)
         self._catalogs.add(cat)
@@ -547,6 +585,184 @@ class Engine:
             self._stage_used.clear()
             self.lib.yawb_destroy(self._h)
             self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class GroupCatalog:
+    """One catalog of a measurement call on the devices of an `EngineGroup`: `parts[d]` is device d's upload (its kept
+    patches, second-role rows masked to its strips), `plan` the `SharePlan` it was made for."""
+
+    def __init__(self, parts: list, plan, resident: list[bool]) -> None:
+        self.parts = parts
+        self.plan = plan
+        self._resident = resident  # parts owned by their engine's catalog cache (not freed here)
+        first = parts[0]
+        self.n_patch, self.n_bins, self.binned, self.weighted = first.n_patch, first.n_bins, first.binned, first.weighted
+        self.n_labels = getattr(first, "n_labels", None)
+
+    def sum_weights(self) -> np.ndarray:
+        """`(n_bins, n_patch)`, every patch from the first device that uploaded it"""
+        out = None
+        done = np.zeros(self.n_patch, dtype=bool)
+        for part, keep in zip(self.parts, self.plan.keep):
+            take = keep.astype(bool) & ~done
+            if not take.any():
+                continue
+            sw = part.sum_weights()
+            if out is None:
+                out = np.zeros_like(sw)
+            out[:, take] = sw[:, take]
+            done |= take
+        return out
+
+    def free(self) -> None:
+        for part, resident in zip(self.parts, self._resident):
+            if not resident:
+                part.free()
+
+
+class EngineGroup:
+    """Several engines driven from one process: a measurement function called with `engine=EngineGroup([0, 1, ...])`
+    splits its pair counts over the devices and returns what the same call on one `Engine` returns.
+
+    Every call cuts the patches of its second catalogs into one share per device (`sharding.plan_shares`: the exact
+    fractional split of the pair costs, a patch at a cut shared as two compact strips of rows).  Each device uploads,
+    of every catalog of the call, only its own patches and the patches linked to them, counts the pairs whose second
+    patch it owns against its strips, and the histograms are summed on the host in device order (integers exactly,
+    float sums to rounding).  No device holds a whole catalog, so a measurement larger than one GPU's memory fits on
+    several.
+
+    `devices`: CUDA device ids (a device may repeat, e.g. `[0, 0]`) or existing engine objects.  One worker thread per
+    engine uploads and counts; the library releases the GIL.  Patch centres (`kmeans`, `assign_patches`) stay on
+    `Engine`.  Not combined with `shard=` (one process per GPU under torchrun)."""
+
+    def __init__(self, devices) -> None:
+        devices = list(devices)
+        if not devices:
+            raise ValueError("an EngineGroup needs at least one device")
+        created = []
+        try:
+            for d in devices:
+                if isinstance(d, (int, np.integer)):
+                    created.append(Engine(int(d)))
+            it = iter(created)
+            self.engines = [next(it) if isinstance(d, (int, np.integer)) else d for d in devices]
+        except Exception:
+            for e in created:
+                e.close()
+            raise
+        self._own = created
+        if len({id(e) for e in self.engines}) != len(self.engines):
+            raise ValueError("an engine object may appear only once in an EngineGroup (a context serves one thread)")
+        self._pool = ThreadPoolExecutor(max_workers=len(self.engines), thread_name_prefix="yawb-group")
+
+    def __len__(self) -> int:
+        return len(self.engines)
+
+    def _map(self, fn):
+        """fn(d, engine) for every device, concurrently; results in device order"""
+        futures = [self._pool.submit(fn, d, e) for d, e in enumerate(self.engines)]
+        return [f.result() for f in futures]
+
+    # ---- uploads --------------------------------------------------------------------------------------
+    def cache_lookup(self, catalog, signature, kappa: bool, plan):
+        """a `GroupCatalog` if every engine keeps this catalog uploaded for its share of `plan`, else None"""
+        parts = []
+        for d, e in enumerate(self.engines):
+            lookup = getattr(e, "cache_lookup", None)
+            dev = lookup(catalog, (signature, plan.signature(d)), kappa) if lookup else None
+            if dev is None:
+                return None
+            parts.append(dev)
+        return GroupCatalog(parts, plan, [True] * len(parts))
+
+    def upload_catalog(self, arrays: dict, plan, cache=None) -> GroupCatalog:
+        """`arrays`: the keyword arguments of `Engine.upload_catalog` for the whole catalog (`xyz`, `patch_off`, ...);
+        device d uploads the patches `plan.keep[d]` with the second-role rows of its strips.  `cache = (catalog,
+        signature, kappa)`: each part is kept in its engine's catalog cache under the signature and its share."""
+        arrays = dict(arrays)
+        xyz, patch_off = arrays.pop("xyz"), arrays.pop("patch_off")
+
+        def one(d, e):
+            dev = e.upload_catalog(xyz, patch_off, keep=plan.keep[d], second_rows=plan.mask(d, xyz, patch_off), **arrays)
+            store = getattr(e, "cache_store", None)
+            resident = bool(cache is not None and store and store(cache[0], (cache[1], plan.signature(d)), cache[2], dev))
+            return dev, resident
+
+        parts = self._map(one)
+        return GroupCatalog([p for p, _ in parts], plan, [r for _, r in parts])
+
+    # ---- counts ---------------------------------------------------------------------------------------
+    @staticmethod
+    def _merge(n_pairs: int, results, n_out: int):
+        """per device (rows, [(counts, sums)] * n_out, stats) -> the outputs over the full pair list, summed in device
+        order; counters summed, times of the slowest device"""
+        outs, stats = [], {}
+        for t in range(n_out):
+            full = [None, None]
+            for rows, dev_outs, _ in results:
+                for k, arr in enumerate(dev_outs[t]):
+                    if full[k] is None:
+                        shape = list(arr.shape)
+                        shape[arr.ndim - 3] = n_pairs  # the pair axis, behind a leading label axis if any
+                        full[k] = np.zeros(shape, dtype=arr.dtype)
+                    idx = (slice(None),) * (arr.ndim - 3) + (rows,)
+                    full[k][idx] += arr
+            outs.append(tuple(full))
+        for _, _, st in results:
+            for key, v in st.items():
+                stats[key] = max(stats.get(key, 0), v) if key.endswith("_ms") else stats.get(key, 0) + v
+        return outs, stats
+
+    def _fan_out(self, second: GroupCatalog, pair_i, pair_j, count_one):
+        """`count_one(d, engine, pair_i, pair_j) -> ([(counts, sums), ...], stats)` on every device over the pairs whose
+        second patch it owns; returns (n_pairs, [(rows, outputs, stats)] in device order)"""
+        pair_i = np.ascontiguousarray(pair_i, dtype=np.int32)
+        pair_j = np.ascontiguousarray(pair_j, dtype=np.int32)
+
+        def one(d, e):
+            rows = np.flatnonzero(second.plan.second[d][pair_j])
+            outs, stats = count_one(d, e, pair_i[rows], pair_j[rows])
+            return rows, outs, stats
+
+        return len(pair_i), self._map(one)
+
+    def count(self, cat1: GroupCatalog, cat2: GroupCatalog, pair_i, pair_j, r2_edges, **kw):
+        """`Engine.count` over the devices: each counts the pairs whose second patch it owns"""
+        def one(d, e, pi, pj):
+            counts, sums, stats = e.count(cat1.parts[d], cat2.parts[d], pi, pj, r2_edges, **kw)
+            return [(counts, sums)], stats
+
+        n, res = self._fan_out(cat2, pair_i, pair_j, one)
+        (out,), stats = self._merge(n, res, 1)
+        return (*out, stats)
+
+    def count2(self, cat1a: GroupCatalog, cat1b: GroupCatalog, cat2: GroupCatalog, pair_i, pair_j, r2_edges, **kw):
+        """`Engine.count2` over the devices"""
+        def one(d, e, pi, pj):
+            a, b, stats = e.count2(cat1a.parts[d], cat1b.parts[d], cat2.parts[d], pi, pj, r2_edges, **kw)
+            return [a, b], stats
+
+        n, res = self._fan_out(cat2, pair_i, pair_j, one)
+        (a, b), stats = self._merge(n, res, 2)
+        return a, b, stats
+
+    def sync(self) -> None:
+        self._map(lambda d, e: e.sync())
+
+    def close(self) -> None:
+        """shut the worker threads down and close the engines the group created (engines passed in stay open)"""
+        if self._pool is not None:
+            self._pool.shutdown(wait=True)
+            self._pool = None
+        for e in self._own:
+            e.close()
+        self._own = []
 
     def __del__(self):
         try:

@@ -32,7 +32,7 @@ from .catalog import InconsistentPatchesError
 from .coordinates import AngularCoordinates, AngularDistances
 from .corrfunc import CorrFunc, ScalarCorrFunc
 from .paircounts import NormalisedCounts, NormalisedScalarCounts, PatchedCounts, PatchedSumWeights
-from .sharding import Shard, assign_pairs_lpt, current_shard, pair_costs
+from .sharding import Shard, assign_pairs_lpt, current_shard, pair_costs, plan_shares
 
 __all__ = ["PatchLinkage", "autocorrelate", "autocorrelate_scalar", "autocorrelate_tomographic",
            "compute_scalar_normalisation", "crosscorrelate", "crosscorrelate_scalar", "crosscorrelate_tomographic",
@@ -262,21 +262,19 @@ def _prepare_for(engine, catalog, binning: Binning | None, kappa: bool) -> dict:
                                   device_digitize=bool(getattr(engine, "device_digitize", False)))
 
 
-def upload_catalog(engine, catalog, binning: Binning | None, *, kappa: bool = False):
-    """Replaces `Catalog.build_trees`: one upload, the index is built on the device."""
-    arrays = _prepare_for(engine, catalog, binning, kappa)
-    return engine.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
-
-
 class _Uploads:
     """Device catalogs of one measurement call, uploaded once and shared by DD/DR/RD/RR.
 
     `enqueue` takes the catalogs of the call in the order they should travel: their host preparation
     (numpy releases the GIL) runs one catalog ahead on a helper thread, so preparing catalog k + 1
-    overlaps with the copy of catalog k, which for pageable host memory blocks the calling thread."""
+    overlaps with the copy of catalog k, which for pageable host memory blocks the calling thread.
 
-    def __init__(self, engine) -> None:
+    On an `EngineGroup` every catalog is prepared once on the host and uploaded in shares: `plan` (the call's
+    `SharePlan`) says which patches and rows each device holds."""
+
+    def __init__(self, engine, plan=None) -> None:
         self.engine = engine
+        self.plan = plan
         self._resident: set = set()  # keys whose device catalog belongs to the engine's cache (not freed here)
         self._cache: dict[tuple[int, bool, bool], object] = {}
         self._pending: dict[tuple[int, bool, bool], object] = {}
@@ -299,12 +297,34 @@ class _Uploads:
 
     def _resident_lookup(self, key, catalog, binning, kappa) -> bool:
         lookup = getattr(self.engine, "cache_lookup", None)
+        if self._group():  # the parts stay with their engines' caches: the GroupCatalog itself is not resident
+            dev = self.engine.cache_lookup(catalog, self._signature(catalog, binning), kappa, self.plan)
+            if dev is not None:
+                self._cache[key] = dev
+            return dev is not None
         dev = lookup(catalog, self._signature(catalog, binning), kappa) if lookup else None
         if dev is None:
             return False
         self._cache[key] = dev
         self._resident.add(key)
         return True
+
+    def _group(self) -> bool:
+        from .engine import EngineGroup
+
+        if not isinstance(self.engine, EngineGroup):
+            return False
+        if self.plan is None:
+            raise ValueError("an EngineGroup counts through the measurement functions, which plan its shares")
+        return True
+
+    def _upload(self, key, catalog, binning, kappa, arrays):
+        if self._group():
+            dev = self.engine.upload_catalog(arrays, self.plan, cache=(catalog, self._signature(catalog, binning), kappa))
+            self._cache[key] = dev
+            return dev
+        dev = self.engine.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
+        return self._store(key, catalog, binning, kappa, dev)
 
     def _store(self, key, catalog, binning, kappa, dev):
         self._cache[key] = dev
@@ -335,16 +355,14 @@ class _Uploads:
 
     def _resolve(self, key):
         fut, catalog, binning, kappa = self._pending.pop(key)
-        arrays = fut.result()
-        dev = self.engine.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
-        return self._store(key, catalog, binning, kappa, dev)
+        return self._upload(key, catalog, binning, kappa, fut.result())
 
     def get(self, catalog, binning: Binning | None, kappa: bool = False):
         key = self._key(catalog, binning, kappa)
         if key in self._pending:
             return self._resolve(key)
         if key not in self._cache and not self._resident_lookup(key, catalog, binning, kappa):
-            self._store(key, catalog, binning, kappa, upload_catalog(self.engine, catalog, binning, kappa=kappa))
+            self._upload(key, catalog, binning, kappa, _prepare_for(self.engine, catalog, binning, kappa))
         return self._cache[key]
 
     def get_labelled(self, catalogs, binning: Binning | None = None):
@@ -354,9 +372,7 @@ class _Uploads:
         catalogs = tuple(catalogs)
         key = (("labelled", *map(id, catalogs)), binning is not None, False)
         if key not in self._cache and not self._resident_lookup(key, catalogs, binning, False):
-            arrays = prepare_labelled_arrays(catalogs, binning)
-            dev = self.engine.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
-            self._store(key, catalogs, binning, False, dev)
+            self._upload(key, catalogs, binning, False, prepare_labelled_arrays(catalogs, binning))
         return self._cache[key]
 
     def free(self) -> None:
@@ -614,6 +630,28 @@ def _own_pairs(shard: Shard, ij, n1_per_patch, n2_per_patch, radii1) -> np.ndarr
     return assign_pairs_lpt(costs, shard.world_size)[shard.rank]
 
 
+def _share_plan(engine, shard: Shard | None, catalogs, counts):
+    """The `SharePlan` of a call on an `EngineGroup` (None on a single engine).  `catalogs`: the catalogs of the
+    linkage (the largest gives the patch centres and radii, as for the links); `counts`: `(pair_i, pair_j, first,
+    second)` of every pair count of the call, `pair_j` the patches of the second catalog, `first` / `second` rows per
+    patch."""
+    from .engine import EngineGroup
+
+    if not isinstance(engine, EngineGroup):
+        return None
+    if (shard or current_shard()).active:
+        raise ValueError("an EngineGroup splits a call over the GPUs of one process; it cannot be combined with an "
+                         "active shard (one process per GPU)")
+    ref = max(catalogs, key=lambda c: tuple(c.get_num_records()))
+    centers = AngularCoordinates(_coords_data(ref.get_centers())).to_3d()
+    counts = [(pi, pj, np.asarray(n1, dtype=np.float64), np.asarray(n2, dtype=np.float64)) for pi, pj, n1, n2 in counts]
+    return plan_shares(counts, _coords_data(ref.get_radii()), centers, len(engine))
+
+
+def _rows(catalog):
+    return np.asarray(catalog.get_num_records(), dtype=np.float64)
+
+
 def _reduce(engine, shard: Shard, hist: np.ndarray, own: np.ndarray, n_pairs: int, *, labelled: bool) -> np.ndarray:
     """the histograms of the pairs `own` placed into the full pair axis (behind the leading label axis if `labelled`)
     and summed over the ranks"""
@@ -677,7 +715,11 @@ def autocorrelate(config, data, random, *, count_rr: bool = True, progress: bool
     `progress` / `max_workers` are accepted and ignored."""
     _ensure_unique_catalogs(data, random)
     links = PatchLinkage.from_catalogs(config, data, random, engine=engine, shard=shard)
-    links._uploads = _Uploads(engine or get_default_engine())
+    auto_ij, cross_ij = links.get_patch_id_pairs(auto=True), links.get_patch_id_pairs(auto=False)
+    nd, nr = _rows(data), _rows(random)
+    plan = _share_plan(engine, shard, (data, random), [(*auto_ij, nd, nd), (*cross_ij, nd, nr)]
+                       + ([(*auto_ij, nr, nr)] if count_rr else []))
+    links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     try:
         binning = _as_binning(config)
@@ -704,7 +746,11 @@ def crosscorrelate(config, reference, unknown, *, ref_rand=None, unk_rand=None, 
     randoms = [cat for cat in (ref_rand, unk_rand) if cat is not None]
 
     links = PatchLinkage.from_catalogs(config, reference, unknown, *randoms, engine=engine, shard=shard)
-    links._uploads = _Uploads(engine or get_default_engine())
+    ij = links.get_patch_id_pairs(auto=False)
+    plan = _share_plan(engine, shard, (reference, unknown, *randoms),
+                       [(*ij, _rows(c1), _rows(c2)) for c1 in (reference, ref_rand) if c1 is not None
+                        for c2 in (unknown, unk_rand) if c2 is not None])
+    links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     kw = dict(binned_second=False)
     try:
@@ -767,6 +813,11 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
         else ref_rand
     own = _own_pairs(shard, ij, first.get_num_records(), np.sum([u.get_num_records() for u in unknowns], axis=0),
                      first.get_radii().data)
+    n_unk = np.sum([_rows(u) for u in unknowns], axis=0)
+    n_ur = None if unk_rand is None else _rows(unk_rand) if shared else np.sum([_rows(r) for r in rands], axis=0)
+    uploads.plan = _share_plan(engine, shard, (reference, *unknowns, *[c for c in (ref_rand, *rands) if c is not None]),
+                               [(*ij, _rows(c1), n2) for c1 in (reference, ref_rand) if c1 is not None
+                                for n2 in (n_unk, n_ur) if n2 is not None])
     fuse = _fuse(eng, reference, ref_rand)
     counts: dict[str, tuple] = {}
     try:
@@ -898,6 +949,10 @@ def autocorrelate_tomographic(config, data, random, *, count_rr: bool = True, pr
     own_auto_dd = _own_pairs(shard, auto_ij, n_data, n_data, radii)
     own_cross = _own_pairs(shard, cross_ij, n_data, n_rand, radii)
     own_auto_rr = _own_pairs(shard, auto_ij, n_rand, n_rand, radii)
+    # with shared randoms DR is counted with the pair lists swapped: the data sample is the second catalog
+    dr_pairs = (cross_ij[1], cross_ij[0], n_rand, n_data) if shared else (*cross_ij, n_data, n_rand)
+    uploads.plan = _share_plan(engine, shard, (*data, *rands), [(*auto_ij, n_data, n_data), dr_pairs]
+                               + ([(*auto_ij, n_rand, n_rand)] if count_rr else []))
 
     counts: dict[str, tuple] = {}
     try:
@@ -931,7 +986,11 @@ def compute_scalar_normalisation(catalog, binning: Binning, *, engine=None, uplo
     """Mean-kappa correction per patch and z-bin: sum(kappa x w) and sum(w) on the diagonal of two
     `PatchedCounts` (`compute_scalar_normalisation`, `measurements.py:634-648`).  Both sums are the
     per-(bin, patch) weight sums the device already computes for its catalogs."""
+    from .engine import EngineGroup
+
     own = uploads is None
+    if own and isinstance(engine, EngineGroup):  # per-patch sums need no share of the devices
+        engine = engine.engines[0]
     uploads = uploads or _Uploads(engine or get_default_engine())
     try:
         num_bins, num_patches = len(binning), len(catalog)
@@ -952,7 +1011,9 @@ def autocorrelate_scalar(config, data, *, progress: bool = False, max_workers=No
     """Angular autocorrelation of a scalar field in z-bins: KK and NN counts of the data sample.
     Signature and result layout of `yaw.autocorrelate_scalar` (`measurements.py:651-705`)."""
     links = PatchLinkage.from_catalogs(config, data, engine=engine, shard=shard)
-    links._uploads = _Uploads(engine or get_default_engine())
+    nd = _rows(data)
+    plan = _share_plan(engine, shard, (data,), [(*links.get_patch_id_pairs(auto=True), nd, nd)])
+    links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     try:
         DD = links.count_scalar_pairs(data, mode="kk", count_type_info="DD")
@@ -971,7 +1032,10 @@ def crosscorrelate_scalar(config, reference, unknown, *, unk_rand=None, progress
     _ensure_unique_catalogs(reference, unknown, unk_rand)
     randoms = [unk_rand] if unk_rand is not None else []
     links = PatchLinkage.from_catalogs(config, reference, unknown, *randoms, engine=engine, shard=shard)
-    links._uploads = _Uploads(engine or get_default_engine())
+    ij = links.get_patch_id_pairs(auto=False)
+    plan = _share_plan(engine, shard, (reference, unknown, *randoms),
+                       [(*ij, _rows(reference), _rows(c2)) for c2 in (unknown, *randoms)])
+    links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     kw = dict(binned_second=False, mode="kn")
     try:

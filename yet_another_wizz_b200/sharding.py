@@ -18,8 +18,8 @@ import os
 
 import numpy as np
 
-__all__ = ["Shard", "assign_pairs_lpt", "assign_patches_contiguous", "assign_patch_fractions", "split_rows", "current_shard",
-           "pair_costs"]
+__all__ = ["SharePlan", "Shard", "assign_pairs_lpt", "assign_patches_contiguous", "assign_patch_fractions", "split_rows",
+           "current_shard", "pair_costs", "plan_shares"]
 
 
 def pair_costs(pair_i, pair_j, n1_per_patch, n2_per_patch, radii1=None) -> np.ndarray:
@@ -150,6 +150,68 @@ def split_rows(xyz: np.ndarray, f0: float, f1: float) -> np.ndarray:
     key = lon if span_lon >= (lat.max() - lat.min() if n else 0.0) else lat
     order = np.argsort(key, kind="stable")
     return np.sort(order[int(round(f0 * n)):int(round(f1 * n))])
+
+
+class SharePlan:
+    """Which device of an `EngineGroup` holds and counts what in one measurement call.
+
+    `shares[d]`: the (patch, f0, f1) of `assign_patch_fractions` -- device d counts the pairs whose second patch is one of
+    these, against the `split_rows` strip [f0, f1) of that patch's rows (a patch split between two devices is counted
+    by both, each on its own strip).  `keep[d]`: the patches device d uploads, its own plus every patch linked to one of
+    them in a pair list of the call, so that one upload per catalog and device serves as first and as second catalog."""
+
+    def __init__(self, shares: list[list[tuple[int, float, float]]], keep: list[np.ndarray]) -> None:
+        self.shares = shares
+        self.keep = keep
+        n_patch = len(keep[0]) if keep else 0
+        self.second = []  # per device: (n_patch,) bool, the second patches it counts
+        for mine in shares:
+            own = np.zeros(n_patch, dtype=bool)
+            own[[p for p, _, _ in mine]] = True
+            self.second.append(own)
+
+    @property
+    def n_devices(self) -> int:
+        return len(self.shares)
+
+    def mask(self, d: int, xyz: np.ndarray, patch_off: np.ndarray) -> np.ndarray:
+        """second-role rows of device d: one byte per row of its kept patches (in patch order), 1 for the rows of its
+        strips.  `xyz` / `patch_off`: the whole catalog."""
+        keep = self.keep[d].astype(bool)
+        sizes = np.diff(patch_off)
+        dev_off = np.concatenate([[0], np.cumsum(np.where(keep, sizes, 0))])
+        out = np.zeros(int(dev_off[-1]), dtype=np.uint8)
+        for p, f0, f1 in self.shares[d]:
+            s, e = int(patch_off[p]), int(patch_off[p + 1])
+            out[dev_off[p] + split_rows(xyz[s:e], f0, f1)] = 1
+        return out
+
+    def signature(self, d: int) -> tuple:
+        """what device d's uploads depend on besides the catalog: its kept patches and strips (they fix the mask)"""
+        return (self.keep[d].tobytes(), tuple(self.shares[d]))
+
+
+def plan_shares(counts, radii1, centers_xyz, n_devices: int) -> SharePlan:
+    """The share plan of one call.  `counts`: the pair counts of the call, each `(pair_i, pair_j, n1_per_patch,
+    n2_per_patch)` with `pair_j` the patches of the second catalog.  The cost of a second patch is the sum of
+    `pair_costs` over every pair that names it; `assign_patch_fractions` cuts the patches, ordered along the curve of
+    their centres, into `n_devices` parts of equal cost."""
+    n_patch = len(centers_xyz)
+    cost = np.zeros(n_patch)
+    for pi, pj, n1, n2 in counts:
+        np.add.at(cost, np.asarray(pj), pair_costs(pi, pj, n1, n2, radii1=radii1))
+    shares = assign_patch_fractions(cost, centers_xyz, n_devices)
+    keep = []
+    for mine in shares:
+        own = np.zeros(n_patch, dtype=bool)
+        own[[p for p, _, _ in mine]] = True
+        k = own.copy()
+        for pi, pj, _, _ in counts:
+            pi, pj = np.asarray(pi), np.asarray(pj)
+            k[pi[own[pj]]] = True
+            k[pj[own[pi]]] = True
+        keep.append(k.astype(np.uint8))
+    return SharePlan(shares, keep)
 
 
 class Shard:
