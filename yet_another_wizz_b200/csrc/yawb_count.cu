@@ -50,10 +50,11 @@ struct FastParams {
     const PatchFrame *sframe;
     int n_types;
     float zeta;  // max | |P|^2 - 1 | over the rows of the second catalog(s), rounded up: part of the FP32 error bound
-    // second catalog (register tiles): 32-byte row records (row j = rx[4 j .. 4 j + 2]) and optional weights;
-    // rx2 / rw2 = second catalog of a joint launch (Item::src == 1, yawb_count4)
+    // second catalog (register tiles): 32-byte row records (row j = rx[4 j .. 4 j + 3], the last double its catalog) and
+    // optional weights; rx2 / rw2 = second index of a joint launch (Item::src == 1, yawb_count4)
     const double *rx, *rw;
     const double *rx2, *rw2;
+    int n_sec;  // second catalogs whose counts a tile splits: 2 for tiles over the union of two catalogs, else 1
     // work items written by the planner: patch-diagonal items first, then the boundary items
     const Item *items_heavy, *items_light;
     long long cap_heavy, cap_light;
@@ -143,6 +144,7 @@ constexpr int HPL = YAWB_RPL / 2;  // row pairs per lane
 // ---- the paths of the streaming kernel; the host picks one per count (yawb_launch_count_fast) ---------------
 enum class CountPath {
     Single,             // unweighted, one sub-bin: saturating ramp (stream_test_sat)
+    SingleUnion,        // the same on tiles over the union of two second catalogs: counts split by each row's catalog
     SingleWeighted,     // weighted, one sub-bin: predicated test, weighted sums (phase2_single)
     Cumulative,         // unweighted, a few sub-bins: cumulative counts with the saturating ramp (phase2_cumul)
     Histogram,          // unweighted, many sub-bins: in-range tests classified into a histogram (phase2_multi_queue)
@@ -151,7 +153,8 @@ enum class CountPath {
 __host__ __device__ constexpr bool path_weighted(CountPath p) {
     return p == CountPath::SingleWeighted || p == CountPath::HistogramWeighted;
 }
-__host__ __device__ constexpr bool path_multi(CountPath p) { return p != CountPath::Single && p != CountPath::SingleWeighted; }
+__host__ __device__ constexpr bool path_sat(CountPath p) { return p == CountPath::Single || p == CountPath::SingleUnion; }
+__host__ __device__ constexpr bool path_multi(CountPath p) { return !path_sat(p) && p != CountPath::SingleWeighted; }
 
 // ---- a warp's block of shared memory in the streaming kernel (yawb_count_stream.cuh) ----------------------
 constexpr int LB = 128;   // rows per raw chunk = capacity of the staged list
@@ -201,7 +204,7 @@ struct StreamSmem {
     SegDesc *seg;              // [n_types * n_bins]
     float4 *binrec;            // [n_bins] half extents of the query box (x, y, z) and mid
     float2 *binthr;            // [n_bins] thresholds of the pair test
-    unsigned long long *acc;   // [n_types][n_bins * nsub]
+    unsigned long long *acc;   // [n_sec][n_types][n_bins * nsub]
     double *accw;              // same (weighted paths)
     unsigned *hist;            // [nsub] scratch histogram of one z-bin segment (sub-bin paths)
     double *histw;             // [nsub] (HistogramWeighted)
@@ -241,6 +244,8 @@ __device__ __forceinline__ void recheck_chunk(const FastParams &P, const StreamS
 // The same for a span [e0, e1) of at most 16 entries (the streaming kernel checks once per <= 16 candidates): lane t
 // takes row t & 7 of lane `src` against candidates t >> 3, t >> 3 + 4, ...; all operands of a lane's (up to four)
 // tests are requested before the first is used, so the warp pays the memory latency once (unweighted single-bin path).
+// The count is returned split by the catalog of the row in the index (the fourth double of its record): pairs with
+// rows of catalog 0 in the low 16 bits, with rows of catalog 1 in the high 16 bits (stream_test_sat).
 __device__ __forceinline__ void recheck_span(const FastParams &P, const StreamSmem &S, int e0, int e1,
                                              const Tile &tl, int lane, int src, double lo, double hi,
                                              unsigned &cnt_out, unsigned &n_recheck) {
@@ -250,8 +255,10 @@ __device__ __forceinline__ void recheck_span(const FastParams &P, const StreamSm
     const int k = src + 32 * (lane & 7);
     const bool row_ok = k < tl.count;
     const int j = tl.start + (row_ok ? k : 0);
-    const double *const trow = YAWB_TILE_ROWS(P, tl);
-    const double bx = trow[(size_t)YAWB_RSTRIDE * j], by = trow[(size_t)YAWB_RSTRIDE * j + 1], bz = trow[(size_t)YAWB_RSTRIDE * j + 2];
+    const double2 *const row = reinterpret_cast<const double2 *>(YAWB_TILE_ROWS(P, tl) + (size_t)YAWB_RSTRIDE * j);
+    const double2 ra = row[0], rb = row[1];
+    const double bx = ra.x, by = ra.y, bz = rb.x;
+    const unsigned one = rb.y != 0.0 ? 0x10000u : 1u;
     double ax[Q], ay[Q], az[Q];
     bool ok[Q];
 #pragma unroll
@@ -265,7 +272,7 @@ __device__ __forceinline__ void recheck_span(const FastParams &P, const StreamSm
     for (int q = 0; q < Q; ++q) {
         const double d2 = exact_d2(ax[q], ay[q], az[q], bx, by, bz);
         if (ok[q]) {
-            if (d2 > lo && d2 <= hi) cnt += 1;
+            if (d2 > lo && d2 <= hi) cnt += one;
             n_recheck += 1;
         }
     }
@@ -277,14 +284,14 @@ __device__ __forceinline__ void recheck_span(const FastParams &P, const StreamSm
 //   unweighted: v = sat(C - K |u|) is a ramp through the uncertainty band: exactly 1 well inside the bin,
 //        exactly 0 well outside, in [0.1, 0.9] wherever FP32 cannot decide (K = 0.4 / eps,
 //        C = 1/2 + h K).  sum(v) and sum(v*v) are equal iff every v of the chunk was 0 or 1 (then
-//        sum(v) is the exact count); an undecidable test makes them differ by >= 0.09;
+//        sum(v) is the exact count); an undecidable test makes them differ by >= 0.09.  With NA = HPL accumulators
+//        sum(v) is kept per register pair (rows 2k, 2k+1), so that the count splits by the catalog of each row;
 //   weighted (predicated): |u| < h - eps, |u| < h + eps (2 FSETP) + 2 predicated FADD, also feeds the weighted sums.
-// Two accumulator pairs (even / odd rows) halve the length of the dependent add chains.
-template <bool WEIGHTED>
-__device__ __forceinline__ void test_candidate(const Cand c, double swt, const float2 (&rx)[HPL],
-                                               const float2 (&ry)[HPL], const float2 (&rz)[HPL],
-                                               float ta, float tb, float2 &acc_a,
-                                               float2 &acc_b, double (&ws)[YAWB_RPL]) {
+//        Two accumulator pairs (even / odd rows) halve the length of the dependent add chains.
+template <int NA>
+__device__ __forceinline__ void test_candidate_sat(const Cand c, const float2 (&rx)[HPL], const float2 (&ry)[HPL],
+                                                   const float2 (&rz)[HPL], float ta, float tb, float2 (&acc_a)[NA],
+                                                   float2 &acc_b) {
     // Blackwell packed FP32: one FFMA2 / FADD2 carries two pair tests (rows 2k and 2k+1 of the lane)
     const float2 sx = make_float2(c.x, c.x), sy = make_float2(c.y, c.y);
     const float2 sz = make_float2(c.z, c.z), sw = make_float2(c.w, c.w);
@@ -293,24 +300,35 @@ __device__ __forceinline__ void test_candidate(const Cand c, double swt, const f
         float2 u = __ffma2_rn(rx[k], sx, sw);
         u = __ffma2_rn(ry[k], sy, u);
         u = __ffma2_rn(rz[k], sz, u);
-        if constexpr (!WEIGHTED) {
-            float2 v;
-            v.x = __saturatef(fmaf(fabsf(u.x), ta, tb));  // ta = -K, tb = C
-            v.y = __saturatef(fmaf(fabsf(u.y), ta, tb));
-            acc_a = __fadd2_rn(acc_a, v);
-            acc_b = __ffma2_rn(v, v, acc_b);
-        } else {
-            const float a0 = fabsf(u.x), a1 = fabsf(u.y);
-            const bool in0 = a0 < ta, in1 = a1 < ta;  // ta = h - eps, tb = h + eps
-            if (in0) acc_a.x += 1.f;
-            if (in1) acc_a.y += 1.f;
-            if (a0 < tb) acc_b.x += 1.f;
-            if (a1 < tb) acc_b.y += 1.f;
-            // ws += [in] * swt as one select on the high word of a 0.0 / 1.0 double plus one DFMA (a
-            // conditional FP64 add is lowered to an add plus two selects)
-            ws[2 * k] = fma(__hiloint2double(in0 ? 0x3ff00000 : 0, 0), swt, ws[2 * k]);
-            ws[2 * k + 1] = fma(__hiloint2double(in1 ? 0x3ff00000 : 0, 0), swt, ws[2 * k + 1]);
-        }
+        float2 v;
+        v.x = __saturatef(fmaf(fabsf(u.x), ta, tb));  // ta = -K, tb = C
+        v.y = __saturatef(fmaf(fabsf(u.y), ta, tb));
+        acc_a[k % NA] = __fadd2_rn(acc_a[k % NA], v);
+        acc_b = __ffma2_rn(v, v, acc_b);
+    }
+}
+
+__device__ __forceinline__ void test_candidate_w(const Cand c, double swt, const float2 (&rx)[HPL],
+                                                 const float2 (&ry)[HPL], const float2 (&rz)[HPL],
+                                                 float ta, float tb, float2 &acc_a,
+                                                 float2 &acc_b, double (&ws)[YAWB_RPL]) {
+    const float2 sx = make_float2(c.x, c.x), sy = make_float2(c.y, c.y);
+    const float2 sz = make_float2(c.z, c.z), sw = make_float2(c.w, c.w);
+#pragma unroll
+    for (int k = 0; k < HPL; ++k) {
+        float2 u = __ffma2_rn(rx[k], sx, sw);
+        u = __ffma2_rn(ry[k], sy, u);
+        u = __ffma2_rn(rz[k], sz, u);
+        const float a0 = fabsf(u.x), a1 = fabsf(u.y);
+        const bool in0 = a0 < ta, in1 = a1 < ta;  // ta = h - eps, tb = h + eps
+        if (in0) acc_a.x += 1.f;
+        if (in1) acc_a.y += 1.f;
+        if (a0 < tb) acc_b.x += 1.f;
+        if (a1 < tb) acc_b.y += 1.f;
+        // ws += [in] * swt as one select on the high word of a 0.0 / 1.0 double plus one DFMA (a
+        // conditional FP64 add is lowered to an add plus two selects)
+        ws[2 * k] = fma(__hiloint2double(in0 ? 0x3ff00000 : 0, 0), swt, ws[2 * k]);
+        ws[2 * k + 1] = fma(__hiloint2double(in1 ? 0x3ff00000 : 0, 0), swt, ws[2 * k + 1]);
     }
 }
 
@@ -330,10 +348,10 @@ __device__ __forceinline__ void phase2_single(const FastParams &P, const StreamS
         if (e1 - e0 == CHUNK) {  // common case: fully unrolled, no loop bookkeeping
 #pragma unroll
             for (int k = 0; k < CHUNK; ++k)
-                test_candidate<true>(S.list[e0 + k], S.lw[e0 + k], rx, ry, rz, ta, tb, acc_a, acc_b, ws);
+                test_candidate_w(S.list[e0 + k], S.lw[e0 + k], rx, ry, rz, ta, tb, acc_a, acc_b, ws);
         } else {
             for (int e = e0; e < e1; ++e)
-                test_candidate<true>(S.list[e], S.lw[e], rx, ry, rz, ta, tb, acc_a, acc_b, ws);
+                test_candidate_w(S.list[e], S.lw[e], rx, ry, rz, ta, tb, acc_a, acc_b, ws);
         }
         const float sa = acc_a.x + acc_a.y, sb = acc_b.x + acc_b.y;
         unsigned c = (unsigned)(sa + 0.5f);
@@ -824,9 +842,10 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
     P.cx[1] = fi->b ? fi->b->x : fi->a->x; P.cy[1] = fi->b ? fi->b->y : fi->a->y; P.cz[1] = fi->b ? fi->b->z : fi->a->z;
     P.sw = fi->sw; P.rec = fi->rec;
     P.cell_start = fi->cell_start; P.sgrid = fi->d_sgrid; P.sframe = fi->d_frames; P.n_types = fi->n_types;
-    P.rx = a.c2->rx; P.rw = a.c2->rw;
+    P.rx = a.r2[0]->rx; P.rw = a.r2[0]->rw;
     P.rx2 = P.rx; P.rw2 = P.rw;
-    if (a.c2b) { P.rx2 = a.c2b->rx; P.rw2 = a.c2b->rw; }
+    if (a.r2[1]) { P.rx2 = a.r2[1]->rx; P.rw2 = a.r2[1]->rw; }
+    P.n_sec = a.r2[0]->b ? 2 : 1;
     {
         // the pair test takes |r|^2 of a tile row from the identity for unit vectors (yawb_count_stream.cuh); rows
         // off the unit sphere by zeta widen the band of tests that are re-evaluated in FP64 (1e-15: the frames'
@@ -861,13 +880,13 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
     P.items_heavy = d_items;
     P.items_light = d_items + cap_heavy;
     P.cap_heavy = cap_heavy; P.cap_light = cap_light;
-    for (int sc = 0; sc < 2; ++sc) {  // one planner launch per second catalog, both append to the same two lists
-        const yawb_cat *c2 = sc ? a.c2b : a.c2;
+    for (int sc = 0; sc < 2; ++sc) {  // one planner launch per second-role index, both append to the same two lists
+        const RIndex *ri = a.r2[sc];
         const long long n_flat = sc ? a.n_items_b : a.n_items;
-        if (!c2 || n_flat == 0) continue;
+        if (!ri || n_flat == 0) continue;
         PlanParams Q{};
-        Q.tiles = c2->d_tiles; Q.tile_box = c2->d_tile_box; Q.ptile_off = c2->d_ptile_off;
-        Q.frames2 = c2->d_frames; Q.frames1 = fi->d_frames; Q.sgrid = fi->d_sgrid;
+        Q.tiles = ri->d_tiles; Q.tile_box = ri->d_tile_box; Q.ptile_off = ri->d_ptile_off;
+        Q.frames2 = ri->d_frames; Q.frames1 = fi->d_frames; Q.sgrid = fi->d_sgrid;
         Q.pair_i = a.d_pair_i; Q.pair_j = a.d_pair_j; Q.pair_item_base = sc ? a.d_pair_item_base_b : a.d_pair_item_base;
         Q.n_pairs = a.n_pairs; Q.n_flat = n_flat; Q.binpar = a.d_binpar; Q.n_bins = a.n_bins; Q.rmax_all = a.rmax_all;
         Q.heavy = d_items; Q.light = d_items + cap_heavy; Q.cap_heavy = cap_heavy; Q.cap_light = cap_light;
@@ -893,7 +912,8 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
         // the general sub-bin path sends every segment histogram straight to global atomics instead
         const size_t acc_bytes = (size_t)fi->n_types * a.n_bins * nsub * (a.weighted ? 16 : 8);
         P.acc_global = multi && !cumul && acc_bytes > 2048;
-        const size_t per_warp = stream_carve(nullptr, nullptr, a.weighted, multi, a.n_bins, nsub, fi->n_types, P.acc_global);
+        const size_t per_warp = stream_carve(nullptr, nullptr, a.weighted, multi, a.n_bins, nsub, fi->n_types, P.n_sec,
+                                             P.acc_global);
         const size_t smem = STREAM_WARPS * per_warp;
         YAWB_REQUIRE(smem <= 227 * 1024, "too many z-bins x sub-bins for the shared-memory accumulators (%zu B)", smem);
         // persistent grid: a multiple of the SM count, warps pull items from a global counter
@@ -911,6 +931,8 @@ int yawb_launch_count_fast(yawb_ctx *ctx, const CountArgs &a, int *launches) {
             LAUNCH(CountPath::Cumulative);
         } else if (multi) {
             LAUNCH(CountPath::Histogram);
+        } else if (P.n_sec == 2) {  // the per-chunk split by catalog costs the single-catalog launches 7 % (C3wt RR)
+            LAUNCH(CountPath::SingleUnion);
         } else {
             LAUNCH(CountPath::Single);
         }
@@ -927,7 +949,7 @@ int yawb_launch_count_exact(yawb_ctx *ctx, const CountArgs &a, int *launches) {
     ExactParams P{};
     P.cx = a.c1_cat->x; P.cy = a.c1_cat->y; P.cz = a.c1_cat->z; P.rec = a.c1->rec;
     P.sw = a.c1->sw; P.s_seg = a.c1_cat->d_seg_off;
-    P.rx = a.c2->rx; P.ry = a.c2->ry; P.rz = a.c2->rz; P.rw = a.c2->rw; P.r_seg = a.c2->second_d_seg_off();
+    P.rx = a.c2->ri.rx; P.ry = a.c2->ri.ry; P.rz = a.c2->ri.rz; P.rw = a.c2->ri.rw; P.r_seg = a.c2->second_d_seg_off();
     P.b1 = a.c1_cat->n_bins; P.b2 = a.c2->n_bins;
     P.pair_i = a.d_pair_i; P.pair_j = a.d_pair_j;
     P.n_pairs = a.n_pairs; P.n_bins = a.n_bins; P.n_edges = a.n_edges;

@@ -28,14 +28,14 @@ __host__ __device__ inline size_t up16(size_t b) { return (b + 15) & ~(size_t)15
 
 // Walks the layout of a warp's block (StreamSmem); with `base == nullptr` only the size is of interest.
 __host__ __device__ inline size_t stream_carve(StreamSmem *S, unsigned char *base, bool weighted, bool multi, int n_bins,
-                                               int nsub, int n_types, bool acc_global) {
+                                               int nsub, int n_types, int n_sec, bool acc_global) {
     size_t o = 0;
     auto take = [&](size_t bytes) {
         unsigned char *p = base + o;
         o += up16(bytes);
         return p;
     };
-    const size_t nacc = acc_global ? 0 : (size_t)n_types * n_bins * nsub;
+    const size_t nacc = acc_global ? 0 : (size_t)n_sec * n_types * n_bins * nsub;
     unsigned char *p;
     p = take(NSLOT * sizeof(Item)); if (S) S->items = (Item *)p;
     p = take(NSLOT * sizeof(ItemAux)); if (S) S->aux = (ItemAux *)p;
@@ -284,7 +284,7 @@ __device__ __forceinline__ void stream_begin(const FastParams &P, const StreamSm
                     k < ne ? fmaf(K, (float)(P.r2[(size_t)b * ne + k] - (double)bp.mid), 0.5f) : -1.0e30f;
         } else if constexpr (path_multi(PATH)) {  // Histogram, HistogramWeighted
             S.binthr[b] = make_float2(bp.h + eps, eps + 4.0f * EPS32 * (float)bp.hi);
-        } else if constexpr (PATH == CountPath::Single) {
+        } else if constexpr (path_sat(PATH)) {
             const float K = 0.4f / eps;  // undecidable tests land in v = [0.1, 0.9]: v (1 - v) >= 0.09
             S.binthr[b] = make_float2(-K, 0.5f + bp.h * K);
         } else {  // SingleWeighted
@@ -373,11 +373,25 @@ __device__ __forceinline__ int stream_segments(const StreamSmem &S, int L0, int 
 // Per z-bin segment: groups of four candidates fully unrolled plus a fall-through tail, the decided /
 // undecided check once per <= 16 candidates, the warp total of a segment added to the accumulator while the
 // next segment is already running.
+// SPLIT (tiles over the union of two second catalogs): Σv is kept per register pair and the count is split by the
+// catalog of each row (bit r of `tmask`: row r of the lane is a row of catalog 1) into the accumulators
+// [catalog][first catalog][z-bin].  The two parts travel packed in one word, catalog 1 in the high 16 bits: a segment
+// holds at most LB candidates, so a warp counts at most LB * YAWB_TILE = 32768 pairs of either catalog in it.
+template <bool SPLIT>
 __device__ __forceinline__ void stream_test_sat(const FastParams &P, const StreamSmem &S, int n_seg,
                                                 const float2 (&rx)[HPL], const float2 (&ry)[HPL], const float2 (&rz)[HPL],
-                                                const Tile &tl, int lane, unsigned &n_recheck) {
+                                                unsigned tmask, const Tile &tl, int lane, unsigned &n_recheck) {
+    static_assert(LB * YAWB_TILE <= 0xffff, "the packed counts of a segment fit 16 bits");
     unsigned pend_tot = 0;
     int pend_acc = -1;
+    auto flush = [&]() {  // the previous segment (its REDUX is long done)
+        if (!SPLIT) {
+            S.acc[pend_acc] += pend_tot;
+            return;
+        }
+        S.acc[pend_acc] += pend_tot & 0xffffu;
+        S.acc[P.n_types * P.n_bins + pend_acc] += pend_tot >> 16;
+    };
     for (int sg = 0; sg < n_seg; ++sg) {
         const SegDesc d = S.seg[sg];
         const float2 thr = S.binthr[d.bin];
@@ -385,10 +399,12 @@ __device__ __forceinline__ void stream_test_sat(const FastParams &P, const Strea
         unsigned cnt_total = 0;
         for (int c0 = d.ea; c0 < d.eb; c0 += 16) {
             const int c1 = min(c0 + 16, (int)d.eb);
-            float2 acc_a = make_float2(0.f, 0.f), acc_b = make_float2(0.f, 0.f);
-            double ws[YAWB_RPL];
+            constexpr int NA = SPLIT ? HPL : 1;
+            float2 acc_a[NA], acc_b = make_float2(0.f, 0.f);
+#pragma unroll
+            for (int k = 0; k < NA; ++k) acc_a[k] = make_float2(0.f, 0.f);
             int e = c0;
-#define YAWB_T(idx) test_candidate<false>(S.list[idx], 0.0, rx, ry, rz, ta, tb, acc_a, acc_b, ws)
+#define YAWB_T(idx) test_candidate_sat<NA>(S.list[idx], rx, ry, rz, ta, tb, acc_a, acc_b)
             for (; e + 4 <= c1; e += 4) {
                 YAWB_T(e); YAWB_T(e + 1); YAWB_T(e + 2); YAWB_T(e + 3);
             }
@@ -399,8 +415,17 @@ __device__ __forceinline__ void stream_test_sat(const FastParams &P, const Strea
                 default: break;
             }
 #undef YAWB_T
-            const float sa = acc_a.x + acc_a.y, sb = acc_b.x + acc_b.y;
+            // a decided chunk has every v at 0 or 1: the sums of v are exact integers
+            float sa = 0.f, sa1 = 0.f;
+#pragma unroll
+            for (int k = 0; k < NA; ++k) {
+                sa += acc_a[k].x + acc_a[k].y;
+                if (SPLIT)
+                    sa1 += ((tmask >> (2 * k)) & 1u ? acc_a[k].x : 0.f) + ((tmask >> (2 * k + 1)) & 1u ? acc_a[k].y : 0.f);
+            }
+            const float sb = acc_b.x + acc_b.y;
             unsigned c = (unsigned)(sa + 0.5f);
+            if (SPLIT) c += 0xffffu * (unsigned)(sa1 + 0.5f);
             unsigned flagged = __ballot_sync(FULL, sa != sb);
             while (flagged) {  // warp-uniform: some lane met the uncertainty band of an edge
                 const int src = __ffs(flagged) - 1;
@@ -411,11 +436,11 @@ __device__ __forceinline__ void stream_test_sat(const FastParams &P, const Strea
             }
             cnt_total += c;
         }
-        if (lane == 0 && pend_acc >= 0) S.acc[pend_acc] += pend_tot;  // the previous segment (its REDUX is long done)
+        if (lane == 0 && pend_acc >= 0) flush();
         pend_tot = __reduce_add_sync(FULL, cnt_total);
         pend_acc = d.type * P.n_bins + d.bin;
     }
-    if (lane == 0 && pend_acc >= 0) S.acc[pend_acc] += pend_tot;
+    if (lane == 0 && pend_acc >= 0) flush();
 }
 
 // ---- every other path: the shared phase-2 functions, one pass per segment ------------------------------
@@ -487,10 +512,10 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
     const int warp = threadIdx.x >> 5;
     const int nsub = P.n_edges - 1;
     const bool acc_global = MULTI && P.acc_global;
-    const int nacc = acc_global ? 0 : P.n_types * P.n_bins * nsub;  // accumulators kept in shared memory
+    const int nacc = acc_global ? 0 : P.n_sec * P.n_types * P.n_bins * nsub;  // accumulators kept in shared memory
     StreamSmem S;
-    const size_t per_warp = stream_carve(nullptr, nullptr, WEIGHTED, MULTI, P.n_bins, nsub, P.n_types, acc_global);
-    stream_carve(&S, smem_raw + warp * per_warp, WEIGHTED, MULTI, P.n_bins, nsub, P.n_types, acc_global);
+    const size_t per_warp = stream_carve(nullptr, nullptr, WEIGHTED, MULTI, P.n_bins, nsub, P.n_types, P.n_sec, acc_global);
+    stream_carve(&S, smem_raw + warp * per_warp, WEIGHTED, MULTI, P.n_bins, nsub, P.n_types, P.n_sec, acc_global);
     for (int k = lane; k < nacc; k += 32) {
         S.acc[k] = 0ull;
         if (WEIGHTED) S.accw[k] = 0.0;
@@ -525,6 +550,7 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
 
     float2 rx[HPL], ry[HPL], rz[HPL];  // rows (2k, 2k+1) of the lane share one register pair, in the tile frame
     double rwt[YAWB_RPL];                       // their weights (weighted kernels only)
+    unsigned tmask = 0;                         // bit r: row r of the lane is a row of catalog 1 of the index (SingleUnion)
 #pragma unroll
     for (int r = 0; r < HPL; ++r) rx[r] = ry[r] = rz[r] = make_float2(0.f, 0.f);
 #pragma unroll
@@ -544,6 +570,7 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
                 // rows of the tile: loads issued now, used after the conversion of the raw chunk
                 tl.start = it.start; tl.count = it.count; tl.patch = it.src; tl.bin = 0;  // patch: the tile's catalog
                 const double *const rxs = it.src ? P.rx2 : P.rx, *const rws = it.src ? P.rw2 : P.rw;
+                tmask = 0;
 #pragma unroll
                 for (int r = 0; r < YAWB_RPL; ++r) {
                     const int k = lane + 32 * r;
@@ -551,8 +578,9 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
                     if (k < it.count) {
                         const int j = it.start + k;
                         const double2 *const row = reinterpret_cast<const double2 *>(rxs + (size_t)YAWB_RSTRIDE * j);
-                        const double2 ra = row[0], rb = row[1];  // 32-byte row record
+                        const double2 ra = row[0], rb = row[1];  // 32-byte row record: x, y, z, catalog
                         dx[r] = ra.x; dy[r] = ra.y; dz[r] = rb.x;
+                        if (PATH == CountPath::SingleUnion && rb.y != 0.0) tmask |= 1u << r;
                         if (WEIGHTED) rwt[r] = rws ? rws[j] : 1.0;
                     }
                 }
@@ -630,19 +658,21 @@ __global__ void __launch_bounds__(STREAM_WARPS * 32, STREAM_CTAS) k_count_stream
         // ---- test ----
         if (c_cnt >= 0) {
             if (n_seg > 0) {
-                if constexpr (PATH == CountPath::Single)
-                    stream_test_sat(P, S, n_seg, rx, ry, rz, tl, lane, n_recheck);
+                if constexpr (path_sat(PATH))
+                    stream_test_sat<PATH == CountPath::SingleUnion>(P, S, n_seg, rx, ry, rz, tmask, tl, lane, n_recheck);
                 else
                     stream_test_generic<PATH>(P, S, n_seg, rx, ry, rz, tl, lane, nsub, n_recheck,
                                               item_offset(P, S.items[c_slot], nsub), rwt);
             }
             if (c_last) {  // the item is complete: its counts go to the result of its patch pair and output block
+                // (accumulator group g = catalog of a union tile's row * n_types + first catalog; the output blocks of
+                // the two catalogs of a union are 0 and 1)
                 __syncwarp();
                 const size_t nacc1 = (size_t)P.n_bins * nsub;
                 const size_t item_off = item_offset(P, S.items[c_slot], nsub);
                 for (int k = lane; k < nacc; k += 32) {
-                    const int type = k >= (int)nacc1 ? 1 : 0;
-                    const size_t o = item_off + (size_t)type * P.type_stride + (k - type * nacc1);
+                    const int g = PATH == CountPath::SingleUnion ? k / (int)nacc1 : k >= (int)nacc1 ? 1 : 0;
+                    const size_t o = item_off + (size_t)g * P.type_stride + (k - g * nacc1);
                     const unsigned long long c = S.acc[k];
                     if (c) {
                         atomicAdd(&P.out_cnt[o], c);

@@ -594,19 +594,19 @@ __global__ void __launch_bounds__(kThreads) k_scan_lookback(int *__restrict__ cu
 // second-role scatter: the row goes to the next free slot of its key
 __global__ void k_scatter_second(const double *__restrict__ x, const double *__restrict__ y, const double *__restrict__ z,
                                  const double *__restrict__ w, const int2 *__restrict__ kr, long long n,
-                                 const int *__restrict__ cur, double *__restrict__ ox, double *__restrict__ oy,
-                                 double *__restrict__ oz, double *__restrict__ ow) {
+                                 const int *__restrict__ cur, double tag, double *__restrict__ ox, double *__restrict__ ow) {
     long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int2 k = kr[i];
     if (k.x < 0) return;
     const double X = x[3 * i], Y = y[3 * i], Z = z[3 * i];
     const int pos = cur[k.x] + k.y;
-    // one 32-byte record per row: a full sector per scattered store (three separate arrays cost three partial ones)
+    // one 32-byte record per row: a full sector per scattered store (three separate arrays cost three partial ones);
+    // its fourth double is the row's catalog in the index (RIndex)
     double2 *const o = reinterpret_cast<double2 *>(ox + (size_t)YAWB_RSTRIDE * pos);
     o[0] = make_double2(X, Y);
-    o[1] = make_double2(Z, 0.0);
-    if (w) ow[pos] = w[i];
+    o[1] = make_double2(Z, tag);
+    if (ow) ow[pos] = w ? w[i] : 1.0;  // union of a weighted and an unweighted catalog
 }
 
 // first-role scatter (rows of one catalog; called twice for a fused index): the exact row plus its fixed-point
@@ -798,23 +798,41 @@ int build_first_counting(FIndex *fi, long long base) {
     return 0;
 }
 
-// second-role rows in (patch, z-bin, Hilbert) order by counting sort
-int build_second_counting(yawb_cat *cat, int hbits, long long n_keys) {
-    yawb_ctx *ctx = cat->ctx;
+template <typename T>
+int ri_alloc(RIndex *ri, T **ptr, size_t count) {
+    *ptr = nullptr;
+    if (count == 0) count = 1;
+    if (yawb_dalloc(ri->ctx, (void **)ptr, count * sizeof(T), ri->ctx->stream)) return 1;
+    ri->device_bytes += (int64_t)(count * sizeof(T));
+    return 0;
+}
+
+// second-role rows of one catalog or of two (RIndex) in (patch, z-bin, Hilbert) order by counting sort; the rows of
+// both catalogs share the Hilbert maps of a's patch frames (the map only orders rows: a row of b outside a's patch
+// box is clamped to its edge)
+int build_second_counting(RIndex *ri, int hbits, long long n_keys) {
+    yawb_ctx *ctx = ri->ctx;
     cudaStream_t st = ctx->stream;
-    if (cat->n_in <= 0) return 0;
+    const yawb_cat *a = ri->a, *b = ri->b;
+    const long long na = a->n_in > 0 ? a->n_in : 0, nb = b && b->n_in > 0 ? b->n_in : 0;
+    if (na + nb == 0) return 0;
     Scratch scr(ctx, st);
     int *cur = scr.get<int>((size_t)n_keys);
-    int2 *keys = scr.get<int2>((size_t)cat->n_in);  // (key, rank among the rows of the key) of every row
-    HMap *maps = scr.get<HMap>((size_t)cat->n_patch);
+    int2 *keys = scr.get<int2>((size_t)(na + nb));  // (key, rank among the rows of the key) of every row
+    HMap *maps = scr.get<HMap>((size_t)a->n_patch);
     YAWB_REQUIRE(cur && keys && maps, "out of device memory (key counts)");
     YAWB_CUDA(cudaMemsetAsync(cur, 0, (size_t)n_keys * sizeof(int), st));
-    k_hilbert_map<<<(cat->n_patch + 127) / 128, 128, 0, st>>>(cat->d_frames, cat->n_patch, hbits, maps);
-    k_hist_second<<<blocks_for(cat->n_in), kThreads, 0, st>>>(cat->x, cat->y, cat->z, cat->bin, cat->patch, cat->n_in,
-                                                              cat->n_bins, hbits, maps, cat->d_second_mask, cur, keys);
+    k_hilbert_map<<<(a->n_patch + 127) / 128, 128, 0, st>>>(a->d_frames, a->n_patch, hbits, maps);
+    for (const yawb_cat *c : {a, b})
+        if (c && c->n_in > 0)
+            k_hist_second<<<blocks_for(c->n_in), kThreads, 0, st>>>(c->x, c->y, c->z, c->bin, c->patch, c->n_in, a->n_bins,
+                                                                    hbits, maps, c->d_second_mask, cur,
+                                                                    keys + (c == b ? na : 0));
     if (exclusive_scan_inplace(ctx, scr, cur, n_keys)) return 1;
-    k_scatter_second<<<blocks_for(cat->n_in), kThreads, 0, st>>>(cat->x, cat->y, cat->z, cat->w, keys, cat->n_in, cur,
-                                                                 cat->rx, cat->ry, cat->rz, cat->rw);
+    for (const yawb_cat *c : {a, b})
+        if (c && c->n_in > 0)
+            k_scatter_second<<<blocks_for(c->n_in), kThreads, 0, st>>>(c->x, c->y, c->z, c->w, keys + (c == b ? na : 0),
+                                                                       c->n_in, cur, c == b ? 1.0 : 0.0, ri->rx, ri->rw);
     return 0;
 }
 
@@ -1172,21 +1190,52 @@ void yawb_findex_drop_fused(yawb_ctx *ctx, const yawb_cat *cat) {
 }
 
 // -------------------------------------------------------------------------------------------
-int yawb_index_build_second(yawb_cat *cat) {
-    if (yawb_cat_finalize(cat)) return 1;
-    if (cat->has_rtiles) return 0;
-    YawbRange range("yawb:index_second");
-    yawb_ctx *ctx = cat->ctx;
-    cudaStream_t st = ctx->stream;
-    const long long n = cat->second_rows();
-    const int P = cat->n_patch, B = cat->n_bins;
-    const std::vector<int> &seg_off = cat->second_seg_off();
+static void rindex_release(RIndex *ri) {
+    for (void *p : {(void *)ri->rrow, (void *)ri->rw, (void *)ri->d_seg_off, (void *)ri->d_tiles, (void *)ri->d_tile_box,
+                    (void *)ri->d_ptile_off})
+        if (p) yawb_dfree(ri->ctx, p, ri->ctx->stream);
+    ri->rrow = ri->rx = ri->ry = ri->rz = ri->rw = nullptr;
+    ri->d_seg_off = ri->d_ptile_off = nullptr;
+    ri->d_tiles = nullptr;
+    ri->d_tile_box = nullptr;
+    ri->h_tiles.clear();
+    ri->h_ptile_off.clear();
+    ri->n = 0;
+    ri->n_tiles = 0;
+    ri->device_bytes = 0;
+    ri->built = false;
+}
 
-    if (dev_alloc(cat, &cat->rrow, (size_t)n * YAWB_RSTRIDE)) return 1;
-    cat->rx = cat->rrow;
-    cat->ry = cat->rrow + 1;
-    cat->rz = cat->rrow + 2;
-    if (cat->weighted && dev_alloc(cat, &cat->rw, n)) return 1;
+// Second-role index over ri->a, or over the union of ri->a and ri->b (same patches and z-bins, both finalized).
+static int rindex_build(RIndex *ri) {
+    yawb_ctx *ctx = ri->ctx;
+    cudaStream_t st = ctx->stream;
+    const yawb_cat *ca = ri->a, *cb = ri->b;
+    const int P = ca->n_patch, B = ca->n_bins;
+    ri->d_frames = ca->d_frames;
+    // (patch, z-bin) segments of the index rows: the catalog's own, or both catalogs' rows of a segment together
+    std::vector<int> union_off;
+    if (cb) {
+        const std::vector<int> &oa = ca->second_seg_off(), &ob = cb->second_seg_off();
+        union_off.resize(oa.size());
+        for (size_t k = 0; k < oa.size(); ++k) union_off[k] = oa[k] + ob[k];
+    }
+    const std::vector<int> &seg_off = cb ? union_off : ca->second_seg_off();
+    const long long n = seg_off.back();
+    YAWB_REQUIRE(ca->second_rows() + (cb ? cb->second_rows() : 0) < (1ll << 31) - 1024,
+                 "a second-role index is limited to 2^31 rows");
+    ri->n = n;
+    if (ri_alloc(ri, &ri->rrow, (size_t)n * YAWB_RSTRIDE)) return 1;
+    ri->rx = ri->rrow;
+    ri->ry = ri->rrow + 1;
+    ri->rz = ri->rrow + 2;
+    if ((ca->weighted || (cb && cb->weighted)) && ri_alloc(ri, &ri->rw, n)) return 1;
+    const int *d_seg_off = ca->second_d_seg_off();
+    if (cb) {
+        if (ri_alloc(ri, &ri->d_seg_off, seg_off.size())) return 1;
+        if (yawb_h2d_small(ctx, ri->d_seg_off, seg_off.data(), seg_off.size() * sizeof(int))) return 1;
+        d_seg_off = ri->d_seg_off;
+    }
     // The curve only has to order the rows down to about one row per Hilbert cell: with m rows in the largest
     // (patch, bin) segment, 2^k x 2^k >= 1.5 m cells are enough.  The counting sort takes one count per (patch, bin,
     // Hilbert cell), so the resolution is capped at about ONE key per row (the cells then hold 1-4 rows, in arbitrary
@@ -1198,47 +1247,46 @@ int yawb_index_build_second(yawb_cat *cat) {
             m = std::max<long long>(m, seg_off[sgm + 1] - seg_off[sgm]);
         int k = 4;
         while (k < 16 && (1ll << (2 * k)) < m + m / 2) ++k;
-        const long long key_budget = std::max<long long>(cat->n_in, 1 << 16);
+        const long long key_budget = std::max<long long>(ca->n_in + (cb ? cb->n_in : 0), 1 << 16);
         while (k > 1 && (((long long)P * B) << (2 * k)) > key_budget) --k;
-        if (build_second_counting(cat, 2 * k, ((long long)P * B) << (2 * k))) return 1;
+        if (build_second_counting(ri, 2 * k, ((long long)P * B) << (2 * k))) return 1;
     }
 
     // tiles: chunks of YAWB_TILE rows inside each (patch, bin) segment; the host only needs their number per segment
     // (the table itself is written on the device, k_make_tiles) and per patch
-    std::vector<Tile> &tiles = cat->h_tiles;  // filled only if tiles have to be split (straggler guard below)
+    std::vector<Tile> &tiles = ri->h_tiles;  // filled only if tiles have to be split (straggler guard below)
     tiles.clear();
-    cat->h_ptile_off.assign(P + 1, 0);
+    ri->h_ptile_off.assign(P + 1, 0);
     std::vector<int> seg_tile_off((size_t)P * B + 1, 0);
     for (int p = 0; p < P; ++p) {
-        cat->h_ptile_off[p] = seg_tile_off[(size_t)p * B];
+        ri->h_ptile_off[p] = seg_tile_off[(size_t)p * B];
         for (int b = 0; b < B; ++b) {
             const int len = seg_off[(size_t)p * B + b + 1] - seg_off[(size_t)p * B + b];
             seg_tile_off[(size_t)p * B + b + 1] = seg_tile_off[(size_t)p * B + b] + (len + YAWB_TILE - 1) / YAWB_TILE;
         }
     }
     const int n_tiles0 = seg_tile_off[(size_t)P * B];
-    cat->h_ptile_off[P] = n_tiles0;
+    ri->h_ptile_off[P] = n_tiles0;
 
     // Straggler guard: a chunk of consecutive rows can straddle a place where the Hilbert curve leaves the
     // populated part of the patch box and re-enters elsewhere (irregular footprints, masks).  Such a tile
     // has a bounding sphere several times the typical one and would be worth many average work items.
-    // Tiles whose radius exceeds 3x the radius expected from the patch's mean density are cut into
-    // sub-tiles of 32 rows (rare; they run the same kernel with most register rows padded).  The common
+    // Tiles whose radius exceeds 3x the radius expected from the patch's mean density (of the index rows) are cut
+    // into sub-tiles of 32 rows (rare; they run the same kernel with most register rows padded).  The common
     // case costs one 4-byte read-back.
     bool table_on_device = false;
     int n_tiles_final = n_tiles0;
     if (n_tiles0 > 0) {
         Scratch scr(ctx, st);
-        if (dev_alloc(cat, &cat->d_tiles, (size_t)n_tiles0)) return 1;  // becomes the final table unless tiles are split
-        Tile *d_tmp = cat->d_tiles;
-        const size_t n_tmp = (size_t)n_tiles0;
+        if (ri_alloc(ri, &ri->d_tiles, (size_t)n_tiles0)) return 1;  // becomes the final table unless tiles are split
+        Tile *d_tmp = ri->d_tiles;
         float *d_thr = scr.get<float>(P);
         unsigned *d_nbig = scr.get<unsigned>(1);
         int *d_seg_tile_off = scr.get<int>((size_t)P * B + 1);
         YAWB_REQUIRE(d_thr && d_nbig && d_seg_tile_off, "out of device memory (tile table)");
         std::vector<float> thr(P, 3.0e38f);
         for (int p = 0; p < P; ++p) {
-            const PatchFrame &f = cat->h_frames[p];
+            const PatchFrame &f = ca->h_frames[p];
             const long long np = seg_off[(size_t)(p + 1) * B] - seg_off[(size_t)p * B];
             const double area = std::max(f.umax - f.umin, 0.0) * std::max(f.vmax - f.vmin, 0.0);
             if (np >= 8 * YAWB_TILE && area > 0.0)  // radius of a disc holding YAWB_TILE rows of one z-bin
@@ -1247,13 +1295,11 @@ int yawb_index_build_second(yawb_cat *cat) {
         if (yawb_h2d_small(ctx, d_seg_tile_off, seg_tile_off.data(), seg_tile_off.size() * sizeof(int))) return 1;
         if (yawb_h2d_small(ctx, d_thr, thr.data(), P * sizeof(float))) return 1;
         YAWB_CUDA(cudaMemsetAsync(d_nbig, 0, sizeof(unsigned), st));
-        k_make_tiles<<<blocks_for((long long)n_tiles0), kThreads, 0, st>>>(cat->second_d_seg_off(), d_seg_tile_off, P * B, B,
-                                                                          cat->binned ? 1 : 0, n_tiles0, d_tmp);
-        TileBox *d_box_tmp = nullptr;
-        if (dev_alloc(cat, &d_box_tmp, (size_t)n_tiles0)) return 1;
-        cat->d_tile_box = d_box_tmp;
-        k_tile_spheres<<<blocks_for((long long)n_tiles0 * 32), kThreads, 0, st>>>(cat->rx, cat->ry, cat->rz, d_tmp, n_tiles0,
-                                                                                 cat->d_frames, d_box_tmp);
+        k_make_tiles<<<blocks_for((long long)n_tiles0), kThreads, 0, st>>>(d_seg_off, d_seg_tile_off, P * B, B,
+                                                                          ca->binned ? 1 : 0, n_tiles0, d_tmp);
+        if (ri_alloc(ri, &ri->d_tile_box, (size_t)n_tiles0)) return 1;
+        k_tile_spheres<<<blocks_for((long long)n_tiles0 * 32), kThreads, 0, st>>>(ri->rx, ri->ry, ri->rz, d_tmp, n_tiles0,
+                                                                                 ri->d_frames, ri->d_tile_box);
         k_count_oversized<<<blocks_for((long long)n_tiles0), kThreads, 0, st>>>(d_tmp, n_tiles0, d_thr, d_nbig);
         unsigned n_big = 0;
         YAWB_CUDA(cudaMemcpyAsync(&n_big, d_nbig, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
@@ -1263,14 +1309,17 @@ int yawb_index_build_second(yawb_cat *cat) {
             tiles.resize((size_t)n_tiles0);
             YAWB_CUDA(cudaMemcpyAsync(tiles.data(), d_tmp, tiles.size() * sizeof(Tile), cudaMemcpyDeviceToHost, st));
             YAWB_CUDA(cudaStreamSynchronize(st));
-            dev_free(cat, cat->d_tiles, n_tmp);
-            dev_free(cat, cat->d_tile_box, n_tmp);
+            for (void **p : {(void **)&ri->d_tiles, (void **)&ri->d_tile_box}) {
+                yawb_dfree(ctx, *p, st);
+                *p = nullptr;
+            }
+            ri->device_bytes -= (int64_t)n_tiles0 * (int64_t)(sizeof(Tile) + sizeof(TileBox));
             std::vector<Tile> out;
             out.reserve(tiles.size() + 8 * (size_t)n_big);
             std::vector<int> new_off(P + 1, 0);
             for (int p = 0; p < P; ++p) {
                 new_off[p] = (int)out.size();
-                for (int t = cat->h_ptile_off[p]; t < cat->h_ptile_off[p + 1]; ++t) {
+                for (int t = ri->h_ptile_off[p]; t < ri->h_ptile_off[p + 1]; ++t) {
                     const Tile &tl = tiles[t];
                     if (tl.rad > thr[p] && tl.count > 32) {
                         for (int s0 = 0; s0 < tl.count; s0 += 32) {
@@ -1286,34 +1335,82 @@ int yawb_index_build_second(yawb_cat *cat) {
             }
             new_off[P] = (int)out.size();
             tiles.swap(out);
-            cat->h_ptile_off = new_off;
+            ri->h_ptile_off = new_off;
             n_tiles_final = (int)tiles.size();
         }
     }
-    cat->n_tiles = n_tiles_final;
-    if (!table_on_device && dev_alloc(cat, &cat->d_tiles, (size_t)n_tiles_final)) return 1;
-    if (dev_alloc(cat, &cat->d_ptile_off, P + 1)) return 1;
-    if (yawb_h2d_small(ctx, cat->d_ptile_off, cat->h_ptile_off.data(), (P + 1) * sizeof(int))) return 1;
-    if (!table_on_device && dev_alloc(cat, &cat->d_tile_box, tiles.size())) return 1;
+    ri->n_tiles = n_tiles_final;
+    if (!table_on_device && ri_alloc(ri, &ri->d_tiles, (size_t)n_tiles_final)) return 1;
+    if (ri_alloc(ri, &ri->d_ptile_off, P + 1)) return 1;
+    if (yawb_h2d_small(ctx, ri->d_ptile_off, ri->h_ptile_off.data(), (P + 1) * sizeof(int))) return 1;
+    if (!table_on_device && ri_alloc(ri, &ri->d_tile_box, tiles.size())) return 1;
     if (!table_on_device && !tiles.empty()) {  // the split tiles need their own spheres and boxes
-        if (yawb_h2d_small(ctx, cat->d_tiles, tiles.data(), tiles.size() * sizeof(Tile))) return 1;
-        k_tile_spheres<<<blocks_for((long long)cat->n_tiles * 32), kThreads, 0, st>>>(cat->rx, cat->ry, cat->rz, cat->d_tiles,
-                                                                                      cat->n_tiles, cat->d_frames, cat->d_tile_box);
+        if (yawb_h2d_small(ctx, ri->d_tiles, tiles.data(), tiles.size() * sizeof(Tile))) return 1;
+        k_tile_spheres<<<blocks_for((long long)ri->n_tiles * 32), kThreads, 0, st>>>(ri->rx, ri->ry, ri->rz, ri->d_tiles,
+                                                                                     ri->n_tiles, ri->d_frames, ri->d_tile_box);
     }
     YAWB_CUDA(cudaGetLastError());
-    cat->has_rtiles = true;
+    ri->built = true;
+    return 0;
+}
+
+int yawb_index_build_second(yawb_cat *cat) {
+    if (yawb_cat_finalize(cat)) return 1;
+    if (cat->ri.built) return 0;
+    YawbRange range("yawb:index_second");
+    RIndex &ri = cat->ri;
+    ri.ctx = cat->ctx;
+    ri.a = cat;
+    ri.b = nullptr;
+    if (int rc = rindex_build(&ri)) {
+        rindex_release(&ri);
+        return rc;
+    }
+    cat->device_bytes += ri.device_bytes;
     return 0;
 }
 
 void yawb_index_free_second(yawb_cat *cat) {
-    const size_t n = (size_t)cat->second_rows(), P = (size_t)cat->n_patch;
-    dev_free(cat, cat->rrow, n * YAWB_RSTRIDE);
-    cat->rx = cat->ry = cat->rz = nullptr;
-    dev_free(cat, cat->rw, n);
-    dev_free(cat, cat->d_tiles, (size_t)cat->n_tiles);
-    dev_free(cat, cat->d_tile_box, (size_t)cat->n_tiles);
-    dev_free(cat, cat->d_ptile_off, P + 1);
-    cat->has_rtiles = false;
+    cat->device_bytes -= cat->ri.device_bytes;
+    if (cat->ri.ctx) rindex_release(&cat->ri);
+}
+
+int yawb_rindex_get_union(yawb_ctx *ctx, yawb_cat *a, yawb_cat *b, RIndex **out, bool *built) {
+    *built = false;
+    for (RIndex *ri : ctx->unions)
+        if (ri->a == a && ri->b == b) {
+            *out = ri;
+            return 0;
+        }
+    if (yawb_cat_finalize(a) || yawb_cat_finalize(b)) return 1;
+    YawbRange range("yawb:index_second_union");
+    RIndex *ri = new (std::nothrow) RIndex();
+    YAWB_REQUIRE(ri != nullptr, "out of host memory");
+    ri->ctx = ctx;
+    ri->a = a;
+    ri->b = b;
+    if (int rc = rindex_build(ri)) {
+        rindex_release(ri);
+        delete ri;
+        return rc;
+    }
+    ctx->unions.push_back(ri);
+    *out = ri;
+    *built = true;
+    return 0;
+}
+
+void yawb_rindex_drop_union(yawb_ctx *ctx, const yawb_cat *cat) {
+    for (size_t k = 0; k < ctx->unions.size();) {
+        RIndex *ri = ctx->unions[k];
+        if (ri->a == cat || ri->b == cat) {
+            rindex_release(ri);
+            delete ri;
+            ctx->unions.erase(ctx->unions.begin() + k);
+        } else {
+            ++k;
+        }
+    }
 }
 
 // The mask is copied to the device and its rows are counted per (z-bin, patch) right away: the second-role index
@@ -1325,6 +1422,7 @@ int yawb_index_set_second_rows(yawb_cat *cat, const uint8_t *mask) {
     const int P = cat->n_patch, B = cat->n_bins;
     YAWB_CUDA(cudaStreamSynchronize(st));  // nothing in flight still reads the second-role index
     yawb_index_free_second(cat);
+    yawb_rindex_drop_union(ctx, cat);
     dev_free(cat, cat->d_second_mask, (size_t)cat->n_in);
     dev_free(cat, cat->d_seg_off2, (size_t)P * B + 1);
     cat->h_counts2.clear();
@@ -1382,7 +1480,8 @@ void yawb_index_free(yawb_cat *cat, bool everything) {
         cat->findex = nullptr;
     }
     yawb_findex_drop_fused(cat->ctx, cat);
-    if (cat->has_rtiles || everything) yawb_index_free_second(cat);
+    yawb_rindex_drop_union(cat->ctx, cat);
+    yawb_index_free_second(cat);
     if (everything) {
         release_staging(cat);
         // a catalog that was never used may still have copies in flight: frees are ordered behind them

@@ -96,8 +96,9 @@ struct __align__(16) Item {
     int b_lo, b_hi;        // z-bins of the first catalog covered by this item
     int row_lo, row_hi;    // cell rows of the query covered, relative to its first row (whole query: 0, INT_MAX);
                            // a restriction only occurs on items of a single z-bin
-    int src;               // second catalog of a joint launch (0 or 1): where the tile's rows live
-    int blk;               // output block of the item's counts: second catalog, then label (YAWB_FLAG_SECOND_LABELS)
+    int src;               // second-role index of a joint launch (CountArgs::r2, 0 or 1): where the tile's rows live
+    int blk;               // output block of the item's counts: second catalog, then label (YAWB_FLAG_SECOND_LABELS);
+                           // a union tile's counts go to block 0 + (catalog of the row)
     int b_off;             // first-catalog id of z-bin 0 of the item's label (label * B when both catalogs carry
                            // binned labels, else 0): the cell rows of z-bin b are those of id b + b_off
     int pad;
@@ -127,7 +128,7 @@ struct BinPar {
 constexpr int YAWB_RPL = 8;               // second-role points per lane
 constexpr int YAWB_TILE = 32 * YAWB_RPL;  // points per register tile (one warp)
 constexpr int YAWB_LG_CELLS_PER_EDGE = 4;  // cells of the lg2(d2) lookup per edge (sub-bin paths): finer cells = fewer fix-up steps
-constexpr int YAWB_RSTRIDE = 4;           // doubles per second-role row record (x, y, z, unused): one 32-byte sector
+constexpr int YAWB_RSTRIDE = 4;           // doubles per second-role row record (x, y, z, catalog): one 32-byte sector
 constexpr int YAWB_MAX_EDGES = 256;
 
 struct yawb_ctx {
@@ -153,6 +154,30 @@ struct yawb_ctx {
     unsigned char *h2d_base = nullptr;
     size_t h2d_size = 0, h2d_used = 0;
     std::vector<struct FIndex *> fused;  // first-role indexes over pairs of catalogs (yawb_count2)
+    std::vector<struct RIndex *> unions;  // second-role indexes over pairs of catalogs (yawb_count4)
+};
+
+// Second-role index: rows sorted by (patch, z-bin, Hilbert index) and cut into register tiles of YAWB_TILE rows.
+// Over the rows of one catalog (yawb_cat::ri), or over the union of two catalogs with the same patches and z-bins
+// (the single-bin path of yawb_count4): a tile of YAWB_TILE rows of both catalogs covers about half the sky of a tile
+// of one, so every query box of the count shrinks.  The catalog of a row (0 / 1) is the fourth double of its record.
+struct RIndex {
+    yawb_ctx *ctx = nullptr;
+    const yawb_cat *a = nullptr, *b = nullptr;  // sources (b == nullptr: single catalog)
+    bool built = false;
+    long long n = 0;                            // rows
+    const PatchFrame *d_frames = nullptr;       // frames the tile boxes live in (a's)
+    double *rrow = nullptr;                     // rows in tile order, one 32-byte record (x, y, z, catalog) per row
+    double *rx = nullptr, *ry = nullptr, *rz = nullptr;  // views of rrow: row j is rx[4 j], ry[4 j], rz[4 j]
+    double *rw = nullptr;                       // weights (1.0 for rows of an unweighted catalog), or nullptr
+    int *d_seg_off = nullptr;                   // union only: [(n_patch * n_bins) + 1] segments of the union rows
+    Tile *d_tiles = nullptr;
+    TileBox *d_tile_box = nullptr;  // [n_tiles] bounding boxes in the frame of the tile's own patch
+    std::vector<Tile> h_tiles;      // host copy of the tile table (source of an async upload)
+    std::vector<int> h_ptile_off;   // [n_patch + 1] first tile of each patch
+    int *d_ptile_off = nullptr;
+    int n_tiles = 0;
+    int64_t device_bytes = 0;
 };
 
 struct yawb_cat {
@@ -213,17 +238,8 @@ struct yawb_cat {
     const std::vector<long long> &second_counts() const { return d_second_mask ? h_counts2 : h_counts; }
     int *second_d_seg_off() const { return d_second_mask ? d_seg_off2 : d_seg_off; }
 
-    // second-role index: rows sorted by (patch, bin, Hilbert index), cut into register tiles
-    bool has_rtiles = false;
-    double *rrow = nullptr;                   // second-role rows in tile order, one 32-byte record (x, y, z, -) per row
-    double *rx = nullptr, *ry = nullptr, *rz = nullptr;  // views of rrow: row j is rx[4 j], ry[4 j], rz[4 j]
-    double *rw = nullptr;
-    Tile *d_tiles = nullptr;
-    TileBox *d_tile_box = nullptr;  // [n_tiles] bounding boxes in the frame of the tile's own patch
-    std::vector<Tile> h_tiles;     // host copy of the tile table (source of an async upload)
-    std::vector<int> h_ptile_off;  // [n_patch + 1] first tile of each patch
-    int *d_ptile_off = nullptr;
-    int n_tiles = 0;
+    // second-role index over this catalog alone (built on first use)
+    RIndex ri;
 };
 
 // First-role ("sky-cell") index over the rows of one catalog, or over the union of two catalogs with the
@@ -273,6 +289,9 @@ int yawb_findex_get_fused(yawb_ctx *ctx, yawb_cat *a, yawb_cat *b, FIndex **out,
 void yawb_findex_drop_fused(yawb_ctx *ctx, const yawb_cat *cat);
 void yawb_findex_free(FIndex *fi);
 int yawb_index_build_second(yawb_cat *cat);
+// second-role index over the union of (a, b); cached in the context until either catalog is dropped or freed
+int yawb_rindex_get_union(yawb_ctx *ctx, yawb_cat *a, yawb_cat *b, RIndex **out, bool *built);
+void yawb_rindex_drop_union(yawb_ctx *ctx, const yawb_cat *cat);
 void yawb_index_free(yawb_cat *cat, bool everything);
 
 // pair counting (yawb_count.cu)
@@ -280,11 +299,14 @@ struct CountArgs {
     const FIndex *c1;    // first-role index (one catalog, or two fused)
     const yawb_cat *c2;
     const yawb_cat *c2b = nullptr;       // second second-role catalog of a joint launch (yawb_count4), or nullptr
+    // where the tiles come from: c2's index and c2b's (Item::src 0 / 1), or ONE index over the union of c2 and c2b
+    // (r2[1] == nullptr; the rows' catalogs split every count, Item::blk = 0)
+    const RIndex *r2[2] = {nullptr, nullptr};
     const int *d_pair_i;
     const int *d_pair_j;
-    const long long *d_pair_item_base;  // [n_pairs + 1] prefix of tiles per pair
+    const long long *d_pair_item_base;  // [n_pairs + 1] prefix of tiles of r2[0] per pair
     long long n_items;                  // (patch pair, tile) combinations = threads of the planner
-    const long long *d_pair_item_base_b = nullptr;  // the same for c2b
+    const long long *d_pair_item_base_b = nullptr;  // the same for r2[1]
     long long n_items_b = 0;
     bool labels = false;    // YAWB_FLAG_SECOND_LABELS: the z-bin ids of a binned second catalog are sample labels
     int blk_b = 1;          // first output block of c2b (= labels of c2)
