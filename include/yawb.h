@@ -283,6 +283,54 @@ int yawb_assign_patches(yawb_ctx *ctx, const double *xyz, int64_t n, const doubl
 int yawb_kmeans(yawb_ctx *ctx, const double *xyz, const double *w, int64_t n, int k, int max_iter,
                 double *centers_xyz, int32_t *labels, int *n_iter, int *converged);
 
+/* Device memory (library version >= 104).
+ *
+ * yawb_catalog_footprint: host arithmetic only, no device access.  An upper bound on the device bytes one catalog of
+ * n_rows rows in n_patch patches and n_bins z-bins (1: unbinned; labelled: labels x z-bins) holds: `what` is an OR of
+ * the YAWB_FOOT_* flags below, naming the columns that travel and the indexes to cover.  Every block the upload, its
+ * per-patch frames and sums, the second-role row mask and the index builds request is summed -- scratch freed
+ * again included -- each rounded as the context's allocator rounds it, so yawb_memory_stats' `peak` of a context
+ * that starts empty stays at or below the bound.  The first-role sky-cell grid is bounded from the row counts alone
+ * (4 (n_rows + n_patch n_bins) / 5.5 + 10241 n_patch n_bins cells, at most 2^30), the tile table by
+ * n_rows / 256 + n_patch n_bins tiles.  Not covered: the rare re-cut of oversized tiles of a second-role index
+ * (tiles whose bounding sphere is more than three times the expected one are cut into pieces of 32 rows).
+ * YAWB_FOOT_NO_UPLOAD with one index flag bounds an index over rows uploaded by other catalogs: the fused first-role
+ * index of yawb_count2 / yawb_count4 (n_rows = rows of both first catalogs) or the union second-role index of
+ * yawb_count4 (rows of both second catalogs).
+ *
+ * yawb_count_footprint: the workspace of one yawb_count / yawb_count2 / yawb_count4 call on a device with `sms`
+ * SMs (the SM count sizes the work-item lists; yawb_device_sms); host arithmetic only: the table of pair lists and thresholds, the work-item lists of the
+ * planner, and the output counts (and sums if `weighted`) of n_blocks x n_pairs x n_bins x (n_edges - 1) entries,
+ * where n_blocks = (first catalogs) x (labels of the second catalogs, 1 each without labels).  n_items: the planner's
+ * (patch pair, tile) combinations, i.e. the sum over the pair list of the tiles of the second patch, at most
+ * rows / 256 + n_bins per patch.  The bound does not decrease with n_items, so an overestimate of n_items gives
+ * an upper bound, also across the count at which the planner switches to the longer lists of a small job.
+ * Not covered: the repeat of a count whose work-item lists overflowed (the
+ * lists are then sized exactly).
+ *
+ * yawb_memory_stats: `held` = bytes the context's allocator holds (blocks in use and blocks parked for reuse), `peak`
+ * = the high-water mark of `held` since the context was created or since yawb_memory_reset_peak, `device_free` =
+ * free bytes of the device (cudaMemGetInfo).  Any pointer may be NULL.
+ * yawb_memory_parked: the bytes of the blocks the allocator holds parked for reuse (part of `held`; they go back to
+ * the driver when a cudaMalloc fails).
+ * yawb_memory_release: parked blocks go back to the driver (blocks in use stay). */
+#define YAWB_FOOT_WEIGHTED 1u   /* weights travel                                     */
+#define YAWB_FOOT_BINNED 2u     /* int32 z-bin ids (yawb_upload_catalog)              */
+#define YAWB_FOOT_U8 4u         /* byte z-bin ids (yawb_upload_catalog_u8)            */
+#define YAWB_FOOT_Z 8u          /* raw redshifts binned on the device (yawb_upload_catalog_z) */
+#define YAWB_FOOT_LABELLED 16u  /* binned labels (yawb_catalog_set_labels): ids as YAWB_FOOT_BINNED / _U8 */
+#define YAWB_FOOT_MASK 32u      /* a second-role row mask (yawb_catalog_set_second_rows) */
+#define YAWB_FOOT_FIRST 64u     /* the first-role index                               */
+#define YAWB_FOOT_SECOND 128u   /* the second-role index                              */
+#define YAWB_FOOT_NO_UPLOAD 256u /* leave out the upload: an index over other catalogs' rows */
+int yawb_catalog_footprint(int64_t n_rows, int n_patch, int n_bins, uint32_t what, int64_t *bytes);
+int yawb_count_footprint(int sms, int64_t n_items, int n_pairs, int n_bins, int n_edges, int n_blocks, int weighted,
+                         int64_t *bytes);
+int yawb_memory_stats(yawb_ctx *ctx, int64_t *held, int64_t *peak, int64_t *device_free);
+int yawb_memory_parked(yawb_ctx *ctx, int64_t *parked);
+int yawb_memory_reset_peak(yawb_ctx *ctx);
+int yawb_memory_release(yawb_ctx *ctx);
+
 /* Library version and number of SMs of the context's device. */
 int yawb_version(void);
 int yawb_device_sms(const yawb_ctx *ctx);

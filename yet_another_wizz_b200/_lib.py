@@ -22,6 +22,16 @@ FLAG_SECOND_LABELS = 4
 LABELS_MIN_VERSION = 101  # first library version that knows FLAG_SECOND_LABELS
 BINNED_LABELS_MIN_VERSION = 102  # first library version with yawb_catalog_set_labels
 PARTIAL_MIN_VERSION = 103  # first library version with partial uploads and second-role row masks
+# yawb_catalog_footprint flags (library version >= 104)
+FOOT_WEIGHTED = 1
+FOOT_BINNED = 2
+FOOT_U8 = 4
+FOOT_Z = 8
+FOOT_LABELLED = 16
+FOOT_MASK = 32
+FOOT_FIRST = 64
+FOOT_SECOND = 128
+FOOT_NO_UPLOAD = 256
 ROLE_FIRST = 1
 ROLE_SECOND = 2
 
@@ -33,6 +43,9 @@ EXPORTS = (
     "yawb_timer_start", "yawb_timer_stop", "yawb_assign_patches", "yawb_upload_catalog_u8", "yawb_count2",
     "yawb_upload_catalog_z", "yawb_patch_metadata", "yawb_jackknife", "yawb_count4", "yawb_kmeans",
     "yawb_catalog_set_labels", "yawb_upload_catalog_patches", "yawb_catalog_set_second_rows",
+    "yawb_catalog_footprint", "yawb_count_footprint", "yawb_memory_stats", "yawb_memory_reset_peak",
+    "yawb_memory_parked",
+    "yawb_memory_release",
 )
 
 
@@ -120,6 +133,12 @@ def load(build_if_missing: bool = False) -> ctypes.CDLL:
         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_uint32,
         POINTER(c_void_p), POINTER(c_void_p), POINTER(YawbStats),
     ]
+    lib.yawb_catalog_footprint.argtypes = [c_int64, c_int, c_int, c_uint32, POINTER(c_int64)]
+    lib.yawb_count_footprint.argtypes = [c_int, c_int64, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]
+    lib.yawb_memory_stats.argtypes = [c_void_p, POINTER(c_int64), POINTER(c_int64), POINTER(c_int64)]
+    lib.yawb_memory_parked.argtypes = [c_void_p, POINTER(c_int64)]
+    lib.yawb_memory_reset_peak.argtypes = [c_void_p]
+    lib.yawb_memory_release.argtypes = [c_void_p]
     if hasattr(lib, "yawb_catalog_set_labels"):  # older libraries lack it: Engine.upload_catalog(n_labels=) refuses
         lib.yawb_catalog_set_labels.argtypes = [c_void_p, c_int]
         lib.yawb_catalog_set_labels.restype = c_int

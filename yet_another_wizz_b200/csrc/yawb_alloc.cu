@@ -11,6 +11,7 @@
 //     It never makes a stream wait for another stream; if nothing fits it calls cudaMalloc, and when the
 //     device is full it returns every parked block to the driver and tries once more.
 // One context is used by one host thread at a time (include/yawb.h), so there is no locking.
+#include <algorithm>
 #include <map>
 #include <unordered_map>
 
@@ -26,7 +27,8 @@ struct DevBlock {
 struct yawb_devcache {
     std::multimap<size_t, DevBlock> parked;
     std::unordered_map<void *, DevBlock> live;
-    size_t bytes_total = 0;
+    size_t bytes_total = 0;  // every block cudaMalloc'ed and not yet returned, parked ones included
+    size_t bytes_peak = 0;   // high-water mark of bytes_total since the last yawb_dcache_reset_peak
 };
 
 static size_t round_size(size_t bytes) {
@@ -81,6 +83,7 @@ int yawb_dalloc(yawb_ctx *ctx, void **out, size_t bytes, cudaStream_t st) {
     }
     YAWB_CUDA(cudaEventCreateWithFlags(&blk.ev, cudaEventDisableTiming));
     c->bytes_total += size;
+    c->bytes_peak = std::max(c->bytes_peak, c->bytes_total);
     c->live.emplace(blk.ptr, blk);
     *out = blk.ptr;
     return 0;
@@ -111,3 +114,22 @@ void yawb_dcache_destroy(yawb_ctx *ctx) {
 }
 
 size_t yawb_dcache_bytes(const yawb_ctx *ctx) { return ctx->cache ? ctx->cache->bytes_total : 0; }
+
+size_t yawb_dcache_parked(const yawb_ctx *ctx) {
+    size_t n = 0;
+    if (ctx->cache)
+        for (const auto &kv : ctx->cache->parked) n += kv.second.size;
+    return n;
+}
+
+size_t yawb_dcache_peak(const yawb_ctx *ctx) { return ctx->cache ? ctx->cache->bytes_peak : 0; }
+
+void yawb_dcache_reset_peak(yawb_ctx *ctx) {
+    if (ctx->cache) ctx->cache->bytes_peak = ctx->cache->bytes_total;
+}
+
+void yawb_dcache_release(yawb_ctx *ctx) {
+    if (ctx->cache) release_parked(ctx->cache);
+}
+
+size_t yawb_dcache_round(size_t bytes) { return round_size(bytes); }

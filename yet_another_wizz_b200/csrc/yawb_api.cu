@@ -144,7 +144,7 @@ int yawb_assign_patches(yawb_ctx *ctx, const double *xyz, int64_t n, const doubl
 
 const char *yawb_last_error(void) { return g_err; }
 
-int yawb_version(void) { return 103; }
+int yawb_version(void) { return 104; }
 
 int yawb_create(int device, yawb_ctx **out) {
     YAWB_REQUIRE(out != nullptr, "yawb_create: out is NULL");
@@ -211,6 +211,56 @@ int yawb_destroy(yawb_ctx *ctx) {
 }
 
 int yawb_device_sms(const yawb_ctx *ctx) { return ctx ? ctx->sms : 0; }
+
+int yawb_catalog_footprint(int64_t n_rows, int n_patch, int n_bins, uint32_t what, int64_t *bytes) {
+    YAWB_REQUIRE(bytes != nullptr, "yawb_catalog_footprint: bytes is NULL");
+    YAWB_REQUIRE(n_rows >= 0 && n_patch >= 1 && n_bins >= 1, "yawb_catalog_footprint: n_rows >= 0, n_patch >= 1 and "
+                 "n_bins >= 1 required (got %lld, %d, %d)", (long long)n_rows, n_patch, n_bins);
+    YAWB_REQUIRE(what < 2 * YAWB_FOOT_NO_UPLOAD, "yawb_catalog_footprint: unknown flag bits 0x%x", what);
+    *bytes = yawb_index_footprint(n_rows, n_patch, n_bins, what);
+    return 0;
+}
+
+int yawb_count_footprint(int sms, int64_t n_items, int n_pairs, int n_bins, int n_edges, int n_blocks, int weighted,
+                         int64_t *bytes) {
+    YAWB_REQUIRE(bytes != nullptr, "yawb_count_footprint: bytes is NULL");
+    YAWB_REQUIRE(sms >= 1 && n_items >= 0 && n_pairs >= 0 && n_bins >= 1 && n_edges >= 2 && n_blocks >= 1,
+                 "yawb_count_footprint: invalid sizes");
+    *bytes = yawb_count_workspace(sms, n_items, n_pairs, n_bins, n_edges, n_blocks, weighted != 0);
+    return 0;
+}
+
+int yawb_memory_stats(yawb_ctx *ctx, int64_t *held, int64_t *peak, int64_t *device_free) {
+    YAWB_REQUIRE(ctx != nullptr, "yawb_memory_stats: ctx is NULL");
+    if (held) *held = (int64_t)yawb_dcache_bytes(ctx);
+    if (peak) *peak = (int64_t)yawb_dcache_peak(ctx);
+    if (device_free) {
+        YAWB_CUDA(cudaSetDevice(ctx->device));
+        size_t free_b = 0, total_b = 0;
+        YAWB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        *device_free = (int64_t)free_b;
+    }
+    return 0;
+}
+
+int yawb_memory_parked(yawb_ctx *ctx, int64_t *parked) {
+    YAWB_REQUIRE(ctx != nullptr && parked != nullptr, "yawb_memory_parked: ctx or parked is NULL");
+    *parked = (int64_t)yawb_dcache_parked(ctx);
+    return 0;
+}
+
+int yawb_memory_reset_peak(yawb_ctx *ctx) {
+    YAWB_REQUIRE(ctx != nullptr, "yawb_memory_reset_peak: ctx is NULL");
+    yawb_dcache_reset_peak(ctx);
+    return 0;
+}
+
+int yawb_memory_release(yawb_ctx *ctx) {
+    YAWB_REQUIRE(ctx != nullptr, "yawb_memory_release: ctx is NULL");
+    YAWB_CUDA(cudaSetDevice(ctx->device));
+    yawb_dcache_release(ctx);
+    return 0;
+}
 
 int yawb_sync(yawb_ctx *ctx) {
     YAWB_REQUIRE(ctx != nullptr, "yawb_sync: ctx is NULL");

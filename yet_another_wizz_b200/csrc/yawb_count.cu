@@ -972,3 +972,27 @@ int yawb_launch_count_exact(yawb_ctx *ctx, const CountArgs &a, int *launches) {
     *launches += 1;
     return 0;
 }
+
+// Upper bound on the device bytes of one count call (yawb_count_footprint): the blocks count_impl (yawb_api.cu) and
+// yawb_launch_count_fast request, rounded as the allocator rounds them.
+int64_t yawb_count_workspace(int sms, int64_t n_items, int n_pairs, int n_bins, int n_edges, int n_blocks, bool weighted) {
+    const size_t np = (size_t)std::max(n_pairs, 1), B = (size_t)std::max(n_bins, 1), ne = (size_t)std::max(n_edges, 2);
+    const size_t lg_cells = ne > 2 ? YAWB_LG_CELLS_PER_EDGE * ne : 0;
+    const size_t r2f_words = B * ne + 2 * B + (B * lg_cells + 1) / 2;
+    auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+    const size_t tab = 2 * up16(np * sizeof(int)) + up16(2 * (np + 1) * sizeof(long long)) + up16(B * ne * sizeof(double)) +
+                       up16(r2f_words * sizeof(float)) + up16(B * sizeof(BinPar));
+    const size_t n_out = std::max<size_t>((size_t)std::max(n_blocks, 1) * np * B * (ne - 1), 1);
+    // work-item lists: 4 per diagonal and 2 per other (pair, tile) combination plus 1024 each; a job below
+    // SMALL_JOB_ITEMS items per warp gets lists CCAP / CCAP_SMALL times longer.  The launch decides from the real item
+    // count, the caller knows an upper bound n of it, so the bound takes the larger of both regimes up to n: the
+    // result does not decrease with n and covers every real count up to n on either side of the threshold
+    const size_t items = (size_t)std::max<int64_t>(n_items, 0);
+    const size_t small = (size_t)SMALL_JOB_ITEMS * std::max(sms, 1) * STREAM_CTAS * STREAM_WARPS - 1;
+    const size_t scale = (CCAP + CCAP_SMALL - 1) / CCAP_SMALL;
+    const size_t item_bytes = std::max(4 * items + 2048, scale * (4 * std::min(items, small) + 2048)) * sizeof(Item);
+    size_t total = yawb_dcache_round(tab) + yawb_dcache_round(n_out * sizeof(unsigned long long)) +
+                   yawb_dcache_round(item_bytes);
+    if (weighted) total += yawb_dcache_round(n_out * sizeof(double));
+    return (int64_t)total;
+}

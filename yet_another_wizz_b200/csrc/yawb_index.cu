@@ -1502,3 +1502,73 @@ void yawb_index_free(yawb_cat *cat, bool everything) {
         dev_free(cat, cat->d_seg_off2, P * (size_t)cat->n_bins + 1);
     }
 }
+
+// -------------------------------------------------------------------------------------------
+// Upper bound on the device bytes of one catalog (yawb_catalog_footprint): every block the upload, the second-role
+// mask and the two index builds above request, scratch included, each rounded as the allocator rounds it.  Blocks
+// freed along the way are counted as well, so the bound also holds for the allocator's high-water mark of a context
+// that starts empty (a freed block is only handed out again for a request it was counted for, or a smaller one).
+int64_t yawb_index_footprint(int64_t n_rows, int n_patch, int n_bins, uint32_t what) {
+    const size_t n = (size_t)std::max<int64_t>(n_rows, 0);
+    const size_t P = (size_t)std::max(n_patch, 1), B = (size_t)std::max(n_bins, 1), PB = P * B;
+    const bool w = what & YAWB_FOOT_WEIGHTED;
+    size_t total = 0;
+    auto blk = [&](size_t count, size_t size) { total += yawb_dcache_round(std::max<size_t>(count, 1) * size); };
+    if (!(what & YAWB_FOOT_NO_UPLOAD)) {
+        // yawb_index_upload
+        blk(3 * n, sizeof(double));
+        blk(n, sizeof(int32_t));
+        if (w) blk(n, sizeof(double));
+        if (what & (YAWB_FOOT_BINNED | YAWB_FOOT_U8 | YAWB_FOOT_Z | YAWB_FOOT_LABELLED)) blk(n, sizeof(int32_t));
+        if (what & YAWB_FOOT_U8) blk(n, 1);
+        if (what & YAWB_FOOT_Z) blk(n, sizeof(double));
+        blk(P, sizeof(PatchFrame));
+        blk(PB + 1, sizeof(int));
+        blk(P + 1, sizeof(long long));
+        // yawb_cat_finalize
+        blk(3 * P, sizeof(double));
+        blk(PB, sizeof(double));
+        blk(PB, sizeof(unsigned long long));
+        blk(P * kBox, sizeof(unsigned long long));
+        if (what & YAWB_FOOT_Z) blk(B + 1, sizeof(double));
+        // yawb_index_set_second_rows
+        if (what & YAWB_FOOT_MASK) {
+            blk(PB, sizeof(unsigned long long));
+            blk(n, 1);
+            blk(PB + 1, sizeof(int));
+        }
+    }
+    if (what & YAWB_FOOT_FIRST) {
+        // findex_build: the grid of a (patch, z-bin) has gu x gv cells with gu <= 4 du / c + 1, gv <= dv / c + 1,
+        // c^2 = kTargetPerCell du dv / max(rows / B, 1) and c >= max(du, dv) / 2048, so gu gv <= 4 max(rows / B, 1) /
+        // kTargetPerCell + 4 * 2048 + 2048 + 1 (growing the cells only lowers it); at most kMaxGridCells in all
+        const double cells = std::ceil(4.0 * (double)(n + PB) / kTargetPerCell) + (double)PB * (4 * 2048 + 2048 + 1);
+        const size_t base = (size_t)std::min<double>(cells, (double)kMaxGridCells);
+        blk(P, sizeof(PatchFrame));
+        blk(P, sizeof(SGrid));
+        blk(n, sizeof(SRec));
+        if (w) blk(n, sizeof(double));
+        blk(base + 1, sizeof(int));
+        blk(n, sizeof(int2));
+        blk((base + 1 + kScanBlock - 1) / kScanBlock + 1, sizeof(unsigned long long));
+    }
+    if (what & YAWB_FOOT_SECOND) {
+        // rindex_build: tiles are chunks of YAWB_TILE rows within each (patch, z-bin) segment
+        const size_t n_keys = std::max<size_t>(std::max<size_t>(n, 1 << 16), 4 * PB);
+        const size_t n_tiles = n / YAWB_TILE + PB;
+        blk(n * YAWB_RSTRIDE, sizeof(double));
+        if (w) blk(n, sizeof(double));
+        if (what & YAWB_FOOT_NO_UPLOAD) blk(PB + 1, sizeof(int));  // the segments of a union index
+        blk(n_keys, sizeof(int));
+        blk(n, sizeof(int2));
+        blk(P, sizeof(HMap));
+        blk((n_keys + kScanBlock - 1) / kScanBlock + 1, sizeof(unsigned long long));
+        blk(n_tiles, sizeof(Tile));
+        blk(P, sizeof(float));
+        blk(1, sizeof(unsigned));
+        blk(PB + 1, sizeof(int));
+        blk(n_tiles, sizeof(TileBox));
+        blk(P + 1, sizeof(int));
+    }
+    return (int64_t)total;
+}

@@ -278,6 +278,14 @@ int yawb_dalloc(yawb_ctx *ctx, void **out, size_t bytes, cudaStream_t st);
 void yawb_dfree(yawb_ctx *ctx, void *ptr, cudaStream_t st);
 void yawb_dcache_destroy(yawb_ctx *ctx);
 size_t yawb_dcache_bytes(const yawb_ctx *ctx);
+size_t yawb_dcache_peak(const yawb_ctx *ctx);
+size_t yawb_dcache_parked(const yawb_ctx *ctx);  // bytes of the parked blocks
+void yawb_dcache_reset_peak(yawb_ctx *ctx);
+void yawb_dcache_release(yawb_ctx *ctx);   // parked blocks back to the driver
+size_t yawb_dcache_round(size_t bytes);    // the size of the block a request of `bytes` gets
+// upper bounds on device bytes (yawb_index.cu / yawb_count.cu; see yawb_catalog_footprint in include/yawb.h)
+int64_t yawb_index_footprint(int64_t n_rows, int n_patch, int n_bins, uint32_t what);
+int64_t yawb_count_workspace(int sms, int64_t n_items, int n_pairs, int n_bins, int n_edges, int n_blocks, bool weighted);
 
 int yawb_cat_finalize(yawb_cat *cat);
 // Small host table -> device on the main stream WITHOUT the copy engine: staged in pinned memory and

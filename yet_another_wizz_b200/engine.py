@@ -108,7 +108,7 @@ class Engine:
     """One context on one CUDA device.  Raises if the device or library is missing."""
 
     def __init__(self, device: int = 0, *, staging: bool | None = None, cache_catalogs: bool | None = None,
-                 cache_bytes: int | None = None):
+                 cache_bytes: int | None = None, memory_limit: int | None = None):
         """`cache_catalogs` (default on; YAWB_CACHE=0 turns it off): device catalogs uploaded by the measurement
         functions stay resident, with their indexes, keyed by (catalog, z-binning) -- the counterpart of the
         reference's on-disk tree cache (`BinnedTrees.build` skips the rebuild while the `binning` file matches,
@@ -121,7 +121,15 @@ class Engine:
         `staging=True` (or YAWB_STAGING=1): measurement calls prepare large catalogs straight into a
         cache of page-locked buffers, so their copies are asynchronous and run at full PCIe rate.  Worth it
         for loops of many calls (C3: 225 -> 118 ms per call), not for a single one: page-locking the cache
-        costs ~1.5 s per GB once."""
+        costs ~1.5 s per GB once.
+
+        `memory_limit` (bytes): the device memory a measurement call may plan for.  A call whose predicted footprint
+        (`footprint`, `count_footprint`) exceeds it is counted in several passes over shares of its patches, one
+        after the other, each uploading only its share (`sharding.plan_passes`).  Default: what the context can
+        obtain when the call starts (`memory_available`): the device's free bytes, the allocator's parked blocks and
+        the engine's cached catalogs.  Under the default a call that fits drops the cached catalogs it does not use,
+        least recently used first, until it fits (`make_room`); a call that needs passes drops the whole cache."""
+        self.memory_limit = None if memory_limit is None else int(memory_limit)
         self.staging = bool(int(os.environ.get("YAWB_STAGING", "0"))) if staging is None else bool(staging)
         self.staging_min_rows = 1_000_000  # smaller catalogs are not worth a page-locked detour
         # YAWB_DEVICE_DIGITIZE=1: measurement calls ship raw redshifts and the device assigns the z-bins
@@ -144,6 +152,85 @@ class Engine:
     @property
     def num_sms(self) -> int:
         return self.lib.yawb_device_sms(self._h)
+
+    # ---- device memory --------------------------------------------------------------------------------
+    def footprint(self, n_rows: int, n_patch: int, n_bins: int = 1, *, weighted: bool = False, zbin: str | None = None,
+                  labelled: bool = False, mask: bool = False, first: bool = True, second: bool = True,
+                  upload: bool = True) -> int:
+        """Upper bound on the device bytes of one catalog (`yawb_catalog_footprint`, host arithmetic): `zbin` is how
+        the z-bin ids travel, None (unbinned), "i32", "u8" or "z" (raw redshifts); `mask` a second-role row mask;
+        `first` / `second` the indexes to cover; `upload=False` an index over rows uploaded by other catalogs (fused
+        first-role index, union second-role index)."""
+        what = ((_lib.FOOT_WEIGHTED if weighted else 0) | (_lib.FOOT_LABELLED if labelled else 0)
+                | (_lib.FOOT_MASK if mask else 0) | (_lib.FOOT_FIRST if first else 0) | (_lib.FOOT_SECOND if second else 0)
+                | (0 if upload else _lib.FOOT_NO_UPLOAD)
+                | {None: 0, "i32": _lib.FOOT_BINNED, "u8": _lib.FOOT_U8, "z": _lib.FOOT_Z}[zbin])
+        out = c_int64()
+        _lib.check(self.lib.yawb_catalog_footprint(int(n_rows), int(n_patch), int(n_bins), what, byref(out)))
+        return out.value
+
+    def count_footprint(self, n_items: int, n_pairs: int, n_bins: int, n_edges: int, *, n_blocks: int = 1,
+                        weighted: bool = False) -> int:
+        """Upper bound on the workspace of one count call (`yawb_count_footprint`): `n_items` (patch pair, tile)
+        combinations, `n_blocks` = first catalogs x labels of the second catalogs."""
+        out = c_int64()
+        _lib.check(self.lib.yawb_count_footprint(self.num_sms, int(n_items), int(n_pairs), int(n_bins), int(n_edges),
+                                                 int(n_blocks), int(bool(weighted)), byref(out)))
+        return out.value
+
+    def memory_stats(self) -> dict:
+        """`held`: bytes the allocator holds (parked blocks included), `peak`: its high-water mark since the last
+        `memory_reset_peak`, `device_free`: free bytes of the device"""
+        held, peak, free = c_int64(), c_int64(), c_int64()
+        _lib.check(self.lib.yawb_memory_stats(self._h, byref(held), byref(peak), byref(free)))
+        return dict(held=held.value, peak=peak.value, device_free=free.value)
+
+    def memory_reset_peak(self) -> None:
+        _lib.check(self.lib.yawb_memory_reset_peak(self._h))
+
+    def memory_release(self) -> None:
+        """blocks parked by the allocator go back to the driver"""
+        _lib.check(self.lib.yawb_memory_release(self._h))
+
+    def memory_parked(self) -> int:
+        """bytes of the blocks the allocator holds parked for reuse (they go back to the driver when it runs out)"""
+        out = c_int64()
+        _lib.check(self.lib.yawb_memory_parked(self._h, byref(out)))
+        return out.value
+
+    def _cache_entry_bytes(self, entry) -> int:
+        dev = entry[1]
+        return max(dev.info()[1], 0) if dev._h is not None else 0
+
+    def memory_available(self) -> int:
+        """The bytes a measurement call plans for: `memory_limit`, or what the context can obtain for it -- the
+        device's free bytes, the parked blocks of the allocator and the catalogs in the engine's cache (those the
+        call uses are part of its footprint, the others are dropped by `make_room` when the call needs their
+        memory).  Catalogs uploaded outside the cache are not counted."""
+        if self.memory_limit is not None:
+            return self.memory_limit
+        return (self.memory_stats()["device_free"] + self.memory_parked()
+                + sum(self._cache_entry_bytes(e) for e in self._cat_cache.values()))
+
+    def make_room(self, nbytes: int, catalogs=()) -> None:
+        """Under the default limit: drop cached catalogs that are none of `catalogs` (and no labelled upload of
+        them), least recently used first, until the free bytes, the parked blocks and the cached catalogs of
+        `catalogs` add up to `nbytes`.  With an explicit `memory_limit` nothing is dropped."""
+        if self.memory_limit is not None or not self._cat_cache:
+            return
+        mine = {id(c) for c in catalogs}
+
+        def used(key) -> bool:
+            kind, ident = key[0]
+            return ident in mine if kind == "id" else any(i in mine for i in ident)
+
+        have = self.memory_stats()["device_free"] + self.memory_parked()
+        have += sum(self._cache_entry_bytes(e) for k, e in self._cat_cache.items() if used(k))
+        for key in sorted((k for k in self._cat_cache if not used(k)), key=lambda k: self._cat_cache[k][4]):
+            if have >= nbytes:
+                break
+            have += self._cache_entry_bytes(self._cat_cache[key])
+            self._cache_drop(key)
 
     def upload_catalog(
         self,
@@ -601,6 +688,7 @@ class GroupCatalog:
         self.parts = parts
         self.plan = plan
         self._resident = resident  # parts owned by their engine's catalog cache (not freed here)
+        self.sums_hook = None  # a call counted in passes: sum_weights goes through it (sums over the passes)
         first = parts[0]
         self.n_patch, self.n_bins, self.binned, self.weighted = first.n_patch, first.n_bins, first.binned, first.weighted
         self.n_labels = getattr(first, "n_labels", None)
@@ -618,7 +706,7 @@ class GroupCatalog:
                 out = np.zeros_like(sw)
             out[:, take] = sw[:, take]
             done |= take
-        return out
+        return out if self.sums_hook is None else self.sums_hook(out, done)
 
     def free(self) -> None:
         for part, resident in zip(self.parts, self._resident):
@@ -657,6 +745,8 @@ class EngineGroup:
                 e.close()
             raise
         self._own = created
+        # raw redshifts travel when every engine asks for it (`Engine.device_digitize`), as on a single engine
+        self.device_digitize = all(getattr(e, "device_digitize", False) for e in self.engines)
         if len({id(e) for e in self.engines}) != len(self.engines):
             raise ValueError("an engine object may appear only once in an EngineGroup (a context serves one thread)")
         self._pool = ThreadPoolExecutor(max_workers=len(self.engines), thread_name_prefix="yawb-group")

@@ -18,8 +18,10 @@ Both this package's `Configuration` / `Catalog` and genuine `yaw.Configuration` 
 
 from __future__ import annotations
 
+import functools
 import logging
 import os
+import threading
 from collections.abc import Sequence
 from copy import deepcopy
 from itertools import compress
@@ -32,7 +34,7 @@ from .catalog import InconsistentPatchesError
 from .coordinates import AngularCoordinates, AngularDistances
 from .corrfunc import CorrFunc, ScalarCorrFunc
 from .paircounts import NormalisedCounts, NormalisedScalarCounts, PatchedCounts, PatchedSumWeights
-from .sharding import Shard, assign_pairs_lpt, current_shard, pair_costs, plan_shares
+from .sharding import Shard, assign_pairs_lpt, current_shard, pair_costs, plan_passes, plan_shares
 
 __all__ = ["PatchLinkage", "autocorrelate", "autocorrelate_scalar", "autocorrelate_tomographic",
            "compute_scalar_normalisation", "crosscorrelate", "crosscorrelate_scalar", "crosscorrelate_tomographic",
@@ -275,6 +277,7 @@ class _Uploads:
     def __init__(self, engine, plan=None) -> None:
         self.engine = engine
         self.plan = plan
+        self.run = _current_run()  # a call counted in passes: host arrays prepared once, no resident catalogs
         self._resident: set = set()  # keys whose device catalog belongs to the engine's cache (not freed here)
         self._cache: dict[tuple[int, bool, bool], object] = {}
         self._pending: dict[tuple[int, bool, bool], object] = {}
@@ -296,6 +299,8 @@ class _Uploads:
         return (rows, tuple(np.asarray(binning.edges, dtype=np.float64).tolist()), str(binning.closed))
 
     def _resident_lookup(self, key, catalog, binning, kappa) -> bool:
+        if self.run is not None:
+            return False
         lookup = getattr(self.engine, "cache_lookup", None)
         if self._group():  # the parts stay with their engines' caches: the GroupCatalog itself is not resident
             dev = self.engine.cache_lookup(catalog, self._signature(catalog, binning), kappa, self.plan)
@@ -320,7 +325,10 @@ class _Uploads:
 
     def _upload(self, key, catalog, binning, kappa, arrays):
         if self._group():
-            dev = self.engine.upload_catalog(arrays, self.plan, cache=(catalog, self._signature(catalog, binning), kappa))
+            cache = None if self.run is not None else (catalog, self._signature(catalog, binning), kappa)
+            dev = self.engine.upload_catalog(arrays, self.plan, cache=cache)
+            if self.run is not None:
+                dev.sums_hook = self.run.sums
             self._cache[key] = dev
             return dev
         dev = self.engine.upload_catalog(arrays.pop("xyz"), arrays.pop("patch_off"), **arrays)
@@ -349,7 +357,7 @@ class _Uploads:
         if self._pool is None:
             self._pool = ThreadPoolExecutor(max_workers=1)
         for key, catalog, binning, kappa in todo:
-            self._pending[key] = (self._pool.submit(_prepare_for, self.engine, catalog, binning, kappa), catalog, binning, kappa)
+            self._pending[key] = (self._pool.submit(self._prepare, key, catalog, binning, kappa), catalog, binning, kappa)
         for key, *_ in todo:  # upload in order; each wait overlaps with the preparation of the next catalog
             self._resolve(key)
 
@@ -357,12 +365,22 @@ class _Uploads:
         fut, catalog, binning, kappa = self._pending.pop(key)
         return self._upload(key, catalog, binning, kappa, fut.result())
 
+    def _prepare(self, key, catalog, binning, kappa, make=None):
+        """host arrays of one catalog; in a call counted in passes prepared once and kept for every pass"""
+        make = make or (lambda: _prepare_for(self.engine, catalog, binning, kappa))
+        if self.run is None:
+            return make()
+        with self.run.lock:
+            if key not in self.run.prepared:
+                self.run.prepared[key] = make()
+            return self.run.prepared[key]
+
     def get(self, catalog, binning: Binning | None, kappa: bool = False):
         key = self._key(catalog, binning, kappa)
         if key in self._pending:
             return self._resolve(key)
         if key not in self._cache and not self._resident_lookup(key, catalog, binning, kappa):
-            self._upload(key, catalog, binning, kappa, _prepare_for(self.engine, catalog, binning, kappa))
+            self._upload(key, catalog, binning, kappa, self._prepare(key, catalog, binning, kappa))
         return self._cache[key]
 
     def get_labelled(self, catalogs, binning: Binning | None = None):
@@ -372,7 +390,8 @@ class _Uploads:
         catalogs = tuple(catalogs)
         key = (("labelled", *map(id, catalogs)), binning is not None, False)
         if key not in self._cache and not self._resident_lookup(key, catalogs, binning, False):
-            self._upload(key, catalogs, binning, False, prepare_labelled_arrays(catalogs, binning))
+            arrays = self._prepare(key, catalogs, binning, False, lambda: prepare_labelled_arrays(catalogs, binning))
+            self._upload(key, catalogs, binning, False, arrays)
         return self._cache[key]
 
     def free(self) -> None:
@@ -630,22 +649,194 @@ def _own_pairs(shard: Shard, ij, n1_per_patch, n2_per_patch, radii1) -> np.ndarr
     return assign_pairs_lpt(costs, shard.world_size)[shard.rank]
 
 
-def _share_plan(engine, shard: Shard | None, catalogs, counts):
+def _share_plan(engine, shard: Shard | None, catalogs, counts, footprint=None):
     """The `SharePlan` of a call on an `EngineGroup` (None on a single engine).  `catalogs`: the catalogs of the
     linkage (the largest gives the patch centres and radii, as for the links); `counts`: `(pair_i, pair_j, first,
     second)` of every pair count of the call, `pair_j` the patches of the second catalog, `first` / `second` rows per
-    patch."""
+    patch; `footprint`: a `_Footprint` of the call's uploads.
+
+    When the predicted footprint of the call exceeds the memory of an engine (`Engine.memory_available`), the call
+    is planned in passes (`sharding.plan_passes`) and `_PassesNeeded` hands them to `_in_passes`, before anything is
+    uploaded; while a pass runs, this returns that pass's plan."""
     from .engine import EngineGroup
 
-    if not isinstance(engine, EngineGroup):
-        return None
+    run = _current_run()
+    if run is not None:
+        return run.steps[run.k]
+    group = isinstance(engine, EngineGroup)
     if (shard or current_shard()).active:
-        raise ValueError("an EngineGroup splits a call over the GPUs of one process; it cannot be combined with an "
-                         "active shard (one process per GPU)")
+        if group:
+            raise ValueError("an EngineGroup splits a call over the GPUs of one process; it cannot be combined with an "
+                             "active shard (one process per GPU)")
+        return None
+    eng = engine if engine is not None else get_default_engine()
+    members = eng.engines if group else [eng]
     ref = max(catalogs, key=lambda c: tuple(c.get_num_records()))
     centers = AngularCoordinates(_coords_data(ref.get_centers())).to_3d()
     counts = [(pi, pj, np.asarray(n1, dtype=np.float64), np.asarray(n2, dtype=np.float64)) for pi, pj, n1, n2 in counts]
-    return plan_shares(counts, _coords_data(ref.get_radii()), centers, len(engine))
+    radii = _coords_data(ref.get_radii())
+    if footprint is None or not all(hasattr(e, "memory_available") for e in members):
+        return plan_shares(counts, radii, centers, len(members)) if group else None
+    fp = footprint.bind(members[0], counts, bool(getattr(eng, "device_digitize", False)))
+    steps = plan_passes(counts, radii, centers, fp, [e.memory_available() for e in members])
+    if len(steps) == 1:
+        # the default limit counted the engines' cached catalogs as obtainable: drop the ones this call does not use
+        # (least recently used first) until its footprint fits
+        for d, e in enumerate(members):
+            if hasattr(e, "make_room"):
+                e.make_room(fp(steps[0].keep[d].astype(bool)), catalogs)
+        return steps[0] if group else None
+    raise _PassesNeeded(eng, steps, default_limit=any(e.memory_limit is None for e in members))
+
+
+class _Footprint:
+    """The device memory model of one call: its uploads, as `_Uploads` makes them (with a second-role row mask and
+    both indexes), the fused first-role indexes of `Engine.count2`, and the workspace of every count."""
+
+    def __init__(self, links: "PatchLinkage") -> None:
+        r2 = links._get_plan().r2
+        self.n_bins, self.n_edges = r2.shape
+        self.uploads: list[tuple[np.ndarray, int, dict]] = []
+        self.fused: list[np.ndarray] = []
+        self.n_labels = 1
+
+    def upload(self, catalog, binning: Binning | None, kappa: bool = False):
+        # how binned ids travel depends on the engine (`bind`): "binned" stands for byte / int32 ids or raw redshifts
+        zbin = None if binning is None else "binned" if len(binning) <= 254 else "i32"
+        self.uploads.append((_rows(catalog), len(binning) if binning is not None else 1,
+                             dict(weighted=bool(catalog.has_weights) or kappa, zbin=zbin)))
+        return self
+
+    def labelled(self, catalogs, binning: Binning | None = None):
+        catalogs = list(catalogs)
+        n_ids = len(catalogs) * (len(binning) if binning is not None else 1)
+        self.uploads.append((np.sum([_rows(c) for c in catalogs], axis=0), n_ids,
+                             dict(weighted=bool(catalogs[0].has_weights), zbin="u8" if n_ids <= 254 else "i32",
+                                  labelled=binning is not None)))
+        self.n_labels = max(self.n_labels, len(catalogs))
+        return self
+
+    def fuse(self, *catalogs):
+        self.fused.append(np.sum([_rows(c) for c in catalogs], axis=0))
+        return self
+
+    def bind(self, engine, counts, device_digitize: bool):
+        """`footprint(keep)` for `sharding.plan_passes`: device bytes of a pass keeping the patches `keep`.
+        `device_digitize`: the engine ships raw redshifts (`_prepare_for`)"""
+        n_edges = self.n_edges
+        uploads = [(rows, nb, dict(kw, zbin=("z" if device_digitize else "u8") if kw["zbin"] == "binned" else kw["zbin"]))
+                   for rows, nb, kw in self.uploads]
+        b2 = max(nb for _, nb, _ in uploads) if uploads else 1
+
+        def footprint(keep: np.ndarray) -> int:
+            n_patch = len(keep)
+            total = sum(engine.footprint(int(rows[keep].sum()), n_patch, nb, mask=True, **kw)
+                        for rows, nb, kw in uploads)
+            total += sum(engine.footprint(int(rows[keep].sum()), n_patch, self.n_bins, weighted=True, second=False,
+                                          upload=False) for rows in self.fused)
+            for pi, pj, _, n2 in counts:  # tiles of a second patch: at most rows / 256 + one per segment
+                pj = np.asarray(pj)
+                mine = keep[pj]
+                n_items = int(np.sum(np.ceil(n2[pj[mine]] / 256.0) + b2))
+                total += engine.count_footprint(n_items, int(mine.sum()), self.n_bins, n_edges,
+                                                n_blocks=2 * self.n_labels, weighted=True)
+            return total
+
+        return footprint
+
+
+class _PassesNeeded(Exception):
+    """raised by `_share_plan` before anything is uploaded: the call does not fit and runs in these passes"""
+
+    def __init__(self, engine, steps, default_limit: bool) -> None:
+        super().__init__(f"{len(steps)} passes")
+        self.engine, self.steps, self.default_limit = engine, steps, default_limit
+
+
+_pass_state = threading.local()
+
+
+def _current_run():
+    return getattr(_pass_state, "run", None)
+
+
+class _PassRun:
+    """One call counted in passes.  The body of a measurement function runs once per pass and makes the same
+    requests in the same order every time, so the n-th count of a pass adds to the n-th count of the passes before
+    (histograms placed in the full pair axis, summed in pass order; counters and times summed), and the n-th sums of
+    weights take every patch from the first pass that kept it.  What the last pass returns is the whole call."""
+
+    def __init__(self, steps) -> None:
+        self.steps = steps
+        self.k = 0
+        self.prepared: dict = {}  # host arrays of every catalog, prepared once for all passes
+        self.lock = threading.Lock()
+        self._counts: list = []
+        self._sums: list = []
+        self._nc = self._ns = 0
+
+    def begin(self, k: int) -> None:
+        self.k, self._nc, self._ns = k, 0, 0
+
+    def counts(self, hists: list, stats: dict) -> tuple[list, dict]:
+        i, self._nc = self._nc, self._nc + 1
+        if i == len(self._counts):
+            self._counts.append(([h.copy() for h in hists], dict(stats)))
+        else:
+            acc, st = self._counts[i]
+            for a, h in zip(acc, hists):
+                a += h
+            for key, v in stats.items():
+                st[key] = st.get(key, 0) + v
+        acc, st = self._counts[i]
+        st["passes"] = self.k + 1
+        return [a.copy() for a in acc], dict(st)
+
+    def sums(self, sw, kept: np.ndarray):
+        i, self._ns = self._ns, self._ns + 1
+        if i == len(self._sums):
+            self._sums.append((sw.copy(), kept.copy()))
+        else:
+            acc, done = self._sums[i]
+            take = kept & ~done
+            acc[:, take] = sw[:, take]
+            done |= take
+        return self._sums[i][0].copy()
+
+
+def _in_passes(fn):
+    """A measurement function that runs in passes when `_share_plan` finds that its call does not fit: the body runs
+    once per pass on an `EngineGroup` (a single engine is wrapped in a group of one), every pass uploads its share of
+    the catalogs and frees it before the next one, and the allocator returns its parked blocks to the driver so the
+    next pass starts from the same memory.  A call that fits runs the body once, as it is."""
+
+    @functools.wraps(fn)
+    def call(*args, **kw):
+        from .engine import EngineGroup
+
+        try:
+            return fn(*args, **kw)
+        except _PassesNeeded as need:
+            engine, steps, default_limit = need.engine, need.steps, need.default_limit
+        group = engine if isinstance(engine, EngineGroup) else EngineGroup([engine])
+        run = _PassRun(steps)
+        try:
+            if default_limit:  # the default limit counts the memory of the engine's cached catalogs as available
+                group._map(lambda d, e: e.cache_clear() if hasattr(e, "cache_clear") else None)
+            _pass_state.run = run
+            # blocks parked by earlier calls go back to the driver first, so every pass starts from the same level
+            group._map(lambda d, e: e.memory_release() if hasattr(e, "memory_release") else None)
+            for k in range(len(steps)):
+                run.begin(k)
+                result = fn(*args, **{**kw, "engine": group})
+                group._map(lambda d, e: e.memory_release() if hasattr(e, "memory_release") else None)
+        finally:
+            _pass_state.run = None
+            if group is not engine:
+                group.close()
+        return result
+
+    return call
 
 
 def _rows(catalog):
@@ -679,10 +870,13 @@ def _count(engine, shard: Shard, tag: str, first, second, ij, own: np.ndarray, r
     else:
         *out, stats = engine.count(first, second, pi, pj, r2, **kw)
         outs = [out]
-    _last_stats[tag] = stats
     weighted = any(c.weighted for c in (*(first if fused else (first,)), second))
     labelled = labels or getattr(second, "n_labels", None) is not None  # a leading label axis
     hists = [_reduce(engine, shard, out[1] if weighted else out[0], own, len(ij[0]), labelled=labelled) for out in outs]
+    run = _current_run()
+    if run is not None:
+        hists, stats = run.counts(hists, stats)
+    _last_stats[tag] = stats
     return tuple(hists) if fused else hists[0]
 
 
@@ -708,6 +902,7 @@ def _ensure_unique_catalogs(*catalogs) -> None:
         raise ValueError("each catalog must have a separate cache directory to avoid interference.")
 
 
+@_in_passes
 def autocorrelate(config, data, random, *, count_rr: bool = True, progress: bool = False, max_workers=None,
                   engine=None, shard: Shard | None = None) -> list[CorrFunc]:
     """Angular autocorrelation pair counts (DD, DR, optional RR) of a z-binned sample.
@@ -717,12 +912,13 @@ def autocorrelate(config, data, random, *, count_rr: bool = True, progress: bool
     links = PatchLinkage.from_catalogs(config, data, random, engine=engine, shard=shard)
     auto_ij, cross_ij = links.get_patch_id_pairs(auto=True), links.get_patch_id_pairs(auto=False)
     nd, nr = _rows(data), _rows(random)
+    binning = _as_binning(config)
     plan = _share_plan(engine, shard, (data, random), [(*auto_ij, nd, nd), (*cross_ij, nd, nr)]
-                       + ([(*auto_ij, nr, nr)] if count_rr else []))
+                       + ([(*auto_ij, nr, nr)] if count_rr else []),
+                       _Footprint(links).upload(data, binning).upload(random, binning))
     links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     try:
-        binning = _as_binning(config)
         links._uploads.enqueue(((data, binning), (random, binning)))
         DD = links.count_pairs(data, count_type_info="DD")
         DR = links.count_pairs(data, random, count_type_info="DR", binned_second=True)
@@ -733,6 +929,7 @@ def autocorrelate(config, data, random, *, count_rr: bool = True, progress: bool
     return [CorrFunc(dd, dr, None, rr) for dd, dr, rr in zip(DD, DR, RR)]
 
 
+@_in_passes
 def crosscorrelate(config, reference, unknown, *, ref_rand=None, unk_rand=None, progress: bool = False,
                    max_workers=None, engine=None, shard: Shard | None = None) -> list[CorrFunc]:
     """Angular cross-correlation pair counts (DD and DR / RD / RR as randoms allow) between the
@@ -747,9 +944,16 @@ def crosscorrelate(config, reference, unknown, *, ref_rand=None, unk_rand=None, 
 
     links = PatchLinkage.from_catalogs(config, reference, unknown, *randoms, engine=engine, shard=shard)
     ij = links.get_patch_id_pairs(auto=False)
+    binning = _as_binning(config)
+    fp = _Footprint(links).upload(reference, binning).upload(unknown, None)
+    for cat, bins in ((ref_rand, binning), (unk_rand, None)):
+        if cat is not None:
+            fp.upload(cat, bins)
+    if ref_rand is not None:
+        fp.fuse(reference, ref_rand)
     plan = _share_plan(engine, shard, (reference, unknown, *randoms),
                        [(*ij, _rows(c1), _rows(c2)) for c1 in (reference, ref_rand) if c1 is not None
-                        for c2 in (unknown, unk_rand) if c2 is not None])
+                        for c2 in (unknown, unk_rand) if c2 is not None], fp)
     links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     kw = dict(binned_second=False)
@@ -758,7 +962,6 @@ def crosscorrelate(config, reference, unknown, *, ref_rand=None, unk_rand=None, 
         # count in the order in which the inputs become complete -- DD gets the GPU going a few ms into the
         # transfer, RD / DR follow, and only RR waits for the last catalog (same schedule as
         # `pipeline.count_cross_pipelined`)
-        binning = _as_binning(config)
         links._uploads.enqueue(((reference, binning), (unknown, None), (ref_rand, binning), (unk_rand, None)))
         if _fuse(links.engine or get_default_engine(), reference, ref_rand):
             DD, RD = links.count_pairs_fused(reference, ref_rand, unknown, count_type_info=("DD", "RD"))
@@ -777,6 +980,7 @@ def crosscorrelate(config, reference, unknown, *, ref_rand=None, unk_rand=None, 
     return [CorrFunc(dd, dr, rd, rr) for dd, dr, rd, rr in zip(DD, DR, RD, RR)]
 
 
+@_in_passes
 def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, unk_rand=None, progress: bool = False,
                                max_workers=None, engine=None, shard: Shard | None = None) -> list[list[CorrFunc]]:
     """`crosscorrelate` of the reference sample with every tomographic bin of the unknown sample in one pass:
@@ -815,9 +1019,14 @@ def crosscorrelate_tomographic(config, reference, unknowns, *, ref_rand=None, un
                      first.get_radii().data)
     n_unk = np.sum([_rows(u) for u in unknowns], axis=0)
     n_ur = None if unk_rand is None else _rows(unk_rand) if shared else np.sum([_rows(r) for r in rands], axis=0)
+    fp = _Footprint(links[0]).upload(reference, binning).labelled(unknowns)
+    if ref_rand is not None:
+        fp.upload(ref_rand, binning).fuse(reference, ref_rand)
+    if unk_rand is not None:
+        fp.upload(unk_rand, None) if shared else fp.labelled(rands)
     uploads.plan = _share_plan(engine, shard, (reference, *unknowns, *[c for c in (ref_rand, *rands) if c is not None]),
                                [(*ij, _rows(c1), n2) for c1 in (reference, ref_rand) if c1 is not None
-                                for n2 in (n_unk, n_ur) if n2 is not None])
+                                for n2 in (n_unk, n_ur) if n2 is not None], fp)
     fuse = _fuse(eng, reference, ref_rand)
     counts: dict[str, tuple] = {}
     try:
@@ -905,6 +1114,7 @@ def _package_bin(count, i: int, rows: np.ndarray, pairs, auto: bool, plan, binni
     return PatchLinkage._package(hist[rows], plan, binning, num_patches, *pairs, sw1, sw2, auto)
 
 
+@_in_passes
 def autocorrelate_tomographic(config, data, random, *, count_rr: bool = True, progress: bool = False,
                               max_workers=None, engine=None, shard: Shard | None = None) -> list[list[CorrFunc]]:
     """`autocorrelate` of every tomographic bin of a sample in one pass: `result[i]` is `autocorrelate(config,
@@ -951,8 +1161,10 @@ def autocorrelate_tomographic(config, data, random, *, count_rr: bool = True, pr
     own_auto_rr = _own_pairs(shard, auto_ij, n_rand, n_rand, radii)
     # with shared randoms DR is counted with the pair lists swapped: the data sample is the second catalog
     dr_pairs = (cross_ij[1], cross_ij[0], n_rand, n_data) if shared else (*cross_ij, n_data, n_rand)
+    fp = _Footprint(links[0]).labelled(data, binning)
+    fp.upload(random, binning) if shared else fp.labelled(rands, binning)
     uploads.plan = _share_plan(engine, shard, (*data, *rands), [(*auto_ij, n_data, n_data), dr_pairs]
-                               + ([(*auto_ij, n_rand, n_rand)] if count_rr else []))
+                               + ([(*auto_ij, n_rand, n_rand)] if count_rr else []), fp)
 
     counts: dict[str, tuple] = {}
     try:
@@ -1006,13 +1218,16 @@ def compute_scalar_normalisation(catalog, binning: Binning, *, engine=None, uplo
                                   PatchedCounts(binning, sum_weights, auto=False))
 
 
+@_in_passes
 def autocorrelate_scalar(config, data, *, progress: bool = False, max_workers=None, engine=None,
                          shard: Shard | None = None) -> list[ScalarCorrFunc]:
     """Angular autocorrelation of a scalar field in z-bins: KK and NN counts of the data sample.
     Signature and result layout of `yaw.autocorrelate_scalar` (`measurements.py:651-705`)."""
     links = PatchLinkage.from_catalogs(config, data, engine=engine, shard=shard)
     nd = _rows(data)
-    plan = _share_plan(engine, shard, (data,), [(*links.get_patch_id_pairs(auto=True), nd, nd)])
+    binning = _as_binning(config)
+    plan = _share_plan(engine, shard, (data,), [(*links.get_patch_id_pairs(auto=True), nd, nd)],
+                       _Footprint(links).upload(data, binning, kappa=True).upload(data, binning))
     links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     try:
@@ -1023,6 +1238,7 @@ def autocorrelate_scalar(config, data, *, progress: bool = False, max_workers=No
     return [ScalarCorrFunc(dd) for dd in DD]
 
 
+@_in_passes
 def crosscorrelate_scalar(config, reference, unknown, *, unk_rand=None, progress: bool = False,
                           max_workers=None, engine=None, shard: Shard | None = None) -> list[ScalarCorrFunc]:
     """Angular cross-correlation between a z-binned scalar-field sample (`reference`, carries
@@ -1033,8 +1249,12 @@ def crosscorrelate_scalar(config, reference, unknown, *, unk_rand=None, progress
     randoms = [unk_rand] if unk_rand is not None else []
     links = PatchLinkage.from_catalogs(config, reference, unknown, *randoms, engine=engine, shard=shard)
     ij = links.get_patch_id_pairs(auto=False)
+    binning = _as_binning(config)
+    fp = _Footprint(links).upload(reference, binning, kappa=True).upload(reference, binning)
+    for cat in (unknown, *randoms):
+        fp.upload(cat, None)
     plan = _share_plan(engine, shard, (reference, unknown, *randoms),
-                       [(*ij, _rows(reference), _rows(c2)) for c2 in (unknown, *randoms)])
+                       [(*ij, _rows(reference), _rows(c2)) for c2 in (unknown, *randoms)], fp)
     links._uploads = _Uploads(engine or get_default_engine(), plan)
     _last_stats.clear()
     kw = dict(binned_second=False, mode="kn")

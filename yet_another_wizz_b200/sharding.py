@@ -19,7 +19,7 @@ import os
 import numpy as np
 
 __all__ = ["SharePlan", "Shard", "assign_pairs_lpt", "assign_patches_contiguous", "assign_patch_fractions", "split_rows",
-           "current_shard", "pair_costs", "plan_shares"]
+           "current_shard", "pair_costs", "plan_passes", "plan_shares"]
 
 
 def pair_costs(pair_i, pair_j, n1_per_patch, n2_per_patch, radii1=None) -> np.ndarray:
@@ -201,17 +201,65 @@ def plan_shares(counts, radii1, centers_xyz, n_devices: int) -> SharePlan:
     for pi, pj, n1, n2 in counts:
         np.add.at(cost, np.asarray(pj), pair_costs(pi, pj, n1, n2, radii1=radii1))
     shares = assign_patch_fractions(cost, centers_xyz, n_devices)
-    keep = []
-    for mine in shares:
-        own = np.zeros(n_patch, dtype=bool)
-        own[[p for p, _, _ in mine]] = True
-        k = own.copy()
-        for pi, pj, _, _ in counts:
-            pi, pj = np.asarray(pi), np.asarray(pj)
-            k[pi[own[pj]]] = True
-            k[pj[own[pi]]] = True
-        keep.append(k.astype(np.uint8))
+    keep = [_keep_for(counts, n_patch, [p for p, _, _ in mine]) for mine in shares]
     return SharePlan(shares, keep)
+
+
+def plan_passes(counts, radii1, centers_xyz, footprint, limits) -> list[SharePlan]:
+    """The passes of one call whose catalogs may not fit its devices at once.  `counts`, `radii1`, `centers_xyz`: as
+    for `plan_shares`; `footprint(keep)`: predicted device bytes of a pass that uploads the patches flagged in `keep`
+    (`(n_patch,)` bool) of every catalog of the call and counts there; `limits`: bytes per device.
+
+    The second patches are cut into `n_devices x K` shares of equal cost (`plan_shares`) and device d takes the K
+    consecutive shares d K .. d K + K - 1, one per pass; K grows until every pass fits its device.  Past one share
+    per patch the cuts stop helping (a pass keeps every patch linked to a patch it owns, whole), and the passes are
+    one second patch each, device d taking the patches of its share of `plan_shares`.  Returns one `SharePlan` per
+    pass step: share d of step k is device d's k-th pass (K = 1: the plan of `plan_shares`; a device with fewer
+    passes has empty shares at the end).  If one patch with its linked patches exceeds a device's limit,
+    ValueError is raised."""
+    limits = [int(x) for x in limits]
+    n_dev, n_patch = len(limits), len(centers_xyz)
+
+    def steps_of(plan, k):
+        return [SharePlan([plan.shares[d * k + s] for d in range(n_dev)], [plan.keep[d * k + s] for d in range(n_dev)])
+                for s in range(k)]
+
+    k = 1
+    while k < n_patch:
+        plan = plan_shares(counts, radii1, centers_xyz, n_dev * k)
+        need = [int(footprint(keep.astype(bool))) for keep in plan.keep]
+        if all(b <= limits[i // k] for i, b in enumerate(need)):
+            return steps_of(plan, k)
+        k = min(k + max(1, k // 4), n_patch)
+    # the smallest passes there are: one second patch each, with its linked patches
+    whole = plan_shares(counts, radii1, centers_xyz, n_dev)
+    seen: set = set()  # a patch cut between two devices goes to the first
+    own = [[p for p, _, _ in mine if not (p in seen or seen.add(p))] for mine in whole.shares]
+    k = max(len(o) for o in own)
+    shares, keep = [], []
+    for d in range(n_dev):
+        for s in range(k):
+            mine = [(own[d][s], 0.0, 1.0)] if s < len(own[d]) else []
+            one = _keep_for(counts, n_patch, [p for p, _, _ in mine])
+            b = int(footprint(one.astype(bool))) if mine else 0  # an empty pass uploads nothing
+            if b > limits[d]:
+                raise ValueError(f"one pass over patch {mine[0][0]} and its linked patches needs {b} bytes of device "
+                                 f"memory, more than the limit of {limits[d]} bytes")
+            shares.append(mine)
+            keep.append(one)
+    return steps_of(SharePlan(shares, keep), k)
+
+
+def _keep_for(counts, n_patch: int, own_patches) -> np.ndarray:
+    """the patches a device uploads to count the second patches `own_patches`: those and every patch linked to one"""
+    own = np.zeros(n_patch, dtype=bool)
+    own[list(own_patches)] = True
+    k = own.copy()
+    for pi, pj, _, _ in counts:
+        pi, pj = np.asarray(pi), np.asarray(pj)
+        k[pi[own[pj]]] = True
+        k[pj[own[pi]]] = True
+    return k.astype(np.uint8)
 
 
 class Shard:
