@@ -1,6 +1,8 @@
 """
 The pair-count kernels against the host oracle, at every place where `yawb_launch_count_fast` or the streaming kernel
-switches to other code or other constants: the five kernel paths and where their accumulators live, the group size of
+switches to other code or other constants: the kernel paths and where their accumulators live (the union-tile path
+of `count4`, `SingleUnion`, has its cases in `test_gpu_union_vs_oracle.py`; the repeat of a count whose work-item
+lists overflowed is in `test_gpu_item_lists.py`), the group size of
 the cumulative path, sub-bin counts up to `YAWB_MAX_EDGES`, z-bin counts around the 32 lanes of a warp, small and
 large jobs (items of `CCAP_SMALL` or `CCAP` cell-row runs) with the row-range split of the planner, weights on either
 side, per-bin thresholds with lower edges of 0, equal edges and empty z-bins, extreme geometry, short tiles and tiles cut
@@ -35,8 +37,15 @@ TILE = 256  # YAWB_TILE: rows of a register tile of the second catalog
 TARGET_PER_CELL, MAX_GRID_SPAN_CELLS = 5.5, 2048
 
 
-def kernel_path(weighted: bool, n_edges: int, n_bins: int, n_types: int) -> tuple[str, bool]:
-    """the choice of `yawb_launch_count_fast`: (CountPath, acc_global)"""
+def kernel_path(weighted: bool, n_edges: int, n_bins: int, n_types: int, n_second: int = 1, labels: bool = False,
+                exact: bool = False) -> tuple[str, bool]:
+    """the choice of `count_impl` and `yawb_launch_count_fast`: (CountPath, acc_global), or ("Exact", False) for the
+    exact kernel.  Two second catalogs (`count4`) share tiles cut from their union only on the single-bin path without
+    weights and labels; every other joint launch keeps per-catalog tiles and the path of one second catalog."""
+    if exact:
+        return "Exact", False
+    if n_second == 2 and not weighted and n_edges == 2 and not labels:
+        return "SingleUnion", False
     multi = n_edges > 2
     cumul = multi and not weighted and n_edges <= CUM_MAX_EDGES
     acc_bytes = n_types * n_bins * (n_edges - 1) * (16 if weighted else 8)
@@ -178,12 +187,25 @@ def _case_path(case):
 
 
 def test_path_cases_cover_every_launch():
-    """the cases below reach every (CountPath, acc_global) combination that can be launched, every cumulative
-    group size (7 and 8 edges in two passes), the listed edge and z-bin counts, and both sides of the 2048-byte
-    accumulator limit for one and two first catalogs, weighted and unweighted"""
-    combos = {_case_path(c) for c in PATH_CASES}
+    """the cases below and the union cases of `test_gpu_union_vs_oracle` reach every (CountPath, acc_global)
+    combination that can be launched, every cumulative group size (7 and 8 edges in two passes), the listed edge and
+    z-bin counts, and both sides of the 2048-byte accumulator limit for one and two first catalogs, weighted and
+    unweighted"""
+    from test_gpu_union_vs_oracle import UNION_CASES, union_case_path
+
+    union = {union_case_path(c) for c in UNION_CASES}
+    assert union == {("SingleUnion", False)}
+    assert {1, 31, 32, 33, 64} <= {c[1] for c in UNION_CASES} and {c[2] for c in UNION_CASES} == {False, True}
+    combos = {_case_path(c) for c in PATH_CASES} | union
     assert combos == {("Single", False), ("SingleWeighted", False), ("Cumulative", False), ("Histogram", False),
-                      ("Histogram", True), ("HistogramWeighted", False), ("HistogramWeighted", True)}
+                      ("Histogram", True), ("HistogramWeighted", False), ("HistogramWeighted", True),
+                      ("SingleUnion", False)}
+    # count4 keeps per-catalog tiles with a weighted catalog, sub-bins or labels (test_four_counts_against_oracle,
+    # test_second_labels_against_oracle), and the exact kernel counts one pair of catalogs at a time
+    assert kernel_path(True, 2, 5, 2, n_second=2) == ("SingleWeighted", False)
+    assert kernel_path(False, 5, 5, 2, n_second=2) == ("Cumulative", False)
+    assert kernel_path(False, 2, 5, 2, n_second=2, labels=True) == ("Single", False)
+    assert kernel_path(False, 2, 5, 1, exact=True) == ("Exact", False)
     cum = [c[1] for c in PATH_CASES if _case_path(c)[0] == "Cumulative"]
     assert {cumul_group(e) for e in cum} == {3, 4, 6} and {7, 8} <= set(cum)
     assert {2, 3, 4, 5, 6, 7, 8, 9, 33, 34, 256} <= {c[1] for c in PATH_CASES}
